@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the routing + assimilation hot path (driver contract).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -28,6 +28,13 @@ One bench "step" is one whole 7-day run.  The metric is reach*timestep*member up
 
 --impl reference times the CPU arm alone: the reference's kernels from oracle/_ref when present, else the
 port, on all the host cores of the box, on the same workload configuration the GPU arm reports at --gpus N.
+
+--dump-outputs DIR writes, after the timed steps of the GPU arm, the state the last timed step left (what
+`Muskingum.o_t_next` / `i_t_next` would hand a caller), float64, on rank 0, as DIR/<name>.npy:
+  c3_outflow, c3_inflow : [32,768 reaches][members] of the C3 ensemble (`value`)
+  c4_outflow, c4_inflow : [262,144 reaches] of the C4 forest (`c4_basins`, rank 0's shard), unless --no-extras
+The reaches are a fixed sorted sample (numpy default_rng(0), independent of --seed), in ascending reach order; all
+inputs derive from --seed, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -69,13 +76,40 @@ def parse_args():
     ap.add_argument("--no-extras", action="store_true", help="skip the C4 (basin-partitioned) and member-sharded arms")
     ap.add_argument("--c4-reaches", type=int, default=2_700_000)
     ap.add_argument("--no-e2e", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the state of the last timed step as DIR/<name>.npy (see the module docstring)")
+    a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    return a
 
 
 def algorithmic_bytes_per_update(M):
     """SURVEY.md section 8d: read o_prev, i_prev, write o_next, i_next (32 B) + per reach*step terms
     shared by the members: 4 coefficients (32 B), forcing (8 B), one index (4 B)."""
     return 32.0 + 44.0 / M
+
+
+DUMP_C3_REACHES = 32768           # x 64 members x 8 B x 2 arrays = 33.6 MB
+DUMP_C4_REACHES = 262144          # x 8 B x 2 arrays = 4.2 MB
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def sample_reaches(n, k):
+    """A fixed sorted sample of k of n reach indices (all of them when k >= n): the same in every run and build."""
+    if k >= n:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0).choice(n, size=k, replace=False))
+
+
+def write_outputs(out_dir, arrays):
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(v.nbytes for v in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"bench.py: --dump-outputs would write {total} bytes (limit {DUMP_LIMIT_BYTES})")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -433,8 +467,9 @@ def gpu_arm(a):
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
     from tx_fast_hydrology_b200 import build
     build.build_lib()
+    dump = {} if (a.dump_outputs and rank == 0) else None
     # the headline line: C3 on one GPU, or one independent C3 basin per GPU (weak scaling, no collective)
-    line = c3_arm(a, rank, world, local, full=True)
+    line = c3_arm(a, rank, world, local, full=True, dump=dump)
     if world > 1 and not a.no_extras and a.sharding == "basins":
         # BASELINE.json configs[2] as written: ONE 64-member ensemble with its members sharded over the ranks
         # (strong scaling: 64 / N members per GPU), EnKF statistics combined over NVLink
@@ -446,11 +481,13 @@ def gpu_arm(a):
                 line["members"] = {k: sub[k] for k in ("value", "unit", "ms_per_step", "scaling", "config", "gpu_launches",
                                                        "roofline", "update_path")}
     if not a.no_extras:
-        c4 = c4_arm(a, rank, world, local)
+        c4 = c4_arm(a, rank, world, local, dump=dump)
         if rank == 0:
             line["c4_basins"] = c4
     if rank == 0:
         line["host_affinity"] = numa
+        if dump is not None:
+            write_outputs(a.dump_outputs, dump)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.barrier()
@@ -485,7 +522,7 @@ def pin_to_gpu_numa_node(local):
         return {"pinned": False, "why": str(e)[:120]}
 
 
-def c4_arm(a, rank, world, local):
+def c4_arm(a, rank, world, local, dump=None):
     """BASELINE.json configs[3]: the CONUS-scale forest (2.7M reaches, 64 independent basins, seed 3), deterministic,
     24 hours at a 5-min step (288 steps), whole basins bin-packed over the ranks (sharding.shard_basins) and routed
     with no collective: strong scaling of a fixed forest.  Device-resident timing like `value`."""
@@ -547,6 +584,10 @@ def c4_arm(a, rank, world, local):
         counts = [int(x[1]) for x in allv]
     o_fin = mdl.download_state()[0]
     ok = bool(np.isfinite(o_fin).all())
+    if dump is not None:
+        keep = sample_reaches(n, DUMP_C4_REACHES)
+        dump["c4_outflow"] = o_fin[keep, 0]
+        dump["c4_inflow"] = mdl.network.unpack_host(I, 1)[keep, 0]
     f.close()
     del mdl, O0, I0, flush
     torch.cuda.empty_cache()
@@ -561,9 +602,10 @@ def c4_arm(a, rank, world, local):
             "l2": "256 MiB buffer written between bench steps (inside the timed region)"}
 
 
-def c3_arm(a, rank, world, local, full):
+def c3_arm(a, rank, world, local, full, dump=None):
     """One C3 measurement (see the module docstring).  `full`: also the end-to-end arm, the CPU baseline and the
-    in-run parity number (rank 0, single GPU).  Returns the JSON line as a dict (meaningful on rank 0)."""
+    in-run parity number (rank 0, single GPU).  `dump`: a dict that receives samples of the final state of the timed
+    steps.  Returns the JSON line as a dict (meaningful on rank 0)."""
     import torch
     import torch.distributed as dist
     from tx_fast_hydrology_b200 import _lib
@@ -696,6 +738,10 @@ def c3_arm(a, rank, world, local, full):
     final_o = mdl.download_state()[0]
     if not np.isfinite(final_o).all():
         raise SystemExit("bench.py: non-finite ensemble state after the run")
+    if dump is not None:
+        keep = sample_reaches(n, DUMP_C3_REACHES)
+        dump["c3_outflow"] = final_o[keep]
+        dump["c3_inflow"] = mdl.network.unpack_host(mdl.device_state[1], M)[keep]
 
     # routing kernel roofline: mean CUDA-event duration of one launch (one hourly window)
     # (an unsharded ensemble runs inside the library, which keeps the event pairs; the member-sharded loop hands
@@ -740,7 +786,7 @@ def c3_arm(a, rank, world, local, full):
         e2e_parts.clear()
         barrier()
         t0 = time.perf_counter()
-        reps = max(1, min(a.steps, 3))
+        reps = a.steps
         for _ in range(reps):
             e2e_run()
         barrier()
