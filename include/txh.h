@@ -240,6 +240,19 @@ int txh_run_assimilating(txh_net* net, double* O_dev, double* I_dev, int64_t M, 
                          double* T_dev, double* G_dev, int64_t time_every,
                          void* obs_ready_event /* cudaEvent_t or NULL: Zp_dev is complete once it has fired (an upload
                          on another stream); only the first update waits for it */, void* stream);
+/* txh_run_assimilating, also recording ensemble hydrographs at `rec_count` reaches (reference order, distinct):
+ *   rec_out_dev[s / rec_every - 1][k][M] after every step s (1-based over the call) with s % rec_every == 0 holds
+ *   what the state holds after that step: the forecast, or the posterior (o + gain) at an update step;
+ *   prior_out_dev (NULL: not wanted) [nsteps / every][k][M] holds the forecast the j-th update started from.
+ * rec_count == 0 is txh_run_assimilating.  TXH_E_INVALID before any device work for a reach out of range or listed
+ * twice, rec_every < 1, or rec_count > 0 without rec_reach_host / rec_out_dev. */
+int txh_run_assimilating_rec(txh_net* net, double* O_dev, double* I_dev, int64_t M, const txh_forcing* forcing,
+                             int64_t t0_ns, int64_t dt_ns, int64_t nsteps, int64_t every, int method,
+                             const int64_t* obs_reach_host, int64_t m, const double* Zp_dev, const double* qs_dev,
+                             const double* R_dev, const double* Dinv_dev, int dinv_kind, double* rowsum_dev,
+                             double* HX_dev, double* work_dev, double* W_dev, double* T_dev, double* G_dev,
+                             int64_t time_every, void* obs_ready_event, const int64_t* rec_reach_host, int64_t rec_count,
+                             int64_t rec_every, double* rec_out_dev, double* prior_out_dev, void* stream);
 int txh_get_route_timings(txh_net* net, double* ms_out, int64_t capacity, int64_t* count);
 
 /* Dense products of KalmanFilter.filter for small n (da.py:115-122): C = alpha op(A) op(B) + beta C,

@@ -75,6 +75,9 @@ SIGNATURES = {
     "txh_run_assimilating": (ctypes.c_int, [c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_i64, c_i64, c_i64, ctypes.c_int,
                                             p_i64, c_i64, c_vp, c_vp, c_vp, c_vp, ctypes.c_int, c_vp, c_vp, c_vp, c_vp,
                                             c_vp, c_vp, c_i64, c_vp, c_vp]),
+    "txh_run_assimilating_rec": (ctypes.c_int, [c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_i64, c_i64, c_i64, ctypes.c_int,
+                                                p_i64, c_i64, c_vp, c_vp, c_vp, c_vp, ctypes.c_int, c_vp, c_vp, c_vp, c_vp,
+                                                c_vp, c_vp, c_i64, c_vp, p_i64, c_i64, c_i64, c_vp, c_vp, c_vp]),
     "txh_get_route_timings": (ctypes.c_int, [c_vp, p_f64, c_i64, p_i64]),
     "txh_dgemm": (ctypes.c_int, [ctypes.c_int, ctypes.c_int, c_i64, c_i64, c_i64, c_f64, c_vp, c_i64, c_vp, c_i64,
                                  c_f64, c_vp, c_i64, c_vp]),

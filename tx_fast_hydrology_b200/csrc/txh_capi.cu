@@ -70,6 +70,7 @@ struct txh_net {
     StepInterp* d_steps = nullptr; size_t steps_cap = 0;
     StepInterp* d_unit_step = nullptr;
     int32_t* d_rec_slot = nullptr;
+    int32_t* d_rec_pos = nullptr; size_t rec_pos_cap = 0;   // positions of the recorded reaches (txh_run_assimilating_rec)
     int32_t* d_tmp_idx = nullptr; size_t tmp_idx_cap = 0;
     int32_t* h_status = nullptr;        // pinned mirror of d_status (word 0) and the solver info (word 1)
     std::vector<int64_t> obs_cached;    // gauge list whose positions are resident in d_obs
@@ -78,14 +79,16 @@ struct txh_net {
     // ensemble update applied by the next window launch while it loads its tasks (txh_run_assimilating, txh_window.cu)
     int32_t* d_gfix_off = nullptr;      // [window tasks + 1] gauge terms per task, for the gauges in obs_cached
     int2* d_gfix = nullptr; size_t gfix_cap = 0; bool gfix_ok = false;
-    struct { const double* T = nullptr; const double* W = nullptr; const double* qs = nullptr; int64_t M = 0; } pending;
+    struct {
+        const double* T = nullptr; const double* W = nullptr; const double* qs = nullptr; int64_t M = 0;
+        double* rec_prior = nullptr; double* rec_post = nullptr; const double* rec_mean = nullptr;   // (REC launches)
+    } pending;
     // window-mode kernel
     WTaskDesc* d_wtasks = nullptr;
     uint32_t *d_whdr = nullptr, *d_winw = nullptr;
     int32_t* d_wprod = nullptr;
     double* d_ring = nullptr; size_t ring_cap = 0; int ring_ld = 0;
-    int route_kernel = 0;               // 0 auto (lane for small ensembles, else window; dataflow when recording
-                                        // a large ensemble), 1 dataflow, 2 window, 3 lane
+    int route_kernel = 0;               // 0 auto (lane for small ensembles, else window), 1 dataflow, 2 window, 3 lane
     // lane kernel (txh_lane.cu): one schedule per member tile, built on first use
     struct LaneDev {
         LaneSchedule sched;
@@ -264,7 +267,7 @@ struct StepPlan {                   // forcing interpolation resolved by the ini
 
 int run_dataflow(txh_net* net, double* O, double* I, int64_t M, const double* F, const double* W, int wm_ld,
                  const StepPlan& plan, int64_t nsteps, const int32_t* rec_slot, double* rec_out,
-                 int rec_every, int rec_count, cudaStream_t st)
+                 int rec_every, int rec_count, int64_t rec_base, cudaStream_t st)
 {
     const Schedule& s = net->sched;
     const int ld = (int)txh_row_stride(M);
@@ -279,8 +282,6 @@ int run_dataflow(txh_net* net, double* O, double* I, int64_t M, const double* F,
     // the ready queue never wraps: one slot per (pair, step); long runs go out in several launches
     const int64_t max_entries = int64_t(1) << 25;
     int64_t steps_per_launch = std::max<int64_t>(1, std::min<int64_t>(nsteps, max_entries / (int64_t)pairs));
-    if (rec_slot && rec_every > 1 && steps_per_launch < nsteps)
-        steps_per_launch = std::max<int64_t>(rec_every, steps_per_launch / rec_every * rec_every);
     const size_t qneed = pairs * (size_t)steps_per_launch;
     const size_t side_need = (size_t)std::max(1, s.n_side) * ld;
     if (side_need > net->side_cap) {
@@ -316,18 +317,13 @@ int run_dataflow(txh_net* net, double* O, double* I, int64_t M, const double* F,
         a.tasks = net->d_tasks; a.notify = net->d_notify; a.hdr = net->d_hdr; a.inw = net->d_inw;
         a.coef = net->d_coef; a.cumA = net->d_coef + 4 * net->topo.n; a.linkA = net->d_coef + 5 * net->topo.n;
         a.O = O; a.I = I; a.Side = net->d_side; a.F = F; a.steps = d_steps; a.Wmul = W;
-        a.rec_slot = rec_slot;
-        a.rec_out = rec_out;
-        if (rec_slot && s0 > 0) {
-            if (s0 % rec_every != 0) return fail(TXH_E_INVALID, "internal: launch split not aligned with rec_every");
-            a.rec_out = rec_out + (size_t)(s0 / rec_every) * rec_count * M;
-        }
+        a.rec_slot = rec_slot; a.rec_out = rec_out; a.rec_step_base = rec_base + s0;
         a.pending = ia.pending; a.queue = net->d_queue; a.q_head = net->d_qctl;
         a.status = net->d_status; a.watchdog_ns = net->watchdog_ns;
         a.total = (long long)pairs * ns;
         a.n = net->topo.n; a.n_tasks = ia.n_tasks; a.n_mblocks = nmb; a.nsteps = (int32_t)ns;
         a.slots = std::max(1, s.slots_used); a.ld = ld; a.M = (int32_t)M;
-        a.wm_ld = wm_ld; a.rec_every = rec_every; a.rec_count = rec_count;
+        a.wm_ld = wm_ld; a.rec_every = std::max(1, rec_every); a.rec_count = rec_count;
         // per-warp shared memory: [scratch slots][staging][row ring].  Staging of a walking task:
         // [coef][f0][f1][hdr][words]; of a LINK task: [A_last per segment][records]; 16-byte aligned parts.
         auto up16 = [](int x) { return (x + 15) & ~15; };
@@ -374,7 +370,9 @@ int run_dataflow(txh_net* net, double* O, double* I, int64_t M, const double* F,
 // Returns 1 when the schedule does not fit it (rows of a task x 1 KB per warp) and the caller should fall
 // back to the dataflow kernel.
 int run_window(txh_net* net, double* O, double* I, int64_t M, const double* F, const double* W, int wm_ld,
-               const StepPlan& plan, int64_t nsteps, cudaStream_t st, bool probe_only = false)
+               const StepPlan& plan, int64_t nsteps, cudaStream_t st, bool probe_only = false,
+               const int32_t* rec_slot = nullptr, double* rec_out = nullptr, int rec_every = 1, int rec_count = 0,
+               int64_t rec_base = 0)
 {
     const Schedule& s = net->sched;
     const int ld = (int)txh_row_stride(M);
@@ -464,11 +462,15 @@ int run_window(txh_net* net, double* O, double* I, int64_t M, const double* F, c
             // the ensemble update owed to the state is applied by this launch while it loads its tasks
             a.upT = net->pending.T; a.upW = net->pending.W; a.upQs = net->pending.qs;
             a.gfix_off = net->d_gfix_off; a.gfix = net->d_gfix;
+            if (rec_slot) { a.rec_prior = net->pending.rec_prior; a.rec_post = net->pending.rec_post; a.rec_mean = net->pending.rec_mean; }
+            net->pending.rec_prior = net->pending.rec_post = nullptr;
             layout(2, 6);
             a.off_T = wpc_upd * a.smem_per_warp;
             net->pending.T = nullptr;
         } else layout(4, 8);
         a.off_steps = a.upT ? a.off_T + 64 * 64 * (int)sizeof(double) + 16 : wpc * a.smem_per_warp;
+        a.rec_slot = rec_slot; a.rec_out = rec_out; a.rec_step_base = rec_base + s0;
+        a.rec_every = std::max(1, rec_every); a.rec_count = rec_count;
         a.nap_min = 32; a.nap_max = 256;
         if (const char* k = getenv("TXH_WINDOW_NAP")) { int lo = 32, hi = 256; if (sscanf(k, "%d,%d", &lo, &hi) >= 1) { a.nap_min = std::max(0, lo); a.nap_max = std::max(a.nap_min, hi); } }
         a.trace = nullptr;
@@ -539,7 +541,7 @@ txh_net::LaneDev* lane_schedule(txh_net* net, int ti, int num_sms)
 // Returns 1 when the lane schedule cannot be built for this network (the caller falls back).
 int run_lane(txh_net* net, double* O, double* I, int64_t M, const double* F, const double* W, int wm_ld,
              const StepPlan& plan, int64_t nsteps, const int32_t* rec_slot, double* rec_out, int rec_every,
-             int rec_count, cudaStream_t st)
+             int rec_count, int64_t rec_base, cudaStream_t st)
 {
     const int ti = lane_tile_index(M), mt = 1 << ti;
     if (M > 16) return 1;
@@ -571,7 +573,6 @@ int run_lane(txh_net* net, double* O, double* I, int64_t M, const double* F, con
     int64_t spl = std::min<int64_t>(nsteps, 4096);
     if (const char* k = getenv("TXH_LANE_SPL")) { const long v = atol(k); if (v > 0) spl = std::min<int64_t>(spl, v); }
     while (spl > 16 && streams * (size_t)((spl + 15) & ~int64_t(15)) * sizeof(double) > (size_t(128) << 20)) spl = (spl + 1) / 2;
-    if (rec_slot && rec_every > 1 && spl < nsteps) spl = std::max<int64_t>(rec_every, spl / rec_every * rec_every);
     const size_t ring_need = streams * (size_t)((spl + 15) & ~int64_t(15));
     if (ring_need > net->lring_cap) {
         if (net->d_lring) { CU(cudaStreamSynchronize(st)); CU(cudaFree(net->d_lring)); }
@@ -623,7 +624,7 @@ int run_lane(txh_net* net, double* O, double* I, int64_t M, const double* F, con
         a.coef = net->d_coef; a.O = O; a.I = I; a.F = F; a.steps = d_steps; a.Wmul = W;
         a.ring = net->d_lring; a.ticket = net->d_qctl + 6; a.done = net->d_qctl + 7;
         a.status = net->d_status; a.watchdog_ns = net->watchdog_ns;
-        a.rec_slot = rec_slot; a.rec_out = rec_out; a.rec_step_base = s0;
+        a.rec_slot = rec_slot; a.rec_out = rec_out; a.rec_step_base = rec_base + s0;
         a.rec_every = std::max(1, rec_every); a.rec_count = rec_count;
         a.n = net->topo.n; a.n_regions = (int32_t)s.regions.size(); a.nsteps = (int32_t)ns;
         a.splp = (int32_t)((ns + 15) & ~int64_t(15)); a.ld = ld; a.M = (int32_t)M; a.wm_ld = wm_ld;
@@ -676,26 +677,28 @@ bool lane_wanted(txh_net* net, int64_t M, int64_t nsteps)
     return t_lane <= t_win;
 }
 
-// routing entry: the lane kernel for small ensembles, else the window kernel unless recording was asked for
-// (or the environment says otherwise)
+// routing entry: the lane kernel for small ensembles, else the window kernel (or what the environment says); the
+// dataflow kernel where the window kernel declines the schedule.  rec_slot: [n] recording slot per position or nullptr;
+// rec_base: steps of the call before this one (the step that ends this call's step s is rec_base + s + 1)
 int run_routing(txh_net* net, double* O, double* I, int64_t M, const double* F, const double* W, int wm_ld,
                 const StepPlan& plan, int64_t nsteps, const int32_t* rec_slot, double* rec_out, int rec_every,
-                int rec_count, cudaStream_t st)
+                int rec_count, cudaStream_t st, int64_t rec_base = 0)
 {
     const int ld = (int)txh_row_stride(M);
     if (lane_wanted(net, M, nsteps)) {
-        const int rc = run_lane(net, O, I, M, F, W, wm_ld, plan, nsteps, rec_slot, rec_out, rec_every, rec_count, st);
+        const int rc = run_lane(net, O, I, M, F, W, wm_ld, plan, nsteps, rec_slot, rec_out, rec_every, rec_count, rec_base, st);
         if (rc == TXH_OK && net->stats_rowsum)
             CU(launch_enkf_stats(O, ld, (int)M, net->topo.n, net->stats_scale, nullptr, net->stats_rowsum, nullptr, st));
         if (rc != 1) return rc;
     }
-    if (net->route_kernel != 1 && !rec_slot) {
-        const int rc = run_window(net, O, I, M, F, W, wm_ld, plan, nsteps, st);
+    if (net->route_kernel != 1) {
+        const int rc = run_window(net, O, I, M, F, W, wm_ld, plan, nsteps, st, false, rec_slot, rec_out, rec_every, rec_count,
+                                  rec_base);
         if (rc == TXH_OK && net->stats_rowsum && ld > kMemberBlock)
             CU(launch_enkf_stats(O, ld, (int)M, net->topo.n, net->stats_scale, nullptr, net->stats_rowsum, nullptr, st));
         if (rc != 1) return rc;
     }
-    const int rc = run_dataflow(net, O, I, M, F, W, wm_ld, plan, nsteps, rec_slot, rec_out, rec_every, rec_count, st);
+    const int rc = run_dataflow(net, O, I, M, F, W, wm_ld, plan, nsteps, rec_slot, rec_out, rec_every, rec_count, rec_base, st);
     if (rc == TXH_OK && net->stats_rowsum)
         CU(launch_enkf_stats(O, ld, (int)M, net->topo.n, net->stats_scale, nullptr, net->stats_rowsum, nullptr, st));
     return rc;
@@ -705,14 +708,14 @@ int run_routing(txh_net* net, double* O, double* I, int64_t M, const double* F, 
 int run_one_step(txh_net* net, double* O, double* I, int64_t M, const double* q, cudaStream_t st)
 {
     if (lane_wanted(net, M, 1)) {
-        const int rc = run_lane(net, O, I, M, q, nullptr, 0, StepPlan(), 1, nullptr, nullptr, 1, 0, st);
+        const int rc = run_lane(net, O, I, M, q, nullptr, 0, StepPlan(), 1, nullptr, nullptr, 1, 0, 0, st);
         if (rc != 1) return rc;
     }
     if (net->route_kernel != 1) {
         const int rc = run_window(net, O, I, M, q, nullptr, 0, StepPlan(), 1, st);
         if (rc != 1) return rc;
     }
-    return run_dataflow(net, O, I, M, q, nullptr, 0, StepPlan(), 1, nullptr, nullptr, 1, 0, st);
+    return run_dataflow(net, O, I, M, q, nullptr, 0, StepPlan(), 1, nullptr, nullptr, 1, 0, 0, st);
 }
 
 }  // namespace
@@ -760,6 +763,7 @@ void txh_destroy(txh_net* net)
         cudaFree(net->d_reach_of_pos); cudaFree(net->d_pos_of_reach); cudaFree(net->d_outlet);
         cudaFree(net->d_coef); cudaFree(net->d_qtmp); cudaFree(net->d_qctl); cudaFree(net->d_rec_slot);
         cudaFree(net->d_unit_step);
+        if (net->d_rec_pos) cudaFree(net->d_rec_pos);
         if (net->d_pending) cudaFree(net->d_pending);
         if (net->d_queue) cudaFree(net->d_queue);
         if (net->d_side) cudaFree(net->d_side);
@@ -1135,18 +1139,28 @@ void txh_forcing_destroy(txh_forcing* f)
     delete f;
 }
 
-int txh_route_run(txh_net* net, double* O, double* I, int64_t M, const txh_forcing* fo, int64_t t0_ns,
-                  int64_t dt_ns, int64_t nsteps, int method, const int64_t* rec_reach, int64_t rec_count,
-                  int64_t rec_every, double* rec_out, void* stream)
+}  // extern "C"
+
+namespace {
+// Recording slot of every schedule position (-1: not recorded) -> net->d_rec_slot, once per call.  A reach listed twice
+// keeps its last slot (txh_route_run's rule; txh_run_assimilating_rec refuses duplicates before it gets here).
+int upload_rec_slots(txh_net* net, const int64_t* rec_reach, int64_t rec_count, cudaStream_t st)
 {
-    if (!net || !O || !I) return fail(TXH_E_INVALID, "null argument");
-    if (nsteps < 0 || nsteps > (1 << 24)) return fail(TXH_E_INVALID, "nsteps out of range");
-    if (fo && fo->net != net) return fail(TXH_E_INVALID, "forcing belongs to another network");
-    if (fo && fo->d_W && fo->M != M) return fail(TXH_E_INVALID, "forcing member multipliers do not match M");
-    if (rec_count > 0 && (!rec_reach || !rec_out || rec_every < 1)) return fail(TXH_E_INVALID, "bad recording arguments");
-    int rc;
-    cudaStream_t st = (cudaStream_t)stream;
-    if ((rc = check_M(M)) || (rc = ensure_device(net)) || (rc = ensure_coef(net, st))) return rc;
+    std::vector<int32_t> slot(net->topo.n, -1);
+    for (int64_t k = 0; k < rec_count; ++k) {
+        if (rec_reach[k] < 0 || rec_reach[k] >= net->topo.n) return fail(TXH_E_INVALID, "recorded reach out of range");
+        slot[net->sched.pos_of_reach[rec_reach[k]]] = (int32_t)k;
+    }
+    CU(cudaMemcpyAsync(net->d_rec_slot, slot.data(), sizeof(int32_t) * net->topo.n, cudaMemcpyHostToDevice, st));
+    CU(cudaStreamSynchronize(st));
+    return TXH_OK;
+}
+
+// txh_route_run once the arguments are checked and the recording slots are on the device
+int route_run_impl(txh_net* net, double* O, double* I, int64_t M, const txh_forcing* fo, int64_t t0_ns, int64_t dt_ns,
+                   int64_t nsteps, int method, const int32_t* rec_slot, int64_t rec_count, int64_t rec_every,
+                   double* rec_out, int64_t rec_base, cudaStream_t st)
+{
     if (nsteps == 0) return TXH_OK;
     StepPlan plan;
     if (fo) { plan.times = fo->d_times; plan.R = fo->R; plan.t0_ns = t0_ns; plan.dt_ns = dt_ns; plan.method = method; }
@@ -1160,19 +1174,29 @@ int txh_route_run(txh_net* net, double* O, double* I, int64_t M, const txh_forci
             ++fw->waited;
         }
     }
-    const int32_t* rec_slot = nullptr;
-    if (rec_count > 0) {
-        std::vector<int32_t> slot(net->topo.n, -1);
-        for (int64_t k = 0; k < rec_count; ++k) {
-            if (rec_reach[k] < 0 || rec_reach[k] >= net->topo.n) return fail(TXH_E_INVALID, "recorded reach out of range");
-            slot[net->sched.pos_of_reach[rec_reach[k]]] = (int32_t)k;
-        }
-        CU(cudaMemcpyAsync(net->d_rec_slot, slot.data(), sizeof(int32_t) * net->topo.n, cudaMemcpyHostToDevice, st));
-        CU(cudaStreamSynchronize(st));
-        rec_slot = net->d_rec_slot;
-    }
     return run_routing(net, O, I, M, fo ? fo->d_F : nullptr, fo ? fo->d_W : nullptr, fo ? (int)fo->M : 0,
-                       plan, nsteps, rec_slot, rec_out, (int)rec_every, (int)rec_count, st);
+                       plan, nsteps, rec_slot, rec_out, (int)rec_every, (int)rec_count, st, rec_base);
+}
+}  // namespace
+
+extern "C" {
+
+int txh_route_run(txh_net* net, double* O, double* I, int64_t M, const txh_forcing* fo, int64_t t0_ns,
+                  int64_t dt_ns, int64_t nsteps, int method, const int64_t* rec_reach, int64_t rec_count,
+                  int64_t rec_every, double* rec_out, void* stream)
+{
+    if (!net || !O || !I) return fail(TXH_E_INVALID, "null argument");
+    if (nsteps < 0 || nsteps > (1 << 24)) return fail(TXH_E_INVALID, "nsteps out of range");
+    if (fo && fo->net != net) return fail(TXH_E_INVALID, "forcing belongs to another network");
+    if (fo && fo->d_W && fo->M != M) return fail(TXH_E_INVALID, "forcing member multipliers do not match M");
+    if (rec_count > 0 && (!rec_reach || !rec_out || rec_every < 1)) return fail(TXH_E_INVALID, "bad recording arguments");
+    int rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    if ((rc = check_M(M)) || (rc = ensure_device(net)) || (rc = ensure_coef(net, st))) return rc;
+    if (nsteps == 0) return TXH_OK;
+    if (rec_count > 0 && (rc = upload_rec_slots(net, rec_reach, rec_count, st))) return rc;
+    return route_run_impl(net, O, I, M, fo, t0_ns, dt_ns, nsteps, method, rec_count > 0 ? net->d_rec_slot : nullptr,
+                          rec_count, rec_every, rec_out, 0, st);
 }
 
 int txh_route_step(txh_net* net, double* O, double* I, int64_t M, const double* q, void* stream)
@@ -1465,8 +1489,31 @@ int txh_run_assimilating(txh_net* net, double* O, double* I, int64_t M, const tx
                          double* rowsum, double* HX, double* work, double* W, double* T, double* G, int64_t time_every,
                          void* obs_ready_event, void* stream)
 {
+    return txh_run_assimilating_rec(net, O, I, M, fo, t0_ns, dt_ns, nsteps, every, method, obs, m, Zp, qs, R, Dinv, dinv_kind,
+                                    rowsum, HX, work, W, T, G, time_every, obs_ready_event, nullptr, 0, 1, nullptr, nullptr,
+                                    stream);
+}
+
+int txh_run_assimilating_rec(txh_net* net, double* O, double* I, int64_t M, const txh_forcing* fo, int64_t t0_ns,
+                             int64_t dt_ns, int64_t nsteps, int64_t every, int method, const int64_t* obs, int64_t m,
+                             const double* Zp, const double* qs, const double* R, const double* Dinv, int dinv_kind,
+                             double* rowsum, double* HX, double* work, double* W, double* T, double* G, int64_t time_every,
+                             void* obs_ready_event, const int64_t* rec_reach, int64_t rec_count, int64_t rec_every,
+                             double* rec_out, double* prior_out, void* stream)
+{
     if (!net || !O || !I || !obs || !Zp || !qs || !R || !rowsum || !HX || !work || !W || !T || !G || every < 1 || m < 1)
         return fail(TXH_E_INVALID, "bad argument");
+    if (rec_count < 0 || rec_every < 1 || (rec_count > 0 && (!rec_reach || !rec_out)))
+        return fail(TXH_E_INVALID, "bad recording arguments");
+    if (rec_count > 0) {
+        if (fo && fo->net != net) return fail(TXH_E_INVALID, "forcing belongs to another network");
+        if (check_M(M)) return TXH_E_INVALID;
+        std::vector<char> seen(net->topo.n, 0);
+        for (int64_t k = 0; k < rec_count; ++k) {
+            if (rec_reach[k] < 0 || rec_reach[k] >= net->topo.n) return fail(TXH_E_INVALID, "recorded reach out of range");
+            if (seen[rec_reach[k]]++) return fail(TXH_E_INVALID, "recorded reach listed twice");
+        }
+    }
     cudaStream_t st = (cudaStream_t)stream;
     double* const rowsum_before = net->stats_rowsum;
     const double scale_before = net->stats_scale;
@@ -1484,8 +1531,54 @@ int txh_run_assimilating(txh_net* net, double* O, double* I, int64_t M, const tx
     if (rc == TXH_OK && fuse_load_ok && ld <= kMemberBlock && (rc = ensure_device(net)) == TXH_OK)
         fuse_load = (net->route_kernel == 0 || net->route_kernel == 2) && !lane_wanted(net, M, every) &&
                     run_window(net, O, I, M, nullptr, nullptr, 0, StepPlan(), every, st, true) == TXH_OK;
+    // recording: the slots once per call; after update k (step (k+1) every) the forecast rows go to prior_out[k] and the
+    // posterior ones -- what the state holds after that step -- to their rec_out slot (the window kernel recorded the
+    // forecast there).  In every path O still holds the forecast when enkf_record runs.
+    const bool rec = rec_count > 0;
+    if (rc == TXH_OK && rec) {
+        // (the arguments were checked above; the routing calls below go past txh_route_run's checks)
+        rc = ensure_device(net);
+        if (rc == TXH_OK) rc = ensure_coef(net, st);
+        if (rc == TXH_OK) rc = upload_rec_slots(net, rec_reach, rec_count, st);
+        if (rc == TXH_OK && (size_t)rec_count > net->rec_pos_cap) {
+            if (net->d_rec_pos) CU(cudaFree(net->d_rec_pos));
+            CU(cudaMalloc((void**)&net->d_rec_pos, sizeof(int32_t) * rec_count));
+            net->rec_pos_cap = (size_t)rec_count;
+        }
+        if (rc == TXH_OK) {
+            std::vector<int32_t> pos(rec_count);
+            for (int64_t k = 0; k < rec_count; ++k) pos[k] = net->sched.pos_of_reach[rec_reach[k]];
+            CU(cudaMemcpyAsync(net->d_rec_pos, pos.data(), sizeof(int32_t) * rec_count, cudaMemcpyHostToDevice, st));
+            CU(cudaStreamSynchronize(st));
+        }
+    }
+    const int32_t* rec_slot = rec ? net->d_rec_slot : nullptr;
+    // where update k's recorded rows go: the forecast to prior_out[k], the posterior to the slot of step (k+1) every
+    auto rec_prior_of = [&](int64_t k) -> double* { return prior_out ? prior_out + (size_t)k * rec_count * M : nullptr; };
+    auto rec_post_of = [&](int64_t k) -> double* {
+        const int64_t s_end = (k + 1) * every;
+        return s_end % rec_every == 0 ? rec_out + (size_t)(s_end / rec_every - 1) * rec_count * M : nullptr;
+    };
+    // update k applied by the stand-alone kernels: its rows recorded first, while O still holds the forecast
+    auto record_update = [&](int64_t k) -> int {
+        double *prior = rec_prior_of(k), *post = rec_post_of(k);
+        if (rec && (post || prior))
+            CU(launch_enkf_record(O, ld, (int)M, rowsum, T, net->d_gauge_of_pos, qs, W, net->d_rec_pos, (int)rec_count,
+                                  prior, post, st));
+        return TXH_OK;
+    };
+    // update k applied by the next window launch while it loads its tasks: that launch records its rows
+    auto set_pending = [&](int64_t k) {
+        net->pending.T = T; net->pending.W = W; net->pending.qs = qs; net->pending.M = M;
+        net->pending.rec_prior = rec ? rec_prior_of(k) : nullptr;
+        net->pending.rec_post = rec ? rec_post_of(k) : nullptr;
+        net->pending.rec_mean = rowsum;
+    };
     bool owed = false;                                     // an update computed (T, W) but not yet applied to O, I
+    int64_t owed_k = 0;                                    // ... and which one
     auto apply_owed = [&]() -> int {
+        int rc2 = record_update(owed_k);
+        if (rc2 != TXH_OK) return rc2;
         CU(launch_enkf_update(O, ld, (int)M, rowsum, T, (int)M, (int)M, O, nullptr, ld, net->topo.n, net->d_gauge_of_pos,
                               qs, W, 0, net->num_sms, (int)M, 0, st));
         CU(launch_inflow_rebuild(net->d_inner_rec, net->n_inner, net->d_up_off, net->d_up_pos, O, I, ld, st));
@@ -1497,10 +1590,12 @@ int txh_run_assimilating(txh_net* net, double* O, double* I, int64_t M, const tx
         const bool timed = time_every > 0 && k % time_every == 0 && net->route_events.size() < 4096;
         if (timed) { CU(cudaEventCreate(&e0)); CU(cudaEventCreate(&e1)); CU(cudaEventRecord(e0, st)); }
         if (owed) {
-            if (net->gfix_ok) { net->pending.T = T; net->pending.W = W; net->pending.qs = qs; net->pending.M = M; }
+            if (net->gfix_ok) set_pending(owed_k);
             else rc = apply_owed();
         }
-        if (rc == TXH_OK) rc = txh_route_run(net, O, I, M, fo, t, dt_ns, every, method, nullptr, 0, 1, nullptr, stream);
+        if (rc == TXH_OK) rc = rec ? route_run_impl(net, O, I, M, fo, t, dt_ns, every, method, rec_slot, rec_count, rec_every,
+                                                    rec_out, k * every, st)
+                                   : txh_route_run(net, O, I, M, fo, t, dt_ns, every, method, nullptr, 0, 1, nullptr, stream);
         if (rc == TXH_OK && owed) {
             if (net->pending.T) { net->pending.T = nullptr; rc = fail(TXH_E_STATE, "the routing launch did not take the pending ensemble update"); }
             owed = false;
@@ -1514,25 +1609,28 @@ int txh_run_assimilating(txh_net* net, double* O, double* I, int64_t M, const tx
         if (rc == TXH_OK) rc = enkf_solve_impl(net, m, M, HX, O, Zp + (size_t)k * m * M, rowsum, obs, qs, R, Dinv, dinv_kind, work, W, T, stream);
         if (rc != TXH_OK) break;
         if (ld <= kMemberBlock) {
-            owed = true;
+            owed = true; owed_k = k;
             if (!fuse_load) rc = apply_owed();
         } else {
-            rc = txh_enkf_apply(net, O, I, M, nullptr, 0, 0, M, 0, rowsum, T, obs, m, qs, W, G, stream);
+            rc = record_update(k);
+            if (rc == TXH_OK) rc = txh_enkf_apply(net, O, I, M, nullptr, 0, 0, M, 0, rowsum, T, obs, m, qs, W, G, stream);
         }
     }
     net->stats_rowsum = nullptr;
     if (rc == TXH_OK && nsteps > nwin * every) {
-        if (owed && net->gfix_ok && !lane_wanted(net, M, nsteps - nwin * every)) {
-            net->pending.T = T; net->pending.W = W; net->pending.qs = qs; net->pending.M = M;
-        } else if (owed) rc = apply_owed();
-        if (rc == TXH_OK) rc = txh_route_run(net, O, I, M, fo, t, dt_ns, nsteps - nwin * every, method, nullptr, 0, 1, nullptr, stream);
+        if (owed && net->gfix_ok && !lane_wanted(net, M, nsteps - nwin * every)) set_pending(owed_k);
+        else if (owed) rc = apply_owed();
+        if (rc == TXH_OK)
+            rc = rec ? route_run_impl(net, O, I, M, fo, t, dt_ns, nsteps - nwin * every, method, rec_slot, rec_count, rec_every,
+                                      rec_out, nwin * every, st)
+                     : txh_route_run(net, O, I, M, fo, t, dt_ns, nsteps - nwin * every, method, nullptr, 0, 1, nullptr, stream);
         if (rc == TXH_OK && owed) {
             if (net->pending.T) { net->pending.T = nullptr; rc = fail(TXH_E_STATE, "the routing launch did not take the pending ensemble update"); }
             owed = false;
         }
     }
     if (rc == TXH_OK && owed) rc = apply_owed();           // after the last window the posterior goes to memory
-    net->pending.T = nullptr;
+    net->pending.T = nullptr; net->pending.rec_prior = net->pending.rec_post = nullptr;
     net->stats_rowsum = rowsum_before; net->stats_scale = scale_before;
     return rc;
 }

@@ -1173,6 +1173,59 @@ inflow_rebuild_kernel(const int4* __restrict__ rec, long long n_inner, const int
 
 inline unsigned nblk(long long work, int threads) { return (unsigned)((work + threads - 1) / threads); }
 
+// Hydrographs of txh_run_assimilating_rec at an update: the forecast of the recorded rows (prior_out) and what the
+// update makes of them (post_out), o + (o - mean) T + qs_g W_g [row gauged] -- the rows of enkf_update_kernel, for a
+// few rows and in plain FP64, read from O while it still holds the forecast.
+// Used where the update is applied by the stand-alone kernels (TXH_ENKF_FUSE_LOAD=0, M > 64, the lane kernel, the update
+// after the last window); where the next window applies it, that launch records the rows itself (record_posterior,
+// txh_window.cu).  A CTA holds T in shared memory (M <= 64) and the anomalies of RG rows: one thread per (row, member).
+
+__global__ void __launch_bounds__(256)
+enkf_record_kernel(const double* __restrict__ O, int ld, int M, const double* __restrict__ mean,
+                   const double* __restrict__ T, const int32_t* __restrict__ gauge_of_pos, const double* __restrict__ qs,
+                   const double* __restrict__ W, const int32_t* __restrict__ rec_pos, int rec_count,
+                   double* __restrict__ prior_out, double* __restrict__ post_out)
+{
+    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+    extern __shared__ double rs_sm[];
+    const int tid = threadIdx.x;
+    const int Mc = M < 256 ? M : 256;                 // threads per row
+    const int RG = 256 / Mc;                          // rows per pass
+    const int q = tid / Mc, cl = tid - q * Mc;
+    const bool stage_a = M <= 4096, stage_t = M <= 64;
+    double* sa = rs_sm;                               // [RG][M] anomalies o - mean
+    double* sT = rs_sm + (stage_a ? RG * M : 0);      // [M][M]
+    asm volatile("griddepcontrol.wait;" ::: "memory");
+    if (stage_t)
+        for (int e = tid; e < M * M; e += blockDim.x) sT[e] = __ldcg(T + e);
+    for (int k0 = blockIdx.x * RG; k0 < rec_count; k0 += gridDim.x * RG) {
+        const int k = k0 + q;
+        const bool on = q < RG && k < rec_count;
+        const int pos = on ? __ldg(rec_pos + k) : 0;
+        const double* o = O + (size_t)pos * ld;
+        const double mu = on ? __ldcg(mean + pos) : 0.0;
+        __syncthreads();                              // the previous pass is done with sa (and T is staged)
+        if (on && stage_a)
+            for (int c = cl; c < M; c += Mc) sa[q * M + c] = __ldcg(o + c) - mu;
+        __syncthreads();
+        if (!on) continue;
+        const int gi = __ldg(gauge_of_pos + pos);
+        for (int c = cl; c < M; c += Mc) {
+            const double oc = __ldcg(o + c);
+            const size_t at = (size_t)k * M + c;
+            if (prior_out) prior_out[at] = oc;
+            if (!post_out) continue;
+            double g = 0.0;
+            for (int j = 0; j < M; ++j) {
+                const double a = stage_a ? sa[q * M + j] : __ldcg(o + j) - mu;
+                g = fma(a, stage_t ? sT[j * M + c] : __ldcg(T + (size_t)j * M + c), g);
+            }
+            if (gi >= 0) g += __ldcg(qs + gi) * __ldcg(W + (size_t)gi * M + c);
+            post_out[at] = oc + g;
+        }
+    }
+}
+
 }  // namespace
 
 cudaError_t launch_dgemm(int transA, int transB, int M, int N, int K, double alpha, const double* A, int lda,
@@ -1411,6 +1464,28 @@ cudaError_t launch_inflow_rebuild(const int4* rec, int64_t n_inner, const int32_
     inflow_rebuild_kernel<<<nblk(((n_inner + 1) >> 1) * (ld >> 1), 256), 256, 0, st>>>(rec, n_inner, up_off, up_pos, O, I, ld);
     count_launch();
     return cudaGetLastError();
+}
+
+cudaError_t launch_enkf_record(const double* O, int ld, int M, const double* mean, const double* T,
+                               const int32_t* gauge_of_pos, const double* qs, const double* W, const int32_t* rec_pos,
+                               int rec_count, double* prior_out, double* post_out, cudaStream_t st)
+{
+    const long long work = (long long)rec_count * M;
+    if (work == 0 || (!prior_out && !post_out)) return cudaSuccess;
+    static const bool pdl = [] { const char* k = getenv("TXH_PDL"); return !(k && atoi(k) == 0); }();
+    const int Mc = M < 256 ? M : 256, RG = 256 / Mc;
+    const size_t smem = sizeof(double) * ((M <= 4096 ? (size_t)RG * M : 0) + (M <= 64 ? (size_t)M * M : 0));
+    const int grid = (int)((rec_count + RG - 1) / RG);
+    cudaLaunchConfig_t cfg{};
+    cfg.gridDim = dim3(grid); cfg.blockDim = dim3(256); cfg.dynamicSmemBytes = smem; cfg.stream = st;
+    cudaLaunchAttribute attr{};
+    attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr.val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = &attr; cfg.numAttrs = pdl ? 1 : 0;
+    cudaError_t e = cudaLaunchKernelEx(&cfg, enkf_record_kernel, O, ld, M, mean, T, gauge_of_pos, qs, W, rec_pos, rec_count,
+                                       prior_out, post_out);
+    count_launch();
+    return e != cudaSuccess ? e : cudaGetLastError();
 }
 
 cudaError_t launch_inflow_gain(const int32_t* inner, int64_t n_inner, const int32_t* up_off, const int32_t* up_pos,

@@ -66,6 +66,7 @@ struct RouteArgs {
     const double* Wmul;                   // [R][wm_ld] member multipliers, or nullptr
     const int32_t* rec_slot;              // [n] recording slot of each position or -1; nullptr = off
     double* rec_out;                      // [nrec_steps][rec_count][M]
+    long long rec_step_base;              // steps of the call before this launch
     // dataflow runtime state (one entry per (task, member block) pair)
     int32_t* pending;                     // outstanding dependencies of the pair's next step
     unsigned long long* queue;            // ready queue: (step << 32) | (pair + 1), 0 = not yet pushed
@@ -137,6 +138,16 @@ struct WinArgs {
     const double* upQs;                   // [gauges]
     const int32_t* gfix_off;              // [n_tasks + 1] gauge terms per task
     const int2* gfix;                     // {row in task | kind << 16 (0: the row's own gauge, chi; 1: an upstream gauge, beta), gauge}
+    // optional recording (REC variant): the outflow of every recorded row after every rec_every-th step of the call
+    const int32_t* rec_slot;              // [n] recording slot of each position or -1; nullptr = off
+    double* rec_out;                      // [steps recorded][rec_count][M]
+    long long rec_step_base;              // steps of the call before this launch
+    int32_t rec_every, rec_count;
+    // UPD + REC: the recorded rows of the update this launch applies, [rec_count][M] each (nullptr = not wanted):
+    // the forecast (rec_prior) and the posterior o + (o - mean) T + qs W (rec_post); rec_mean = the forecast's row means
+    double* rec_prior;
+    double* rec_post;
+    const double* rec_mean;
 };
 
 // route_lane_kernel (txh_lane.cu): lanes = reaches, time-skewed regions, state in shared memory
@@ -247,6 +258,11 @@ cudaError_t launch_enkf_update(const double* Xall, int ldx, int Mtot, const doub
                                cudaStream_t st, const PeerBlocks* peers = nullptr, double* Oout = nullptr);
 cudaError_t launch_inflow_rebuild(const int4* rec, int64_t n_inner, const int32_t* up_off, const int32_t* up_pos,
                                   const double* O, double* I, int ld, cudaStream_t st);
+// prior_out[k][:] = O[rec_pos[k]][:] (forecast), post_out[k][:] = the same row after the update of (T, W) (da.py:124-126);
+// either may be nullptr.  Launched between the ensemble-space system and the next routing launch (PDL chain).
+cudaError_t launch_enkf_record(const double* O, int ld, int M, const double* mean, const double* T,
+                               const int32_t* gauge_of_pos, const double* qs, const double* W, const int32_t* rec_pos,
+                               int rec_count, double* prior_out, double* post_out, cudaStream_t st);
 cudaError_t launch_inflow_gain(const int32_t* inner, int64_t n_inner, const int32_t* up_off, const int32_t* up_pos,
                                const double* G, double* I, int ld, cudaStream_t st);
 

@@ -125,8 +125,9 @@ __device__ __forceinline__ void record(const RouteArgs& a, int k, int s, int col
 {
     if (REC) {
         const int rs = a.rec_slot[k];
-        if (rs >= 0 && ((s + 1) % a.rec_every) == 0 && col < a.M) {
-            double* dst = a.rec_out + ((size_t)((s + 1) / a.rec_every - 1) * a.rec_count + rs) * a.M + col;
+        const long long gs = a.rec_step_base + s + 1;
+        if (rs >= 0 && (gs % a.rec_every) == 0 && col < a.M) {
+            double* dst = a.rec_out + ((size_t)(gs / a.rec_every - 1) * a.rec_count + rs) * a.M + col;
             dst[0] = on.x;
             if (col + 1 < a.M) dst[1] = on.y;
         }

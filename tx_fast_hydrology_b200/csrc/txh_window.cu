@@ -23,6 +23,12 @@
 // freshly loaded p rows with the 64 x 64 matrix T on the FP64 tensor cores (transform_p_rows) and the posterior state
 // never goes through global memory.  Such a launch may start while the kernel that computes T still runs
 // (programmatic dependent launch): it loads its first tasks and waits for T only then (stage_T).
+//
+// Recording variant (template parameter REC; txh_route_run / txh_run_assimilating_rec with rec_*): after every step of
+// the call that is a multiple of rec_every the outflow of each recorded row goes to rec_out[step / rec_every - 1][k][M].
+// A row's slot k rides in the spare word of its per-row record.  A pocket row has its outflow in registers every step;
+// a segment's interior rows never form theirs before the last step of a launch (only p0 is kept, the FIX loop folds
+// C_k o_in into it), so PRE stores B_k into the row's rec_out cell and the same lane adds A_k o_in in the FIX loop.
 #include <cstdlib>
 
 #include "txh_kernels.cuh"
@@ -231,9 +237,21 @@ __device__ __forceinline__ void emit_rowsum(const WinArgs& a, int pos, int col, 
     if (lane == 0) a.rowsum[pos] = v * a.rowsum_scale;
 }
 
+// this lane's columns (< M) of a recorded row: rj = index of the recorded step, rs = the row's slot
+__device__ __forceinline__ double* rec_cell(const WinArgs& a, int rj, int rs, int col)
+{
+    return a.rec_out + ((size_t)rj * a.rec_count + rs) * a.M + col;
+}
+__device__ __forceinline__ void rec_store(const WinArgs& a, int rj, int rs, int col, double2 v)
+{
+    double* d = rec_cell(a, rj, rs, col);
+    if (col < a.M) d[0] = v.x;
+    if (col + 1 < a.M) d[1] = v.y;
+}
+
 // Per-row record in shared memory (48 bytes): everything a row update needs besides its state row, read with
 // three 128-bit loads one row ahead of the arithmetic.
-//   +0 header word   +8 alpha   +16 beta   +24 chi   +32 gamma*F[r0]   +40 gamma*F[r1]
+//   +0 header word   +4 recording slot (REC)   +8 alpha   +16 beta   +24 chi   +32 gamma*F[r0]   +40 gamma*F[r1]
 constexpr unsigned kRec = 48u;
 struct RowIn {
     uint32_t h;
@@ -278,6 +296,9 @@ struct Tk {
     size_t step_bytes;
 };
 
+// recording slot of row r of the task (-1: not recorded), staged at task load
+__device__ __forceinline__ int rec_slot_of(const Tk& tk, int r) { return (int)lds_u32(tk.sRec + kRec * r + 4u); }
+
 // p + gamma*q of this lane's two members, accumulated with fused multiply-adds (one operation less per member than
 // forming q first)
 template <bool HAS_F, bool HAS_W>
@@ -296,9 +317,10 @@ __device__ __forceinline__ double2 forcing_add(const FCtx& c, double g0, double 
 }
 
 // One row of a pocket step (see pocket_step)
-template <bool LAST, bool HAS_F, bool HAS_W, int IR>
+template <bool LAST, bool HAS_F, bool HAS_W, int IR, bool REC>
 __device__ __forceinline__ void pocket_row(const WinArgs& a, const Tk& tk, InStream& ist, const FCtx& fc, char* ringS,
-                                           const RowIn& x, double2& acc, unsigned& aW, unsigned aP, double* ig, double* og, int r)
+                                           const RowIn& x, double2& acc, unsigned& aW, unsigned aP, double* ig, double* og, int r,
+                                           int rj)
 {
     const uint32_t h = x.h;
     double2 inflow = (h & HDR_ACC) ? acc : make_double2(0.0, 0.0);
@@ -322,6 +344,10 @@ __device__ __forceinline__ void pocket_row(const WinArgs& a, const Tk& tk, InStr
         if (tk.active) { st_row(ig, inflow); st_row(og, on); }
         if (a.rowsum) emit_rowsum(a, tk.begin + r, tk.col, on, tk.lane);
     }
+    if (REC && rj >= 0) {
+        const int rs = rec_slot_of(tk, r);
+        if (rs >= 0) rec_store(a, rj, rs, tk.col, on);
+    }
     if (h & (HDR_PUSH | 0x3eu)) {                               // published and / or parked in a scratch row
         if (h & HDR_PUSH) {
             const uint32_t slot = lds_u32(aW);
@@ -338,8 +364,9 @@ __device__ __forceinline__ void pocket_row(const WinArgs& a, const Tk& tk, InStr
 // a row (RowIn) is read one row ahead of the arithmetic.  (Unrolling the walk by two rows with the two records
 // alternating removes the 17 register moves at the loop edge -- and was 8 % slower: the kernel is sensitive to its code
 // size.)
-template <bool LAST, bool HAS_F, bool HAS_W, int IR>
-__device__ __forceinline__ void pocket_step(const WinArgs& a, const Tk& tk, InStream& ist, const FCtx& fc, char* ringS)
+template <bool LAST, bool HAS_F, bool HAS_W, int IR, bool REC>
+__device__ __forceinline__ void pocket_step(const WinArgs& a, const Tk& tk, InStream& ist, const FCtx& fc, char* ringS,
+                                            int rj)
 {
     unsigned aRec = tk.sRec, aP = tk.sP, aW = tk.sWords;
     double* ig = tk.Ig;
@@ -349,7 +376,7 @@ __device__ __forceinline__ void pocket_step(const WinArgs& a, const Tk& tk, InSt
     for (int r = 0; r < tk.len; ++r) {
         const RowIn x = nx;
         if (r + 1 < tk.len) nx = load_rowin(aRec + kRec, aP + 512u);
-        pocket_row<LAST, HAS_F, HAS_W, IR>(a, tk, ist, fc, ringS, x, acc, aW, aP, ig, og, r);
+        pocket_row<LAST, HAS_F, HAS_W, IR, REC>(a, tk, ist, fc, ringS, x, acc, aW, aP, ig, og, r, rj);
         aRec += kRec; aP += 512u;
         ig += tk.ld; og += tk.ld;
     }
@@ -361,9 +388,9 @@ __device__ __forceinline__ void pocket_step(const WinArgs& a, const Tk& tk, InSt
 //   C_k = beta_k A_{k-1} + chi_k A_k  (A = prefix product of alpha, A_{-1} = 1; precomputed).
 // Hop: out = A_last * o_in + B_last, handed on before anything else.  In the last step (side_k, B_k) are
 // parked in the global I / O rows for the final fix-up o_k = B_k + A_k o_in, i_k = o_{k-1} + side_k.
-template <bool LAST, bool HAS_F, bool HAS_W, int SR>
+template <bool LAST, bool HAS_F, bool HAS_W, int SR, bool REC>
 __device__ __forceinline__ void segment_step(const WinArgs& a, const Tk& tk, InStream& ist, const FCtx& fc, char* ringS,
-                                             int out_slot, unsigned long long* trs)
+                                             int out_slot, unsigned long long* trs, int rj)
 {
     unsigned aRec = tk.sRec, aP = tk.sP;
     double* ig = tk.Ig;
@@ -389,6 +416,10 @@ __device__ __forceinline__ void segment_step(const WinArgs& a, const Tk& tk, InS
             p0.x = x.be * inflow.x + x.ch * B.x;
             p0.y = x.be * inflow.y + x.ch * B.y;
             sts_row(aP, p0);
+            if (REC && rj >= 0) {                                   // B_k; the FIX loop adds A_k o_in
+                const int rs = rec_slot_of(tk, r);
+                if (rs >= 0) rec_store(a, rj, rs, tk.col, B);
+            }
         } else {
             if (tk.active) { st_row(ig, side); st_row(og, B); }
             ig += tk.ld; og += tk.ld;
@@ -419,6 +450,21 @@ __device__ __forceinline__ void segment_step(const WinArgs& a, const Tk& tk, InS
             p0.x = C * oin.x + p0.x;
             p0.y = C * oin.y + p0.y;
             sts_row(aQ, p0);
+            if (REC && rj >= 0) {
+                // o_k = B_k + A_k o_in (B_k parked in the row's cell by PRE); the last row's is `out`
+                const int rs = rec_slot_of(tk, r);
+                if (rs >= 0) {
+                    double2 o = out;
+                    if (r + 1 < tk.len) {
+                        const double A = lds_f64(tk.sCum + 8u * r);
+                        const double* d = rec_cell(a, rj, rs, tk.col);
+                        const double b0 = tk.col < a.M ? d[0] : 0.0, b1 = tk.col + 1 < a.M ? d[1] : 0.0;
+                        o.x = A * oin.x + b0;
+                        o.y = A * oin.y + b1;
+                    }
+                    rec_store(a, rj, rs, tk.col, o);
+                }
+            }
             aQ += 512u; aC += 8u;
         }
     } else {
@@ -439,6 +485,10 @@ __device__ __forceinline__ void segment_step(const WinArgs& a, const Tk& tk, InS
             it.y = op.y + side.y;
             if (tk.active) { st_row(og, on); st_row(ig, it); }
             if (a.rowsum) emit_rowsum(a, tk.begin + r, tk.col, on, tk.lane);
+            if (REC && rj >= 0) {
+                const int rs = rec_slot_of(tk, r);
+                if (rs >= 0) rec_store(a, rj, rs, tk.col, on);
+            }
             op = on;
             ig += tk.ld; og += tk.ld;
         }
@@ -510,10 +560,56 @@ __device__ __noinline__ void transform_p_rows(const WinArgs& a, unsigned sb, uns
     }
 }
 
+// UPD + REC: the forecast and the posterior of the task's recorded rows for the update this launch applies (the posterior
+// of the fused loop never reaches HBM otherwise).  Runs at task load, T staged, before the task writes any row of O: the
+// forecast row is still in O.  A lane loads its two members and forms o + sum_j (o_j - mean) T[j][c] + qs_g W_g[c] (own
+// gauge) with the other members shuffled in: one memory latency per row, not one per member.
+__device__ __noinline__ void record_posterior(const WinArgs& a, unsigned sRec, unsigned sT, int task, int begin, int len,
+                                              int lane)
+{
+    const int M = a.M, c0 = 2 * lane, c1 = c0 + 1;
+    for (int r = 0; r < len; ++r) {
+        const int rs = (int)lds_u32(sRec + kRec * r + 4u);
+        if (rs < 0) continue;
+        const double* o = a.O + (size_t)(begin + r) * a.ld;
+        const double mu = __ldcg(a.rec_mean + begin + r);
+        // this lane's two members of the row in one load; member j comes from lane j / 2 by a shuffle
+        const double2 ov = c0 < a.ld ? ld_row(o + c0) : make_double2(0.0, 0.0);
+        double g0 = 0.0, g1 = 0.0;
+#pragma unroll 4
+        for (int j = 0; j < M; j += 2) {
+            const double oa = __shfl_sync(0xffffffffu, ov.x, j >> 1) - mu, ob = __shfl_sync(0xffffffffu, ov.y, j >> 1) - mu;
+            g0 = fma(oa, lds_f64(sT + t_swz(j, c0 & 63)), g0);
+            g1 = fma(oa, lds_f64(sT + t_swz(j, c1 & 63)), g1);
+            if (j + 1 < M) {
+                g0 = fma(ob, lds_f64(sT + t_swz(j + 1, c0 & 63)), g0);
+                g1 = fma(ob, lds_f64(sT + t_swz(j + 1, c1 & 63)), g1);
+            }
+        }
+        for (int e = __ldg(a.gfix_off + task), e1 = __ldg(a.gfix_off + task + 1); e < e1; ++e) {
+            const int2 x = __ldg(a.gfix + e);
+            if ((x.x >> 16) != 0 || (x.x & 0xffff) != r) continue;      // the row's own gauge only
+            const double q = __ldg(a.upQs + x.y);
+            const double* wr = a.upW + (size_t)x.y * M;
+            if (c0 < M) g0 += q * __ldg(wr + c0);
+            if (c1 < M) g1 += q * __ldg(wr + c1);
+        }
+        const size_t at = (size_t)rs * M;
+        if (c0 < M) {
+            if (a.rec_prior) a.rec_prior[at + c0] = ov.x;
+            if (a.rec_post) a.rec_post[at + c0] = ov.x + g0;
+        }
+        if (c1 < M) {
+            if (a.rec_prior) a.rec_prior[at + c1] = ov.y;
+            if (a.rec_post) a.rec_post[at + c1] = ov.y + g1;
+        }
+    }
+}
+
 // Shared-memory state of a task: ONE row per reach, p = beta*i + chi*o, the part of the next update that
 // depends on the old state (o' = alpha*inflow + (gamma*q + p)); the outflows and inflows themselves only
 // exist in registers, and are written to global memory in the last step of the launch.
-template <bool HAS_F, bool HAS_W, bool UPD>
+template <bool HAS_F, bool HAS_W, bool UPD, bool REC>
 __global__ void __launch_bounds__(kWinThreads, 1)
 route_window_kernel(const WinArgs a)
 {
@@ -633,6 +729,7 @@ route_window_kernel(const WinArgs a)
             const double2 cg = *reinterpret_cast<const double2*>(a.coef + 4 * (size_t)(td.begin + i) + 2);
             const unsigned rec = tk.sRec + kRec * i;
             sts_u32(rec, a.hdr[td.begin + i]);
+            if (REC) sts_u32(rec + 4u, (uint32_t)__ldg(a.rec_slot + td.begin + i));
             sts_f64(rec + 8u, ab.x);
             sts_row(rec + 16u, make_double2(ab.y, cg.x));
             sts_row(rec + 32u, make_double2(0.0, 0.0));
@@ -688,6 +785,7 @@ route_window_kernel(const WinArgs a)
                 }
             }
             __syncwarp();
+            if (REC && (a.rec_prior || a.rec_post)) record_posterior(a, tk.sRec, sT, task, td.begin, len, lane);
         }
         // rows of other tasks consumed through the input ring, in consumption order: byte offsets of their slots
         int nL = 0;
@@ -739,6 +837,11 @@ route_window_kernel(const WinArgs a)
             const bool last = s + 1 == a.nsteps;                   // outflows and inflows go to global memory
             char* ringS = reinterpret_cast<char*>(a.ring + ccol) + (size_t)s * tk.step_bytes;
             const FCtx fc = fc_next;
+            int rj = -1;                                          // index of this step in rec_out, if it is recorded
+            if (REC) {
+                const long long gs = a.rec_step_base + s + 1;
+                if (gs % a.rec_every == 0) rj = (int)(gs / a.rec_every - 1);
+            }
             if (HAS_F) {
                 const int2 rr = step_rows(s);
                 const int r0 = rr.x, r1 = rr.y;
@@ -757,13 +860,13 @@ route_window_kernel(const WinArgs a)
                 if (!last) fc_next = load_fctx(s + 1);           // in flight during this step
             }
             if (!seg) {
-                if (last) pocket_step<true, HAS_F, HAS_W, IR>(a, tk, ist, fc, ringS);
-                else pocket_step<false, HAS_F, HAS_W, IR>(a, tk, ist, fc, ringS);
+                if (last) pocket_step<true, HAS_F, HAS_W, IR, REC>(a, tk, ist, fc, ringS, rj);
+                else pocket_step<false, HAS_F, HAS_W, IR, REC>(a, tk, ist, fc, ringS, rj);
                 if (tr && lane == 0) tr[4 + s] = globaltimer_ns();
             } else {
                 unsigned long long* trs = tr ? tr + 4 + s : nullptr;
-                if (last) segment_step<true, HAS_F, HAS_W, SR>(a, tk, ist, fc, ringS, td.out_slot, trs);
-                else segment_step<false, HAS_F, HAS_W, SR>(a, tk, ist, fc, ringS, td.out_slot, trs);
+                if (last) segment_step<true, HAS_F, HAS_W, SR, REC>(a, tk, ist, fc, ringS, td.out_slot, trs, rj);
+                else segment_step<false, HAS_F, HAS_W, SR, REC>(a, tk, ist, fc, ringS, td.out_slot, trs, rj);
             }
             if (ist.dead) break;
         }
@@ -800,6 +903,14 @@ __global__ void __launch_bounds__(256) window_init_kernel(const InitArgs a, unsi
     }
 }
 
+template <bool REC>
+auto pick_window_kernel(bool f, bool w, bool u) -> void (*)(const WinArgs)
+{
+    if (!f) return u ? route_window_kernel<false, false, true, REC> : route_window_kernel<false, false, false, REC>;
+    if (!w) return u ? route_window_kernel<true, false, true, REC> : route_window_kernel<true, false, false, REC>;
+    return u ? route_window_kernel<true, true, true, REC> : route_window_kernel<true, true, false, REC>;
+}
+
 }  // namespace
 
 cudaError_t launch_window_init(const InitArgs& a, unsigned long long* ticket, cudaStream_t st)
@@ -814,12 +925,9 @@ cudaError_t launch_route_window(const WinArgs& a, int warps_per_cta, int num_sms
     const size_t smem = (size_t)a.off_steps + 16 * 24;          // [per-warp areas][T + counter (update variant)][step records]
     (void)warps_per_cta;
     static const bool pdl = [] { const char* k = getenv("TXH_PDL"); return !(k && atoi(k) == 0); }();
-    void (*kern)(const WinArgs) = nullptr;
     const bool f = a.F != nullptr, w = a.Wmul != nullptr;
     const bool u = a.upT != nullptr;
-    if (!f) kern = u ? route_window_kernel<false, false, true> : route_window_kernel<false, false, false>;
-    else if (!w) kern = u ? route_window_kernel<true, false, true> : route_window_kernel<true, false, false>;
-    else kern = u ? route_window_kernel<true, true, true> : route_window_kernel<true, true, false>;
+    void (*kern)(const WinArgs) = a.rec_slot ? pick_window_kernel<true>(f, w, u) : pick_window_kernel<false>(f, w, u);
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     const long long pairs = (long long)a.n_tasks * a.n_mblocks;

@@ -443,7 +443,25 @@ class Muskingum:
         self.datetime = self.datetime + nsteps * self.timedelta
         return rec
 
-    def run_assimilating(self, forcing, nsteps, enkf, every, observations, timers=None, observations_ready=None):
+    def _record_reaches(self, record_reaches, record_every, nsteps):
+        """Checked reach list (reference order) of a recording run, as int64 numpy."""
+        if isinstance(record_every, bool) or int(record_every) != record_every or record_every < 1:
+            raise ValueError(f'`record_every` must be a positive integer, got {record_every!r}')
+        idx = np.asarray(record_reaches.cpu() if hasattr(record_reaches, 'cpu') else record_reaches)
+        if idx.ndim != 1 or idx.size == 0 or not np.issubdtype(idx.dtype, np.integer):
+            raise ValueError('`record_reaches` must be a non-empty 1-D list of integer reach indices')
+        idx = idx.astype(np.int64)
+        n = len(self.reach_ids)
+        if idx.min() < 0 or idx.max() >= n:
+            raise ValueError(f'`record_reaches` out of range [0, {n})')
+        if np.unique(idx).size != idx.size:
+            raise ValueError('`record_reaches` lists a reach twice')
+        if nsteps // int(record_every) < 1:
+            raise ValueError(f'`record_every` = {record_every} records nothing in {nsteps} steps')
+        return idx
+
+    def run_assimilating(self, forcing, nsteps, enkf, every, observations, timers=None, observations_ready=None,
+                         record_reaches=None, record_every=1, record_prior=False):
         """Device-resident run with periodic ensemble assimilation: `every` routing steps in one
         persistent launch, then one `EnsembleKalmanFilter` update with `observations[k]` ([m][Mtot]
         CUDA tensor of per-member observations for the k-th update), repeated; nothing returns to
@@ -453,13 +471,30 @@ class Muskingum:
         keeps them in the library (`network.route_timings()` returns their durations), the sharded one appends
         (start, end) torch event pairs.
         `observations_ready`: optional `torch.cuda.Event` recorded after an upload of `observations` on another
-        stream; the first update waits for it (the first routing window does not)."""
+        stream; the first update waits for it (the first routing window does not).
+        `record_reaches` (reach indices, reference order): also record the ensemble hydrographs there and return
+        `rec`, a CUDA tensor [nsteps // record_every][k][members]: after every `record_every`-th step what a simulate
+        loop with the filter bound sees in `o_t_next` -- the forecast, or the posterior at an update step.  With
+        `record_prior`, returns (rec, prior), prior [nsteps // every][k][members] the forecast each update started from.
+        A member-sharded filter records this rank's members.  Without `record_reaches`, returns None.
+        The Python loop (observations as a list, or a member-sharded filter) records every step of a window into a
+        scratch buffer and copies the wanted steps out, and each of its routing calls uploads the slot map again and
+        synchronises: correct, with per-window host work on a path that already has it; the in-library loop does this
+        once per call."""
+        ridx = None if record_reaches is None else self._record_reaches(record_reaches, record_every, nsteps)
         torch = self._ensure_device()
         self._sync_coeffs()
         d, net, M = self._dev, self.network, self.members
         step_ns = int(self.timedelta.value)
         t = int(self.datetime.value)
         nwin = nsteps // every
+        rec = prior = None
+        if ridx is not None:
+            record_every = int(record_every)
+            rec = torch.zeros((nsteps // record_every, ridx.size, M), dtype=torch.float64, device='cuda')
+            if record_prior:
+                prior = torch.zeros((nwin, ridx.size, M), dtype=torch.float64, device='cuda')
+        result = None if rec is None else ((rec, prior) if record_prior else rec)
         if torch.is_tensor(observations) or isinstance(observations, np.ndarray):
             want = (enkf.num_measurements, enkf.Mtot)
             if observations.ndim != 3 or observations.shape[0] < nwin or tuple(observations.shape[1:]) != want:
@@ -470,14 +505,28 @@ class Muskingum:
             net.run_assimilating(d['O'], d['I'], M, forcing, t, step_ns, nsteps, every, enkf.reach_indices,
                                  observations, enkf._qs, enkf._R, enkf._Dinv, enkf._dinv_kind, enkf._rowsum, enkf._HX,
                                  enkf._work, enkf._W, enkf._T, enkf._G, time_every=8 if timers is not None else 0,
-                                 obs_ready=observations_ready)
+                                 obs_ready=observations_ready, rec_reach=ridx, rec_every=record_every, rec_out=rec,
+                                 prior_out=prior)
             enkf.n_updates += nwin
             self._datetime = pd.Timestamp(t + nsteps * step_ns, tz='UTC')
             enkf.datetime = self._datetime
             self._device_advanced()
-            return
+            return result
         if observations_ready is not None:
             torch.cuda.current_stream().wait_event(observations_ready)
+        # recording: every step of a window into `win`, the steps that are multiples of record_every copied out of it
+        win = None if rec is None else torch.empty((every, ridx.size, M), dtype=torch.float64, device='cuda')
+
+        def route(nst, s0):
+            if rec is None:
+                net.route_run(d['O'], d['I'], M, forcing, t, step_ns, nst)
+                return
+            net.route_run(d['O'], d['I'], M, forcing, t, step_ns, nst, rec_reach=ridx, rec_every=1, rec_out=win)
+            first = (s0 // record_every + 1) * record_every         # first recorded step of the window (1-based)
+            steps = torch.arange(first, s0 + nst + 1, record_every, device='cuda')
+            if steps.numel():
+                rec.index_copy_(0, steps // record_every - 1, win.index_select(0, steps - s0 - 1))
+
         # the ensemble row sums ride on the last step of every routing launch
         net.set_stats_output(enkf._rowsum, enkf.stats_scale())
         for k in range(nwin):
@@ -485,20 +534,27 @@ class Muskingum:
             if timed:
                 e0 = torch.cuda.Event(enable_timing=True); e1 = torch.cuda.Event(enable_timing=True)
                 e0.record()
-            net.route_run(d['O'], d['I'], M, forcing, t, step_ns, every)
+            route(every, k * every)
             if timed:
                 e1.record()
                 timers.append((e0, e1))
             t += every * step_ns
             self._datetime = pd.Timestamp(t, tz='UTC')
+            if prior is not None:
+                net.gather_rows(d['O'], M, ridx, prior[k])
             enkf.filter(observations[k], stats_fresh=True)
+            s_end = (k + 1) * every
+            if rec is not None and s_end % record_every == 0:
+                # the posterior; a filter on the peer-read path has swapped the state buffer
+                net.gather_rows(d['O'], M, ridx, rec[s_end // record_every - 1])
         net.set_stats_output(None)
         rest = nsteps - nwin * every
         if rest:
-            net.route_run(d['O'], d['I'], M, forcing, t, step_ns, rest)
+            route(rest, nwin * every)
             t += rest * step_ns
         self._datetime = pd.Timestamp(t, tz='UTC')
         self._device_advanced()
+        return result
 
     def upload_state(self, o_t_next, i_t_next=None):
         """`init_states` (muskingum.py:410-419) without the host round trip: `o_t_next` ([n][members],

@@ -301,15 +301,23 @@ class RiverNetwork:
                                         _stream_ptr()))
 
     def run_assimilating(self, O, I, M, forcing, t0_ns, dt_ns, nsteps, every, obs_reach, Zp, qs, R, Dinv, dinv_kind,
-                         rowsum, HX, work, W, T, G, method=1, time_every=0, obs_ready=None):
-        """`txh_run_assimilating`: routing windows + ensemble updates of an unsharded ensemble, host out of the loop."""
+                         rowsum, HX, work, W, T, G, method=1, time_every=0, obs_ready=None, rec_reach=None, rec_every=1,
+                         rec_out=None, prior_out=None):
+        """`txh_run_assimilating`: routing windows + ensemble updates of an unsharded ensemble, host out of the loop.
+        With `rec_reach`: `txh_run_assimilating_rec`, hydrographs into `rec_out` (and the priors into `prior_out`)."""
         idx = L.as_i64(obs_reach)
-        L.check(self._lib.txh_run_assimilating(
-            self.handle, _cuda_ptr(O), _cuda_ptr(I), int(M), forcing.handle if forcing is not None else None,
-            int(t0_ns), int(dt_ns), int(nsteps), int(every), int(method), L.ptr_i64(idx), idx.size, _cuda_ptr(Zp),
-            _cuda_ptr(qs), _cuda_ptr(R), _cuda_ptr(Dinv) if Dinv is not None else None, int(dinv_kind),
-            _cuda_ptr(rowsum), _cuda_ptr(HX), _cuda_ptr(work), _cuda_ptr(W), _cuda_ptr(T), _cuda_ptr(G),
-            int(time_every), ctypes.c_void_p(obs_ready.cuda_event) if obs_ready is not None else None, _stream_ptr()))
+        args = (self.handle, _cuda_ptr(O), _cuda_ptr(I), int(M), forcing.handle if forcing is not None else None,
+                int(t0_ns), int(dt_ns), int(nsteps), int(every), int(method), L.ptr_i64(idx), idx.size, _cuda_ptr(Zp),
+                _cuda_ptr(qs), _cuda_ptr(R), _cuda_ptr(Dinv) if Dinv is not None else None, int(dinv_kind),
+                _cuda_ptr(rowsum), _cuda_ptr(HX), _cuda_ptr(work), _cuda_ptr(W), _cuda_ptr(T), _cuda_ptr(G),
+                int(time_every), ctypes.c_void_p(obs_ready.cuda_event) if obs_ready is not None else None)
+        if rec_reach is None:
+            L.check(self._lib.txh_run_assimilating(*args, _stream_ptr()))
+            return
+        rr = L.as_i64(rec_reach)
+        L.check(self._lib.txh_run_assimilating_rec(*args, L.ptr_i64(rr), rr.size, int(rec_every), _cuda_ptr(rec_out),
+                                                   _cuda_ptr(prior_out) if prior_out is not None else None,
+                                                   _stream_ptr()))
 
     def route_timings(self):
         """Durations (ms) of the routing launches `run_assimilating(time_every=...)` bracketed; synchronises."""
