@@ -254,6 +254,26 @@ int txh_run_assimilating_rec(txh_net* net, double* O_dev, double* I_dev, int64_t
                              int64_t time_every, void* obs_ready_event, const int64_t* rec_reach_host, int64_t rec_count,
                              int64_t rec_every, double* rec_out_dev, double* prior_out_dev, void* stream);
 int txh_get_route_timings(txh_net* net, double* ms_out, int64_t capacity, int64_t* count);
+/* While set, update k (0-based) of every txh_run_assimilating(_rec) call on the handle solves its ensemble transform
+ * into T_hist_dev + k*M*M ([M][M] row-major) instead of into T_dev, and every consumer of that update reads it there:
+ * the transforms of a call survive it (txh_enks_smooth).  A call whose (nsteps / every) * M * M exceeds
+ * capacity_doubles fails with TXH_E_INVALID before any device work.  NULL switches it off. */
+int txh_set_transform_history(txh_net* net, double* T_hist_dev, int64_t capacity_doubles);
+
+/* ---- ensemble Kalman smoother of recorded hydrographs ----------------------------------------------------------------
+ * Fixed-lag EnKS of the slots txh_run_assimilating_rec recorded, from the transforms it kept (txh_set_transform_history):
+ * update u (0-based) happened after step (u+1)*every with transform T_u = T_hist_dev + u*M*M; slot j of rec_dev
+ * ([nslots][rec_count][M]) holds the ensemble X_j after step s_j = (j+1)*rec_every.  Every update with
+ * s_j < (u+1)*every <= s_j + lag is applied to the slot, in increasing u:
+ *     X_j <- X_j + (X_j - mean over the members of X_j) T_u
+ * which is the EnKS gain A_j HA^T S^-1 dz/(M-1) of the update's innovation solve (the Q[:,s] W term of the filter gain
+ * is not: model noise added at the update is uncorrelated with earlier states).  Result in out_dev, the same shape as
+ * rec_dev and a buffer of its own (rec_dev is left alone).  lag = 0 or a slot no later update reaches: a copy.
+ * TXH_E_INVALID before any device work for M < 2, nupd < 0, every, rec_every < 1, lag < 0, a null buffer or out
+ * overlapping rec; TXH_E_NODEVICE without a device.  Asynchronous. */
+int64_t txh_enks_work_size(int64_t M, int64_t nupd);           /* doubles of work_dev */
+int txh_enks_smooth(int64_t M, int64_t nupd, int64_t every, const double* T_hist_dev, int64_t nslots, int64_t rec_count,
+                    int64_t rec_every, int64_t lag, const double* rec_dev, double* out_dev, double* work_dev, void* stream);
 
 /* Dense products of KalmanFilter.filter for small n (da.py:115-122): C = alpha op(A) op(B) + beta C,
  * row-major FP64 on the tensor cores (mma.sync m8n8k4 = DMMA). */

@@ -108,6 +108,8 @@ struct txh_net {
     double* d_stage = nullptr; size_t stage_cap = 0;   // reach-order staging of txh_pack_host / txh_unpack_host
     double* stats_rowsum = nullptr;     // txh_set_stats_output: row sums of the final outflows of every routing call
     double stats_scale = 1.0;
+    double* T_hist = nullptr;           // txh_set_transform_history: update k of a run_assimilating call solves into
+    int64_t T_hist_cap = 0;             // T_hist + k*M*M (capacity in doubles)
     std::vector<std::pair<cudaEvent_t, cudaEvent_t>> route_events;   // txh_run_assimilating(time_every > 0)
 };
 
@@ -1505,6 +1507,8 @@ int txh_run_assimilating_rec(txh_net* net, double* O, double* I, int64_t M, cons
         return fail(TXH_E_INVALID, "bad argument");
     if (rec_count < 0 || rec_every < 1 || (rec_count > 0 && (!rec_reach || !rec_out)))
         return fail(TXH_E_INVALID, "bad recording arguments");
+    if (net->T_hist && (nsteps / every) * M * M > net->T_hist_cap)
+        return fail(TXH_E_INVALID, "the transform history holds fewer than nsteps / every transforms of M x M");
     if (rec_count > 0) {
         if (fo && fo->net != net) return fail(TXH_E_INVALID, "forcing belongs to another network");
         if (check_M(M)) return TXH_E_INVALID;
@@ -1535,6 +1539,8 @@ int txh_run_assimilating_rec(txh_net* net, double* O, double* I, int64_t M, cons
     // posterior ones -- what the state holds after that step -- to their rec_out slot (the window kernel recorded the
     // forecast there).  In every path O still holds the forecast when enkf_record runs.
     const bool rec = rec_count > 0;
+    // where update k's transform goes and where its consumers read it
+    auto T_of = [&](int64_t k) -> double* { return net->T_hist ? net->T_hist + (size_t)k * M * M : T; };
     if (rc == TXH_OK && rec) {
         // (the arguments were checked above; the routing calls below go past txh_route_run's checks)
         rc = ensure_device(net);
@@ -1563,13 +1569,13 @@ int txh_run_assimilating_rec(txh_net* net, double* O, double* I, int64_t M, cons
     auto record_update = [&](int64_t k) -> int {
         double *prior = rec_prior_of(k), *post = rec_post_of(k);
         if (rec && (post || prior))
-            CU(launch_enkf_record(O, ld, (int)M, rowsum, T, net->d_gauge_of_pos, qs, W, net->d_rec_pos, (int)rec_count,
+            CU(launch_enkf_record(O, ld, (int)M, rowsum, T_of(k), net->d_gauge_of_pos, qs, W, net->d_rec_pos, (int)rec_count,
                                   prior, post, st));
         return TXH_OK;
     };
     // update k applied by the next window launch while it loads its tasks: that launch records its rows
     auto set_pending = [&](int64_t k) {
-        net->pending.T = T; net->pending.W = W; net->pending.qs = qs; net->pending.M = M;
+        net->pending.T = T_of(k); net->pending.W = W; net->pending.qs = qs; net->pending.M = M;
         net->pending.rec_prior = rec ? rec_prior_of(k) : nullptr;
         net->pending.rec_post = rec ? rec_post_of(k) : nullptr;
         net->pending.rec_mean = rowsum;
@@ -1579,7 +1585,7 @@ int txh_run_assimilating_rec(txh_net* net, double* O, double* I, int64_t M, cons
     auto apply_owed = [&]() -> int {
         int rc2 = record_update(owed_k);
         if (rc2 != TXH_OK) return rc2;
-        CU(launch_enkf_update(O, ld, (int)M, rowsum, T, (int)M, (int)M, O, nullptr, ld, net->topo.n, net->d_gauge_of_pos,
+        CU(launch_enkf_update(O, ld, (int)M, rowsum, T_of(owed_k), (int)M, (int)M, O, nullptr, ld, net->topo.n, net->d_gauge_of_pos,
                               qs, W, 0, net->num_sms, (int)M, 0, st));
         CU(launch_inflow_rebuild(net->d_inner_rec, net->n_inner, net->d_up_off, net->d_up_pos, O, I, ld, st));
         owed = false;
@@ -1606,14 +1612,15 @@ int txh_run_assimilating_rec(txh_net* net, double* O, double* I, int64_t M, cons
         // window does not
         if (k == 0 && obs_ready_event) CU(cudaStreamWaitEvent(st, (cudaEvent_t)obs_ready_event, 0));
         if (rc == TXH_OK) rc = check_M(M);
-        if (rc == TXH_OK) rc = enkf_solve_impl(net, m, M, HX, O, Zp + (size_t)k * m * M, rowsum, obs, qs, R, Dinv, dinv_kind, work, W, T, stream);
+        if (rc == TXH_OK) rc = enkf_solve_impl(net, m, M, HX, O, Zp + (size_t)k * m * M, rowsum, obs, qs, R, Dinv, dinv_kind, work, W,
+                                                  T_of(k), stream);
         if (rc != TXH_OK) break;
         if (ld <= kMemberBlock) {
             owed = true; owed_k = k;
             if (!fuse_load) rc = apply_owed();
         } else {
             rc = record_update(k);
-            if (rc == TXH_OK) rc = txh_enkf_apply(net, O, I, M, nullptr, 0, 0, M, 0, rowsum, T, obs, m, qs, W, G, stream);
+            if (rc == TXH_OK) rc = txh_enkf_apply(net, O, I, M, nullptr, 0, 0, M, 0, rowsum, T_of(k), obs, m, qs, W, G, stream);
         }
     }
     net->stats_rowsum = nullptr;
@@ -1633,6 +1640,34 @@ int txh_run_assimilating_rec(txh_net* net, double* O, double* I, int64_t M, cons
     net->pending.T = nullptr; net->pending.rec_prior = net->pending.rec_post = nullptr;
     net->stats_rowsum = rowsum_before; net->stats_scale = scale_before;
     return rc;
+}
+
+int txh_set_transform_history(txh_net* net, double* T_hist, int64_t capacity)
+{
+    if (!net) return fail(TXH_E_INVALID, "null argument");
+    if (T_hist && capacity < 0) return fail(TXH_E_INVALID, "negative transform history capacity");
+    net->T_hist = T_hist; net->T_hist_cap = T_hist ? capacity : 0;
+    return TXH_OK;
+}
+
+int64_t txh_enks_work_size(int64_t M, int64_t nupd) { return M < 1 || nupd < 0 ? 0 : 6 * nupd * M * M; }
+
+int txh_enks_smooth(int64_t M, int64_t nupd, int64_t every, const double* T_hist, int64_t nslots, int64_t rec_count,
+                    int64_t rec_every, int64_t lag, const double* rec, double* out, double* work, void* stream)
+{
+    if (M < 2 || M > 4096) return fail(TXH_E_INVALID, "member count out of range [2, 4096]");
+    if (nupd < 0 || nupd > (int64_t(1) << 30) || every < 1) return fail(TXH_E_INVALID, "bad update count or cadence");
+    if (nslots < 0 || rec_count < 0 || rec_every < 1) return fail(TXH_E_INVALID, "bad recording shape");
+    if (lag < 0) return fail(TXH_E_INVALID, "negative smoother lag");
+    if (!T_hist || !rec || !out || !work) return fail(TXH_E_INVALID, "null buffer");
+    const uintptr_t bytes = (uintptr_t)(nslots * rec_count * M) * sizeof(double);
+    const uintptr_t r0 = (uintptr_t)rec, o0 = (uintptr_t)out;
+    if (bytes > 0 && r0 < o0 + bytes && o0 < r0 + bytes)
+        return fail(TXH_E_INVALID, "out overlaps rec: the smoothed hydrographs need a buffer of their own");
+    if (txh_device_count() == 0) return fail(TXH_E_NODEVICE, "no CUDA device visible: libtxh has no CPU fallback");
+    CU(launch_enks_smooth((int)M, (int)nupd, every, T_hist, nslots, rec_count, rec_every, lag, rec, out, work,
+                          (cudaStream_t)stream));
+    return TXH_OK;
 }
 
 int txh_get_route_timings(txh_net* net, double* ms_out, int64_t capacity, int64_t* count)

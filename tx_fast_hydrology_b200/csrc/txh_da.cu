@@ -1226,6 +1226,282 @@ enkf_record_kernel(const double* __restrict__ O, int ld, int M, const double* __
     }
 }
 
+// ---- ensemble Kalman smoother of recorded hydrographs (txh_enks_smooth) ------------------------------------------------
+// An update maps a past ensemble X to X (I + C T_u), C = I - 11^T/M the centring matrix.  Products keep that form:
+//     (I + C T1)(I + C T2) = I + C compose(T1, T2),   compose(T1, T2) = T1 + T2 + (T1 C) T2
+// so the updates a slot receives collapse into one cumulative transform.  Stage (a) forms one per range of updates
+// [a, b] the slots need (at most two per first update a: a lag that is not a multiple of `every` splits a group), from
+// in-block prefix and suffix products over blocks of Bs = ceil(sqrt(nupd)) updates: a range inside one block is a
+// prefix or a suffix of it or a chain of at most Bs - 2 products, any other range is a suffix, the totals of the blocks
+// in between and a prefix.  The longest chain of dependent products is about 2 sqrt(nupd) (26 at 168 updates) instead
+// of nupd.  Stage (b) streams the recorded rows once: X + (X - mean) T_cum on the tensor cores.
+constexpr int SM_K = 16;
+
+// out = T1 + T2 + (T1 - rowmean(T1)) T2 for M x M row-major matrices in global memory (written by this CTA or an
+// earlier launch), by a whole CTA of 256 threads: 64 x 64 output tiles, 8 warps x 16 x 32 DMMA tiles, k tiles of 16.
+// out must not alias T1 or T2.  mu: M doubles of shared memory.  Ends in a barrier: out is visible to the CTA.
+__device__ void enks_compose(const double* T1, const double* T2, double* out, int M, double* mu, double* sA, double* sB)
+{
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int g = lane >> 2, t = lane & 3;
+    const int wm = (warp >> 1) * 16, wn = (warp & 1) * 32;
+    for (int i = warp; i < M; i += 8) {
+        double s = 0.0;
+        for (int c = lane; c < M; c += 32) s += __ldcg(T1 + (size_t)i * M + c);
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+        if (lane == 0) mu[i] = s / M;
+    }
+    __syncthreads();
+    for (int i0 = 0; i0 < M; i0 += 64)
+        for (int j0 = 0; j0 < M; j0 += 64) {
+            double acc[2][4][2];
+#pragma unroll
+            for (int i = 0; i < 2; ++i)
+#pragma unroll
+                for (int j = 0; j < 4; ++j) acc[i][j][0] = acc[i][j][1] = 0.0;
+            for (int k0 = 0; k0 < M; k0 += SM_K) {
+#pragma unroll
+                for (int u = 0; u < 4; ++u) {
+                    const int e = tid + 256 * u;
+                    const int r = e / SM_K, k = e % SM_K, gi = i0 + r, gk = k0 + k;
+                    sA[r * (SM_K + 1) + k] = (gi < M && gk < M) ? __ldcg(T1 + (size_t)gi * M + gk) - mu[gi] : 0.0;
+                    const int kb = e / 64, c = e % 64, gkb = k0 + kb, gc = j0 + c;
+                    sB[kb * 65 + c] = (gkb < M && gc < M) ? __ldcg(T2 + (size_t)gkb * M + gc) : 0.0;
+                }
+                __syncthreads();
+#pragma unroll
+                for (int kk = 0; kk < SM_K; kk += 4) {
+                    double a[2], b[4];
+#pragma unroll
+                    for (int i = 0; i < 2; ++i) a[i] = sA[(wm + 8 * i + g) * (SM_K + 1) + kk + t];
+#pragma unroll
+                    for (int j = 0; j < 4; ++j) b[j] = sB[(kk + t) * 65 + wn + 8 * j + g];
+#pragma unroll
+                    for (int i = 0; i < 2; ++i)
+#pragma unroll
+                        for (int j = 0; j < 4; ++j) dmma8x8x4(acc[i][j][0], acc[i][j][1], a[i], b[j]);
+                }
+                __syncthreads();
+            }
+#pragma unroll
+            for (int i = 0; i < 2; ++i)
+#pragma unroll
+                for (int j = 0; j < 4; ++j)
+#pragma unroll
+                    for (int c = 0; c < 2; ++c) {
+                        const int gi = i0 + wm + 8 * i + g, gc = j0 + wn + 8 * j + 2 * t + c;
+                        if (gi < M && gc < M) {
+                            const size_t at = (size_t)gi * M + gc;
+                            out[at] = __ldcg(T1 + at) + __ldcg(T2 + at) + acc[i][j][c];
+                        }
+                    }
+        }
+    __syncthreads();
+}
+
+__device__ void enks_copy(const double* src, double* dst, size_t count)
+{
+    for (size_t e = threadIdx.x; e < count; e += blockDim.x) dst[e] = __ldcg(src + e);
+    __syncthreads();
+}
+
+// stage (a), part 1: CTA (block, 0) forms the prefix products P[u] = T_b0 o ... o T_u of its block of updates, CTA
+// (block, 1) the suffix products S[u] = T_u o ... o T_b1
+__global__ void __launch_bounds__(256)
+enks_block_scan_kernel(const double* __restrict__ Th, int M, int nupd, int Bs, double* P, double* S)
+{
+    extern __shared__ double enks_mu[];
+    __shared__ double sA[64 * (SM_K + 1)], sB[SM_K * 65];
+    const size_t MM = (size_t)M * M;
+    const int u0 = blockIdx.x * Bs, u1 = min(nupd, u0 + Bs) - 1;
+    if (blockIdx.y == 0) {
+        enks_copy(Th + u0 * MM, P + u0 * MM, MM);
+        for (int u = u0 + 1; u <= u1; ++u) enks_compose(P + (u - 1) * MM, Th + u * MM, P + u * MM, M, enks_mu, sA, sB);
+    } else {
+        enks_copy(Th + u1 * MM, S + u1 * MM, MM);
+        for (int u = u1 - 1; u >= u0; --u) enks_compose(Th + u * MM, S + (u + 1) * MM, S + u * MM, M, enks_mu, sA, sB);
+    }
+}
+
+// the range of updates [a, b] of slots whose first update is a; which = 1: the longer of the two a lag that is not a
+// multiple of `every` gives (b one further).  -1: no update reaches the slot.
+__device__ __forceinline__ void enks_range(long long a, int which, int nupd, long long lag_q, int* b_out)
+{
+    const long long bmin = min((long long)nupd - 1, a + lag_q - 1);
+    const long long b = min((long long)nupd - 1, a + lag_q - 1 + which);
+    *b_out = (b < a || (which == 1 && b == bmin)) ? -1 : (int)b;
+}
+
+// stage (a), part 2: CTA r forms the cumulative transform Tc[r] of the range (a = r / 2, which = r % 2), ping-ponging
+// between Tc[r] and the scratch X[r] so that the last product lands in Tc[r]
+__global__ void __launch_bounds__(256)
+enks_range_kernel(const double* __restrict__ Th, int M, int nupd, int Bs, long long lag_q, const double* P,
+                  const double* S, double* Tc, double* X)
+{
+    extern __shared__ double enks_mu[];
+    __shared__ double sA[64 * (SM_K + 1)], sB[SM_K * 65];
+    const size_t MM = (size_t)M * M;
+    const int r = blockIdx.x, a = r >> 1;
+    int b;
+    enks_range(a, r & 1, nupd, lag_q, &b);
+    if (b < 0) return;
+    const int ka = a / Bs, kb = b / Bs;
+    const double* first;
+    int n;                                            // products after `first`
+    if (ka == kb && a == ka * Bs) { first = P + b * MM; n = 0; }
+    else if (ka == kb && b == min(nupd, (ka + 1) * Bs) - 1) { first = S + a * MM; n = 0; }
+    else if (ka == kb) { first = Th + a * MM; n = b - a; }
+    else { first = S + a * MM; n = kb - ka; }
+    double* dst = Tc + r * MM;
+    if (n == 0) { enks_copy(first, dst, MM); return; }
+    const double* cur = first;
+    for (int i = 0; i < n; ++i) {
+        const double* rhs = ka == kb ? Th + (a + 1 + i) * MM                          // chain inside the block
+                                     : (i < n - 1 ? S + (size_t)(ka + 1 + i) * Bs * MM : P + b * MM);   // block totals, prefix
+        double* o = ((n - 1 - i) & 1) ? X + r * MM : dst;
+        enks_compose(cur, rhs, o, M, enks_mu, sA, sB);
+        cur = o;
+    }
+}
+
+// stage (b): out = X + (X - mean) Tc for every recorded row, a copy for slots no update reaches.  Work items are
+// (slot, 128-row tile), CTA b takes a contiguous run of them and stages Tc only when the range changes.  A warp owns 16
+// rows (two 8-row MMA tiles) as in enkf_update_kernel: its lanes hold the members 8j+2t, 8j+2t+1 of a row, which are
+// both the permuted A fragment and the C fragment positions of output tile j, so X + gain needs no second read when
+// M <= 64.  The row mean is the sum of a lane's 16 values over the 4 lanes of the row.
+constexpr int ES_ROWS = 16 * 8;
+
+template <bool ONE>                               // ONE: M <= 64, a single member block
+__global__ void __launch_bounds__(256)
+enks_apply_kernel(const double* __restrict__ rec, double* __restrict__ out, const double* __restrict__ Tc, int M, int nupd,
+                  long long every, long long lag_c, long long rec_every, long long rec_count, long long nitems,
+                  long long per_cta, int tiles_per_slot, int resident)
+{
+    extern __shared__ double sT_all[];
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int g = lane >> 2, t = lane & 3;
+    const int nkc = ONE ? 1 : (M + 63) / 64;
+    const bool vec = (M & 1) == 0;
+    const size_t MM = (size_t)M * M;
+    int staged = -1;
+    const long long it0 = (long long)blockIdx.x * per_cta, it1 = min(nitems, it0 + per_cta);
+    for (long long it = it0; it < it1; ++it) {
+        const long long j = it / tiles_per_slot;
+        const long long tile = it - j * tiles_per_slot;
+        const long long s = (j + 1) * rec_every, a = s / every;
+        // updates a .. b reach the slot, b = the last with (b+1) every <= s + lag; r as enks_range_kernel numbers them
+        int r = -1;
+        const long long b = min((long long)nupd - 1, (s + lag_c) / every - 1);
+        if (a < nupd && b >= a) r = (int)(2 * a + (b > min((long long)nupd - 1, a + lag_c / every - 1) ? 1 : 0));
+        const long long lr0 = tile * ES_ROWS + warp * 16;                    // this warp's rows in the slot
+        const double* xs = rec + (size_t)j * rec_count * M;
+        double* os = out + (size_t)j * rec_count * M;
+        if (r < 0) {
+            for (long long q = lr0; q < lr0 + 16 && q < rec_count; ++q)
+                for (int c = lane; c < M; c += 32) __stcs(os + q * M + c, __ldcs(xs + q * M + c));
+            continue;
+        }
+        if (resident && r != staged) {
+            __syncthreads();
+            for (int blk = 0; blk < nkc * nkc; ++blk)
+                for (int e = tid; e < 64 * 64; e += 256) {
+                    const int k = e >> 6, c = e & 63, gk = (blk / nkc) * 64 + k, gc = (blk % nkc) * 64 + c;
+                    sT_all[blk * 64 * EU_LDT + k * EU_LDT + c] = (gk < M && gc < M) ? __ldg(Tc + r * MM + (size_t)gk * M + gc) : 0.0;
+                }
+            __syncthreads();
+            staged = r;
+        }
+        const long long rows[2] = {lr0 + g, lr0 + 8 + g};
+        // this lane's members of chunk kc of its two rows (0 beyond the matrix)
+        auto load_chunk = [&](int kc, double (&x)[2][16]) {
+#pragma unroll
+            for (int i = 0; i < 2; ++i) {
+                const bool ok = rows[i] < rec_count;
+                const double* xr = xs + (size_t)(ok ? rows[i] : 0) * M;
+#pragma unroll
+                for (int jj = 0; jj < 8; ++jj) {
+                    const int k = kc * 64 + 8 * jj + 2 * t;
+                    double x0 = 0.0, x1 = 0.0;
+                    if (ok && vec && k < M) {
+                        const double2 v = __ldcs(reinterpret_cast<const double2*>(xr + k));
+                        x0 = v.x; x1 = v.y;
+                    } else if (ok) {
+                        if (k < M) x0 = __ldcs(xr + k);
+                        if (k + 1 < M) x1 = __ldcs(xr + k + 1);
+                    }
+                    x[i][2 * jj] = x0; x[i][2 * jj + 1] = x1;
+                }
+            }
+        };
+        double x[2][16], mu[2] = {0.0, 0.0};
+        for (int kc = 0; kc < nkc; ++kc) {
+            load_chunk(kc, x);
+#pragma unroll
+            for (int i = 0; i < 2; ++i)
+#pragma unroll
+                for (int q = 0; q < 16; ++q) mu[i] += x[i][q];
+        }
+#pragma unroll
+        for (int i = 0; i < 2; ++i) {
+            mu[i] += __shfl_xor_sync(0xffffffffu, mu[i], 1);
+            mu[i] += __shfl_xor_sync(0xffffffffu, mu[i], 2);
+            mu[i] /= M;
+        }
+        for (int cg = 0; cg < nkc; ++cg) {
+            const int njt = min(8, (M - cg * 64 + 7) >> 3);
+            double acc[2][8][2];
+#pragma unroll
+            for (int i = 0; i < 2; ++i)
+#pragma unroll
+                for (int jj = 0; jj < 8; ++jj) acc[i][jj][0] = acc[i][jj][1] = 0.0;
+            for (int kc = 0; kc < nkc; ++kc) {
+                if (nkc > 1) load_chunk(kc, x);
+                const double* sT = sT_all + (resident ? (kc * nkc + cg) * 64 * EU_LDT : 0);
+                if (!resident) {
+                    __syncthreads();
+                    for (int e = tid; e < 64 * 64; e += 256) {
+                        const int k = e >> 6, c = e & 63, gk = kc * 64 + k, gc = cg * 64 + c;
+                        sT_all[k * EU_LDT + c] = (gk < M && gc < M) ? __ldg(Tc + r * MM + (size_t)gk * M + gc) : 0.0;
+                    }
+                    __syncthreads();
+                }
+#pragma unroll
+                for (int ks = 0; ks < 16; ++ks) {
+                    const int k = 8 * (ks >> 1) + 2 * t + (ks & 1);
+                    const bool in = kc * 64 + k < M;          // the anomaly is formed here: x stays for the epilogue
+                    const double a0 = in ? x[0][ks] - mu[0] : 0.0, a1 = in ? x[1][ks] - mu[1] : 0.0;
+                    const double* bt = sT + k * EU_LDT + g;
+#pragma unroll
+                    for (int jj = 0; jj < 8; ++jj)
+                        if (jj < njt) {
+                            const double bv = bt[8 * jj];
+                            dmma8x8x4(acc[0][jj][0], acc[0][jj][1], a0, bv);
+                            dmma8x8x4(acc[1][jj][0], acc[1][jj][1], a1, bv);
+                        }
+                }
+            }
+            if (nkc > 1) load_chunk(cg, x);
+#pragma unroll
+            for (int i = 0; i < 2; ++i) {
+                if (rows[i] >= rec_count) continue;
+                double* orow = os + (size_t)rows[i] * M;
+#pragma unroll
+                for (int jj = 0; jj < 8; ++jj) {
+                    const int col = cg * 64 + 8 * jj + 2 * t;
+                    if (vec && col < M) {
+                        __stcs(reinterpret_cast<double2*>(orow + col),
+                               make_double2(x[i][2 * jj] + acc[i][jj][0], x[i][2 * jj + 1] + acc[i][jj][1]));
+                    } else {
+                        if (col < M) __stcs(orow + col, x[i][2 * jj] + acc[i][jj][0]);
+                        if (col + 1 < M) __stcs(orow + col + 1, x[i][2 * jj + 1] + acc[i][jj][1]);
+                    }
+                }
+            }
+        }
+    }
+}
+
 }  // namespace
 
 cudaError_t launch_dgemm(int transA, int transB, int M, int N, int K, double alpha, const double* A, int lda,
@@ -1493,6 +1769,47 @@ cudaError_t launch_inflow_gain(const int32_t* inner, int64_t n_inner, const int3
 {
     if (n_inner == 0) return cudaSuccess;
     inflow_gain_kernel<<<nblk(n_inner * (ld >> 1), 256), 256, 0, st>>>(inner, n_inner, up_off, up_pos, G, I, ld);
+    count_launch();
+    return cudaGetLastError();
+}
+
+// work: P [nupd], S [nupd], Tc [2 nupd], X [2 nupd] matrices of M x M (txh_enks_work_size)
+cudaError_t launch_enks_smooth(int M, int nupd, long long every, const double* T_hist, long long nslots, long long rec_count,
+                               long long rec_every, long long lag, const double* rec, double* out, double* work,
+                               cudaStream_t st)
+{
+    if (nslots == 0 || rec_count == 0) return cudaSuccess;
+    const size_t MM = (size_t)M * M;
+    double *P = work, *S = P + nupd * MM, *Tc = S + nupd * MM, *X = Tc + 2 * nupd * MM;
+    if (lag == 0) nupd = 0;                               // nothing reaches any slot: stage (b) copies
+    const long long lag_c = lag < (nupd + 1LL) * every ? lag : (nupd + 1LL) * every;   // beyond: the same ranges
+    cudaError_t e;
+    if (nupd > 0) {
+        int Bs = 1;
+        while ((long long)Bs * Bs < nupd) ++Bs;
+        const size_t smem = sizeof(double) * M;
+        enks_block_scan_kernel<<<dim3((nupd + Bs - 1) / Bs, 2), 256, smem, st>>>(T_hist, M, nupd, Bs, P, S);
+        count_launch();
+        if ((e = cudaGetLastError()) != cudaSuccess) return e;
+        enks_range_kernel<<<2 * nupd, 256, smem, st>>>(T_hist, M, nupd, Bs, lag_c / every, P, S, Tc, X);
+        count_launch();
+        if ((e = cudaGetLastError()) != cudaSuccess) return e;
+    }
+    const int nkc = (M + 63) / 64;
+    const int resident = nkc <= 2 ? 1 : 0;               // every 64 x 64 block of Tc in shared memory (<= 135 KB)
+    const size_t smem = (size_t)(resident ? nkc * nkc : 1) * 64 * EU_LDT * sizeof(double);
+    auto kern = nkc == 1 ? enks_apply_kernel<true> : enks_apply_kernel<false>;
+    if ((e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess) return e;
+    int dev = 0, num_sms = 0;
+    if ((e = cudaGetDevice(&dev)) != cudaSuccess) return e;
+    if ((e = cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, dev)) != cudaSuccess) return e;
+    const int tiles_per_slot = (int)((rec_count + ES_ROWS - 1) / ES_ROWS);
+    const long long nitems = nslots * tiles_per_slot;
+    const long long want = (long long)num_sms * 2;      // 168-198 registers: one CTA of 8 warps per SM
+    const long long grid = nitems < want ? nitems : want;
+    const long long per_cta = (nitems + grid - 1) / grid;
+    kern<<<(unsigned)((nitems + per_cta - 1) / per_cta), 256, smem, st>>>(
+        rec, out, Tc, M, nupd, every, lag_c, rec_every, rec_count, nitems, per_cta, tiles_per_slot, resident);
     count_launch();
     return cudaGetLastError();
 }

@@ -263,6 +263,10 @@ cudaError_t launch_inflow_rebuild(const int4* rec, int64_t n_inner, const int32_
 cudaError_t launch_enkf_record(const double* O, int ld, int M, const double* mean, const double* T,
                                const int32_t* gauge_of_pos, const double* qs, const double* W, const int32_t* rec_pos,
                                int rec_count, double* prior_out, double* post_out, cudaStream_t st);
+// txh_enks_smooth (arguments checked by the caller): cumulative transforms, then one pass over rec
+cudaError_t launch_enks_smooth(int M, int nupd, long long every, const double* T_hist, long long nslots, long long rec_count,
+                               long long rec_every, long long lag, const double* rec, double* out, double* work,
+                               cudaStream_t st);
 cudaError_t launch_inflow_gain(const int32_t* inner, int64_t n_inner, const int32_t* up_off, const int32_t* up_pos,
                                const double* G, double* I, int ld, cudaStream_t st);
 

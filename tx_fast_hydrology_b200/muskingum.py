@@ -461,7 +461,7 @@ class Muskingum:
         return idx
 
     def run_assimilating(self, forcing, nsteps, enkf, every, observations, timers=None, observations_ready=None,
-                         record_reaches=None, record_every=1, record_prior=False):
+                         record_reaches=None, record_every=1, record_prior=False, smooth_lag=None):
         """Device-resident run with periodic ensemble assimilation: `every` routing steps in one
         persistent launch, then one `EnsembleKalmanFilter` update with `observations[k]` ([m][Mtot]
         CUDA tensor of per-member observations for the k-th update), repeated; nothing returns to
@@ -480,7 +480,20 @@ class Muskingum:
         The Python loop (observations as a list, or a member-sharded filter) records every step of a window into a
         scratch buffer and copies the wanted steps out, and each of its routing calls uploads the slot map again and
         synchronises: correct, with per-window host work on a path that already has it; the in-library loop does this
-        once per call."""
+        once per call.
+        `smooth_lag` (steps, needs `record_reaches`): also return the hydrographs of the fixed-lag ensemble Kalman
+        smoother, `smoothed` shaped like `rec`, as (rec, smoothed) or (rec, prior, smoothed): slot j (after step
+        s = (j+1) record_every) conditioned on every update of the call after s up to s + smooth_lag, from the
+        transforms the updates solved (txh_enks_smooth; DESIGN.md §4.4).  `rec` keeps the filtered hydrographs.  A
+        lag of at least `nsteps` gives the fixed-interval smoother.  Not for a member-sharded filter."""
+        if smooth_lag is not None:
+            if isinstance(smooth_lag, bool) or not isinstance(smooth_lag, (int, np.integer)) or smooth_lag < 0:
+                raise ValueError(f'`smooth_lag` must be a non-negative integer number of steps, got {smooth_lag!r}')
+            if record_reaches is None:
+                raise ValueError('`smooth_lag` smooths recorded hydrographs: it needs `record_reaches`')
+            if getattr(enkf, 'world', 1) > 1:
+                raise ValueError('`smooth_lag` is not available for a member-sharded filter (smoothing one rank\'s '
+                                 'members needs every rank\'s)')
         ridx = None if record_reaches is None else self._record_reaches(record_reaches, record_every, nsteps)
         torch = self._ensure_device()
         self._sync_coeffs()
@@ -494,7 +507,16 @@ class Muskingum:
             rec = torch.zeros((nsteps // record_every, ridx.size, M), dtype=torch.float64, device='cuda')
             if record_prior:
                 prior = torch.zeros((nwin, ridx.size, M), dtype=torch.float64, device='cuda')
-        result = None if rec is None else ((rec, prior) if record_prior else rec)
+        # smoothing: update k's transform kept in T_hist[k]
+        T_hist = None if smooth_lag is None else torch.empty((max(nwin, 1), M, M), dtype=torch.float64, device='cuda')
+
+        def result():
+            if rec is None:
+                return None
+            out = (rec, prior) if record_prior else (rec,)
+            if T_hist is not None:
+                out += (net.enks_smooth(M, nwin, every, T_hist, rec, record_every, smooth_lag, torch.empty_like(rec)),)
+            return out if len(out) > 1 else rec
         if torch.is_tensor(observations) or isinstance(observations, np.ndarray):
             want = (enkf.num_measurements, enkf.Mtot)
             if observations.ndim != 3 or observations.shape[0] < nwin or tuple(observations.shape[1:]) != want:
@@ -502,16 +524,24 @@ class Muskingum:
         if (enkf.world == 1 and torch.is_tensor(observations) and observations.is_cuda and observations.is_contiguous()
                 and observations.shape[0] >= nwin and observations.dtype == torch.float64):
             # one call: the loop below, in the library (txh_run_assimilating)
-            net.run_assimilating(d['O'], d['I'], M, forcing, t, step_ns, nsteps, every, enkf.reach_indices,
-                                 observations, enkf._qs, enkf._R, enkf._Dinv, enkf._dinv_kind, enkf._rowsum, enkf._HX,
-                                 enkf._work, enkf._W, enkf._T, enkf._G, time_every=8 if timers is not None else 0,
-                                 obs_ready=observations_ready, rec_reach=ridx, rec_every=record_every, rec_out=rec,
-                                 prior_out=prior)
+            if T_hist is not None:
+                net.set_transform_history(T_hist)
+            try:
+                net.run_assimilating(d['O'], d['I'], M, forcing, t, step_ns, nsteps, every, enkf.reach_indices,
+                                     observations, enkf._qs, enkf._R, enkf._Dinv, enkf._dinv_kind, enkf._rowsum,
+                                     enkf._HX, enkf._work, enkf._W, enkf._T, enkf._G,
+                                     time_every=8 if timers is not None else 0, obs_ready=observations_ready,
+                                     rec_reach=ridx, rec_every=record_every, rec_out=rec, prior_out=prior)
+            finally:
+                if T_hist is not None:
+                    net.set_transform_history(None)
+            if T_hist is not None and nwin:
+                enkf._T.copy_(T_hist[nwin - 1])             # the filter's last transform, as without smoothing
             enkf.n_updates += nwin
             self._datetime = pd.Timestamp(t + nsteps * step_ns, tz='UTC')
             enkf.datetime = self._datetime
             self._device_advanced()
-            return result
+            return result()
         if observations_ready is not None:
             torch.cuda.current_stream().wait_event(observations_ready)
         # recording: every step of a window into `win`, the steps that are multiples of record_every copied out of it
@@ -543,6 +573,8 @@ class Muskingum:
             if prior is not None:
                 net.gather_rows(d['O'], M, ridx, prior[k])
             enkf.filter(observations[k], stats_fresh=True)
+            if T_hist is not None:
+                T_hist[k].copy_(enkf._T)
             s_end = (k + 1) * every
             if rec is not None and s_end % record_every == 0:
                 # the posterior; a filter on the peer-read path has swapped the state buffer
@@ -554,7 +586,7 @@ class Muskingum:
             t += rest * step_ns
         self._datetime = pd.Timestamp(t, tz='UTC')
         self._device_advanced()
-        return result
+        return result()
 
     def upload_state(self, o_t_next, i_t_next=None):
         """`init_states` (muskingum.py:410-419) without the host round trip: `o_t_next` ([n][members],

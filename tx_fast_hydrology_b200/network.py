@@ -15,6 +15,12 @@ def _cuda_ptr(t):
     return ctypes.c_void_p(t.data_ptr())
 
 
+def _check_f64_cuda(t, name):
+    import torch
+    if not (torch.is_tensor(t) and t.is_cuda and t.dtype == torch.float64 and t.is_contiguous()):
+        raise ValueError(f"`{name}` must be a contiguous float64 CUDA tensor")
+
+
 _raw_stream = None
 
 
@@ -318,6 +324,43 @@ class RiverNetwork:
         L.check(self._lib.txh_run_assimilating_rec(*args, L.ptr_i64(rr), rr.size, int(rec_every), _cuda_ptr(rec_out),
                                                    _cuda_ptr(prior_out) if prior_out is not None else None,
                                                    _stream_ptr()))
+
+    def set_transform_history(self, T_hist=None):
+        """While set, update k of every `run_assimilating` call solves its ensemble transform into `T_hist[k]`
+        ([>= updates][M][M] float64 contiguous CUDA tensor) instead of into `T`; None switches it off."""
+        if T_hist is not None:
+            _check_f64_cuda(T_hist, "T_hist")
+            if T_hist.dim() != 3 or T_hist.shape[1] != T_hist.shape[2]:
+                raise ValueError(f"set_transform_history: `T_hist` must be [updates][M][M], got {tuple(T_hist.shape)}")
+        self._T_hist_keep = T_hist
+        L.check(self._lib.txh_set_transform_history(self.handle, _cuda_ptr(T_hist) if T_hist is not None else None,
+                                                    T_hist.numel() if T_hist is not None else 0))
+
+    @staticmethod
+    def enks_work_size(M, nupd):
+        return int(L.load().txh_enks_work_size(int(M), int(nupd)))
+
+    def enks_smooth(self, M, nupd, every, T_hist, rec, rec_every, lag, out, work=None):
+        """`txh_enks_smooth`: the fixed-lag ensemble Kalman smoother of recorded hydrographs `rec`
+        ([slots][k][M], slot j after step (j+1)*rec_every) from the transforms `T_hist[:nupd]` of updates after every
+        `every`-th step; `lag` in steps.  Writes `out` (same shape as `rec`, a buffer of its own) and returns it."""
+        for name, t in (("T_hist", T_hist), ("rec", rec), ("out", out)):
+            _check_f64_cuda(t, name)
+        M, nupd = int(M), int(nupd)
+        if T_hist.dim() != 3 or T_hist.shape[0] < nupd or tuple(T_hist.shape[1:]) != (M, M):
+            raise ValueError(f"enks_smooth: `T_hist` must be [>= {nupd}][{M}][{M}], got {tuple(T_hist.shape)}")
+        if rec.dim() != 3 or rec.shape[2] != M or tuple(out.shape) != tuple(rec.shape):
+            raise ValueError(f"enks_smooth: `rec` and `out` must both be [slots][k][{M}], got {tuple(rec.shape)} and "
+                             f"{tuple(out.shape)}")
+        if work is None:
+            import torch
+            work = torch.empty(max(1, self.enks_work_size(M, nupd)), dtype=torch.float64, device=rec.device)
+        elif work.numel() < self.enks_work_size(M, nupd):
+            raise ValueError("enks_smooth: `work` is smaller than enks_work_size(M, nupd)")
+        L.check(self._lib.txh_enks_smooth(M, nupd, int(every), _cuda_ptr(T_hist), rec.shape[0], rec.shape[1],
+                                          int(rec_every), int(lag), _cuda_ptr(rec), _cuda_ptr(out), _cuda_ptr(work),
+                                          _stream_ptr()))
+        return out
 
     def route_timings(self):
         """Durations (ms) of the routing launches `run_assimilating(time_every=...)` bracketed; synchronises."""
