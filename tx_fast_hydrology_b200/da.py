@@ -342,7 +342,12 @@ class EnsembleKalmanFilter(_MeasurementTable, BaseCallback):
             self.world = torch.distributed.get_world_size(group)
         self.M = model.members
         self.Mtot = self.M * self.world
-        Rp = np.asarray(R_cov, dtype=np.float64)[perm, :][:, perm]
+        if self.Mtot < 2:
+            # the sample covariance divides by Mtot - 1: refused here, before any device work, rather than by the
+            # first solve, after the assimilation loop has already routed a window
+            raise ValueError(f'an ensemble Kalman filter needs at least 2 members in all, got {self.Mtot} '
+                             f'({self.M} per rank x {self.world} ranks)')
+        Rp =np.asarray(R_cov, dtype=np.float64)[perm, :][:, perm]
         q = np.broadcast_to(np.asarray(Q_diag, dtype=np.float64), (model.n,))
         self._R = torch.as_tensor(np.ascontiguousarray(Rp), device='cuda')
         self._qs = torch.as_tensor(np.ascontiguousarray(q[self.reach_indices]), device='cuda')
