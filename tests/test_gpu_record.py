@@ -266,6 +266,40 @@ def test_run_assimilating_recording_leaves_state_alone():
     assert (out[0][0] == out[1][0]).all() and (out[0][1] == out[1][1]).all()
 
 
+def test_run_assimilating_recording_refuses_multipliers_for_another_M():
+    """A forcing whose member multipliers were made for another member count is refused with TXH_E_INVALID before
+    any device work when the in-library loop records, as it is without recording: state and clock stay as they were."""
+    import torch
+    from tx_fast_hydrology_b200 import synthetic as S
+    from tx_fast_hydrology_b200._lib import TxhError
+    from tx_fast_hydrology_b200.muskingum import Muskingum
+    from tx_fast_hydrology_b200.da import EnsembleKalmanFilter
+    n, M, m, seed, every, nwin = 1500, 16, 20, 57, 6, 2
+    net = S.make_network(n, seed); prm = S.make_params(n, seed, well_posed=True)
+    rng = np.random.default_rng(seed)
+    d = S.model_dict(net, prm, dt_s=300.0); d["o_t"] = prm["o_t"][:, None] * rng.uniform(0.5, 1.5, size=(n, M))
+    mdl = Muskingum(d, members=M); t0 = mdl.datetime
+    times, table = S.make_forcing(n, every * nwin, 300.0, seed, t0_ns=int(t0.value), rows_every=4)
+    g = S.make_gauges(net["endnodes"], m, seed=seed)
+    mt = int(t0.value) + (np.arange(nwin, dtype=np.int64) + 1) * int(every * 300e9)
+    meas = rng.uniform(0.5, 8.0, size=(nwin, m))
+    mdf = pd.DataFrame(meas, index=pd.DatetimeIndex(pd.to_datetime(mt, unit="ns", utc=True)).as_unit("ns"),
+                       columns=[d["reach_ids"][j] for j in g])
+    enkf = EnsembleKalmanFilter(mdl, mdf, rng.uniform(0.5, 2.0, size=n), 1e-2 * np.eye(m))
+    Zp = torch.as_tensor(meas[:, :, None] + 0.1 * rng.standard_normal((nwin, m, M)), device="cuda")
+    # multipliers of M + 3 members: a run that went ahead would read them inside the table, with the wrong stride
+    f = mdl.make_forcing(times_ns=times, table=table, member_mul=S.make_member_multipliers(times.size, M + 3, seed))
+    O, I = mdl.device_state
+    O0, I0 = O.clone(), I.clone()
+    for record in (None, np.arange(0, n, 7)):
+        with pytest.raises(TxhError, match="do not match M") as err:
+            mdl.run_assimilating(f, every * nwin, enkf, every, Zp, record_reaches=record, record_prior=record is not None)
+        assert err.value.code == -1                             # TXH_E_INVALID
+        torch.cuda.synchronize()
+        assert torch.equal(O, O0) and torch.equal(I, I0)
+        assert mdl.datetime == t0 and enkf.n_updates == 0
+
+
 def test_run_assimilating_recording_variants_agree():
     """With the fused stages switched off (TXH_ENKF_FUSED=0 TXH_ENKF_FUSE_LOAD=0 TXH_PDL=0, read once per process: a
     child process), the recorded hydrographs and priors agree with the default path to 1e-10."""

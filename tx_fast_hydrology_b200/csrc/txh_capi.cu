@@ -42,6 +42,45 @@ int upload(T** dptr, const std::vector<T>& v)
     return TXH_OK;
 }
 
+// Grow-only device buffer of a handle: reallocated when `count` elements do not fit, once the handle's stream has
+// drained (a queued launch may still read the old one); new memory is filled with the byte `fill` unless it is < 0.
+template <class T>
+int grow(T** buf, size_t* cap, size_t count, cudaStream_t st, int fill = -1)
+{
+    if (count <= *cap) return TXH_OK;
+    if (*buf) { CU(cudaStreamSynchronize(st)); CU(cudaFree(*buf)); *buf = nullptr; *cap = 0; }
+    CU(cudaMalloc((void**)buf, count * sizeof(T)));
+    *cap = count;
+    if (fill >= 0) CU(cudaMemsetAsync(*buf, fill, count * sizeof(T), st));
+    return TXH_OK;
+}
+
+// Development aid (TXH_TRACE_FILE, TXH_LANE_TRACE): when the environment variable `env` names a file, `launch` runs
+// with a zeroed device timeline of `words` counters in `trace`, which is then written to that file behind the header
+// `hd` and `extra_bytes` of `extra` (synchronous).  Otherwise `launch` runs with trace == nullptr.
+template <class Launch>
+int traced_launch(const char* env, unsigned long long*& trace, size_t words, const long long (&hd)[4], const void* extra,
+                  size_t extra_bytes, cudaStream_t st, Launch&& launch)
+{
+    const char* file = getenv(env);
+    trace = nullptr;
+    if (!file || !*file) { CU(launch()); return TXH_OK; }
+    CU(cudaMalloc((void**)&trace, words * sizeof(unsigned long long)));
+    CU(cudaMemsetAsync(trace, 0, words * sizeof(unsigned long long), st));
+    CU(launch());
+    std::vector<unsigned long long> h(words);
+    CU(cudaMemcpyAsync(h.data(), trace, words * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    CU(cudaFree(trace));
+    if (FILE* fp = fopen(file, "wb")) {
+        fwrite(hd, sizeof(hd), 1, fp);
+        if (extra_bytes) fwrite(extra, 1, extra_bytes, fp);
+        fwrite(h.data(), sizeof(unsigned long long), h.size(), fp);
+        fclose(fp);
+    }
+    return TXH_OK;
+}
+
 }  // namespace
 
 struct txh_net {
@@ -79,10 +118,6 @@ struct txh_net {
     // ensemble update applied by the next window launch while it loads its tasks (txh_run_assimilating, txh_window.cu)
     int32_t* d_gfix_off = nullptr;      // [window tasks + 1] gauge terms per task, for the gauges in obs_cached
     int2* d_gfix = nullptr; size_t gfix_cap = 0; bool gfix_ok = false;
-    struct {
-        const double* T = nullptr; const double* W = nullptr; const double* qs = nullptr; int64_t M = 0;
-        double* rec_prior = nullptr; double* rec_post = nullptr; const double* rec_mean = nullptr;   // (REC launches)
-    } pending;
     // window-mode kernel
     WTaskDesc* d_wtasks = nullptr;
     uint32_t *d_whdr = nullptr, *d_winw = nullptr;
@@ -106,7 +141,7 @@ struct txh_net {
     int lane_ctas = 1;                  // regions (CTAs) per SM the schedule is sized for (measured: 1 is best, DESIGN.md)
     double* d_lring = nullptr; size_t lring_cap = 0;
     double* d_stage = nullptr; size_t stage_cap = 0;   // reach-order staging of txh_pack_host / txh_unpack_host
-    double* stats_rowsum = nullptr;     // txh_set_stats_output: row sums of the final outflows of every routing call
+    double* stats_rowsum = nullptr;     // txh_set_stats_output: row sums of the final outflows of every txh_route_run
     double stats_scale = 1.0;
     double* T_hist = nullptr;           // txh_set_transform_history: update k of a run_assimilating call solves into
     int64_t T_hist_cap = 0;             // T_hist + k*M*M (capacity in doubles)
@@ -214,18 +249,6 @@ int ensure_coef(txh_net* net, cudaStream_t st)
     return TXH_OK;
 }
 
-// grow-only device staging buffer in reach order (stream-ordered reuse: one stream per handle)
-int stage_buffer(txh_net* net, size_t doubles, cudaStream_t st, double** out)
-{
-    if (doubles > net->stage_cap) {
-        if (net->d_stage) { CU(cudaStreamSynchronize(st)); CU(cudaFree(net->d_stage)); net->d_stage = nullptr; }
-        CU(cudaMalloc((void**)&net->d_stage, doubles * sizeof(double)));
-        net->stage_cap = doubles;
-    }
-    *out = net->d_stage;
-    return TXH_OK;
-}
-
 // Synchronise `st` and report what the device recorded since the last report: a watchdog bail-out (status word)
 // or a failed factorisation (info word).  Both words are cleared once reported, so the handle is usable again
 // after the caller has re-uploaded a sane state; the rings of the persistent kernels are re-armed with them
@@ -260,72 +283,75 @@ int check_M(int64_t M)
     return TXH_OK;
 }
 
-// common launcher for the persistent dataflow kernel
 struct StepPlan {                   // forcing interpolation resolved by the init kernel (times == nullptr: unit step)
     const double* times = nullptr;
     int64_t R = 0, t0_ns = 0, dt_ns = 0;
     int method = 1;
 };
 
+// Outflows of the rows with a slot (slot == nullptr: off) recorded after every `every`-th step of a call; `base` steps
+// of the call came before this routing call (the step that ends its step s is base + s + 1).
+struct Recording {
+    const int32_t* slot = nullptr;
+    double* out = nullptr;
+    int every = 1, count = 0;
+    int64_t base = 0;
+};
+
+// An ensemble update still owed to the state (txh_run_assimilating): the first window launch of a routing call applies
+// it while it loads its tasks, and a recording launch also writes the update's recorded rows (rec_prior, rec_post).
+struct OwedUpdate {
+    const double* T; const double* W; const double* qs; int64_t M;
+    double* rec_prior; double* rec_post; const double* rec_mean;
+};
+
+// the forcing interpolation fields of the InitArgs of a launch's steps [s0, s0 + ns)
+InitArgs step_init(const txh_net* net, const StepPlan& plan, int64_t s0, int64_t ns)
+{
+    InitArgs ia{};
+    ia.times = plan.times; ia.steps_out = net->d_steps; ia.t0_ns = plan.t0_ns; ia.dt_ns = plan.dt_ns;
+    ia.step_base = s0; ia.R = (int32_t)plan.R; ia.nsteps = (int32_t)ns; ia.method = plan.method;
+    return ia;
+}
+
+// common launcher for the persistent dataflow kernel
 int run_dataflow(txh_net* net, double* O, double* I, int64_t M, const double* F, const double* W, int wm_ld,
-                 const StepPlan& plan, int64_t nsteps, const int32_t* rec_slot, double* rec_out,
-                 int rec_every, int rec_count, int64_t rec_base, cudaStream_t st)
+                 const StepPlan& plan, int64_t nsteps, const Recording& rec, cudaStream_t st)
 {
     const Schedule& s = net->sched;
     const int ld = (int)txh_row_stride(M);
     const int nmb = (ld + kMemberBlock - 1) / kMemberBlock;
     const size_t pairs = (size_t)s.tasks.size() * nmb;
     if (pairs >= (size_t(1) << 31)) return fail(TXH_E_INVALID, "too many (task, member block) pairs");
-    if (pairs > net->pairs_cap) {
-        if (net->d_pending) CU(cudaFree(net->d_pending));
-        CU(cudaMalloc((void**)&net->d_pending, pairs * sizeof(int32_t)));
-        net->pairs_cap = pairs;
-    }
     // the ready queue never wraps: one slot per (pair, step); long runs go out in several launches
     const int64_t max_entries = int64_t(1) << 25;
-    int64_t steps_per_launch = std::max<int64_t>(1, std::min<int64_t>(nsteps, max_entries / (int64_t)pairs));
-    const size_t qneed = pairs * (size_t)steps_per_launch;
-    const size_t side_need = (size_t)std::max(1, s.n_side) * ld;
-    if (side_need > net->side_cap) {
-        if (net->d_side) CU(cudaFree(net->d_side));
-        CU(cudaMalloc((void**)&net->d_side, side_need * sizeof(double)));
-        net->side_cap = side_need;
-    }
-    if (qneed > net->queue_cap) {
-        if (net->d_queue) CU(cudaFree(net->d_queue));
-        CU(cudaMalloc((void**)&net->d_queue, qneed * sizeof(unsigned long long)));
-        net->queue_cap = qneed;
-    }
-    const StepInterp* d_steps = net->d_unit_step;
-    if (plan.times) {
-        if ((size_t)steps_per_launch > net->steps_cap) {
-            if (net->d_steps) CU(cudaFree(net->d_steps));
-            CU(cudaMalloc((void**)&net->d_steps, sizeof(StepInterp) * steps_per_launch));
-            net->steps_cap = steps_per_launch;
-        }
-        d_steps = net->d_steps;
-    }
+    const int64_t steps_per_launch = std::max<int64_t>(1, std::min<int64_t>(nsteps, max_entries / (int64_t)pairs));
+    int rc;
+    if ((rc = grow(&net->d_pending, &net->pairs_cap, pairs, st)) ||
+        (rc = grow(&net->d_side, &net->side_cap, (size_t)std::max(1, s.n_side) * ld, st)) ||   // [n_side][ld]
+        (rc = grow(&net->d_queue, &net->queue_cap, pairs * (size_t)steps_per_launch, st)))
+        return rc;
+    if (plan.times && (rc = grow(&net->d_steps, &net->steps_cap, (size_t)steps_per_launch, st))) return rc;
+    const StepInterp* d_steps = plan.times ? net->d_steps : net->d_unit_step;
     for (int64_t s0 = 0; s0 < nsteps; s0 += steps_per_launch) {
         const int64_t ns = std::min<int64_t>(steps_per_launch, nsteps - s0);
-        InitArgs ia{};
+        InitArgs ia = step_init(net, plan, s0, ns);
         ia.tasks = net->d_tasks; ia.init_ready = net->d_init_ready; ia.pending = net->d_pending;
         ia.queue = net->d_queue; ia.q_head = net->d_qctl;
         ia.n_tasks = (int32_t)s.tasks.size(); ia.n_mblocks = nmb; ia.n_init = (int32_t)s.init_ready.size();
         ia.queue_entries = (long long)pairs * ns;
-        ia.times = plan.times; ia.steps_out = net->d_steps; ia.t0_ns = plan.t0_ns; ia.dt_ns = plan.dt_ns;
-        ia.step_base = s0; ia.R = (int32_t)plan.R; ia.nsteps = (int32_t)ns; ia.method = plan.method;
         CU(launch_dataflow_init(ia, st));
         RouteArgs a{};
         a.tasks = net->d_tasks; a.notify = net->d_notify; a.hdr = net->d_hdr; a.inw = net->d_inw;
         a.coef = net->d_coef; a.cumA = net->d_coef + 4 * net->topo.n; a.linkA = net->d_coef + 5 * net->topo.n;
         a.O = O; a.I = I; a.Side = net->d_side; a.F = F; a.steps = d_steps; a.Wmul = W;
-        a.rec_slot = rec_slot; a.rec_out = rec_out; a.rec_step_base = rec_base + s0;
+        a.rec_slot = rec.slot; a.rec_out = rec.out; a.rec_step_base = rec.base + s0;
         a.pending = ia.pending; a.queue = net->d_queue; a.q_head = net->d_qctl;
         a.status = net->d_status; a.watchdog_ns = net->watchdog_ns;
         a.total = (long long)pairs * ns;
         a.n = net->topo.n; a.n_tasks = ia.n_tasks; a.n_mblocks = nmb; a.nsteps = (int32_t)ns;
         a.slots = std::max(1, s.slots_used); a.ld = ld; a.M = (int32_t)M;
-        a.wm_ld = wm_ld; a.rec_every = std::max(1, rec_every); a.rec_count = rec_count;
+        a.wm_ld = wm_ld; a.rec_every = std::max(1, rec.every); a.rec_count = rec.count;
         // per-warp shared memory: [scratch slots][staging][row ring].  Staging of a walking task:
         // [coef][f0][f1][hdr][words]; of a LINK task: [A_last per segment][records]; 16-byte aligned parts.
         auto up16 = [](int x) { return (x + 15) & ~15; };
@@ -342,111 +368,96 @@ int run_dataflow(txh_net* net, double* O, double* I, int64_t M, const double* F,
         const int end_link = a.off_inw_link + up16(a.max_words_link * (int)sizeof(uint32_t));
         a.off_ring = std::max(end_walk, end_link);
         a.smem_per_warp = a.off_ring + kRingBytes;
-        a.trace = nullptr;
-        const char* trace_file = getenv("TXH_TRACE_FILE");
-        unsigned long long* d_trace = nullptr;
-        if (trace_file && *trace_file) {
-            CU(cudaMalloc((void**)&d_trace, (size_t)a.total * 4 * sizeof(unsigned long long)));
-            CU(cudaMemsetAsync(d_trace, 0, (size_t)a.total * 4 * sizeof(unsigned long long), st));
-            a.trace = d_trace;
-        }
-        CU(launch_route_dataflow(a, net->num_sms, st));
-        if (d_trace) {
-            // development aid: dump the per-task timeline of this launch (synchronous)
-            std::vector<unsigned long long> h((size_t)a.total * 4);
-            CU(cudaMemcpyAsync(h.data(), d_trace, h.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-            CU(cudaStreamSynchronize(st));
-            CU(cudaFree(d_trace));
-            if (FILE* fp = fopen(trace_file, "wb")) {
-                const long long hd[4] = {(long long)pairs, (long long)ns, (long long)s.tasks.size(), (long long)nmb};
-                fwrite(hd, sizeof(hd), 1, fp);
-                fwrite(h.data(), sizeof(unsigned long long), h.size(), fp);
-                fclose(fp);
-            }
-        }
+        // the per-task timeline of this launch
+        const long long hd[4] = {(long long)pairs, (long long)ns, (long long)s.tasks.size(), (long long)nmb};
+        if ((rc = traced_launch("TXH_TRACE_FILE", a.trace, (size_t)a.total * 4, hd, nullptr, 0, st,
+                                [&] { return launch_route_dataflow(a, net->num_sms, st); })))
+            return rc;
     }
     return TXH_OK;
 }
 
-// The window-resident kernel (txh_window.cu): state in shared memory for all steps of a launch.
-// Returns 1 when the schedule does not fit it (rows of a task x 1 KB per warp) and the caller should fall
+// Per-warp shared-memory layout of route_window_kernel.  A launch that applies an ensemble update keeps the 64 x 64
+// transform in shared memory and runs shorter input rings (txh_window.cu: kInRingUpd, kSegRingUpd) to keep its warps:
+// at the headline shape 16 x 12,432 B + 33,168 B of the 232,448 B a CTA may have.
+void window_smem_layout(const Schedule& s, bool upd, WinArgs& a)
+{
+    auto up16 = [](int x) { return (x + 15) & ~15; };
+    const int rc = std::max(1, s.w_max_len), slots = std::max(1, s.slots_used);
+    // `seg_ring` rows for the input stream of a segment ([scratch | ring]), `in_ring` for a pocket's
+    const int in_ring = upd ? 2 : 4, seg_ring = upd ? 6 : 8;
+    a.off_scr = rc * 512;
+    a.off_in = a.off_scr + slots * 512;
+    a.off_rec = a.off_in + std::max(in_ring, seg_ring - slots) * 512;
+    a.off_cum = a.off_rec + rc * 48;
+    a.off_cumc = a.off_cum + up16(rc * 8);
+    a.off_words = a.off_cumc + up16(rc * 8);
+    a.off_list = a.off_words + up16(std::max(1, s.w_max_words) * 4);
+    a.off_mbar = a.off_list + up16(std::max(1, s.w_max_words) * 4);
+    a.smem_per_warp = a.off_mbar + 16;                        // + the warp's mbarrier (bulk staging of the state rows)
+    const char* bulk = getenv("TXH_WINDOW_BULK");
+    if (bulk && atoi(bulk) == 0) a.off_mbar = 0;
+}
+
+// Whether route_window_kernel takes the schedule at M members (ok), and the warps per CTA of a launch without (wpc) and
+// with (wpc_upd) an ensemble update to apply.  The kernel declines when a CTA would hold fewer than two warps (rows of
+// a task x 1 KB per warp), when the schedule has rows it would own, and when ring slots need offsets beyond 32 bits.
+// Allocates and launches nothing.
+struct WindowFit {
+    bool ok;
+    int wpc, wpc_upd;
+};
+WindowFit window_fit(const txh_net* net, int64_t M)
+{
+    const Schedule& s = net->sched;
+    const int steps_bytes = 16 * 24;                          // StepInterp records of one launch (<= 16 steps), once per CTA
+    const int smem_max = 227 * 1024;
+    int warps_cap = 16;
+    if (const char* k = getenv("TXH_WINDOW_WARPS")) warps_cap = std::max(1, std::min(16, atoi(k)));
+    WinArgs a{};
+    window_smem_layout(s, true, a);
+    const int wpc_upd = std::min(warps_cap, (smem_max - steps_bytes - 64 * 64 * (int)sizeof(double) - 16) / a.smem_per_warp);
+    window_smem_layout(s, false, a);
+    const int wpc = std::min(warps_cap, (smem_max - 1024 - steps_bytes) / a.smem_per_warp);
+    const bool ok = wpc >= 2 && s.w_n_own == 0 &&
+                    (size_t)std::max(1, s.n_wslots) * txh_row_stride(M) * sizeof(double) < (size_t(1) << 32);
+    return {ok, wpc, wpc_upd};
+}
+
+// The window-resident kernel (txh_window.cu): state in shared memory for all steps of a launch; its first launch
+// applies `upd`.  Returns 1 when the kernel declines the schedule (window_fit) or cannot apply `upd`; the caller falls
 // back to the dataflow kernel.
 int run_window(txh_net* net, double* O, double* I, int64_t M, const double* F, const double* W, int wm_ld,
-               const StepPlan& plan, int64_t nsteps, cudaStream_t st, bool probe_only = false,
-               const int32_t* rec_slot = nullptr, double* rec_out = nullptr, int rec_every = 1, int rec_count = 0,
-               int64_t rec_base = 0)
+               const StepPlan& plan, int64_t nsteps, const Recording& rec, double* rowsum, double rowsum_scale,
+               const OwedUpdate* upd, cudaStream_t st)
 {
     const Schedule& s = net->sched;
     const int ld = (int)txh_row_stride(M);
     const int nmb = (ld + kMemberBlock - 1) / kMemberBlock;
     const size_t pairs = (size_t)s.wtasks.size() * nmb;
     if (pairs >= (size_t(1) << 31)) return fail(TXH_E_INVALID, "too many (task, member block) pairs");
-    WinArgs a{};
-    auto up16 = [](int x) { return (x + 15) & ~15; };
-    const int rc = std::max(1, s.w_max_len), slots = std::max(1, s.slots_used);
-    const bool bulk_off = [] { const char* k = getenv("TXH_WINDOW_BULK"); return k && atoi(k) == 0; }();
-    // per-warp layout; `seg_ring` rows for the input stream of a segment ([scratch | ring]), `in_ring` for a pocket's
-    auto layout = [&](int in_ring, int seg_ring) {
-        a.off_scr = rc * 512;
-        a.off_in = a.off_scr + slots * 512;
-        a.off_rec = a.off_in + std::max(in_ring, seg_ring - slots) * 512;
-        a.off_cum = a.off_rec + rc * 48;
-        a.off_cumc = a.off_cum + up16(rc * 8);
-        a.off_words = a.off_cumc + up16(rc * 8);
-        a.off_list = a.off_words + up16(std::max(1, s.w_max_words) * 4);
-        a.off_mbar = a.off_list + up16(std::max(1, s.w_max_words) * 4);
-        a.smem_per_warp = a.off_mbar + 16;                    // + the warp's mbarrier (bulk staging of the state rows)
-        if (bulk_off) a.off_mbar = 0;
-    };
-    const int steps_bytes = 16 * 24;                          // StepInterp records of one launch (<= 16 steps), once per CTA
-    if ((size_t)std::max(1, s.n_wslots) * ld * sizeof(double) >= (size_t(1) << 32)) return 1;   // 32-bit slot offsets
-    const int smem_max = 227 * 1024;
-    int warps_cap = 16;
-    if (const char* k = getenv("TXH_WINDOW_WARPS")) warps_cap = std::max(1, std::min(16, atoi(k)));
-    // a launch that applies an ensemble update keeps the 64 x 64 transform in shared memory and runs shorter input rings
-    // (txh_window.cu: kInRingUpd, kSegRingUpd) to keep its warps: at the headline shape 16 x 12,432 B + 33,168 B of the
-    // 232,448 B a CTA may have
-    layout(2, 6);
-    const int wpc_upd = std::min(warps_cap, (smem_max - steps_bytes - 64 * 64 * (int)sizeof(double) - 16) / a.smem_per_warp);
-    layout(4, 8);
-    const int wpc = std::min(warps_cap, (smem_max - 1024 - steps_bytes) / a.smem_per_warp);
-    if (wpc < 2 || s.w_n_own > 0) return 1;
-    if (probe_only) return wpc_upd >= 2 ? TXH_OK : 1;
+    const WindowFit fit = window_fit(net, M);
+    if (!fit.ok || (upd && (nmb != 1 || upd->M != M || fit.wpc_upd < 2))) return 1;
     // ring[step][slot][ld]: one launch covers 16 steps, up to 64 while the ring stays below 64 MiB (few members):
     // a launch costs the critical path of one step before its pipeline is full, so longer launches amortise it
     const size_t slot_row = (size_t)std::max(1, s.n_wslots) * ld;
     const int64_t spl_max = std::min<int64_t>(64, std::max<int64_t>(16, (int64_t)((size_t(64) << 20) / (slot_row * sizeof(double)))));
     int64_t spl = std::min<int64_t>(spl_max, nsteps);
     while (spl > 1 && slot_row * spl * sizeof(double) > (size_t(1) << 30)) --spl;
-    if (slot_row * spl > net->ring_cap) {
-        // every cell starts EMPTY (all bits set); consumers put EMPTY back, so a finished launch leaves the whole
-        // ring EMPTY again whatever row stride the next launch lays over it
-        if (net->d_ring) CU(cudaFree(net->d_ring));
-        CU(cudaMalloc((void**)&net->d_ring, slot_row * spl * sizeof(double)));
-        net->ring_cap = slot_row * spl;
-        CU(cudaMemsetAsync(net->d_ring, 0xff, net->ring_cap * sizeof(double), st));
-    }
+    // every cell starts EMPTY (all bits set); consumers put EMPTY back, so a finished launch leaves the whole
+    // ring EMPTY again whatever row stride the next launch lays over it
+    int rc;
+    if ((rc = grow(&net->d_ring, &net->ring_cap, slot_row * spl, st, 0xff))) return rc;
     net->ring_ld = ld;
-    const StepInterp* d_steps = net->d_unit_step;
-    if (plan.times) {
-        if ((size_t)spl > net->steps_cap) {
-            if (net->d_steps) CU(cudaFree(net->d_steps));
-            CU(cudaMalloc((void**)&net->d_steps, sizeof(StepInterp) * spl));
-            net->steps_cap = spl;
-        }
-        d_steps = net->d_steps;
-    }
+    if (plan.times && (rc = grow(&net->d_steps, &net->steps_cap, (size_t)spl, st))) return rc;
+    const StepInterp* d_steps = plan.times ? net->d_steps : net->d_unit_step;
+    WinArgs a{};
     for (int64_t s0 = 0; s0 < nsteps; s0 += spl) {
         const int64_t ns = std::min<int64_t>(spl, nsteps - s0);
         // up to 16 steps every warp resolves the forcing interpolation itself (no init launch: the kernel re-arms
         // its own ticket); longer launches read the records an init kernel leaves in global memory
         const bool own_steps = ns <= 16;
-        if (!own_steps) {
-            InitArgs ia{};
-            ia.times = plan.times; ia.steps_out = net->d_steps; ia.t0_ns = plan.t0_ns; ia.dt_ns = plan.dt_ns;
-            ia.step_base = s0; ia.R = (int32_t)plan.R; ia.nsteps = (int32_t)ns; ia.method = plan.method;
-            CU(launch_window_init(ia, net->d_qctl + 3, st));
-        }
+        if (!own_steps) CU(launch_window_init(step_init(net, plan, s0, ns), net->d_qctl + 3, st));
         a.times = plan.times; a.t0_ns = plan.t0_ns; a.dt_ns = plan.dt_ns; a.step_base = s0; a.R = (int32_t)plan.R;
         a.method = plan.method; a.done = net->d_qctl + 5;
         a.tasks = net->d_wtasks; a.hdr = net->d_whdr; a.inw = net->d_winw; a.prod = net->d_wprod;
@@ -457,47 +468,27 @@ int run_window(txh_net* net, double* O, double* I, int64_t M, const double* F, c
         a.n = net->topo.n; a.n_tasks = (int32_t)s.wtasks.size(); a.n_mblocks = nmb; a.nsteps = (int32_t)ns;
         a.n_slots = std::max(1, s.n_wslots); a.ld = ld; a.M = (int32_t)M; a.wm_ld = wm_ld;
         // the row sums ride on the last step of the call when one warp covers all members of a row
-        a.rowsum = (net->stats_rowsum && nmb == 1 && s0 + ns == nsteps) ? net->stats_rowsum : nullptr;
-        a.rowsum_scale = net->stats_scale;
+        a.rowsum = (rowsum && nmb == 1 && s0 + ns == nsteps) ? rowsum : nullptr;
+        a.rowsum_scale = rowsum_scale;
         a.upT = nullptr;
-        if (s0 == 0 && net->pending.T && nmb == 1 && net->pending.M == M && wpc_upd >= 2) {
+        if (s0 == 0 && upd) {
             // the ensemble update owed to the state is applied by this launch while it loads its tasks
-            a.upT = net->pending.T; a.upW = net->pending.W; a.upQs = net->pending.qs;
+            a.upT = upd->T; a.upW = upd->W; a.upQs = upd->qs;
             a.gfix_off = net->d_gfix_off; a.gfix = net->d_gfix;
-            if (rec_slot) { a.rec_prior = net->pending.rec_prior; a.rec_post = net->pending.rec_post; a.rec_mean = net->pending.rec_mean; }
-            net->pending.rec_prior = net->pending.rec_post = nullptr;
-            layout(2, 6);
-            a.off_T = wpc_upd * a.smem_per_warp;
-            net->pending.T = nullptr;
-        } else layout(4, 8);
-        a.off_steps = a.upT ? a.off_T + 64 * 64 * (int)sizeof(double) + 16 : wpc * a.smem_per_warp;
-        a.rec_slot = rec_slot; a.rec_out = rec_out; a.rec_step_base = rec_base + s0;
-        a.rec_every = std::max(1, rec_every); a.rec_count = rec_count;
+            if (rec.slot) { a.rec_prior = upd->rec_prior; a.rec_post = upd->rec_post; a.rec_mean = upd->rec_mean; }
+            window_smem_layout(s, true, a);
+            a.off_T = fit.wpc_upd * a.smem_per_warp;
+        } else window_smem_layout(s, false, a);
+        a.off_steps = a.upT ? a.off_T + 64 * 64 * (int)sizeof(double) + 16 : fit.wpc * a.smem_per_warp;
+        a.rec_slot = rec.slot; a.rec_out = rec.out; a.rec_step_base = rec.base + s0;
+        a.rec_every = std::max(1, rec.every); a.rec_count = rec.count;
         a.nap_min = 32; a.nap_max = 256;
         if (const char* k = getenv("TXH_WINDOW_NAP")) { int lo = 32, hi = 256; if (sscanf(k, "%d,%d", &lo, &hi) >= 1) { a.nap_min = std::max(0, lo); a.nap_max = std::max(a.nap_min, hi); } }
-        a.trace = nullptr;
-        const char* trace_file = getenv("TXH_TRACE_FILE");
-        unsigned long long* d_trace = nullptr;
-        const size_t trace_words = pairs * (size_t)(4 + ns);
-        if (trace_file && *trace_file) {
-            CU(cudaMalloc((void**)&d_trace, trace_words * sizeof(unsigned long long)));
-            CU(cudaMemsetAsync(d_trace, 0, trace_words * sizeof(unsigned long long), st));
-            a.trace = d_trace;
-        }
-        CU(launch_route_window(a, a.upT ? wpc_upd : wpc, net->num_sms, st));
-        if (d_trace) {
-            // development aid: dump the per-task timeline of this launch (synchronous)
-            std::vector<unsigned long long> h(trace_words);
-            CU(cudaMemcpyAsync(h.data(), d_trace, h.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-            CU(cudaStreamSynchronize(st));
-            CU(cudaFree(d_trace));
-            if (FILE* fp = fopen(trace_file, "wb")) {
-                const long long hd[4] = {(long long)pairs, (long long)ns, (long long)s.wtasks.size(), -(long long)nmb};
-                fwrite(hd, sizeof(hd), 1, fp);
-                fwrite(h.data(), sizeof(unsigned long long), h.size(), fp);
-                fclose(fp);
-            }
-        }
+        // the per-task timeline of this launch
+        const long long hd[4] = {(long long)pairs, (long long)ns, (long long)s.wtasks.size(), -(long long)nmb};
+        if ((rc = traced_launch("TXH_TRACE_FILE", a.trace, pairs * (size_t)(4 + ns), hd, nullptr, 0, st,
+                                [&] { return launch_route_window(a, a.upT ? fit.wpc_upd : fit.wpc, net->num_sms, st); })))
+            return rc;
     }
     return TXH_OK;
 }
@@ -542,14 +533,14 @@ txh_net::LaneDev* lane_schedule(txh_net* net, int ti, int num_sms)
 
 // Returns 1 when the lane schedule cannot be built for this network (the caller falls back).
 int run_lane(txh_net* net, double* O, double* I, int64_t M, const double* F, const double* W, int wm_ld,
-             const StepPlan& plan, int64_t nsteps, const int32_t* rec_slot, double* rec_out, int rec_every,
-             int rec_count, int64_t rec_base, cudaStream_t st)
+             const StepPlan& plan, int64_t nsteps, const Recording& rec, cudaStream_t st)
 {
     const int ti = lane_tile_index(M), mt = 1 << ti;
     if (M > 16) return 1;
     txh_net::LaneDev* L = lane_schedule(net, ti, net->num_sms);
     if (!L->ok) return 1;
     const LaneSchedule& s = L->sched;
+    int rc;
     if (!L->on_dev) {
         std::vector<int4> meta(s.row_reach.size());
         for (size_t i = 0; i < meta.size(); ++i) {
@@ -557,7 +548,6 @@ int run_lane(txh_net* net, double* O, double* I, int64_t M, const double* F, con
             meta[i] = make_int4(j >= 0 ? net->sched.pos_of_reach[j] : -1, s.row_off[i] | (s.row_nx[i] << 16), s.row_c01[i],
                                 s.row_slot[i]);
         }
-        int rc;
         if ((rc = upload(&L->d_regions, s.regions))) return rc;
         if ((rc = upload(&L->d_meta, meta))) return rc;
         if ((rc = upload(&L->d_xbeg, s.row_xbeg))) return rc;
@@ -576,23 +566,13 @@ int run_lane(txh_net* net, double* O, double* I, int64_t M, const double* F, con
     if (const char* k = getenv("TXH_LANE_SPL")) { const long v = atol(k); if (v > 0) spl = std::min<int64_t>(spl, v); }
     while (spl > 16 && streams * (size_t)((spl + 15) & ~int64_t(15)) * sizeof(double) > (size_t(128) << 20)) spl = (spl + 1) / 2;
     const size_t ring_need = streams * (size_t)((spl + 15) & ~int64_t(15));
-    if (ring_need > net->lring_cap) {
-        if (net->d_lring) { CU(cudaStreamSynchronize(st)); CU(cudaFree(net->d_lring)); }
-        CU(cudaMalloc((void**)&net->d_lring, ring_need * sizeof(double)));
-        net->lring_cap = ring_need;
-        CU(cudaMemsetAsync(net->d_lring, 0xff, ring_need * sizeof(double), st));   // every cell starts EMPTY
-    }
-    const LaneStep* d_steps = net->d_unit_lstep;
+    if ((rc = grow(&net->d_lring, &net->lring_cap, ring_need, st, 0xff))) return rc;   // every cell starts EMPTY
     if (plan.times) {
-        if ((size_t)spl > net->lsteps_cap) {
-            if (net->d_lsteps) { CU(cudaStreamSynchronize(st)); CU(cudaFree(net->d_lsteps)); }
-            CU(cudaMalloc((void**)&net->d_lsteps, sizeof(LaneStep) * spl));
-            net->lsteps_cap = spl;
-        }
-        d_steps = net->d_lsteps;
+        if ((rc = grow(&net->d_lsteps, &net->lsteps_cap, (size_t)spl, st))) return rc;
     } else if (nsteps != 1) {
         return fail(TXH_E_INVALID, "internal: a launch without a forcing table covers one step");
     }
+    const LaneStep* d_steps = plan.times ? net->d_lsteps : net->d_unit_lstep;
     // shared memory: the largest region (every CTA lays its region out itself, LaneSchedule::region_bytes)
     LaneArgs a{};
     size_t smem = (s.max_bytes + 31) & ~size_t(15);
@@ -616,44 +596,22 @@ int run_lane(txh_net* net, double* O, double* I, int64_t M, const double* F, con
     const int grid = (int)std::min<int64_t>((int64_t)net->num_sms * per_sm, (int64_t)s.regions.size());
     for (int64_t s0 = 0; s0 < nsteps; s0 += spl) {
         const int64_t ns = std::min<int64_t>(spl, nsteps - s0);
-        if (plan.times) {
-            InitArgs ia{};
-            ia.times = plan.times; ia.steps_out = net->d_steps; ia.t0_ns = plan.t0_ns; ia.dt_ns = plan.dt_ns;
-            ia.step_base = s0; ia.R = (int32_t)plan.R; ia.nsteps = (int32_t)ns; ia.method = plan.method;
-            CU(launch_lane_init(ia, net->d_lsteps, net->d_qctl + 6, st));
-        }
+        if (plan.times) CU(launch_lane_init(step_init(net, plan, s0, ns), net->d_lsteps, net->d_qctl + 6, st));
         a.regions = L->d_regions; a.meta = L->d_meta; a.xbeg = L->d_xbeg; a.child = L->d_child;
         a.coef = net->d_coef; a.O = O; a.I = I; a.F = F; a.steps = d_steps; a.Wmul = W;
         a.ring = net->d_lring; a.ticket = net->d_qctl + 6; a.done = net->d_qctl + 7;
         a.status = net->d_status; a.watchdog_ns = net->watchdog_ns;
-        a.rec_slot = rec_slot; a.rec_out = rec_out; a.rec_step_base = rec_base + s0;
-        a.rec_every = std::max(1, rec_every); a.rec_count = rec_count;
+        a.rec_slot = rec.slot; a.rec_out = rec.out; a.rec_step_base = rec.base + s0;
+        a.rec_every = std::max(1, rec.every); a.rec_count = rec.count;
         a.n = net->topo.n; a.n_regions = (int32_t)s.regions.size(); a.nsteps = (int32_t)ns;
         a.splp = (int32_t)((ns + 15) & ~int64_t(15)); a.ld = ld; a.M = (int32_t)M; a.wm_ld = wm_ld;
         a.R = plan.times ? (int32_t)plan.R : 1;
-        // development aid: TXH_LANE_TRACE=<file> dumps the region timeline of this launch (synchronous)
-        const char* trace_file = getenv("TXH_LANE_TRACE");
-        unsigned long long* d_trace = nullptr;
-        const size_t trace_words = 8 * s.regions.size();
-        if (trace_file && *trace_file) {
-            CU(cudaMalloc((void**)&d_trace, trace_words * sizeof(unsigned long long)));
-            CU(cudaMemsetAsync(d_trace, 0, trace_words * sizeof(unsigned long long), st));
-            a.trace = d_trace;
-        }
-        CU(launch_route_lane(a, mt, threads, smem, grid, st));
-        if (d_trace) {
-            std::vector<unsigned long long> h(trace_words);
-            CU(cudaMemcpyAsync(h.data(), d_trace, h.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-            CU(cudaStreamSynchronize(st));
-            CU(cudaFree(d_trace));
-            if (FILE* fp = fopen(trace_file, "wb")) {
-                const long long hd[4] = {(long long)s.regions.size(), (long long)ns, (long long)threads, (long long)grid};
-                fwrite(hd, sizeof(hd), 1, fp);
-                fwrite(s.regions.data(), sizeof(LaneRegionDesc), s.regions.size(), fp);
-                fwrite(h.data(), sizeof(unsigned long long), h.size(), fp);
-                fclose(fp);
-            }
-        }
+        // the region timeline of this launch, behind the region descriptors
+        const long long hd[4] = {(long long)s.regions.size(), (long long)ns, (long long)threads, (long long)grid};
+        if ((rc = traced_launch("TXH_LANE_TRACE", a.trace, 8 * s.regions.size(), hd, s.regions.data(),
+                                s.regions.size() * sizeof(LaneRegionDesc), st,
+                                [&] { return launch_route_lane(a, mt, threads, smem, grid, st); })))
+            return rc;
     }
     return TXH_OK;
 }
@@ -680,44 +638,26 @@ bool lane_wanted(txh_net* net, int64_t M, int64_t nsteps)
 }
 
 // routing entry: the lane kernel for small ensembles, else the window kernel (or what the environment says); the
-// dataflow kernel where the window kernel declines the schedule.  rec_slot: [n] recording slot per position or nullptr;
-// rec_base: steps of the call before this one (the step that ends this call's step s is rec_base + s + 1)
+// dataflow kernel where the window kernel declines the schedule.  rowsum (nullptr: off) receives rowsum_scale * the
+// member sums of the final outflows.  upd (nullptr: none) is applied by the first window launch; a routing call that
+// cannot apply it fails.
 int run_routing(txh_net* net, double* O, double* I, int64_t M, const double* F, const double* W, int wm_ld,
-                const StepPlan& plan, int64_t nsteps, const int32_t* rec_slot, double* rec_out, int rec_every,
-                int rec_count, cudaStream_t st, int64_t rec_base = 0)
+                const StepPlan& plan, int64_t nsteps, cudaStream_t st, const Recording& rec = Recording(),
+                double* rowsum = nullptr, double rowsum_scale = 1.0, const OwedUpdate* upd = nullptr)
 {
     const int ld = (int)txh_row_stride(M);
-    if (lane_wanted(net, M, nsteps)) {
-        const int rc = run_lane(net, O, I, M, F, W, wm_ld, plan, nsteps, rec_slot, rec_out, rec_every, rec_count, rec_base, st);
-        if (rc == TXH_OK && net->stats_rowsum)
-            CU(launch_enkf_stats(O, ld, (int)M, net->topo.n, net->stats_scale, nullptr, net->stats_rowsum, nullptr, st));
-        if (rc != 1) return rc;
+    int rc = 1;                                           // 1: the kernel declined, the next one routes
+    bool sums_done = false;                               // by the window kernel, on its last step
+    if (!upd && lane_wanted(net, M, nsteps)) rc = run_lane(net, O, I, M, F, W, wm_ld, plan, nsteps, rec, st);
+    if (rc == 1 && net->route_kernel != 1) {
+        rc = run_window(net, O, I, M, F, W, wm_ld, plan, nsteps, rec, rowsum, rowsum_scale, upd, st);
+        sums_done = rc == TXH_OK && ld <= kMemberBlock;
     }
-    if (net->route_kernel != 1) {
-        const int rc = run_window(net, O, I, M, F, W, wm_ld, plan, nsteps, st, false, rec_slot, rec_out, rec_every, rec_count,
-                                  rec_base);
-        if (rc == TXH_OK && net->stats_rowsum && ld > kMemberBlock)
-            CU(launch_enkf_stats(O, ld, (int)M, net->topo.n, net->stats_scale, nullptr, net->stats_rowsum, nullptr, st));
-        if (rc != 1) return rc;
-    }
-    const int rc = run_dataflow(net, O, I, M, F, W, wm_ld, plan, nsteps, rec_slot, rec_out, rec_every, rec_count, rec_base, st);
-    if (rc == TXH_OK && net->stats_rowsum)
-        CU(launch_enkf_stats(O, ld, (int)M, net->topo.n, net->stats_scale, nullptr, net->stats_rowsum, nullptr, st));
+    if (rc == 1 && upd) return fail(TXH_E_STATE, "the routing launch did not take the pending ensemble update");
+    if (rc == 1) rc = run_dataflow(net, O, I, M, F, W, wm_ld, plan, nsteps, rec, st);
+    if (rc == TXH_OK && rowsum && !sums_done)
+        CU(launch_enkf_stats(O, ld, (int)M, net->topo.n, rowsum_scale, nullptr, rowsum, nullptr, st));
     return rc;
-}
-
-// one step without a forcing table (q: [n] schedule order or nullptr): window kernel first, dataflow otherwise
-int run_one_step(txh_net* net, double* O, double* I, int64_t M, const double* q, cudaStream_t st)
-{
-    if (lane_wanted(net, M, 1)) {
-        const int rc = run_lane(net, O, I, M, q, nullptr, 0, StepPlan(), 1, nullptr, nullptr, 1, 0, 0, st);
-        if (rc != 1) return rc;
-    }
-    if (net->route_kernel != 1) {
-        const int rc = run_window(net, O, I, M, q, nullptr, 0, StepPlan(), 1, st);
-        if (rc != 1) return rc;
-    }
-    return run_dataflow(net, O, I, M, q, nullptr, 0, StepPlan(), 1, nullptr, nullptr, 1, 0, 0, st);
 }
 
 }  // namespace
@@ -952,8 +892,8 @@ int txh_pack_host(txh_net* net, const double* src, int64_t M, int layout, double
     if ((rc = check_M(M)) || (rc = ensure_device(net))) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     const int64_t n = net->topo.n;
-    double* tmp = nullptr;
-    if ((rc = stage_buffer(net, (size_t)n * M, st, &tmp))) return rc;
+    if ((rc = grow(&net->d_stage, &net->stage_cap, (size_t)n * M, st))) return rc;
+    double* tmp = net->d_stage;
     CU(cudaMemcpyAsync(tmp, src, sizeof(double) * n * M, cudaMemcpyHostToDevice, st));
     CU(launch_pack(net->d_reach_of_pos, tmp, dst, n, (int)M, (int)txh_row_stride(M), layout, st));
     return TXH_OK;
@@ -966,8 +906,8 @@ int txh_unpack_host(txh_net* net, const double* src, int64_t M, int layout, doub
     if ((rc = check_M(M)) || (rc = ensure_device(net))) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     const int64_t n = net->topo.n;
-    double* tmp = nullptr;
-    if ((rc = stage_buffer(net, (size_t)n * M, st, &tmp))) return rc;
+    if ((rc = grow(&net->d_stage, &net->stage_cap, (size_t)n * M, st))) return rc;
+    double* tmp = net->d_stage;
     CU(launch_unpack(net->d_reach_of_pos, src, tmp, n, (int)M, (int)txh_row_stride(M), layout, st));
     CU(cudaMemcpyAsync(dst, tmp, sizeof(double) * n * M, cudaMemcpyDeviceToHost, st));
     return report_status(net, st);
@@ -1004,11 +944,7 @@ int txh_gather_rows(txh_net* net, const double* X, int64_t M, const int64_t* idx
         if (idx[k] < 0 || idx[k] >= net->topo.n) return fail(TXH_E_INVALID, "reach index out of range");
         pos[k] = net->sched.pos_of_reach[idx[k]];
     }
-    if ((size_t)count > net->tmp_idx_cap) {
-        if (net->d_tmp_idx) CU(cudaFree(net->d_tmp_idx));
-        CU(cudaMalloc((void**)&net->d_tmp_idx, sizeof(int32_t) * count));
-        net->tmp_idx_cap = count;
-    }
+    if ((rc = grow(&net->d_tmp_idx, &net->tmp_idx_cap, (size_t)count, st))) return rc;
     CU(cudaMemcpyAsync(net->d_tmp_idx, pos.data(), sizeof(int32_t) * count, cudaMemcpyHostToDevice, st));
     CU(cudaStreamSynchronize(st));      // `pos` is a stack-lifetime buffer
     CU(launch_gather_rows(net->d_tmp_idx, count, X, (int)txh_row_stride(M), (int)M, out, st));
@@ -1041,8 +977,8 @@ int txh_forcing_create(txh_net* net, int64_t R, const double* times, const doubl
     f->times.assign(times, times + R);
     // one H2D copy of the table as given (pinned or pageable) into the handle's staging buffer, columns
     // permuted into schedule order on the device
-    double* tmp = nullptr;
-    if ((rc = stage_buffer(net, (size_t)R * n, st, &tmp))) { delete f; return rc; }
+    if ((rc = grow(&net->d_stage, &net->stage_cap, (size_t)R * n, st))) { delete f; return rc; }
+    double* tmp = net->d_stage;
     cudaError_t e = cudaMalloc((void**)&f->d_F, sizeof(double) * R * n);
     if (e == cudaSuccess) e = cudaMalloc((void**)&f->d_times, sizeof(double) * R);
     if (e == cudaSuccess) e = cudaMemcpyAsync(f->d_times, f->times.data(), sizeof(double) * R, cudaMemcpyHostToDevice, st);
@@ -1070,8 +1006,8 @@ int txh_forcing_update(txh_forcing* f, const double* times, const double* table,
         if (!(times[r] >= times[r - 1])) return fail(TXH_E_INVALID, "forcing times must be sorted ascending");
     int rc;
     if ((rc = txh_forcing_wait(f))) return rc;
-    double* tmp = nullptr;
-    if ((rc = stage_buffer(net, (size_t)R * n, st, &tmp))) return rc;
+    if ((rc = grow(&net->d_stage, &net->stage_cap, (size_t)R * n, st))) return rc;
+    double* tmp = net->d_stage;
     f->times.assign(times, times + R);
     CU(cudaMemcpyAsync(f->d_times, f->times.data(), sizeof(double) * R, cudaMemcpyHostToDevice, st));
     CU(cudaMemcpyAsync(tmp, table, sizeof(double) * R * n, cudaMemcpyHostToDevice, st));
@@ -1160,8 +1096,8 @@ int upload_rec_slots(txh_net* net, const int64_t* rec_reach, int64_t rec_count, 
 
 // txh_route_run once the arguments are checked and the recording slots are on the device
 int route_run_impl(txh_net* net, double* O, double* I, int64_t M, const txh_forcing* fo, int64_t t0_ns, int64_t dt_ns,
-                   int64_t nsteps, int method, const int32_t* rec_slot, int64_t rec_count, int64_t rec_every,
-                   double* rec_out, int64_t rec_base, cudaStream_t st)
+                   int64_t nsteps, int method, const Recording& rec, double* rowsum, double rowsum_scale,
+                   const OwedUpdate* upd, cudaStream_t st)
 {
     if (nsteps == 0) return TXH_OK;
     StepPlan plan;
@@ -1177,7 +1113,7 @@ int route_run_impl(txh_net* net, double* O, double* I, int64_t M, const txh_forc
         }
     }
     return run_routing(net, O, I, M, fo ? fo->d_F : nullptr, fo ? fo->d_W : nullptr, fo ? (int)fo->M : 0,
-                       plan, nsteps, rec_slot, rec_out, (int)rec_every, (int)rec_count, st, rec_base);
+                       plan, nsteps, st, rec, rowsum, rowsum_scale, upd);
 }
 }  // namespace
 
@@ -1197,8 +1133,9 @@ int txh_route_run(txh_net* net, double* O, double* I, int64_t M, const txh_forci
     if ((rc = check_M(M)) || (rc = ensure_device(net)) || (rc = ensure_coef(net, st))) return rc;
     if (nsteps == 0) return TXH_OK;
     if (rec_count > 0 && (rc = upload_rec_slots(net, rec_reach, rec_count, st))) return rc;
-    return route_run_impl(net, O, I, M, fo, t0_ns, dt_ns, nsteps, method, rec_count > 0 ? net->d_rec_slot : nullptr,
-                          rec_count, rec_every, rec_out, 0, st);
+    const Recording rec{rec_count > 0 ? net->d_rec_slot : nullptr, rec_out, (int)rec_every, (int)rec_count, 0};
+    return route_run_impl(net, O, I, M, fo, t0_ns, dt_ns, nsteps, method, rec, net->stats_rowsum, net->stats_scale,
+                          nullptr, st);
 }
 
 int txh_route_step(txh_net* net, double* O, double* I, int64_t M, const double* q, void* stream)
@@ -1208,7 +1145,7 @@ int txh_route_step(txh_net* net, double* O, double* I, int64_t M, const double* 
     cudaStream_t st = (cudaStream_t)stream;
     if ((rc = check_M(M)) || (rc = ensure_device(net)) || (rc = ensure_coef(net, st))) return rc;
     if (q) CU(launch_permute_vec(net->d_reach_of_pos, q, net->d_qtmp, net->topo.n, st));
-    return run_one_step(net, O, I, M, q ? net->d_qtmp : nullptr, st);
+    return run_routing(net, O, I, M, q ? net->d_qtmp : nullptr, nullptr, 0, StepPlan(), 1, st);
 }
 
 int txh_route_step_levels(txh_net* net, double* O, double* I, int64_t M, const double* q, void* stream)
@@ -1238,7 +1175,7 @@ int txh_route_apply(txh_net* net, double* X, double* Iscr, int64_t M, void* stre
     // nutils.py:148-154: i_prev = init_inflows(o_prev) (self-loop included), then _ax
     CU(launch_init_inflows(net->d_up_off, net->d_up_pos, net->d_outlet, X, Iscr, net->topo.n,
                            (int)txh_row_stride(M), (int)M, st));
-    return run_one_step(net, X, Iscr, M, nullptr, st);
+    return run_routing(net, X, Iscr, M, nullptr, nullptr, 0, StepPlan(), 1, st);
 }
 
 int txh_apply_gain(txh_net* net, const double* G, double* O, double* I, int64_t M, void* stream)
@@ -1275,11 +1212,8 @@ int obs_positions(txh_net* net, const int64_t* obs, int64_t m, cudaStream_t st, 
         if (k > 0 && obs[k] <= obs[k - 1]) return fail(TXH_E_INVALID, "gauge reach indices must be strictly ascending");
         pos[k] = net->sched.pos_of_reach[obs[k]];
     }
-    if ((size_t)m > net->obs_cap) {
-        if (net->d_obs) CU(cudaFree(net->d_obs));
-        CU(cudaMalloc((void**)&net->d_obs, sizeof(int32_t) * m));
-        net->obs_cap = m;
-    }
+    int rc;
+    if ((rc = grow(&net->d_obs, &net->obs_cap, (size_t)m, st))) return rc;
     std::vector<int32_t> gop(net->topo.n, -1);
     for (int64_t k = 0; k < m; ++k) gop[pos[k]] = (int32_t)k;
     if (!net->d_gauge_of_pos) CU(cudaMalloc((void**)&net->d_gauge_of_pos, sizeof(int32_t) * net->topo.n));
@@ -1308,11 +1242,7 @@ int obs_positions(txh_net* net, const int64_t* obs, int64_t m, cudaStream_t st, 
     if (fix_ok)
         for (size_t k = 0; k < ntask; ++k) { gfix.insert(gfix.end(), per_task[k].begin(), per_task[k].end()); goff[k + 1] = (int32_t)gfix.size(); }
     if (!net->d_gfix_off) CU(cudaMalloc((void**)&net->d_gfix_off, sizeof(int32_t) * (ntask + 1)));
-    if (gfix.size() > net->gfix_cap || !net->d_gfix) {
-        if (net->d_gfix) CU(cudaFree(net->d_gfix));
-        net->gfix_cap = std::max<size_t>(gfix.size(), 16);
-        CU(cudaMalloc((void**)&net->d_gfix, sizeof(int2) * net->gfix_cap));
-    }
+    if ((rc = grow(&net->d_gfix, &net->gfix_cap, std::max<size_t>(gfix.size(), 16), st))) return rc;
     net->gfix_ok = fix_ok;
     CU(cudaMemcpyAsync(net->d_gfix_off, goff.data(), sizeof(int32_t) * (ntask + 1), cudaMemcpyHostToDevice, st));
     if (!gfix.empty()) CU(cudaMemcpyAsync(net->d_gfix, gfix.data(), sizeof(int2) * gfix.size(), cudaMemcpyHostToDevice, st));
@@ -1509,9 +1439,17 @@ int txh_run_assimilating_rec(txh_net* net, double* O, double* I, int64_t M, cons
         return fail(TXH_E_INVALID, "bad recording arguments");
     if (net->T_hist && (nsteps / every) * M * M > net->T_hist_cap)
         return fail(TXH_E_INVALID, "the transform history holds fewer than nsteps / every transforms of M x M");
-    if (rec_count > 0) {
-        if (fo && fo->net != net) return fail(TXH_E_INVALID, "forcing belongs to another network");
-        if (check_M(M)) return TXH_E_INVALID;
+    // segments: nwin windows of `every` steps, each followed by an update, then the remaining steps
+    const int64_t nwin = nsteps / every, nseg = nwin + (nsteps > nwin * every ? 1 : 0);
+    auto seg_steps = [&](int64_t k) { return k < nwin ? every : nsteps - nwin * every; };
+    // the checks txh_route_run makes of every routing call
+    if (nwin > 0 && every > (1 << 24)) return fail(TXH_E_INVALID, "nsteps out of range");
+    if (fo && fo->net != net) return fail(TXH_E_INVALID, "forcing belongs to another network");
+    if (fo && fo->d_W && fo->M != M) return fail(TXH_E_INVALID, "forcing member multipliers do not match M");
+    int rc;
+    if ((rc = check_M(M))) return rc;
+    const bool rec = rec_count > 0;
+    if (rec) {
         std::vector<char> seen(net->topo.n, 0);
         for (int64_t k = 0; k < rec_count; ++k) {
             if (rec_reach[k] < 0 || rec_reach[k] >= net->topo.n) return fail(TXH_E_INVALID, "recorded reach out of range");
@@ -1519,127 +1457,78 @@ int txh_run_assimilating_rec(txh_net* net, double* O, double* I, int64_t M, cons
         }
     }
     cudaStream_t st = (cudaStream_t)stream;
-    double* const rowsum_before = net->stats_rowsum;
-    const double scale_before = net->stats_scale;
-    int rc = txh_set_stats_output(net, rowsum, 1.0 / (double)M);
-    const int64_t nwin = nsteps / every;
-    int64_t t = t0_ns;
+    if ((rc = ensure_device(net)) || (rc = ensure_coef(net, st))) return rc;
+    if (rec) {
+        // the slots and positions of the recorded reaches once per call
+        if ((rc = upload_rec_slots(net, rec_reach, rec_count, st)) ||
+            (rc = grow(&net->d_rec_pos, &net->rec_pos_cap, (size_t)rec_count, st)))
+            return rc;
+        std::vector<int32_t> pos(rec_count);
+        for (int64_t k = 0; k < rec_count; ++k) pos[k] = net->sched.pos_of_reach[rec_reach[k]];
+        CU(cudaMemcpyAsync(net->d_rec_pos, pos.data(), sizeof(int32_t) * rec_count, cudaMemcpyHostToDevice, st));
+        CU(cudaStreamSynchronize(st));
+    }
     const int ld = (int)txh_row_stride(M);
+    // where update k's transform goes and where its consumers read it
+    auto T_of = [&](int64_t k) -> double* { return net->T_hist ? net->T_hist + (size_t)k * M * M : T; };
+    // where update k's recorded rows go: the forecast to prior_out[k], the posterior -- what the state holds after step
+    // (k+1) every -- to that step's rec_out slot (the routing launch recorded the forecast there)
+    auto rec_prior_of = [&](int64_t k) -> double* {
+        return rec && prior_out ? prior_out + (size_t)k * rec_count * M : nullptr;
+    };
+    auto rec_post_of = [&](int64_t k) -> double* {
+        const int64_t s_end = (k + 1) * every;
+        return rec && s_end % rec_every == 0 ? rec_out + (size_t)(s_end / rec_every - 1) * rec_count * M : nullptr;
+    };
     // Right after a routing launch the forecast inflows are exactly the sums of the upstream forecast outflows
     // (nutils.py:84-85), so i + N gain = N (o + gain): the gains are never stored.  When the window kernel routes the
-    // next window, it applies the update itself while it loads its tasks (p is linear in the state rows, txh_window.cu):
+    // next segment, it applies the update itself while it loads its tasks (p is linear in the state rows, txh_window.cu):
     // the posterior state only goes to memory after the last window; otherwise the transform kernel updates O in place
     // and the posterior inflows are rebuilt from the posterior outflows.
     static const bool fuse_load_ok = [] { const char* k = getenv("TXH_ENKF_FUSE_LOAD"); return !(k && atoi(k) == 0); }();
-    bool fuse_load = false;
-    if (rc == TXH_OK && fuse_load_ok && ld <= kMemberBlock && (rc = ensure_device(net)) == TXH_OK)
-        fuse_load = (net->route_kernel == 0 || net->route_kernel == 2) && !lane_wanted(net, M, every) &&
-                    run_window(net, O, I, M, nullptr, nullptr, 0, StepPlan(), every, st, true) == TXH_OK;
-    // recording: the slots once per call; after update k (step (k+1) every) the forecast rows go to prior_out[k] and the
-    // posterior ones -- what the state holds after that step -- to their rec_out slot (the window kernel recorded the
-    // forecast there).  In every path O still holds the forecast when enkf_record runs.
-    const bool rec = rec_count > 0;
-    // where update k's transform goes and where its consumers read it
-    auto T_of = [&](int64_t k) -> double* { return net->T_hist ? net->T_hist + (size_t)k * M * M : T; };
-    if (rc == TXH_OK && rec) {
-        // (the arguments were checked above; the routing calls below go past txh_route_run's checks)
-        rc = ensure_device(net);
-        if (rc == TXH_OK) rc = ensure_coef(net, st);
-        if (rc == TXH_OK) rc = upload_rec_slots(net, rec_reach, rec_count, st);
-        if (rc == TXH_OK && (size_t)rec_count > net->rec_pos_cap) {
-            if (net->d_rec_pos) CU(cudaFree(net->d_rec_pos));
-            CU(cudaMalloc((void**)&net->d_rec_pos, sizeof(int32_t) * rec_count));
-            net->rec_pos_cap = (size_t)rec_count;
-        }
-        if (rc == TXH_OK) {
-            std::vector<int32_t> pos(rec_count);
-            for (int64_t k = 0; k < rec_count; ++k) pos[k] = net->sched.pos_of_reach[rec_reach[k]];
-            CU(cudaMemcpyAsync(net->d_rec_pos, pos.data(), sizeof(int32_t) * rec_count, cudaMemcpyHostToDevice, st));
-            CU(cudaStreamSynchronize(st));
-        }
-    }
-    const int32_t* rec_slot = rec ? net->d_rec_slot : nullptr;
-    // where update k's recorded rows go: the forecast to prior_out[k], the posterior to the slot of step (k+1) every
-    auto rec_prior_of = [&](int64_t k) -> double* { return prior_out ? prior_out + (size_t)k * rec_count * M : nullptr; };
-    auto rec_post_of = [&](int64_t k) -> double* {
-        const int64_t s_end = (k + 1) * every;
-        return s_end % rec_every == 0 ? rec_out + (size_t)(s_end / rec_every - 1) * rec_count * M : nullptr;
-    };
+    const WindowFit fit = window_fit(net, M);
+    const bool fuse_load = fuse_load_ok && ld <= kMemberBlock && (net->route_kernel == 0 || net->route_kernel == 2) &&
+                           !lane_wanted(net, M, every) && fit.ok && fit.wpc_upd >= 2;
     // update k applied by the stand-alone kernels: its rows recorded first, while O still holds the forecast
-    auto record_update = [&](int64_t k) -> int {
+    auto apply_update = [&](int64_t k) -> int {
         double *prior = rec_prior_of(k), *post = rec_post_of(k);
-        if (rec && (post || prior))
+        if (prior || post)
             CU(launch_enkf_record(O, ld, (int)M, rowsum, T_of(k), net->d_gauge_of_pos, qs, W, net->d_rec_pos, (int)rec_count,
                                   prior, post, st));
-        return TXH_OK;
-    };
-    // update k applied by the next window launch while it loads its tasks: that launch records its rows
-    auto set_pending = [&](int64_t k) {
-        net->pending.T = T_of(k); net->pending.W = W; net->pending.qs = qs; net->pending.M = M;
-        net->pending.rec_prior = rec ? rec_prior_of(k) : nullptr;
-        net->pending.rec_post = rec ? rec_post_of(k) : nullptr;
-        net->pending.rec_mean = rowsum;
-    };
-    bool owed = false;                                     // an update computed (T, W) but not yet applied to O, I
-    int64_t owed_k = 0;                                    // ... and which one
-    auto apply_owed = [&]() -> int {
-        int rc2 = record_update(owed_k);
-        if (rc2 != TXH_OK) return rc2;
-        CU(launch_enkf_update(O, ld, (int)M, rowsum, T_of(owed_k), (int)M, (int)M, O, nullptr, ld, net->topo.n, net->d_gauge_of_pos,
+        if (ld > kMemberBlock) return txh_enkf_apply(net, O, I, M, nullptr, 0, 0, M, 0, rowsum, T_of(k), obs, m, qs, W, G, stream);
+        CU(launch_enkf_update(O, ld, (int)M, rowsum, T_of(k), (int)M, (int)M, O, nullptr, ld, net->topo.n, net->d_gauge_of_pos,
                               qs, W, 0, net->num_sms, (int)M, 0, st));
         CU(launch_inflow_rebuild(net->d_inner_rec, net->n_inner, net->d_up_off, net->d_up_pos, O, I, ld, st));
-        owed = false;
         return TXH_OK;
     };
-    for (int64_t k = 0; k < nwin && rc == TXH_OK; ++k) {
+    OwedUpdate owed{};                                     // the update the next routing launch applies, if handed over
+    bool handed_over = false;
+    int64_t t = t0_ns;
+    for (int64_t k = 0; k < nseg; ++k) {
         cudaEvent_t e0 = nullptr, e1 = nullptr;
-        const bool timed = time_every > 0 && k % time_every == 0 && net->route_events.size() < 4096;
+        const bool timed = k < nwin && time_every > 0 && k % time_every == 0 && net->route_events.size() < 4096;
         if (timed) { CU(cudaEventCreate(&e0)); CU(cudaEventCreate(&e1)); CU(cudaEventRecord(e0, st)); }
-        if (owed) {
-            if (net->gfix_ok) set_pending(owed_k);
-            else rc = apply_owed();
-        }
-        if (rc == TXH_OK) rc = rec ? route_run_impl(net, O, I, M, fo, t, dt_ns, every, method, rec_slot, rec_count, rec_every,
-                                                    rec_out, k * every, st)
-                                   : txh_route_run(net, O, I, M, fo, t, dt_ns, every, method, nullptr, 0, 1, nullptr, stream);
-        if (rc == TXH_OK && owed) {
-            if (net->pending.T) { net->pending.T = nullptr; rc = fail(TXH_E_STATE, "the routing launch did not take the pending ensemble update"); }
-            owed = false;
-        }
+        const Recording rk = rec ? Recording{net->d_rec_slot, rec_out, (int)rec_every, (int)rec_count, k * every} : Recording();
+        // the row sums of the forecast ride on the last step of every window (the mean of the update)
+        rc = route_run_impl(net, O, I, M, fo, t, dt_ns, seg_steps(k), method, rk, k < nwin ? rowsum : nullptr,
+                            1.0 / (double)M, handed_over ? &owed : nullptr, st);
         if (timed) { CU(cudaEventRecord(e1, st)); net->route_events.emplace_back(e0, e1); }
+        if (rc != TXH_OK) return rc;
+        if (k == nwin) break;                              // the remaining steps: no update follows
         t += every * dt_ns;
         // observations still on their way (copied on another stream): the first update waits for them, the first
         // window does not
         if (k == 0 && obs_ready_event) CU(cudaStreamWaitEvent(st, (cudaEvent_t)obs_ready_event, 0));
-        if (rc == TXH_OK) rc = check_M(M);
-        if (rc == TXH_OK) rc = enkf_solve_impl(net, m, M, HX, O, Zp + (size_t)k * m * M, rowsum, obs, qs, R, Dinv, dinv_kind, work, W,
-                                                  T_of(k), stream);
-        if (rc != TXH_OK) break;
-        if (ld <= kMemberBlock) {
-            owed = true; owed_k = k;
-            if (!fuse_load) rc = apply_owed();
-        } else {
-            rc = record_update(k);
-            if (rc == TXH_OK) rc = txh_enkf_apply(net, O, I, M, nullptr, 0, 0, M, 0, rowsum, T_of(k), obs, m, qs, W, G, stream);
-        }
+        if ((rc = enkf_solve_impl(net, m, M, HX, O, Zp + (size_t)k * m * M, rowsum, obs, qs, R, Dinv, dinv_kind, work, W,
+                                  T_of(k), stream)))
+            return rc;
+        // the update rides on the next routing launch when that is a window launch with room for it (and every gauge
+        // term falls in a window task); otherwise, and after the last segment, the stand-alone kernels apply it now
+        handed_over = fuse_load && k + 1 < nseg && net->gfix_ok && !lane_wanted(net, M, seg_steps(k + 1));
+        if (handed_over) owed = OwedUpdate{T_of(k), W, qs, M, rec_prior_of(k), rec_post_of(k), rowsum};
+        else if ((rc = apply_update(k))) return rc;
     }
-    net->stats_rowsum = nullptr;
-    if (rc == TXH_OK && nsteps > nwin * every) {
-        if (owed && net->gfix_ok && !lane_wanted(net, M, nsteps - nwin * every)) set_pending(owed_k);
-        else if (owed) rc = apply_owed();
-        if (rc == TXH_OK)
-            rc = rec ? route_run_impl(net, O, I, M, fo, t, dt_ns, nsteps - nwin * every, method, rec_slot, rec_count, rec_every,
-                                      rec_out, nwin * every, st)
-                     : txh_route_run(net, O, I, M, fo, t, dt_ns, nsteps - nwin * every, method, nullptr, 0, 1, nullptr, stream);
-        if (rc == TXH_OK && owed) {
-            if (net->pending.T) { net->pending.T = nullptr; rc = fail(TXH_E_STATE, "the routing launch did not take the pending ensemble update"); }
-            owed = false;
-        }
-    }
-    if (rc == TXH_OK && owed) rc = apply_owed();           // after the last window the posterior goes to memory
-    net->pending.T = nullptr; net->pending.rec_prior = net->pending.rec_post = nullptr;
-    net->stats_rowsum = rowsum_before; net->stats_scale = scale_before;
-    return rc;
+    return TXH_OK;
 }
 
 int txh_set_transform_history(txh_net* net, double* T_hist, int64_t capacity)
@@ -1767,10 +1656,10 @@ int txh_kf_filter(txh_net* net, const double* P_in, double* P_out, double* P_pri
     // P- = A (A P)^T + Q, nutils.py:194-214 (X2 doubles as the inflow scratch of the first pass and vice versa)
     CU(launch_pack(net->d_reach_of_pos, P_in, X, n, (int)n, ld, 0, st));
     CU(launch_init_inflows(net->d_up_off, net->d_up_pos, net->d_outlet, X, X2, n, ld, (int)n, st));
-    if ((rc = run_one_step(net, X, X2, n, nullptr, st))) return rc;
+    if ((rc = run_routing(net, X, X2, n, nullptr, nullptr, 0, StepPlan(), 1, st))) return rc;
     CU(launch_kf_repack_transposed(net->d_reach_of_pos, net->d_pos_of_reach, X, X2, (int)n, ld, st));
     CU(launch_init_inflows(net->d_up_off, net->d_up_pos, net->d_outlet, X2, X, n, ld, (int)n, st));
-    if ((rc = run_one_step(net, X2, X, n, nullptr, st))) return rc;
+    if ((rc = run_routing(net, X2, X, n, nullptr, nullptr, 0, StepPlan(), 1, st))) return rc;
     CU(launch_kf_prior_finish(net->d_reach_of_pos, net->d_pos_of_reach, net->d_gauge_of_pos, X2, ld, Q, R, (int)n, (int)m,
                               Pm, Ps, Prow, S, st));
     // K = P-[:, s] inv(P-[s][:, s] + R)   (da.py:119)
@@ -1928,10 +1817,10 @@ int txh_kfb_filter(txh_kfb* b, const uint8_t* active, const double* z_host, doub
     // P- = A (A P)^T + Q for every block at once: the blocks' columns are the members of two routing launches
     CU(launch_kfb_pack(b->d_blocks, b->d_blk_of_reach, net->d_pos_of_reach, b->d_P, b->d_X, n_u, ld, st));
     CU(launch_init_inflows(net->d_up_off, net->d_up_pos, net->d_outlet, b->d_X, b->d_X2, n_u, ld, M, st));
-    if ((rc = run_one_step(net, b->d_X, b->d_X2, M, nullptr, st))) return rc;
+    if ((rc = run_routing(net, b->d_X, b->d_X2, M, nullptr, nullptr, 0, StepPlan(), 1, st))) return rc;
     CU(launch_kfb_transpose(b->d_blocks, b->d_blk_of_reach, net->d_pos_of_reach, b->d_X, b->d_X2, n_u, ld, st));
     CU(launch_init_inflows(net->d_up_off, net->d_up_pos, net->d_outlet, b->d_X2, b->d_X, n_u, ld, M, st));
-    if ((rc = run_one_step(net, b->d_X2, b->d_X, M, nullptr, st))) return rc;
+    if ((rc = run_routing(net, b->d_X2, b->d_X, M, nullptr, nullptr, 0, StepPlan(), 1, st))) return rc;
     CU(launch_kfb_update(b->d_blocks, (int)b->blocks.size(), b->max_m, b->d_blk_of_reach, net->d_pos_of_reach, b->d_gl_of_reach,
                          b->d_obs_reach, b->d_X2, n_u, ld, b->d_Q, b->d_R, b->d_z, O, (int)txh_row_stride(1), b->d_Pm, b->d_Ps,
                          b->d_Prow, b->d_S, b->d_K, b->d_dz, b->d_gain, b->d_Gp, b->d_P, info_word(net), st));
