@@ -276,7 +276,7 @@ int txh_enks_smooth(int64_t M, int64_t nupd, int64_t every, const double* T_hist
                     int64_t rec_every, int64_t lag, const double* rec_dev, double* out_dev, double* work_dev, void* stream);
 
 /* Dense products of KalmanFilter.filter for small n (da.py:115-122): C = alpha op(A) op(B) + beta C,
- * row-major FP64 on the tensor cores (mma.sync m8n8k4 = DMMA). */
+ * row-major FP64 on the tensor cores (mma.sync m8n8k4 = DMMA).  With K = 0, A and B are not read and may be null. */
 int txh_dgemm(int transA, int transB, int64_t M, int64_t N, int64_t K, double alpha, const double* A_dev,
               int64_t lda, const double* B_dev, int64_t ldb, double beta, double* C_dev, int64_t ldc, void* stream);
 /* In-place Cholesky solve S X = B for SPD S [m][m] (destroyed), B [m][k] -> X.  Synchronous;
@@ -310,8 +310,11 @@ int txh_kf_filter(txh_net* net, const double* P_in, double* P_out, double* P_pri
  * which (txh_kfb_set / _get): 0 P (posterior), 1 Q, 2 R -- settable -- 3 P before the last update, 4 K [n][m], 5 dz [m],
  * 6 gain [n]; matrices row-major in the block's local reach / gauge order.
  * txh_kfb_filter: active[k] = 0 leaves block k alone (its filter is not due, da.py:49-61); z_host: the measurement
- * vectors of all blocks concatenated; O, I: state rows of the UNION model (M = 1).  Asynchronous after its copies. */
+ * vectors of all blocks concatenated; O, I: state rows of the UNION model (M = 1).  Asynchronous after its copies.
+ * A block that is not due keeps P, P before its last update, K, dz and gain.
+ * txh_kfb_max_gauges: the most gauges a block may have (its inverse runs in shared memory); txh_kfb_create refuses more. */
 typedef struct txh_kfb txh_kfb;
+int64_t txh_kfb_max_gauges(void);
 int txh_kfb_create(txh_net* union_net, int64_t nblocks, const int64_t* n_k, const int64_t* m_k, const int64_t* obs_local,
                    txh_kfb** out);
 void txh_kfb_destroy(txh_kfb* b);

@@ -89,6 +89,7 @@ SIGNATURES = {
     "txh_kf_work_size": (c_i64, [c_vp, c_i64]),
     "txh_kf_filter": (ctypes.c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, p_i64, c_i64, p_f64, c_vp, c_vp, c_vp,
                                      c_vp, c_vp, c_vp, c_vp]),
+    "txh_kfb_max_gauges": (c_i64, []),
     "txh_kfb_create": (ctypes.c_int, [c_vp, c_i64, p_i64, p_i64, p_i64, ctypes.POINTER(c_vp)]),
     "txh_kfb_destroy": (None, [c_vp]),
     "txh_kfb_set": (ctypes.c_int, [c_vp, c_i64, ctypes.c_int, p_f64, c_vp]),

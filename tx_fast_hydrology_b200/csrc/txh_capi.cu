@@ -1579,7 +1579,8 @@ int txh_get_route_timings(txh_net* net, double* ms_out, int64_t capacity, int64_
 int txh_dgemm(int transA, int transB, int64_t M, int64_t N, int64_t K, double alpha, const double* A, int64_t lda,
               const double* B, int64_t ldb, double beta, double* C, int64_t ldc, void* stream)
 {
-    if (!A || !B || !C || M < 0 || N < 0 || K < 0) return fail(TXH_E_INVALID, "bad argument");
+    // K = 0: A and B are never read (C = beta C), so empty operands may come without an address
+    if ((K > 0 && (!A || !B)) || !C || M < 0 || N < 0 || K < 0) return fail(TXH_E_INVALID, "bad argument");
     if (txh_device_count() == 0) return fail(TXH_E_NODEVICE, "no CUDA device visible: libtxh has no CPU fallback");
     CU(launch_dgemm(transA, transB, (int)M, (int)N, (int)K, alpha, A, (int)lda, B, (int)ldb, beta, C, (int)ldc,
                     (cudaStream_t)stream));
@@ -1690,6 +1691,14 @@ struct txh_kfb {
 
 extern "C" {
 
+// kfb_inverse_kernel holds a block's m x m system and four m-vectors in 200 KB of shared memory
+int64_t txh_kfb_max_gauges(void)
+{
+    int64_t m = 0;
+    while ((size_t)4 * (m + 1) + (size_t)(m + 1) * (m + 1) <= 200 * 1024 / sizeof(double)) ++m;
+    return m;
+}
+
 int txh_kfb_create(txh_net* net, int64_t nblocks, const int64_t* n_k, const int64_t* m_k, const int64_t* obs_local, txh_kfb** out)
 {
     if (!net || !n_k || !m_k || !obs_local || !out || nblocks < 1) return fail(TXH_E_INVALID, "bad argument");
@@ -1722,7 +1731,7 @@ int txh_kfb_create(txh_net* net, int64_t nblocks, const int64_t* n_k, const int6
         row0 += n_k[k]; g0 += m_k[k];
     }
     if (row0 != net->topo.n) { delete b; return fail(TXH_E_INVALID, "block sizes do not add up to the union network"); }
-    if ((size_t)4 * b->max_m + (size_t)b->max_m * b->max_m > 200 * 1024 / sizeof(double)) {
+    if (b->max_m > txh_kfb_max_gauges()) {
         delete b; return fail(TXH_E_INVALID, "a block has too many gauges for the batched inverse");
     }
     b->n_u = row0; b->m_tot = g0;
@@ -1812,7 +1821,11 @@ int txh_kfb_filter(txh_kfb* b, const uint8_t* active, const double* z_host, doub
         CU(cudaStreamSynchronize(st));
     }
     CU(cudaMemcpyAsync(b->d_z, z_host, sizeof(double) * b->m_tot, cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(b->d_Pprev, b->d_P, sizeof(double) * b->pp, cudaMemcpyDeviceToDevice, st));
+    // P before this update, for the blocks it updates; a block that is not due keeps the P before its last one
+    for (const KfbBlock& k : b->blocks)
+        if (k.active)
+            CU(cudaMemcpyAsync(b->d_Pprev + k.p_off, b->d_P + k.p_off, sizeof(double) * k.n * k.n,
+                               cudaMemcpyDeviceToDevice, st));
     const int n_u = (int)b->n_u, ld = b->ld, M = b->max_n;
     // P- = A (A P)^T + Q for every block at once: the blocks' columns are the members of two routing launches
     CU(launch_kfb_pack(b->d_blocks, b->d_blk_of_reach, net->d_pos_of_reach, b->d_P, b->d_X, n_u, ld, st));

@@ -234,7 +234,8 @@ kfb_inverse_kernel(const KfbBlock* __restrict__ blocks, double* __restrict__ S, 
     inverse_in_cta(S + b.mm_off, b.m, 1, info, sm);
 }
 
-// per reach: K_k[j][:] = P-_k[j, s] S_k^-1 (da.py:119), gain = K dz with dz = z - o[s] (da.py:112, 121)
+// per reach: K_k[j][:] = P-_k[j, s] S_k^-1 (da.py:119), gain = K dz with dz = z - o[s] (da.py:112, 121).
+// An inactive block adds a zero gain to the state and keeps K, dz and gain of its last update.
 __global__ void __launch_bounds__(128)
 kfb_gain_kernel(const KfbBlock* __restrict__ blocks, const int32_t* __restrict__ blk_of_reach,
                 const int32_t* __restrict__ pos_of_reach, const int32_t* __restrict__ obs_reach, const double* __restrict__ z,
@@ -258,8 +259,8 @@ kfb_gain_kernel(const KfbBlock* __restrict__ blocks, const int32_t* __restrict__
             if (j == 0) dz[b.g_off + q] = d;
             g += kq * d;
         }
+        gain[r] = g;
     }
-    gain[r] = g;
     Gp[gp] = g;
     for (int c = 1; c < ldo; ++c) Gp[gp + c] = 0.0;
 }

@@ -579,6 +579,7 @@ class BatchedKalmanFilters:
                 a = L.as_f64(t.cpu().numpy())
                 L.check(lib.txh_kfb_set(h, k, which, L.ptr_f64(a), None))
         self.n_updates = 0
+        self._ran = np.zeros(len(self.filters), dtype=bool)     # the filters that have updated at least once
 
     def close(self):
         if getattr(self, 'handle', None):
@@ -613,7 +614,7 @@ class BatchedKalmanFilters:
                                                self._L.ptr_f64(self._L.as_f64(z)), _cuda_ptr(d['O']), _cuda_ptr(d['I']),
                                                _stream_ptr()))
         u._device_advanced()
-        self._last_active = active
+        self._ran |= active.astype(bool)
         for kf, a in zip(self.filters, active):
             if a:
                 kf.datetime = u.datetime
@@ -631,7 +632,6 @@ class BatchedKalmanFilters:
         times = index.astype(int).astype(float).values
         table = np.ascontiguousarray(np.concatenate([f.values for f in frames], axis=1), dtype=np.float64)
         end_time = index.max()
-        self._last_active = np.zeros(len(self.filters), dtype=np.uint8)
         torch = self._torch
         nsteps = 0 if not end_time > u.datetime else int(-((u.datetime - end_time) // u.timedelta))
         # the hydrographs are recorded on the device (one unpack launch per step, no host round trip in the loop)
@@ -668,8 +668,8 @@ class BatchedKalmanFilters:
             m.datetime = u.datetime
             n, mm = m.n, kf.num_measurements
             kf._P = torch.as_tensor(self._get(k, 0, (n, n)), device='cuda')
-            kf._P_prev = torch.as_tensor(self._get(k, 3, (n, n)), device='cuda')
-            if kf.datetime == u.datetime or self._last_active[k]:
+            if self._ran[k]:                     # P before, K, dz and gain of its last update, as the per-model path
+                kf._P_prev = torch.as_tensor(self._get(k, 3, (n, n)), device='cuda')
                 kf._K_d = torch.as_tensor(self._get(k, 4, (n, mm)), device='cuda')
                 kf._dz_d = torch.as_tensor(self._get(k, 5, (mm,)), device='cuda')
                 kf._gain_d = torch.as_tensor(self._get(k, 6, (n,)), device='cuda')

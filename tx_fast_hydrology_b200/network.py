@@ -451,11 +451,35 @@ class RiverNetwork:
             return False
 
 
+def _check_matrix(name, t, rows=None, cols=None, contiguous=False):
+    """Raw device pointers cross the C ABI below: a matrix must be a 2-D float64 CUDA tensor of the expected shape
+    whose rows are contiguous (row-major with a leading dimension); `contiguous` also rules out a leading dimension
+    wider than a row."""
+    import torch
+    if not isinstance(t, torch.Tensor) or t.dim() != 2:
+        raise ValueError(f'`{name}` must be a 2-D tensor')
+    if (rows is not None and t.shape[0] != rows) or (cols is not None and t.shape[1] != cols):
+        raise ValueError(f'`{name}` must be ({rows}, {cols}), got {tuple(t.shape)}')
+    if t.numel() and ((t.shape[1] > 1 and t.stride(1) != 1) or (t.shape[0] > 1 and t.stride(0) < t.shape[1])):
+        raise ValueError(f'`{name}` must be row-major with contiguous rows, got strides {t.stride()}')
+    if contiguous and not t.is_contiguous():
+        raise ValueError(f'`{name}` must be contiguous')
+    if t.dtype != torch.float64:
+        raise ValueError(f'`{name}` must be float64, got {t.dtype}')
+    if not t.is_cuda:
+        raise ValueError(f'`{name}` must be a CUDA tensor')
+
+
 def dgemm(A, B, C, transA=False, transB=False, alpha=1.0, beta=0.0):
-    """C = alpha op(A) op(B) + beta C on the FP64 tensor cores (row-major CUDA tensors, float64)."""
-    lib = L.load()
+    """C = alpha op(A) op(B) + beta C on the FP64 tensor cores (row-major CUDA tensors, float64; a row slice such as
+    X[:, :k] is fine, a transposed view is not: pass the transpose flag instead)."""
+    _check_matrix('C', C)
     M, N = C.shape
+    _check_matrix('A', A)
     K = A.shape[0] if transA else A.shape[1]
+    _check_matrix('A', A, *((K, M) if transA else (M, K)))
+    _check_matrix('B', B, *((N, K) if transB else (K, N)))
+    lib = L.load()
     L.check(lib.txh_dgemm(int(transA), int(transB), M, N, K, float(alpha), _cuda_ptr(A), A.stride(0),
                           _cuda_ptr(B), B.stride(0), float(beta), _cuda_ptr(C), C.stride(0), _stream_ptr()))
     return C
@@ -463,13 +487,20 @@ def dgemm(A, B, C, transA=False, transB=False, alpha=1.0, beta=0.0):
 
 def spd_solve(S, B):
     """In place: B <- S^-1 B for SPD S (S is overwritten by its Cholesky factor)."""
-    L.check(L.load().txh_spd_solve(S.shape[0], B.shape[1], _cuda_ptr(S), _cuda_ptr(B), _stream_ptr()))
+    _check_matrix('S', S, contiguous=True)
+    m = S.shape[0]
+    _check_matrix('S', S, m, m, contiguous=True)
+    _check_matrix('B', B, m, None, contiguous=True)
+    L.check(L.load().txh_spd_solve(m, B.shape[1], _cuda_ptr(S), _cuda_ptr(B), _stream_ptr()))
     return B
 
 
 def inverse(A):
     """In place: A <- inv(A), Gauss-Jordan with partial pivoting."""
     import torch
+    _check_matrix('A', A, contiguous=True)
+    m = A.shape[0]
+    _check_matrix('A', A, m, m, contiguous=True)
     work = torch.empty_like(A)
-    L.check(L.load().txh_inverse(A.shape[0], _cuda_ptr(A), _cuda_ptr(work), _stream_ptr()))
+    L.check(L.load().txh_inverse(m, _cuda_ptr(A), _cuda_ptr(work), _stream_ptr()))
     return A

@@ -95,13 +95,18 @@ class AsyncSimulation(Simulation):
 
     def _batchable(self, names):
         """The ready sub-models whose filters can run as ONE chain of launches (da.BatchedKalmanFilters): a single
-        plain KalmanFilter callback, one member, a whole-second step, the same clock and forcing index."""
+        plain KalmanFilter callback with no more gauges than a batched block takes, one member, a whole-second step,
+        the same clock and forcing index."""
+        from . import _lib
         from .da import KalmanFilter
+        max_gauges = _lib.load().txh_kfb_max_gauges()
         out = []
         for name in names:
             m = self.models[name]
             cbs = list(m.callbacks.values())
             if len(cbs) != 1 or type(cbs[0]) is not KalmanFilter or m.members != 1:
+                continue
+            if cbs[0].num_measurements > max_gauges:
                 continue
             if m.timedelta.value != int(round(m.dt * 1e9)):
                 continue
