@@ -280,7 +280,8 @@ def test_forcing_update_in_place(torch_cuda, libtxh):
 def test_forcing_update_overlapped(torch_cuda, libtxh):
     """txh_forcing_update_async: the table arrives in row chunks on the handle's copy stream while routing calls
     that read only its first hours already run; window by window the result equals the synchronous upload.
-    (A 40 MB table: several chunks.)"""
+    (A 40 MB table: several chunks.)  The rows sit at irregular times off the step grid, so the rows a call waits
+    for come from the search of its last step, and the first pass interpolates the nearest row."""
     torch = torch_cuda
     from tx_fast_hydrology_b200 import synthetic as S
     from tx_fast_hydrology_b200.network import Forcing
@@ -290,6 +291,9 @@ def test_forcing_update_overlapped(torch_cuda, libtxh):
     net, _ = _setup(net_d["endnodes"], prm["K"], prm["X"], 300.0)
     t0 = 1_700_000_000 * 10**9
     times, table = S.make_forcing(n, every * nwin, 300.0, seed, t0_ns=t0)
+    # gaps of 1 s to 2 h (mean one hour) from 7 min before t0: some calls need no new row, some several
+    gaps = np.random.default_rng(seed).uniform(1.0 / 3600, 2.0, size=times.size - 1) * 3600 * 10**9
+    times = t0 - 420 * 10**9 + np.concatenate([[0], np.cumsum(gaps.astype(np.int64))])
     mul = S.make_member_multipliers(times.size, M, seed)
     tp = torch.from_numpy(np.ascontiguousarray(table)).pin_memory()
     mp = torch.from_numpy(np.ascontiguousarray(mul)).pin_memory()
@@ -297,14 +301,14 @@ def test_forcing_update_overlapped(torch_cuda, libtxh):
     o0 = prm["o_t"][:, None] * rng.uniform(0.5, 1.5, size=(n, M))
     f = Forcing(net, times, torch.zeros_like(tp), torch.ones_like(mp))
     g = Forcing(net, times, tp, mp)
-    for rep in range(2):                                   # the second pass re-uses the table while it may be in use
+    for rep, method in enumerate((0, 1)):                  # the second pass re-uses the table while it may be in use
         O, I = _upload(torch, net, o0, np.zeros_like(o0), M)
         O2, I2 = _upload(torch, net, o0, np.zeros_like(o0), M)
         f.update(times, tp, mp, overlap=True)
         for k in range(nwin):
-            net.route_run(O, I, M, f, t0 + k * every * int(300e9), int(300e9), every)
+            net.route_run(O, I, M, f, t0 + k * every * int(300e9), int(300e9), every, method=method)
         for k in range(nwin):
-            net.route_run(O2, I2, M, g, t0 + k * every * int(300e9), int(300e9), every)
+            net.route_run(O2, I2, M, g, t0 + k * every * int(300e9), int(300e9), every, method=method)
         net.check()
         assert torch.equal(O, O2) and torch.equal(I, I2)
     f.wait()

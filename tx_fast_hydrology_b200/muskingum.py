@@ -423,7 +423,10 @@ class Muskingum:
         launch: forcing interpolated on the device at t + dt, state updated in HBM, Python out
         of the loop.  Fires no per-step callbacks (bind-free fast path); returns the recorded
         outflows [nsteps // record_every][len(record_reaches)][members] as a CUDA tensor, or None.
-        `o_t_prev` / `i_t_prev` afterwards hold the state before the last step only if nsteps == 1."""
+        `o_t_prev` / `i_t_prev` afterwards hold the state before the last step only if nsteps == 1.
+        `method`: 'linear' or 'nearest' (the row interpolation of nutils.interpolate_sample)."""
+        if method not in ('linear', 'nearest'):
+            raise ValueError(f"`method` must be 'linear' or 'nearest', got {method!r}")
         torch = self._ensure_device()
         self._sync_coeffs()
         d, net, M = self._dev, self.network, self.members

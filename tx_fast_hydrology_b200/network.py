@@ -296,6 +296,9 @@ class RiverNetwork:
     # ---- routing ----------------------------------------------------------------------------
     def route_run(self, O, I, M, forcing, t0_ns, dt_ns, nsteps, method=1, rec_reach=None, rec_every=1,
                   rec_out=None):
+        """`method`: 1 linear, 0 nearest row (nutils.interpolate_sample)."""
+        if isinstance(method, bool) or method not in (0, 1):
+            raise ValueError(f"`method` must be 0 (nearest) or 1 (linear), got {method!r}")
         fh = forcing.handle if forcing is not None else None
         if rec_reach is not None:
             rr = L.as_i64(rec_reach)
