@@ -290,6 +290,7 @@ __device__ __forceinline__ double2 forcing_q(const FCtx& c, double g0, double g1
 struct Tk {
     unsigned sP, sScr, sIn, sRec, sCum, sCumC, sWords, sList;
     int len, n_in, nL, col, lane, begin, ld;
+    unsigned ldb;              // bytes of a ring row (ld doubles; a ring step stays below 4 GiB, see window_fit)
     bool active;
     double* Ig;
     double* Og;
@@ -316,54 +317,14 @@ __device__ __forceinline__ double2 forcing_add(const FCtx& c, double g0, double 
     return p;
 }
 
-// One row of a pocket step (see pocket_step)
-template <bool LAST, bool HAS_F, bool HAS_W, int IR, bool REC>
-__device__ __forceinline__ void pocket_row(const WinArgs& a, const Tk& tk, InStream& ist, const FCtx& fc, char* ringS,
-                                           const RowIn& x, double2& acc, unsigned& aW, unsigned aP, double* ig, double* og, int r,
-                                           int rj)
-{
-    const uint32_t h = x.h;
-    double2 inflow = (h & HDR_ACC) ? acc : make_double2(0.0, 0.0);
-    for (uint32_t k = (h >> 6) & 0x1ffffffu; k > 0; --k) {
-        const uint32_t w = lds_u32(aW);
-        aW += 4u;
-        const double2 v = (w & WIN_SLOT) ? stream_next<IR>(ist, a, tk.sIn, tk.sList, tk.nL, tk.step_bytes, tk.active, tk.lane)
-                                         : lds_row(tk.sScr + (w << 9));
-        inflow.x += v.x; inflow.y += v.y;
-    }
-    const double2 pq = forcing_add<HAS_F, HAS_W>(fc, x.g0, x.g1, x.p);
-    double2 on;
-    on.x = fma(x.al, inflow.x, pq.x);
-    on.y = fma(x.al, inflow.y, pq.y);
-    if (!LAST) {
-        double2 pn;
-        pn.x = x.be * inflow.x + x.ch * on.x;
-        pn.y = x.be * inflow.y + x.ch * on.y;
-        sts_row(aP, pn);
-    } else {
-        if (tk.active) { st_row(ig, inflow); st_row(og, on); }
-        if (a.rowsum) emit_rowsum(a, tk.begin + r, tk.col, on, tk.lane);
-    }
-    if (REC && rj >= 0) {
-        const int rs = rec_slot_of(tk, r);
-        if (rs >= 0) rec_store(a, rj, rs, tk.col, on);
-    }
-    if (h & (HDR_PUSH | 0x3eu)) {                               // published and / or parked in a scratch row
-        if (h & HDR_PUSH) {
-            const uint32_t slot = lds_u32(aW);
-            aW += 4u;
-            if (tk.active) st_row(reinterpret_cast<double*>(ringS + (size_t)slot * tk.ld * sizeof(double)), on);
-        }
-        const uint32_t sl = (h >> 1) & 31u;
-        if (sl) sts_row(tk.sScr + ((sl - 1u) << 9), on);
-    }
-    acc = on;
-}
-
-// One step of a pocket: depth-first walk, o' = alpha*inflow + (p + gamma q), p' = beta*inflow + chi*o'.  The record of
-// a row (RowIn) is read one row ahead of the arithmetic.  (Unrolling the walk by two rows with the two records
-// alternating removes the 17 register moves at the loop edge -- and was 8 % slower: the kernel is sensitive to its code
-// size.)
+// One step of a pocket: depth-first walk, o' = alpha*inflow + (p + gamma q), p' = beta*inflow + chi*o'.
+// Two thirds of the rows (C3) are leaves or chain rows: no input word, no push, at most a scratch row to park in.  One
+// test of the header skips the input loop for them, and the scratch store is predicated (profiles/r05_pocket_row_sass.txt:
+// 40 instructions per such row, 52 / 60 when the record was read one row ahead into registers of its own).  The record
+// of the next row is read into the registers each field of this row frees after its last use, so the loop edge moves
+// only the header instead of the whole record; the arithmetic of the row covers the latency of the loads.  (Unrolling
+// the walk by two rows instead was 8 % slower: the kernel is sensitive to its code size.)  Past the last row the loads
+// read the next area of the warp's shared memory and are not used.
 template <bool LAST, bool HAS_F, bool HAS_W, int IR, bool REC>
 __device__ __forceinline__ void pocket_step(const WinArgs& a, const Tk& tk, InStream& ist, const FCtx& fc, char* ringS,
                                             int rj)
@@ -372,12 +333,59 @@ __device__ __forceinline__ void pocket_step(const WinArgs& a, const Tk& tk, InSt
     double* ig = tk.Ig;
     double* og = tk.Og;
     double2 acc = make_double2(0.0, 0.0);
-    RowIn nx = load_rowin(aRec, aP);
+    RowIn x = load_rowin(aRec, aP);
     for (int r = 0; r < tk.len; ++r) {
-        const RowIn x = nx;
-        if (r + 1 < tk.len) nx = load_rowin(aRec + kRec, aP + 512u);
-        pocket_row<LAST, HAS_F, HAS_W, IR, REC>(a, tk, ist, fc, ringS, x, acc, aW, aP, ig, og, r, rj);
-        aRec += kRec; aP += 512u;
+        const uint32_t h = x.h;
+        const uint32_t park = h & 0x3eu;                         // (scratch row + 1) << 1 the outflow is parked in, 0: none
+        double2 inflow = (h & HDR_ACC) ? acc : make_double2(0.0, 0.0);
+        // the next row, whose record the loads below read (an opaque add: the old addresses die here)
+        asm("add.u32 %0, %0, %1;" : "+r"(aRec) : "n"(kRec));
+        asm("add.u32 %0, %0, 512;" : "+r"(aP));
+        if (h & ~0x3fu) {                                        // input words and / or a push
+            for (uint32_t k = (h >> 6) & 0x1ffffffu; k > 0; --k) {
+                const uint32_t w = lds_u32(aW);
+                aW += 4u;
+                const double2 v = (w & WIN_SLOT) ? stream_next<IR>(ist, a, tk.sIn, tk.sList, tk.nL, tk.step_bytes, tk.active, tk.lane)
+                                                 : lds_row(tk.sScr + (w << 9));
+                inflow.x += v.x; inflow.y += v.y;
+            }
+        }
+        const bool push = (h & HDR_PUSH) != 0u;
+        x.h = lds_u32(aRec);
+        const double2 pq = forcing_add<HAS_F, HAS_W>(fc, x.g0, x.g1, x.p);
+        {
+            const double2 g = lds_row(aRec + 32u);
+            x.g0 = g.x; x.g1 = g.y;
+            x.p = lds_row(aP);
+        }
+        double2 on;
+        on.x = fma(x.al, inflow.x, pq.x);
+        on.y = fma(x.al, inflow.y, pq.y);
+        x.al = lds_f64(aRec + 8u);
+        if (!LAST) {
+            double2 pn;
+            pn.x = x.be * inflow.x + x.ch * on.x;
+            pn.y = x.be * inflow.y + x.ch * on.y;
+            const double2 bc = lds_row(aRec + 16u);
+            x.be = bc.x; x.ch = bc.y;
+            sts_row(aP - 512u, pn);
+        } else {
+            const double2 bc = lds_row(aRec + 16u);
+            x.be = bc.x; x.ch = bc.y;
+            if (tk.active) { st_row(ig, inflow); st_row(og, on); }
+            if (a.rowsum) emit_rowsum(a, tk.begin + r, tk.col, on, tk.lane);
+        }
+        if (REC && rj >= 0) {
+            const int rs = rec_slot_of(tk, r);
+            if (rs >= 0) rec_store(a, rj, rs, tk.col, on);
+        }
+        if (push) {                                              // published: the slot word follows the inputs
+            const uint32_t slot = lds_u32(aW);
+            aW += 4u;
+            if (tk.active) st_row(reinterpret_cast<double*>(ringS + slot * tk.ldb), on);
+        }
+        if (park) sts_row(tk.sScr - 512u + (park << 8), on);
+        acc = on;
         ig += tk.ld; og += tk.ld;
     }
 }
@@ -625,7 +633,7 @@ route_window_kernel(const WinArgs a)
     tk.sP = sb + lane * 16u; tk.sScr = sb + a.off_scr + lane * 16u; tk.sIn = sb + a.off_in + lane * 16u;
     tk.sRec = sb + a.off_rec; tk.sCum = sb + a.off_cum; tk.sCumC = sb + a.off_cumc;
     tk.sWords = sb + a.off_words; tk.sList = sb + a.off_list;
-    tk.lane = lane; tk.ld = ld;
+    tk.lane = lane; tk.ld = ld; tk.ldb = (unsigned)ld * (unsigned)sizeof(double);
     tk.step_bytes = (size_t)a.n_slots * ld * sizeof(double);
     // bulk staging of the state rows (see the helpers above): one mbarrier per warp
     const bool bulk = a.off_mbar > 0 && ld == kMemberBlock;
