@@ -60,7 +60,7 @@ def run(name, net_d, M, nsteps, seed, parity_steps, parity_members, chunk=None):
     tc = time.time() - tc
     eo = float(np.abs(og - o_ref.T).max() / np.abs(o_ref).max()); ei = float(np.abs(ig - i_ref.T).max() / np.abs(i_ref).max())
     upd = float(n) * M * nsteps
-    extra = {k: os.environ[k] for k in ("TXH_ROUTE_KERNEL", "TXH_LANE_CAP", "TXH_LANE_SIDE_MIN", "TXH_LANE_MAX_M", "TXH_LANE_CTAS", "TXH_LANE_LAG") if k in os.environ}
+    extra = {k: os.environ[k] for k in ("TXH_ROUTE_KERNEL",) if k in os.environ}
     out = {"config": name, "env": extra, "reaches": n, "levels": nlev, "members": M, "steps": nsteps, "topology_pass_s": round(tb, 3),
            "gpu_ms": round(ms, 3), "updates_per_s": upd / (ms * 1e-3),
            "algorithmic_GBps": upd * (32 + 44.0 / M) / (ms * 1e-3) / 1e9,

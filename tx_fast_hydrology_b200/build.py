@@ -14,7 +14,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libtxh.so")
 SOURCES = ["txh_topology.cpp", "txh_geojson.cpp", "txh_route.cu", "txh_window.cu", "txh_lane.cu", "txh_da.cu", "txh_kf.cu", "txh_capi.cu"]
-HEADERS = ["txh_topology.hpp", "txh_kernels.cuh", os.path.join("..", "..", "include", "txh.h")]
+HEADERS = ["txh_topology.hpp", "txh_kernels.cuh", "txh_device.cuh", os.path.join("..", "..", "include", "txh.h")]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xcompiler", "-fPIC,-O3",

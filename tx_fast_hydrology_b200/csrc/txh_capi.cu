@@ -136,9 +136,7 @@ struct txh_net {
     LaneStep* d_lsteps = nullptr; size_t lsteps_cap = 0;
     LaneStep* d_unit_lstep = nullptr;
     LaneDev lane[5];                    // member tiles 1, 2, 4, 8, 16
-    int lane_max_members = 4;           // ensembles up to this size may take the lane kernel (row state in registers)
     int lane_cap_rows = 0;              // rows per region; 0 = from the size of the network and the SM count
-    int lane_ctas = 1;                  // regions (CTAs) per SM the schedule is sized for (measured: 1 is best, DESIGN.md)
     double* d_lring = nullptr; size_t lring_cap = 0;
     double* d_stage = nullptr; size_t stage_cap = 0;   // reach-order staging of txh_pack_host / txh_unpack_host
     double* stats_rowsum = nullptr;     // txh_set_stats_output: row sums of the final outflows of every txh_route_run
@@ -214,9 +212,6 @@ int ensure_device(txh_net* net)
         else if (!strcmp(k, "window")) net->route_kernel = 2;
         else if (!strcmp(k, "lane")) net->route_kernel = 3;
     }
-    if (const char* k = getenv("TXH_LANE_MAX_M")) net->lane_max_members = std::max(0, std::min(16, atoi(k)));
-    if (const char* k = getenv("TXH_LANE_CAP")) net->lane_cap_rows = std::max(0, atoi(k));
-    if (const char* k = getenv("TXH_LANE_CTAS")) net->lane_ctas = std::max(1, std::min(8, atoi(k)));
     CU(cudaMalloc((void**)&net->d_coef, sizeof(double) * (6 * net->topo.n + net->sched.link_last.size() + 1)));
     CU(cudaMalloc((void**)&net->d_qtmp, sizeof(double) * net->topo.n));
     CU(cudaMalloc((void**)&net->d_qctl, 64));
@@ -261,8 +256,8 @@ int report_status(txh_net* net, cudaStream_t st)
     if (status == 0 && info == 0) return TXH_OK;
     CU(cudaMemsetAsync(net->d_status, 0, 2 * sizeof(int32_t), st));
     if (status != 0) {
-        if (net->d_ring) CU(cudaMemsetAsync(net->d_ring, 0xff, net->ring_cap * sizeof(double), st));
-        if (net->d_lring) CU(cudaMemsetAsync(net->d_lring, 0xff, net->lring_cap * sizeof(double), st));
+        if (net->d_ring) CU(cudaMemsetAsync(net->d_ring, kEmptyByte, net->ring_cap * sizeof(double), st));
+        if (net->d_lring) CU(cudaMemsetAsync(net->d_lring, kEmptyByte, net->lring_cap * sizeof(double), st));
         CU(cudaMemsetAsync(net->d_qctl, 0, 32, st));                    // queue cursors, tickets
         CU(cudaMemsetAsync(net->d_qctl + 5, 0, 24, st));                // done counters, lane ticket
         CU(cudaStreamSynchronize(st));
@@ -377,6 +372,11 @@ int run_dataflow(txh_net* net, double* O, double* I, int64_t M, const double* F,
     return TXH_OK;
 }
 
+// Launch shapes of route_window_kernel, measured on B200 (DESIGN.md section 4.1): up to 16 warps per CTA; a warp polling
+// for a row another task has not published yet backs off from 32 to 256 ns.
+constexpr int kWindowWarps = 16;
+constexpr int kWindowNapMin = 32, kWindowNapMax = 256;
+
 // Per-warp shared-memory layout of route_window_kernel.  A launch that applies an ensemble update keeps the 64 x 64
 // transform in shared memory and runs shorter input rings (txh_window.cu: kInRingUpd, kSegRingUpd) to keep its warps:
 // at the headline shape 16 x 12,432 B + 33,168 B of the 232,448 B a CTA may have.
@@ -395,8 +395,6 @@ void window_smem_layout(const Schedule& s, bool upd, WinArgs& a)
     a.off_list = a.off_words + up16(std::max(1, s.w_max_words) * 4);
     a.off_mbar = a.off_list + up16(std::max(1, s.w_max_words) * 4);
     a.smem_per_warp = a.off_mbar + 16;                        // + the warp's mbarrier (bulk staging of the state rows)
-    const char* bulk = getenv("TXH_WINDOW_BULK");
-    if (bulk && atoi(bulk) == 0) a.off_mbar = 0;
 }
 
 // Whether route_window_kernel takes the schedule at M members (ok), and the warps per CTA of a launch without (wpc) and
@@ -412,13 +410,11 @@ WindowFit window_fit(const txh_net* net, int64_t M)
     const Schedule& s = net->sched;
     const int steps_bytes = 16 * 24;                          // StepInterp records of one launch (<= 16 steps), once per CTA
     const int smem_max = 227 * 1024;
-    int warps_cap = 16;
-    if (const char* k = getenv("TXH_WINDOW_WARPS")) warps_cap = std::max(1, std::min(16, atoi(k)));
     WinArgs a{};
     window_smem_layout(s, true, a);
-    const int wpc_upd = std::min(warps_cap, (smem_max - steps_bytes - 64 * 64 * (int)sizeof(double) - 16) / a.smem_per_warp);
+    const int wpc_upd = std::min(kWindowWarps, (smem_max - steps_bytes - 64 * 64 * (int)sizeof(double) - 16) / a.smem_per_warp);
     window_smem_layout(s, false, a);
-    const int wpc = std::min(warps_cap, (smem_max - 1024 - steps_bytes) / a.smem_per_warp);
+    const int wpc = std::min(kWindowWarps, (smem_max - 1024 - steps_bytes) / a.smem_per_warp);
     const bool ok = wpc >= 2 && s.w_n_own == 0 &&
                     (size_t)std::max(1, s.n_wslots) * txh_row_stride(M) * sizeof(double) < (size_t(1) << 32);
     return {ok, wpc, wpc_upd};
@@ -447,7 +443,7 @@ int run_window(txh_net* net, double* O, double* I, int64_t M, const double* F, c
     // every cell starts EMPTY (all bits set); consumers put EMPTY back, so a finished launch leaves the whole
     // ring EMPTY again whatever row stride the next launch lays over it
     int rc;
-    if ((rc = grow(&net->d_ring, &net->ring_cap, slot_row * spl, st, 0xff))) return rc;
+    if ((rc = grow(&net->d_ring, &net->ring_cap, slot_row * spl, st, kEmptyByte))) return rc;
     net->ring_ld = ld;
     if (plan.times && (rc = grow(&net->d_steps, &net->steps_cap, (size_t)spl, st))) return rc;
     const StepInterp* d_steps = plan.times ? net->d_steps : net->d_unit_step;
@@ -482,8 +478,7 @@ int run_window(txh_net* net, double* O, double* I, int64_t M, const double* F, c
         a.off_steps = a.upT ? a.off_T + 64 * 64 * (int)sizeof(double) + 16 : fit.wpc * a.smem_per_warp;
         a.rec_slot = rec.slot; a.rec_out = rec.out; a.rec_step_base = rec.base + s0;
         a.rec_every = std::max(1, rec.every); a.rec_count = rec.count;
-        a.nap_min = 32; a.nap_max = 256;
-        if (const char* k = getenv("TXH_WINDOW_NAP")) { int lo = 32, hi = 256; if (sscanf(k, "%d,%d", &lo, &hi) >= 1) { a.nap_min = std::max(0, lo); a.nap_max = std::max(a.nap_min, hi); } }
+        a.nap_min = kWindowNapMin; a.nap_max = kWindowNapMax;
         // the per-task timeline of this launch
         const long long hd[4] = {(long long)pairs, (long long)ns, (long long)s.wtasks.size(), -(long long)nmb};
         if ((rc = traced_launch("TXH_TRACE_FILE", a.trace, pairs * (size_t)(4 + ns), hd, nullptr, 0, st,
@@ -495,6 +490,12 @@ int run_window(txh_net* net, double* O, double* I, int64_t M, const double* F, c
 
 // ---- lane kernel (txh_lane.cu): lanes = reaches, for deterministic runs and small ensembles --------------
 constexpr size_t kLaneSmemBudget = 200 * 1024;
+constexpr int kLaneMaxMembers = 4;      // ensembles up to this size may take the lane kernel (row state in registers)
+constexpr int kLaneSideMin = 32;        // side tributaries of at least this many rows become regions of their own
+// steps a producer region is ahead before its consumer starts / resumes (measured: 24 / 32 / 48 steps -> C2 2.47 / 2.53
+// / 2.69 ms, C4 5.72 / 5.81 / 6.16 ms), and iterations between barrier votes on abandoning a launch
+constexpr int kLaneLag = 24;
+constexpr int kLaneVoteEvery = 64;
 
 int lane_tile_index(int64_t M) { return M <= 1 ? 0 : M <= 2 ? 1 : M <= 4 ? 2 : M <= 8 ? 3 : 4; }
 
@@ -506,21 +507,18 @@ txh_net::LaneDev* lane_schedule(txh_net* net, int ti, int num_sms)
     txh_net::LaneDev& L = net->lane[ti];
     if (!L.built) {
         std::string err;
-        int side_min = 32;
-        if (const char* k = getenv("TXH_LANE_SIDE_MIN")) side_min = atoi(k);
         if (net->lane_cap_rows > 0) {
-            L.ok = L.sched.build(net->topo, net->sched.pos_of_reach, 1 << ti, net->lane_cap_rows, kLaneSmemBudget, side_min, err);
+            L.ok = L.sched.build(net->topo, net->sched.pos_of_reach, 1 << ti, net->lane_cap_rows, kLaneSmemBudget, kLaneSideMin, err);
         } else {
-            // lane_ctas regions per SM, all resident at once while the network is small enough.  Measured on B200
+            // one region per SM, all resident at once while the network is small enough.  Measured on B200
             // (profiles/r02_lane_sweeps.jsonl): the SM's issue rate is set by warps x their dependent-instruction
             // chains, not by the size of a barrier domain, so one large region per SM (fewest streams and hops) wins.
-            const int ctas = std::max(1, net->lane_ctas);
-            const int cap_max = std::max(64, 1024 / ctas - 48);            // threads of a CTA = rows + stream mirrors
-            const int64_t slots = (int64_t)num_sms * ctas;
+            const int cap_max = 1024 - 48;                                 // threads of a CTA = rows + stream mirrors
+            const int64_t slots = num_sms;
             const int64_t per = (net->topo.n + slots - 1) / slots;
-            int cap = (int)std::min<int64_t>(cap_max, std::max<int64_t>(std::min(320, cap_max), per + per / 50));
+            int cap = (int)std::min<int64_t>(cap_max, std::max<int64_t>(320, per + per / 50));
             for (;;) {
-                L.ok = L.sched.build(net->topo, net->sched.pos_of_reach, 1 << ti, cap, kLaneSmemBudget, side_min, err);
+                L.ok = L.sched.build(net->topo, net->sched.pos_of_reach, 1 << ti, cap, kLaneSmemBudget, kLaneSideMin, err);
                 if (!L.ok || (int64_t)L.sched.regions.size() <= slots || cap >= cap_max) break;
                 cap = std::min(cap_max, cap + std::max(4, cap / 12));
             }
@@ -566,7 +564,7 @@ int run_lane(txh_net* net, double* O, double* I, int64_t M, const double* F, con
     if (const char* k = getenv("TXH_LANE_SPL")) { const long v = atol(k); if (v > 0) spl = std::min<int64_t>(spl, v); }
     while (spl > 16 && streams * (size_t)((spl + 15) & ~int64_t(15)) * sizeof(double) > (size_t(128) << 20)) spl = (spl + 1) / 2;
     const size_t ring_need = streams * (size_t)((spl + 15) & ~int64_t(15));
-    if ((rc = grow(&net->d_lring, &net->lring_cap, ring_need, st, 0xff))) return rc;   // every cell starts EMPTY
+    if ((rc = grow(&net->d_lring, &net->lring_cap, ring_need, st, kEmptyByte))) return rc;   // every cell starts EMPTY
     if (plan.times) {
         if ((rc = grow(&net->d_lsteps, &net->lsteps_cap, (size_t)spl, st))) return rc;
     } else if (nsteps != 1) {
@@ -579,10 +577,8 @@ int run_lane(txh_net* net, double* O, double* I, int64_t M, const double* F, con
     if (smem > 227 * 1024) return 1;
     // the per-step interpolation records ride in shared memory too when they fit
     if (plan.times && smem + 32 * (size_t)spl <= 200 * 1024) { a.off_steps = (int32_t)smem; smem += 32 * (size_t)spl; }
-    a.lag = 24;                                            // (measured: 24 / 32 / 48 steps -> C2 2.47 / 2.53 / 2.69 ms, C4 5.72 / 5.81 / 6.16 ms)
-    if (const char* k = getenv("TXH_LANE_LAG")) a.lag = std::max(24, std::min(4096, atoi(k)));
-    a.vote_every = 64;
-    if (const char* k = getenv("TXH_LANE_VOTE_EVERY")) { const int v = atoi(k); if (v > 0 && (v & (v - 1)) == 0) a.vote_every = v; }
+    a.lag = kLaneLag;
+    a.vote_every = kLaneVoteEvery;
     const int tv = s.max_virt > 0 ? std::min(128, (s.max_virt + 31) / 32 * 32) : 0;
     const int tr = (s.max_real + 31) / 32 * 32;                            // one row per thread
     if (tr + tv > 1024) return 1;
@@ -624,7 +620,7 @@ int run_lane(txh_net* net, double* O, double* I, int64_t M, const double* F, con
 bool lane_wanted(txh_net* net, int64_t M, int64_t nsteps)
 {
     if (net->route_kernel == 3) return M <= 16;
-    if (net->route_kernel != 0 || M > net->lane_max_members) return false;
+    if (net->route_kernel != 0 || M > kLaneMaxMembers) return false;
     txh_net::LaneDev* L = lane_schedule(net, lane_tile_index(M), net->num_sms);
     if (!L->ok) return false;
     const LaneSchedule& s = L->sched;
@@ -687,9 +683,6 @@ int txh_create(int64_t n, const int64_t* endnodes, const int32_t* sp, txh_net** 
     if (!net->topo.build(n, endnodes, err)) { delete net; return fail(TXH_E_TOPOLOGY, err); }
     SchedParams p;
     if (sp) { p.long_path_min = sp[0]; p.spine_cap = sp[1]; p.pocket_cap = sp[2]; p.max_slots = sp[3]; p.link_cap = sp[4]; }
-    if (const char* lw = getenv("TXH_LEN_WEIGHT")) p.len_weight = atoi(lw);
-    if (const char* sc = getenv("TXH_SIDE_CAP")) p.side_cap = std::max(1, atoi(sc));
-    if (const char* pc = getenv("TXH_POCKET_CAP")) p.pocket_cap = std::max(4, std::min(16, atoi(pc)));
     if (!net->sched.build(net->topo, p, err)) { delete net; return fail(TXH_E_INVALID, err); }
     *out = net;
     return TXH_OK;

@@ -16,21 +16,11 @@
 #include <cstdio>
 #include <cstdlib>
 
-#include "txh_kernels.cuh"
+#include "txh_device.cuh"
 
 namespace txh {
 
-void count_launch();
-
 namespace {
-
-// D(8x8) += A(8x4) * B(4x8), FP64.  Fragment ownership (lane = 4*g + t):
-//   a = A[g][t], b = B[t][g], c0 = C[g][2t], c1 = C[g][2t+1]
-__device__ __forceinline__ void dmma8x8x4(double& c0, double& c1, double a, double b)
-{
-    asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
-                 : "+d"(c0), "+d"(c1) : "d"(a), "d"(b));
-}
 
 // ---- generic C = alpha * op(A) op(B) + beta * C ------------------------------------------------
 // CTA tile 64x64, K tile 16; 8 warps, each a 16x32 sub-tile = 2x4 DMMA tiles.
@@ -631,11 +621,7 @@ enkf_small_system_kernel(double* __restrict__ HX, const double* __restrict__ O, 
     const int mc = (((m + NC - 1) / NC) + 3) & ~3;                 // gauges per CTA
     const int k_lo = min(m, rank * mc), k_hi = min(m, k_lo + mc);
     auto stamp = [&](int i) {                                      // development aid (TXH_SS_TRACE): phase timeline
-        if (trace && tid == 0) {
-            unsigned long long ns;
-            asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(ns));
-            trace[rank * 8 + i] = ns;
-        }
+        if (trace && tid == 0) trace[rank * 8 + i] = globaltimer_ns();
     };
     // programmatic dependent launch: this kernel may have started before the routing launch in front of it has
     // finished; what it reads is final after the wait, and the routing launch behind it (which reads T and W only
@@ -663,8 +649,8 @@ enkf_small_system_kernel(double* __restrict__ HX, const double* __restrict__ O, 
         }
         const double dk = (tid < SS_KT && kt + tid < k_hi) ? __ldg(dinv + kt + tid) : 0.0;
         if (!waited) {
-            asm volatile("griddepcontrol.wait;" ::: "memory");
-            asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+            griddep_wait();
+            griddep_launch_dependents();
             waited = true;
         }
 #pragma unroll
@@ -993,10 +979,10 @@ enkf_update64_kernel(const double* __restrict__ X, int M, const double* __restri
                 if (r0 + r < n) {
                     const unsigned sa = stage0 + (buf * TR + r) * EU_RS + lane * 16;
                     const double* gp = X + (size_t)(r0 + r) * ld + 2 * lane;
-                    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(sa), "l"(gp) : "memory");
+                    cp_async16(sa, gp);
                 }
         }
-        asm volatile("cp.async.commit_group;" ::: "memory");
+        cp_async_commit();
     };
     prefetch(tile, 0);
     {
@@ -1037,7 +1023,7 @@ enkf_update64_kernel(const double* __restrict__ X, int M, const double* __restri
 #pragma unroll
         for (int i = 0; i < RT; ++i) { mu[i] = mu_n[i]; gi[i] = gi_n[i]; }
         row_meta(tile + tstride, mu_n, gi_n);
-        asm volatile("cp.async.wait_group 1;" ::: "memory");
+        cp_async_wait_group<1>();
         __syncwarp();
         const long long rw = tile * TR;
         long long rows[RT];
@@ -1052,7 +1038,7 @@ enkf_update64_kernel(const double* __restrict__ X, int M, const double* __restri
             for (int j = 0; j < 8; ++j) {
                 const int k = 8 * j + 2 * t;
                 double2 v = make_double2(0.0, 0.0);
-                if (ok && k < ld) asm volatile("ld.shared.v2.f64 {%0, %1}, [%2];" : "=d"(v.x), "=d"(v.y) : "r"(ra + j * 64));
+                if (ok && k < ld) v = lds_row(ra + j * 64);
                 a[i][2 * j] = (ok && k < M) ? v.x - mu[i] : 0.0;
                 a[i][2 * j + 1] = (ok && k + 1 < M) ? v.y - mu[i] : 0.0;
             }
@@ -1090,8 +1076,7 @@ enkf_update64_kernel(const double* __restrict__ X, int M, const double* __restri
                     if (col + 1 < M) gn.y += qg * wr[col + 1];
                 }
                 if (O) {
-                    double2 o;
-                    asm volatile("ld.shared.v2.f64 {%0, %1}, [%2];" : "=d"(o.x), "=d"(o.y) : "r"(ra + j * 64));
+                    double2 o = lds_row(ra + j * 64);
                     o.x += gn.x; o.y += gn.y;
                     *reinterpret_cast<double2*>(O + (size_t)rows[i] * ld + col) = o;
                 }
@@ -1100,7 +1085,7 @@ enkf_update64_kernel(const double* __restrict__ X, int M, const double* __restri
         }
         __syncwarp();                                 // everyone is done with this buffer before it is refilled
     }
-    asm volatile("cp.async.wait_all;" ::: "memory");
+    cp_async_wait_all();
 }
 
 // inflow part of _apply_gain (nutils.py:116-134, da.py:125): I[k] += sum of the gains of the reaches
@@ -1171,8 +1156,6 @@ inflow_rebuild_kernel(const int4* __restrict__ rec, long long n_inner, const int
     }
 }
 
-inline unsigned nblk(long long work, int threads) { return (unsigned)((work + threads - 1) / threads); }
-
 // Hydrographs of txh_run_assimilating_rec at an update: the forecast of the recorded rows (prior_out) and what the
 // update makes of them (post_out), o + (o - mean) T + qs_g W_g [row gauged] -- the rows of enkf_update_kernel, for a
 // few rows and in plain FP64, read from O while it still holds the forecast.
@@ -1186,7 +1169,7 @@ enkf_record_kernel(const double* __restrict__ O, int ld, int M, const double* __
                    const double* __restrict__ W, const int32_t* __restrict__ rec_pos, int rec_count,
                    double* __restrict__ prior_out, double* __restrict__ post_out)
 {
-    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+    griddep_launch_dependents();
     extern __shared__ double rs_sm[];
     const int tid = threadIdx.x;
     const int Mc = M < 256 ? M : 256;                 // threads per row
@@ -1195,7 +1178,7 @@ enkf_record_kernel(const double* __restrict__ O, int ld, int M, const double* __
     const bool stage_a = M <= 4096, stage_t = M <= 64;
     double* sa = rs_sm;                               // [RG][M] anomalies o - mean
     double* sT = rs_sm + (stage_a ? RG * M : 0);      // [M][M]
-    asm volatile("griddepcontrol.wait;" ::: "memory");
+    griddep_wait();
     if (stage_t)
         for (int e = tid; e < M * M; e += blockDim.x) sT[e] = __ldcg(T + e);
     for (int k0 = blockIdx.x * RG; k0 < rec_count; k0 += gridDim.x * RG) {
@@ -1580,9 +1563,7 @@ cudaError_t launch_enkf_small_system(double* HX, const double* O, int ldo, const
     if (nc == 0) {
         if ((e = cudaFuncSetAttribute(k8, cudaFuncAttributeMaxDynamicSharedMemorySize, SS_SMEM)) != cudaSuccess) return e;
         nc = 8;
-        int want = 16;
-        if (const char* k = getenv("TXH_SS_CLUSTER")) want = atoi(k);
-        if (want >= 16 && cudaFuncSetAttribute(k16, cudaFuncAttributeMaxDynamicSharedMemorySize, SS_SMEM) == cudaSuccess &&
+        if (cudaFuncSetAttribute(k16, cudaFuncAttributeMaxDynamicSharedMemorySize, SS_SMEM) == cudaSuccess &&
             cudaFuncSetAttribute(k16, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) == cudaSuccess) {
             cudaLaunchConfig_t q{};
             q.gridDim = dim3(16); q.blockDim = dim3(256); q.dynamicSmemBytes = SS_SMEM;

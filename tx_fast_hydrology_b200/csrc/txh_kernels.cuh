@@ -49,6 +49,12 @@ struct LaneStep {
 constexpr int kWarpsPerCta = 4;
 constexpr int kMemberBlock = 64;          // members per warp: one double2 per lane
 constexpr int kRingBytes = 2 * 12 * 512;  // per-warp row ring: 2 arrays x 12 rows x 512 B (see txh_route.cu)
+// every byte of an EMPTY cell of the window and lane kernels' hand-over rings (txh_device.cuh): the fill of a new ring
+constexpr int kEmptyByte = 0xff;
+
+// launch bookkeeping of the launchers (txh_launch_count) and their grid sizes
+void count_launch();
+inline unsigned nblk(long long work, int threads) { return (unsigned)((work + threads - 1) / threads); }
 
 struct RouteArgs {
     const TaskDesc* tasks;

@@ -19,11 +19,7 @@
 
 namespace txh {
 
-void count_launch();
-
 namespace {
-
-inline unsigned nblk(long long work, int threads) { return (unsigned)((work + threads - 1) / threads); }
 
 // X2[k][c] = X[pos_of_reach[c]][reach_of_pos[k]]  (= pack of the transposed unpacked matrix), pad columns zeroed
 __global__ void __launch_bounds__(256)

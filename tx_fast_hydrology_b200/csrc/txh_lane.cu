@@ -23,32 +23,12 @@
 #include <algorithm>
 #include <type_traits>
 
-#include "txh_kernels.cuh"
+#include "txh_device.cuh"
 
 namespace txh {
 
-void count_launch();
-
 namespace {
 
-__device__ __forceinline__ int ld_relaxed_s32(const int* p)
-{
-    int v;
-    asm volatile("ld.relaxed.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ double ld_relaxed_f64(const double* p)
-{
-    double v;
-    asm volatile("ld.relaxed.gpu.global.f64 %0, [%1];" : "=d"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ unsigned long long globaltimer_ns()
-{
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    return t;
-}
 __device__ __forceinline__ void bar_sync() { asm volatile("bar.sync 0;" ::: "memory"); }
 __device__ __forceinline__ int bar_or(int pred)
 {
@@ -57,10 +37,6 @@ __device__ __forceinline__ int bar_or(int pred)
                  : "=r"(r) : "r"(pred) : "memory");
     return r;
 }
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
-__device__ __forceinline__ bool is_empty(double v) { return __double_as_longlong(v) == -1ll; }
-__device__ __forceinline__ double empty_cell() { return __longlong_as_double(-1ll); }
 
 // Streams are read in batches of kBatch steps (64 bytes), prefetched TWO batches ahead with cp.async into a
 // four-batch window in shared memory.  Producer and consumer regions advance at the same rate, so a consumer
@@ -69,48 +45,6 @@ __device__ __forceinline__ double empty_cell() { return __longlong_as_double(-1l
 // later prefetch lands on cells that are already written.
 constexpr int kBatch = 8;
 constexpr int kExtCells = 4 * kBatch;      // shared-memory window of a stream
-
-// ---- shared memory through 32-bit shared-space addresses (no generic-address arithmetic in the loop) ----
-__device__ __forceinline__ int4 lds_i4(unsigned a)
-{
-    int4 v;
-    asm volatile("ld.shared.v4.s32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(a));
-    return v;
-}
-__device__ __forceinline__ double2 lds_d2(unsigned a)
-{
-    double2 v;
-    asm volatile("ld.shared.v2.f64 {%0, %1}, [%2];" : "=d"(v.x), "=d"(v.y) : "r"(a));
-    return v;
-}
-__device__ __forceinline__ double lds_d(unsigned a)
-{
-    double v;
-    asm volatile("ld.shared.f64 %0, [%1];" : "=d"(v) : "r"(a));
-    return v;
-}
-__device__ __forceinline__ unsigned lds_u16(unsigned a)
-{
-    unsigned short v;
-    asm volatile("ld.shared.u16 %0, [%1];" : "=h"(v) : "r"(a));
-    return v;
-}
-__device__ __forceinline__ void sts_d(unsigned a, double v) { asm volatile("st.shared.f64 [%0], %1;" ::"r"(a), "d"(v) : "memory"); }
-__device__ __forceinline__ void sts_i4(unsigned a, int4 v)
-{
-    asm volatile("st.shared.v4.s32 [%0], {%1, %2, %3, %4};" ::"r"(a), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
-}
-__device__ __forceinline__ void sts_u16(unsigned a, unsigned v) { asm volatile("st.shared.u16 [%0], %1;" ::"r"(a), "h"((unsigned short)v) : "memory"); }
-__device__ __forceinline__ void cp_async8_s(unsigned sa, const void* g)
-{
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(sa), "l"(g) : "memory");
-}
-template <int N>
-__device__ __forceinline__ void cp_async_wait_group() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
-__device__ __forceinline__ void cp_async16_s(unsigned sa, const void* g)
-{
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(sa), "l"(g) : "memory");
-}
 
 // A new forcing bracket for a row: (pr0, pr1) -> (r0, r1).  f0, f1 are the rows of the old bracket at this reach,
 // fn the row after them, requested when the old bracket was entered (a plain load whose register is not touched
@@ -192,7 +126,7 @@ route_lane_kernel(const LaneArgs a)
                 f0 = __ldg(a.F + (size_t)r0s * a.n + pos);
                 f1 = __ldg(a.F + (size_t)r1s * a.n + pos);
                 fn = __ldg(a.F + (size_t)min(max(r0s, r1s) + 1, a.R - 1) * a.n + pos);
-                sts_d(sFn + 8u * (unsigned)tid, fn);
+                sts_f64(sFn + 8u * (unsigned)tid, fn);
             }
             if (a.rec_slot) rec = a.rec_slot[pos];
             const double* og = a.O + (size_t)pos * ld;
@@ -202,7 +136,7 @@ route_lane_kernel(const LaneArgs a)
                 double pm = 0.0;
                 if (m < M) pm = be * __ldcg(ig + m) + ch * __ldcg(og + m);
                 if (PREG) p[m < MR ? m : 0] = pm;
-                else sts_d(sP + 8u * ((unsigned)m * nr + tid), pm);
+                else sts_f64(sP + 8u * ((unsigned)m * nr + tid), pm);
             }
         }
         {
@@ -211,7 +145,7 @@ route_lane_kernel(const LaneArgs a)
             const uint16_t* gc = a.child + rd.child_off;
             for (int i = tid; i < rd.n_child; i += blockDim.x) sts_u16(sChild + 2u * i, gc[i]);
             // the ZERO row of both buffers: what a missing child reads
-            for (int i = tid; i < 2 * MT; i += blockDim.x) sts_d(sOb + 8u * ((unsigned)i * rv + (nr + nv)), 0.0);
+            for (int i = tid; i < 2 * MT; i += blockDim.x) sts_f64(sOb + 8u * ((unsigned)i * rv + (nr + nv)), 0.0);
             if (HAS_F && a.off_steps > 0 && reg == first_region) {
                 const int4* gs = reinterpret_cast<const int4*>(a.steps);
                 for (int i = tid; i < 2 * nsteps; i += blockDim.x) sts_i4(sSteps + 16u * i, gs[i]);
@@ -225,7 +159,7 @@ route_lane_kernel(const LaneArgs a)
                     const unsigned ex = sExt + 256u * ((unsigned)v * MT + m);
                     const double* g = a.ring + ((size_t)vslot * M + m) * splp;
 #pragma unroll
-                    for (int q = 0; q < kBatch; ++q) cp_async16_s(ex + 16u * q, g + 2 * q);
+                    for (int q = 0; q < kBatch; ++q) cp_async16(ex + 16u * q, g + 2 * q);
                 }
             }
             cp_async_commit();
@@ -266,7 +200,7 @@ route_lane_kernel(const LaneArgs a)
                 if (HAS_F) {
                     int r1f;
                     if (SM) {
-                        const double2 ww = lds_d2(sSteps + 32u * s);
+                        const double2 ww = lds_row(sSteps + 32u * s);
                         const int4 rr = lds_i4(sSteps + 32u * s + 16u);
                         w0 = ww.x; w1 = ww.y; fr0 = rr.x; r1f = rr.y;
                     } else {
@@ -281,16 +215,16 @@ route_lane_kernel(const LaneArgs a)
                         if (r1f & 0x40000000) {
                             // the usual case, marked by lane_init_kernel: the bracket moved on by one row -- shift, and
                             // request the row after it
-                            f0 = f1; f1 = lds_d(sFn + ra);
+                            f0 = f1; f1 = lds_f64(sFn + ra);
                             const int nn = min(fr1 + 1, a.R - 1);
-                            if (nn != fr1) { cp_async8_s(sFn + ra, a.F + (size_t)nn * a.n + pos); kreq = k; }
+                            if (nn != fr1) { cp_async8(sFn + ra, a.F + (size_t)nn * a.n + pos); kreq = k; }
                         } else {
                             int pr0, pr1;
                             if (SM) { const int4 pp = lds_i4(sSteps + 32u * (s - 1) + 16u); pr0 = pp.x; pr1 = pp.y; }
                             else { pr0 = __ldg(&a.steps[s - 1].r0); pr1 = __ldg(&a.steps[s - 1].r1); }
-                            fn = lds_d(sFn + ra);
+                            fn = lds_f64(sFn + ra);
                             rotate_bracket(f0, f1, fn, a.F + pos, a.n, a.R, pr0, pr1 & 0x3fffffff, fr0, fr1);
-                            sts_d(sFn + ra, fn);
+                            sts_f64(sFn + ra, fn);
                         }
                     }
                 }
@@ -300,10 +234,10 @@ route_lane_kernel(const LaneArgs a)
 #pragma unroll
                 for (int m = 0; m < MT; ++m) {
                     const unsigned mo = 8u * (unsigned)(m * rv);
-                    double infl = lds_d(obp + mo + c0a) + lds_d(obp + mo + c1a);
+                    double infl = lds_f64(obp + mo + c0a) + lds_f64(obp + mo + c1a);
                     if (nx > 0) {                               // confluences of more than two reaches (rows sorted last)
                         unsigned xa = xa0;
-                        for (int c = 0; c < nx; ++c, xa += 2u) infl += lds_d(obp + mo + 8u * lds_u16(xa));
+                        for (int c = 0; c < nx; ++c, xa += 2u) infl += lds_f64(obp + mo + 8u * lds_u16(xa));
                     }
                     double qm = q;
                     if (HAS_W) {
@@ -313,12 +247,12 @@ route_lane_kernel(const LaneArgs a)
                     }
                     double pm;
                     if (PREG) pm = p[m < MR ? m : 0];
-                    else pm = lds_d(sP + 8u * ((unsigned)m * nr + tid));
+                    else pm = lds_f64(sP + 8u * ((unsigned)m * nr + tid));
                     const double o = al * infl + (pm + qm);
                     pm = be * infl + ch * o;
                     if (PREG) p[m < MR ? m : 0] = pm;
-                    else sts_d(sP + 8u * ((unsigned)m * nr + tid), pm);
-                    sts_d(obc + mo + ra, o);
+                    else sts_f64(sP + 8u * ((unsigned)m * nr + tid), pm);
+                    sts_f64(obc + mo + ra, o);
                     if ((slot >= 0 || last) && (MT == 1 || m < M)) {
                         if (slot >= 0) __stcg(a.ring + ((size_t)slot * M + m) * splp + s, o);
                         if (last) {
@@ -378,7 +312,7 @@ route_lane_kernel(const LaneArgs a)
 #pragma unroll
                             for (int q = 0; q < 3 * kBatch / 2; ++q) {
                                 const int c = b0 + 2 * q;
-                                if (c < (int)splp) cp_async16_s(ex0 + 256u * m + 8u * (c & (kExtCells - 1)), g0 + (size_t)m * splp + c);
+                                if (c < (int)splp) cp_async16(ex0 + 256u * m + 8u * (c & (kExtCells - 1)), g0 + (size_t)m * splp + c);
                             }
                         cp_async_commit();
                         cp_async_wait_all();
@@ -393,7 +327,7 @@ route_lane_kernel(const LaneArgs a)
                                 const unsigned ex = ex0 + 256u * m + 8u * ((sv + 2 * kBatch) & (kExtCells - 1));
                                 const double* g = g0 + (size_t)m * splp + sv + 2 * kBatch;
 #pragma unroll
-                                for (int q = 0; q < kBatch / 2; ++q) cp_async16_s(ex + 16u * q, g + 2 * q);
+                                for (int q = 0; q < kBatch / 2; ++q) cp_async16(ex + 16u * q, g + 2 * q);
                             }
                         }
                         cp_async_commit();
@@ -401,12 +335,12 @@ route_lane_kernel(const LaneArgs a)
                     for (int m = 0; m < M; ++m) {
                         double* cell = a.ring + ((size_t)mt.w * M + m) * splp + sv;
                         const unsigned ea = ex0 + 256u * m + 8u * (sv & (kExtCells - 1));
-                        double val = lds_d(ea);
+                        double val = lds_f64(ea);
                         if (is_empty(val)) {
                             // caught up with the producer: fall back by `lag` steps, then continue from the window
                             if (tr) atomicAdd(tr + 6, 1ull);
                             lag_and_fetch(sv, m);
-                            val = lds_d(ea);
+                            val = lds_f64(ea);
                             unsigned spins = 0, nap = 32;
                             unsigned long long t0 = 0;
                             while (is_empty(val)) {                          // (stores to different cells may land out of order)
@@ -422,8 +356,8 @@ route_lane_kernel(const LaneArgs a)
                                 if (nap < 256u) nap <<= 1;
                             }
                         }
-                        __stcg(cell, empty_cell());
-                        sts_d(obc + 8u * ((unsigned)m * rv + nr + v), val);
+                        __stcg(cell, empty_f64());
+                        sts_f64(obc + 8u * ((unsigned)m * rv + nr + v), val);
                     }
                 }
             }
@@ -434,9 +368,8 @@ route_lane_kernel(const LaneArgs a)
         }
         cp_async_wait_all();
         if (tr && tid == 0) {
-            unsigned smid;
-            asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-            tr[3] = globaltimer_ns(); tr[5] = smid;
+            const unsigned sm = smid();
+            tr[3] = globaltimer_ns(); tr[5] = sm;
         }
         if (abandon) break;
     }
@@ -514,9 +447,6 @@ cudaError_t lane_occupancy(int mt, bool f, bool w, int threads, size_t smem, int
         default: return cudaErrorInvalidValue;
     }
 }
-
-namespace {
-}  // namespace
 
 cudaError_t launch_lane_init(const InitArgs& a, LaneStep* out, unsigned long long* ticket, cudaStream_t st)
 {

@@ -11,7 +11,7 @@
 // reference's walk is honoured.  Ensemble members are the SIMD axis: a lane owns two
 // adjacent member columns (one 128-bit access per row), so a thread only ever
 // reads values of its own columns and intra-task hand-offs need no synchronisation.
-#include "txh_kernels.cuh"
+#include "txh_device.cuh"
 
 #include <atomic>
 
@@ -23,67 +23,9 @@ void count_launch() { g_launches++; }
 
 namespace {
 
-__device__ __forceinline__ int ld_relaxed(const int* p)
-{
-    int v;
-    asm volatile("ld.relaxed.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ unsigned long long globaltimer_ns()
-{
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    return t;
-}
-// state rows are produced and consumed by different SMs inside one launch: bypass L1
-__device__ __forceinline__ double2 ld_row(const double* p) { return __ldcg(reinterpret_cast<const double2*>(p)); }
-__device__ __forceinline__ void st_row(double* p, double2 v) { __stcg(reinterpret_cast<double2*>(p), v); }
 constexpr int kRing = 12;     // rows in flight per warp and state array (cp.async ring in shared memory)
 constexpr int kRingPre = 6;   // PRE tasks stream four arrays (I, O, two side rows): 4 x 6 == 2 x 12 slots
 
-__device__ __forceinline__ void cp_async4(void* s, const void* g)
-{
-    const unsigned sa = (unsigned)__cvta_generic_to_shared(s);
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(sa), "l"(g) : "memory");
-}
-__device__ __forceinline__ void cp_async8(void* s, const void* g)
-{
-    const unsigned sa = (unsigned)__cvta_generic_to_shared(s);
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(sa), "l"(g) : "memory");
-}
-__device__ __forceinline__ void cp_async16(void* s, const void* g)
-{
-    const unsigned sa = (unsigned)__cvta_generic_to_shared(s);
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(sa), "l"(g) : "memory");
-}
-__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait_group() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
-// row copy global -> this lane's 16-byte cell of a ring slot (LDGSTS, L1 bypass)
-__device__ __forceinline__ void cp_row(unsigned saddr, const double* g)
-{
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(saddr), "l"(g) : "memory");
-}
-__device__ __forceinline__ double2 lds_row(unsigned saddr)
-{
-    double2 v;
-    asm volatile("ld.shared.v2.f64 {%0, %1}, [%2];" : "=d"(v.x), "=d"(v.y) : "r"(saddr));
-    return v;
-}
-
-__device__ __forceinline__ double lds_f64(unsigned a)
-{
-    double v;
-    asm volatile("ld.shared.f64 %0, [%1];" : "=d"(v) : "r"(a));
-    return v;
-}
-__device__ __forceinline__ uint32_t lds_u32(unsigned a)
-{
-    uint32_t v;
-    asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(a));
-    return v;
-}
 __device__ __forceinline__ void fence_acq_rel() { asm volatile("fence.acq_rel.gpu;" ::: "memory"); }
 
 // Per-warp shared-memory staging of one task's per-reach metadata: filled once per task by
@@ -154,7 +96,7 @@ __device__ __forceinline__ void run_pocket(const RouteArgs& a, const TaskDesc& t
     const unsigned ringO = ring + kRing * 512u;
 #pragma unroll
     for (int j = 0; j < kRing; ++j) {
-        if (active && j < len) { cp_row(ring + j * 512u, Ir + (size_t)j * ld); cp_row(ringO + j * 512u, Or + (size_t)j * ld); }
+        if (active && j < len) { cp_async16(ring + j * 512u, Ir + (size_t)j * ld); cp_async16(ringO + j * 512u, Or + (size_t)j * ld); }
         cp_async_commit();
     }
     cp_async_wait_group<kRing>();                       // this thread's share of the staged metadata ...
@@ -165,8 +107,8 @@ __device__ __forceinline__ void run_pocket(const RouteArgs& a, const TaskDesc& t
         cp_async_wait_group<kRing - 1>();               // row i has landed
         const double2 io = lds_row(ring + sl * 512u), oo = lds_row(ringO + sl * 512u);
         if (active && i + kRing < len) {
-            cp_row(ring + sl * 512u, Ir + (size_t)(i + kRing) * ld);
-            cp_row(ringO + sl * 512u, Or + (size_t)(i + kRing) * ld);
+            cp_async16(ring + sl * 512u, Ir + (size_t)(i + kRing) * ld);
+            cp_async16(ringO + sl * 512u, Or + (size_t)(i + kRing) * ld);
         }
         cp_async_commit();
         sl = sl + 1 == kRing ? 0 : sl + 1;
@@ -221,9 +163,9 @@ __device__ __forceinline__ void run_pre(const RouteArgs& a, const TaskDesc& td, 
         if (j < len) {
             const int nin = (int)((st.h(j) >> 6) & 0x1fffu);
             if (active) {
-                cp_row(ring + j * 512u, Ir + (size_t)j * ld); cp_row(ringO + j * 512u, Or + (size_t)j * ld);
-                if (nin > 0) cp_row(ringG + j * 512u, Sr + (size_t)cq * ld);
-                if (nin > 1) cp_row(ringH + j * 512u, Sr + (size_t)(cq + 1) * ld);
+                cp_async16(ring + j * 512u, Ir + (size_t)j * ld); cp_async16(ringO + j * 512u, Or + (size_t)j * ld);
+                if (nin > 0) cp_async16(ringG + j * 512u, Sr + (size_t)cq * ld);
+                if (nin > 1) cp_async16(ringH + j * 512u, Sr + (size_t)(cq + 1) * ld);
             }
             cq += nin;
         }
@@ -242,9 +184,9 @@ __device__ __forceinline__ void run_pre(const RouteArgs& a, const TaskDesc& td, 
         if (ip < len) {
             const int np = (int)((st.h(ip) >> 6) & 0x1fffu);
             if (active) {
-                cp_row(ring + sl * 512u, Ir + (size_t)ip * ld); cp_row(ringO + sl * 512u, Or + (size_t)ip * ld);
-                if (np > 0) cp_row(ringG + sl * 512u, Sr + (size_t)cq * ld);
-                if (np > 1) cp_row(ringH + sl * 512u, Sr + (size_t)(cq + 1) * ld);
+                cp_async16(ring + sl * 512u, Ir + (size_t)ip * ld); cp_async16(ringO + sl * 512u, Or + (size_t)ip * ld);
+                if (np > 0) cp_async16(ringG + sl * 512u, Sr + (size_t)cq * ld);
+                if (np > 1) cp_async16(ringH + sl * 512u, Sr + (size_t)(cq + 1) * ld);
             }
             cq += np;
         }
@@ -289,8 +231,8 @@ __device__ __forceinline__ void run_link(const RouteArgs& a, const TaskDesc& td,
             const uint32_t last = st.word(wq) & ~INW_ROW;
             const int nl = (int)st.word(wq + 1);
             if (active) {
-                cp_row(ring + j * 512u, Ob + (size_t)last * ld);
-                if (nl > 0) cp_row(ringG + j * 512u, Ob + (size_t)(st.word(wq + 2) & ~INW_ROW) * ld);
+                cp_async16(ring + j * 512u, Ob + (size_t)last * ld);
+                if (nl > 0) cp_async16(ringG + j * 512u, Ob + (size_t)(st.word(wq + 2) & ~INW_ROW) * ld);
             }
             wq += 2 + nl;
         }
@@ -316,8 +258,8 @@ __device__ __forceinline__ void run_link(const RouteArgs& a, const TaskDesc& td,
             const uint32_t lastp = st.word(wq) & ~INW_ROW;
             const int np = (int)st.word(wq + 1);
             if (active) {
-                cp_row(ring + sl * 512u, Ob + (size_t)lastp * ld);
-                if (np > 0) cp_row(ringG + sl * 512u, Ob + (size_t)(st.word(wq + 2) & ~INW_ROW) * ld);
+                cp_async16(ring + sl * 512u, Ob + (size_t)lastp * ld);
+                if (np > 0) cp_async16(ringG + sl * 512u, Ob + (size_t)(st.word(wq + 2) & ~INW_ROW) * ld);
             }
             wq += 2 + np;
         }
@@ -348,7 +290,7 @@ __device__ __forceinline__ void run_fix(const RouteArgs& a, const TaskDesc& td, 
     const unsigned ringO = ring + kRing * 512u;
 #pragma unroll
     for (int j = 0; j < kRing; ++j) {
-        if (active && j < len) { cp_row(ring + j * 512u, Ir + (size_t)j * ld); cp_row(ringO + j * 512u, Or + (size_t)j * ld); }
+        if (active && j < len) { cp_async16(ring + j * 512u, Ir + (size_t)j * ld); cp_async16(ringO + j * 512u, Or + (size_t)j * ld); }
         cp_async_commit();
     }
     cp_async_wait_group<kRing>();
@@ -366,8 +308,8 @@ __device__ __forceinline__ void run_fix(const RouteArgs& a, const TaskDesc& td, 
         cp_async_wait_group<kRing - 1>();
         const double2 side = lds_row(ring + sl * 512u), B = lds_row(ringO + sl * 512u);
         if (active && i + kRing < len) {
-            cp_row(ring + sl * 512u, Ir + (size_t)(i + kRing) * ld);
-            cp_row(ringO + sl * 512u, Or + (size_t)(i + kRing) * ld);
+            cp_async16(ring + sl * 512u, Ir + (size_t)(i + kRing) * ld);
+            cp_async16(ringO + sl * 512u, Or + (size_t)(i + kRing) * ld);
         }
         cp_async_commit();
         sl = sl + 1 == kRing ? 0 : sl + 1;
@@ -452,7 +394,7 @@ route_dataflow_kernel(const RouteArgs a)
     unsigned long long* n_done = a.q_head + 2;
     const long long pairs = (long long)a.n_tasks * nmb;
 
-    if (ld_relaxed(a.status) != 0) return;          // a previous launch on this handle was poisoned
+    if (ld_relaxed_s32(a.status) != 0) return;          // a previous launch on this handle was poisoned
 
     long long next_entry = 0;                       // task made ready by this warp: run it without queueing
     for (;;) {
@@ -477,7 +419,7 @@ route_dataflow_kernel(const RouteArgs a)
                             unsigned long long fin;
                             asm volatile("ld.relaxed.gpu.global.u64 %0, [%1];" : "=l"(fin) : "l"(n_done) : "memory");
                             if ((long long)fin >= a.total) break;           // everything ran (inline continuations skip the queue)
-                            if (ld_relaxed(a.status) != 0) break;
+                            if (ld_relaxed_s32(a.status) != 0) break;
                             const unsigned long long now = globaltimer_ns();
                             if (t0 == 0) t0 = now;
                             else if (now - t0 > a.watchdog_ns) { atomicExch(a.status, 1); break; }
@@ -601,11 +543,10 @@ route_dataflow_kernel(const RouteArgs a)
         if (lane == 0) {
             atomicAdd(n_done, 1ull);
             if (a.trace) {
-                unsigned smid;
-                asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
+                const unsigned sm = smid();
                 unsigned long long* tr = a.trace + 4 * ((size_t)s * pairs + pair);
                 tr[0] = t_pop; tr[1] = t_begin; tr[2] = t_comp;
-                tr[3] = (globaltimer_ns() << 16) | ((unsigned long long)(smid & 0xffu) << 8) | (unsigned)td.kind;
+                tr[3] = (globaltimer_ns() << 16) | ((unsigned long long)(sm & 0xffu) << 8) | (unsigned)td.kind;
             }
         }
         __syncwarp();
@@ -739,18 +680,16 @@ permute_vec_kernel(const int32_t* reach_of_pos, const double* src, double* dst, 
     if (gid < n) dst[gid] = src[reach_of_pos[gid]];
 }
 
-inline unsigned blocks_for(long long work, int threads) { return (unsigned)((work + threads - 1) / threads); }
-
 }  // namespace
 
 cudaError_t launch_dataflow_init(const InitArgs& a, cudaStream_t st)
 {
     long long work = (long long)a.n_tasks * a.n_mblocks;
     if (a.queue_entries > work) work = a.queue_entries;
-    unsigned blocks = blocks_for(work, 256);
+    unsigned blocks = nblk(work, 256);
     if (blocks > 1184u) blocks = 1184u;                       // grid-stride beyond 8 CTAs per SM
     dataflow_init_kernel<<<blocks, 256, 0, st>>>(a);
-    g_launches++;
+    count_launch();
     return cudaGetLastError();
 }
 
@@ -773,15 +712,15 @@ cudaError_t launch_route_dataflow(const RouteArgs& a, int num_sms, cudaStream_t 
     long long cap = (long long)num_sms * occ;
     const unsigned grid = (unsigned)(want < cap ? (want < 1 ? 1 : want) : cap);
     kern<<<grid, kWarpsPerCta * 32, smem, st>>>(a);
-    g_launches++;
+    count_launch();
     return cudaGetLastError();
 }
 
 cudaError_t launch_route_level(const LevelArgs& a, cudaStream_t st)
 {
     const int half = (a.ld + 1) / 2;
-    route_level_kernel<<<blocks_for((long long)a.count * half, 256), 256, 0, st>>>(a);
-    g_launches++;
+    route_level_kernel<<<nblk((long long)a.count * half, 256), 256, 0, st>>>(a);
+    count_launch();
     return cudaGetLastError();
 }
 
@@ -789,8 +728,8 @@ cudaError_t launch_init_inflows(const int32_t* up_off, const int32_t* up_pos, co
                                 const double* O, double* I, int64_t n, int ld, int M, cudaStream_t st)
 {
     (void)M;
-    init_inflows_kernel<<<blocks_for(n * ((ld + 1) / 2), 256), 256, 0, st>>>(up_off, up_pos, is_outlet, O, I, n, ld);
-    g_launches++;
+    init_inflows_kernel<<<nblk(n * ((ld + 1) / 2), 256), 256, 0, st>>>(up_off, up_pos, is_outlet, O, I, n, ld);
+    count_launch();
     return cudaGetLastError();
 }
 
@@ -798,48 +737,48 @@ cudaError_t launch_apply_gain(const int32_t* up_off, const int32_t* up_pos, cons
                               double* I, int64_t n, int ld, int M, cudaStream_t st)
 {
     (void)M;
-    apply_gain_kernel<<<blocks_for(n * ((ld + 1) / 2), 256), 256, 0, st>>>(up_off, up_pos, G, O, I, n, ld);
-    g_launches++;
+    apply_gain_kernel<<<nblk(n * ((ld + 1) / 2), 256), 256, 0, st>>>(up_off, up_pos, G, O, I, n, ld);
+    count_launch();
     return cudaGetLastError();
 }
 
 cudaError_t launch_pack(const int32_t* reach_of_pos, const double* src, double* dst, int64_t n, int M,
                         int ld, int src_member_major, cudaStream_t st)
 {
-    pack_kernel<<<blocks_for(n * ld, 256), 256, 0, st>>>(reach_of_pos, src, dst, n, M, ld, src_member_major);
-    g_launches++;
+    pack_kernel<<<nblk(n * ld, 256), 256, 0, st>>>(reach_of_pos, src, dst, n, M, ld, src_member_major);
+    count_launch();
     return cudaGetLastError();
 }
 
 cudaError_t launch_unpack(const int32_t* reach_of_pos, const double* src, double* dst, int64_t n, int M,
                           int ld, int dst_member_major, cudaStream_t st)
 {
-    unpack_kernel<<<blocks_for(n * M, 256), 256, 0, st>>>(reach_of_pos, src, dst, n, M, ld, dst_member_major);
-    g_launches++;
+    unpack_kernel<<<nblk(n * M, 256), 256, 0, st>>>(reach_of_pos, src, dst, n, M, ld, dst_member_major);
+    count_launch();
     return cudaGetLastError();
 }
 
 cudaError_t launch_gather_rows(const int32_t* pos, int64_t count, const double* X, int ld, int M,
                                double* out, cudaStream_t st)
 {
-    gather_rows_kernel<<<blocks_for(count * M, 256), 256, 0, st>>>(pos, count, X, ld, M, out);
-    g_launches++;
+    gather_rows_kernel<<<nblk(count * M, 256), 256, 0, st>>>(pos, count, X, ld, M, out);
+    count_launch();
     return cudaGetLastError();
 }
 
 cudaError_t launch_permute_rows(const int32_t* reach_of_pos, const double* src, double* dst, int64_t n, int64_t R,
                                 cudaStream_t st)
 {
-    permute_rows_kernel<<<blocks_for(n * R, 256), 256, 0, st>>>(reach_of_pos, src, dst, n, R);
-    g_launches++;
+    permute_rows_kernel<<<nblk(n * R, 256), 256, 0, st>>>(reach_of_pos, src, dst, n, R);
+    count_launch();
     return cudaGetLastError();
 }
 
 cudaError_t launch_permute_vec(const int32_t* reach_of_pos, const double* src, double* dst, int64_t n,
                                cudaStream_t st)
 {
-    permute_vec_kernel<<<blocks_for(n, 256), 256, 0, st>>>(reach_of_pos, src, dst, n);
-    g_launches++;
+    permute_vec_kernel<<<nblk(n, 256), 256, 0, st>>>(reach_of_pos, src, dst, n);
+    count_launch();
     return cudaGetLastError();
 }
 

@@ -616,11 +616,8 @@ bool Schedule::build(const Topology& t, const SchedParams& p_in, std::string& er
         }
         std::vector<int32_t> worder; worder.reserve(ng);
         {
-            // longest remaining chain first; among equals (and to shorten the ramp-down at the end of a launch,
-            // where the last tasks claimed decide when it ends) the tasks with more rows first
-            std::vector<int64_t> prio(ng);
-            for (int32_t g = 0; g < ng; ++g) prio[g] = wcp[g] + (int64_t)p.len_weight * g_len[g];
-            auto cmp = [&](int32_t a, int32_t b) { return prio[a] != prio[b] ? prio[a] < prio[b] : a > b; };
+            // longest remaining chain first; among equals the lower task index
+            auto cmp = [&](int32_t a, int32_t b) { return wcp[a] != wcp[b] ? wcp[a] < wcp[b] : a > b; };
             std::priority_queue<int32_t, std::vector<int32_t>, decltype(cmp)> pq(cmp);
             std::vector<int32_t> pend(ng);
             for (int32_t g = 0; g < ng; ++g) { pend[g] = (int32_t)allprod[g].size(); if (!pend[g]) pq.push(g); }

@@ -43,7 +43,6 @@ struct SchedParams {
     int pocket_cap = 16;      // reaches per pocket task (bundled side subtrees)
     int max_slots = 8;        // shared-memory scratch rows per warp
     int link_cap = 8;         // segments per LINK task (dataflow kernel: blocks chained along the path)
-    int len_weight = 0;       // window-task order: priority = remaining chain + len_weight * rows of the task
     int side_cap = 10;        // pocket roots joining one spine segment (its serial work per step paces the chain)
 };
 

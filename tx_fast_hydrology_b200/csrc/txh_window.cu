@@ -31,70 +31,11 @@
 // C_k o_in into it), so PRE stores B_k into the row's rec_out cell and the same lane adds A_k o_in in the FIX loop.
 #include <cstdlib>
 
-#include "txh_kernels.cuh"
+#include "txh_device.cuh"
 
 namespace txh {
 
-void count_launch();
-
 namespace {
-
-__device__ __forceinline__ int ld_relaxed_s32(const int* p)
-{
-    int v;
-    asm volatile("ld.relaxed.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ unsigned long long globaltimer_ns()
-{
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    return t;
-}
-__device__ __forceinline__ double2 ld_row(const double* p) { return __ldcg(reinterpret_cast<const double2*>(p)); }
-__device__ __forceinline__ void st_row(double* p, double2 v) { __stcg(reinterpret_cast<double2*>(p), v); }
-__device__ __forceinline__ void cp_async4(unsigned sa, const void* g)
-{
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(sa), "l"(g) : "memory");
-}
-__device__ __forceinline__ void cp_async16(unsigned sa, const void* g)
-{
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(sa), "l"(g) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait_group() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
-__device__ __forceinline__ double2 lds_row(unsigned sa)
-{
-    double2 v;
-    asm volatile("ld.shared.v2.f64 {%0, %1}, [%2];" : "=d"(v.x), "=d"(v.y) : "r"(sa));
-    return v;
-}
-__device__ __forceinline__ void sts_row(unsigned sa, double2 v)
-{
-    asm volatile("st.shared.v2.f64 [%0], {%1, %2};" ::"r"(sa), "d"(v.x), "d"(v.y) : "memory");
-}
-__device__ __forceinline__ double lds_f64(unsigned sa)
-{
-    double v;
-    asm volatile("ld.shared.f64 %0, [%1];" : "=d"(v) : "r"(sa));
-    return v;
-}
-__device__ __forceinline__ void sts_f64(unsigned sa, double v)
-{
-    asm volatile("st.shared.f64 [%0], %1;" ::"r"(sa), "d"(v) : "memory");
-}
-__device__ __forceinline__ uint32_t lds_u32(unsigned sa)
-{
-    uint32_t v;
-    asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(sa));
-    return v;
-}
-__device__ __forceinline__ void sts_u32(unsigned sa, uint32_t v)
-{
-    asm volatile("st.shared.u32 [%0], %1;" ::"r"(sa), "r"(v) : "memory");
-}
 
 // ---- TMA bulk copies (cp.async.bulk, 1-D) + mbarrier: the rows of a task are contiguous in global memory, and with
 // 64 doubles per row (one member block) their shared-memory image is contiguous too, so ONE elected lane moves all
@@ -127,12 +68,6 @@ __device__ __forceinline__ void mbar_wait(unsigned mbar, unsigned phase)
     } while (!ok);
 }
 
-// Programmatic dependent launch: a kernel launched with cudaLaunchAttributeProgrammaticStreamSerialization may start
-// once every CTA of the kernel before it in the stream has executed launch_dependents (or exited); what that kernel
-// wrote is only visible after wait.
-__device__ __forceinline__ void griddep_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ void griddep_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-
 constexpr int kInRing = 4;                 // pockets: rows of other tasks in flight per warp (cp.async ring)
 constexpr int kSegRing = 8;                // segments: the ring also takes the (unused) scratch slots
 constexpr int kInRingUpd = 2;              // the update variant gives two ring rows per warp to the CTA's copy of T (16 warps
@@ -142,26 +77,8 @@ constexpr int kStepsStaged = 16;            // interpolation records of a launch
 constexpr int kWinThreads = 512;           // one CTA per SM, up to 16 warps
 constexpr uint32_t kIdMask = 0x3fffffffu;
 
-// Hand-over protocol: a ring cell that has not been written holds the EMPTY pattern (all bits set -- a NaN no
-// arithmetic produces).  The producer just stores its row; the consumer polls the 16 bytes of its own two
-// member columns until neither is EMPTY, and puts EMPTY back (every cell has exactly one reader), so the
-// ring is clean again when the launch ends.  No flags, no fences: a lane only ever depends on the cell the
-// same lane of the producer wrote.
-__device__ __forceinline__ bool cell_full(double2 v)
-{
-    return __double_as_longlong(v.x) != -1ll && __double_as_longlong(v.y) != -1ll;
-}
-__device__ __forceinline__ double2 ld_cell_relaxed(const double* p)
-{
-    double2 v;
-    asm volatile("ld.relaxed.gpu.global.v2.f64 {%0, %1}, [%2];" : "=d"(v.x), "=d"(v.y) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ double2 empty_cell()
-{
-    return make_double2(__longlong_as_double(-1ll), __longlong_as_double(-1ll));
-}
-
+// Hand-over protocol (EMPTY, txh_device.cuh): the consumer polls the 16 bytes of its own two member columns until
+// neither is EMPTY.  No flags, no fences: a lane only ever depends on the cell the same lane of the producer wrote.
 // Polls `cell` (this lane's 16 bytes of a ring row) until it is full; `v` is what an earlier read saw.
 // Returns false when the launch is being abandoned (watchdog / poisoned handle).  (Moving the polling loop into a
 // function of its own to shrink the dozen walks that inline it costs 40 us per launch: the call spills the walk's
@@ -173,7 +90,7 @@ __device__ __forceinline__ bool wait_cell(const WinArgs& a, const double* cell, 
     unsigned spins = 0, nap = (unsigned)a.nap_min;
     unsigned long long t0 = 0;
     for (;;) {
-        if (!ok) { v = ld_cell_relaxed(cell); ok = cell_full(v); }
+        if (!ok) { v = ld_relaxed_row(cell); ok = cell_full(v); }
         if (__all_sync(0xffffffffu, ok)) return true;
         if ((++spins & 15u) == 0) {
             if (ld_relaxed_s32(a.status) != 0) return false;
@@ -220,7 +137,7 @@ __device__ __forceinline__ double2 stream_next(InStream& st, const WinArgs& a, u
     double2 v = lds_row(ring_sa + st.slot_c);
     double* cell = reinterpret_cast<double*>(st.cbase + lds_u32(list_sa + 4u * st.ci));
     if (!st.dead && !wait_cell(a, cell, active, v, lane)) st.dead = true;
-    if (active) st_row(cell, empty_cell());
+    if (active) st_row(cell, empty_row());
     st.slot_c = st.slot_c + 512u == D * 512u ? 0u : st.slot_c + 512u;
     --st.in_flight;
     if (++st.ci == nL) { st.ci = 0; st.cbase += step_bytes; }
@@ -438,9 +355,9 @@ __device__ __forceinline__ void segment_step(const WinArgs& a, const Tk& tk, InS
     double2 oin = make_double2(0.0, 0.0);
     for (int k = 0; k < tk.n_in; ++k) {
         double* cell = reinterpret_cast<double*>(ringS + (size_t)(lds_u32(tk.sWords + 4u * k) & kIdMask) * tk.ld * sizeof(double));
-        double2 v = tk.active ? ld_cell_relaxed(cell) : make_double2(0.0, 0.0);
+        double2 v = tk.active ? ld_relaxed_row(cell) : make_double2(0.0, 0.0);
         if (!ist.dead && !wait_cell(a, cell, tk.active, v, tk.lane)) ist.dead = true;
-        if (tk.active) st_row(cell, empty_cell());
+        if (tk.active) st_row(cell, empty_row());
         oin.x += v.x; oin.y += v.y;
     }
     const double Al = lds_f64(tk.sCum + 8u * (tk.len - 1));
@@ -501,13 +418,6 @@ __device__ __forceinline__ void segment_step(const WinArgs& a, const Tk& tk, InS
             ig += tk.ld; og += tk.ld;
         }
     }
-}
-
-// D(8x8) += A(8x4) * B(4x8), FP64 tensor cores.  lane = 4g + t: a = A[g][t], b = B[t][g], c0 = C[g][2t], c1 = C[g][2t+1]
-__device__ __forceinline__ void dmma8x8x4(double& c0, double& c1, double a, double b)
-{
-    asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
-                 : "+d"(c0), "+d"(c1) : "d"(a), "d"(b));
 }
 
 // The ensemble update owed to the state, applied to the freshly loaded p rows of a task (da.py:112-126 in ensemble
@@ -880,10 +790,9 @@ route_window_kernel(const WinArgs a)
         }
         cp_async_wait_all();
         if (tr && lane == 0) {
-            unsigned smid;
-            asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
+            const unsigned sm = smid();
             tr[2] = globaltimer_ns();
-            tr[3] = ((unsigned long long)smid << 8) | (unsigned)td.kind;
+            tr[3] = ((unsigned long long)sm << 8) | (unsigned)td.kind;
         }
         __syncwarp();
     }
