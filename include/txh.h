@@ -198,7 +198,13 @@ int txh_set_stats_output(txh_net* net, double* rowsum_dev, double scale);
 int64_t txh_enkf_work_size(int64_t m, int64_t Mtot);
 /* Dinv (optional): the inverse of D = R + diag(qs), which is constant between updates -- dinv_kind 1: its
  * diagonal [m] (R diagonal), 2: dense [m][m], 0: not supplied.  When it is supplied and Mtot < m the m x m
- * solve collapses to an Mtot x Mtot one in ensemble space (Sherman-Morrison-Woodbury; txh_da.cu). */
+ * solve collapses to an Mtot x Mtot one in ensemble space (Sherman-Morrison-Woodbury; txh_da.cu).
+ * Missing observations: gauge g is missing when its row Zp_dev[g][0..Mtot) holds a NaN in any member (only NaN;
+ * +-Inf is not special).  With dinv_kind 1 the solve is then that of the same filter without the missing gauges:
+ * T is the reduced system's transform, W[g][:] = 0.0 at a missing gauge and the reduced W elsewhere, and no NaN
+ * reaches T, W or the state; with every gauge missing T = 0, W = 0 and the posterior is the forecast.  With
+ * dinv_kind 0 or 2 a missing gauge is not left out (R couples it): the solve records it for txh_check, which
+ * reports it, and T, W are not usable. */
 int txh_enkf_solve(txh_net* net, int64_t m, int64_t Mtot, const double* HX_dev /*[m][Mtot]*/,
                    const double* Zp_dev /*[m][Mtot]*/, const double* mean_dev /*[n] schedule order*/,
                    const int64_t* obs_reach_host, const double* qs_dev /*[m] diag(Q) at the gauges*/,
@@ -231,7 +237,9 @@ int txh_enkf_apply_peers(txh_net* net, const double* O_in_dev, double* O_out_dev
  * gated to every `every`-th step (muskingum.py:527-536, da.py:56-61), with the host out of it.
  * time_every > 0: every time_every-th routing launch is bracketed by CUDA events on `stream` (kept over
  * calls, at most 4096); txh_get_route_timings synchronises them, returns their durations (ms) and, when
- * `capacity` covers them all, releases them (capacity 0: just count). */
+ * `capacity` covers them all, releases them (capacity 0: just count).
+ * A NaN in row g of Zp_dev[k] leaves gauge g out of update k as txh_enkf_solve describes (the gauge set of the call
+ * stays fixed; only its weights change per update); with dinv_kind 0 or 2 it is reported by txh_check. */
 int txh_run_assimilating(txh_net* net, double* O_dev, double* I_dev, int64_t M, const txh_forcing* forcing,
                          int64_t t0_ns, int64_t dt_ns, int64_t nsteps, int64_t every, int method,
                          const int64_t* obs_reach_host, int64_t m, const double* Zp_dev /*[nsteps/every][m][M]*/,
@@ -323,7 +331,10 @@ int txh_kfb_get(txh_kfb* b, int64_t block, int which, double* host, void* stream
 int txh_kfb_filter(txh_kfb* b, const uint8_t* active_host, const double* z_host, double* O_dev, double* I_dev, void* stream);
 
 /* Synchronise `stream` and report a poisoned launch (TXH_E_WATCHDOG), an innovation covariance that was
- * not positive definite in an earlier txh_enkf_solve (TXH_E_INVALID), or a CUDA fault. */
+ * not positive definite in an earlier txh_enkf_solve (TXH_E_INVALID), a missing (NaN) observation given to an earlier
+ * txh_enkf_solve or txh_run_assimilating(_rec) with a non-diagonal observation covariance (dinv_kind 0 or 2;
+ * TXH_E_INVALID, "missing observation ... non-diagonal observation covariance"), or a CUDA fault.  The report clears
+ * the record: the next solve on the handle is unaffected. */
 int txh_check(txh_net* net, void* stream);
 
 /* kernel-launch counter (bench.py's gpu_launches claim) */

@@ -265,6 +265,9 @@ int report_status(txh_net* net, cudaStream_t st)
                                     "exceeded TXH_WATCHDOG_MS; the state arrays of that call are undefined)");
     }
     CU(cudaStreamSynchronize(st));
+    if (info == kInfoMissingObs)
+        return fail(TXH_E_INVALID, "a missing observation (NaN) with a non-diagonal observation covariance: an ensemble "
+                                   "update can leave out a gauge only when R is diagonal");
     if (info > 0)
         return fail(TXH_E_INVALID, "an ensemble innovation covariance was not positive definite (Cholesky pivot " +
                                    std::to_string(info) + ")");
@@ -1310,7 +1313,7 @@ int enkf_solve_impl(txh_net* net, int64_t m, int64_t Mtot, double* HX, const dou
         double* Y = Bc + 2 * m * Mtot;                      // [m][2Mt] = D^-1 Bc
         double* Cp = Y + 2 * m * Mtot;                      // [nsplit][Mt][2Mt] split-K partials of HA^T Y
         CU(launch_innovation_cat(HX, O_gather, (int)txh_row_stride(Mtot), Zp, mean, d_pos, dinv_kind == 1 ? Dinv : nullptr,
-                                 (int)m, Mt, Bc, Y, st));
+                                 (int)m, Mt, Bc, Y, info_word(net), st));
         if (dinv_kind == 2)
             CU(launch_dgemm(0, 0, (int)m, 2 * Mt, (int)m, 1.0, Dinv, (int)m, Bc, 2 * Mt, 0.0, Y, 2 * Mt, st));
         CU(launch_dgemm_splitk(1, 0, Mt, 2 * Mt, (int)m, Bc, 2 * Mt, Y, 2 * Mt, Cp, 2 * Mt, nsplit,
@@ -1330,7 +1333,7 @@ int enkf_solve_impl(txh_net* net, int64_t m, int64_t Mtot, double* HX, const dou
         double* HA = S + m * m;
         double* mean_obs = HA + m * Mtot;
         CU(launch_gather_rows(d_pos, m, mean, 1, 1, mean_obs, st));
-        CU(launch_innovation(HX, Zp, mean_obs, (int)m, (int)Mtot, HA, W, st));                    // W <- dz
+        CU(launch_innovation(HX, Zp, mean_obs, (int)m, (int)Mtot, dinv_kind == 1, HA, W, info_word(net), st));  // W <- dz
         CU(launch_dgemm(0, 1, (int)m, (int)m, (int)Mtot, 1.0, HA, (int)Mtot, HA, (int)Mtot, 0.0, S, (int)m, st));
         CU(launch_innov_cov_finish(S, qs, R, (int)m, 1.0 / (double)(Mtot - 1), st));
         CU(launch_spd_solve(S, W, (int)m, (int)Mtot, info_word(net), st));                        // W <- S^-1 dz

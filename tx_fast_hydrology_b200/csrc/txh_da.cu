@@ -131,17 +131,42 @@ enkf_stats_kernel(const double* __restrict__ X, int ld, int M, long long n, doub
     if (lane == 0) rowsum[row] = s * scale;
 }
 
-// HA[k][m] = HX[k][m] - mean_k ; dz[k][m] = Zp[k][m] - HX[k][m]     (da.py:112)
+// ---- missing observations ----------------------------------------------------------------------------------------
+// A gauge is missing at an update when its observation row Zp[k][0..M) holds a NaN in any member (a gap in the feed;
+// only NaN counts, +-Inf is an observation like any other).  With a diagonal D = R + diag(qs) the update must be that of
+// a filter without the gauge, and a zero row of [HA | dz] gives exactly that: it drops out of C = HA^T D^-1 [HA | dz]
+// and of S = HA HA^T/(M-1) + D (whose diagonal keeps the gauge decoupled), and W_k = D^-1_k (dz_k - HA_k Z) = 0.  The
+// NaN entries themselves are replaced -- a zero weight would not do, 0 * NaN being NaN -- and the decision is per row,
+// not per element.  With a dense D a zero row is not the reduced update; the solve reports the row instead
+// (kInfoMissingObs).
+__device__ __forceinline__ bool obs_missing(double zp) { return zp != zp; }
+
+// warp-collective: whether the observation row zp[0..M) is missing (every lane of the warp passes the same row)
+__device__ __forceinline__ bool gauge_row_missing(const double* __restrict__ zp, int M)
+{
+    bool nan = false;
+    for (int c = threadIdx.x & 31; c < M; c += 32) nan |= obs_missing(__ldg(zp + c));
+    return __any_sync(0xffffffffu, nan);
+}
+
+// HA[k][m] = HX[k][m] - mean_k ; dz[k][m] = Zp[k][m] - HX[k][m]     (da.py:112), one warp per gauge.  A missing gauge
+// gets zero rows when R is diagonal (diag_R) and is reported through *info otherwise.
 __global__ void __launch_bounds__(256)
 innovation_kernel(const double* __restrict__ HX, const double* __restrict__ Zp, const double* __restrict__ mean_obs,
-                  int m, int M, double* __restrict__ HA, double* __restrict__ dz)
+                  int m, int M, int diag_R, double* __restrict__ HA, double* __restrict__ dz, int* __restrict__ info)
 {
-    const int gid = blockIdx.x * blockDim.x + threadIdx.x;
-    if (gid >= m * M) return;
-    const int k = gid / M;
-    const double hx = HX[gid];
-    HA[gid] = hx - mean_obs[k];
-    dz[gid] = Zp[gid] - hx;
+    const int k = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+    if (k >= m) return;                                           // (warp-uniform)
+    const size_t r = (size_t)k * M;
+    const bool miss = gauge_row_missing(Zp + r, M);
+    if (miss && !diag_R && lane == 0) *info = kInfoMissingObs;
+    const bool zero = miss && diag_R;
+    const double mu = mean_obs[k];
+    for (int c = lane; c < M; c += 32) {
+        const double hx = HX[r + c];
+        HA[r + c] = zero ? 0.0 : hx - mu;
+        dz[r + c] = zero ? 0.0 : Zp[r + c] - hx;
+    }
 }
 
 // S = S * scale + diag(qs) + R        (P[s][:, s] + R_cov with P = sample covariance + Q, da.py:117-119)
@@ -321,22 +346,31 @@ chol_back_kernel(const double* __restrict__ S, int m, double* __restrict__ B, in
 //     (C0 + (Mt-1) I) Z = C1                   T = HA^T W/(Mt-1) = Z          W = Y_dz - Y_HA Z
 // (HA^T S^-1 = (Mt-1) (C0 + (Mt-1) I)^-1 HA^T D^-1, so the ensemble transform IS the small solve.)
 
-// Bc[k] = [HA_k | dz_k] (2*Mt doubles per gauge); Y = dinv_k * Bc when D is diagonal.
+// Bc[k] = [HA_k | dz_k] (2*Mt doubles per gauge); Y = dinv_k * Bc when D is diagonal.  One warp per gauge: a missing
+// gauge gets zero rows of Bc and Y when D is diagonal and is reported through *info when it is dense.
 __global__ void __launch_bounds__(256)
 innovation_cat_kernel(double* __restrict__ HX, const double* __restrict__ O, int ldo, const double* __restrict__ Zp,
                       const double* __restrict__ mean, const int32_t* __restrict__ obs_pos,
-                      const double* __restrict__ dinv_diag, int m, int Mt, double* __restrict__ Bc, double* __restrict__ Y)
+                      const double* __restrict__ dinv_diag, int m, int Mt, double* __restrict__ Bc, double* __restrict__ Y,
+                      int* __restrict__ info)
 {
-    const int gid = blockIdx.x * blockDim.x + threadIdx.x;
-    if (gid >= m * Mt) return;
-    const int k = gid / Mt, c = gid - k * Mt;
-    double hx;
-    if (O) { hx = O[(size_t)obs_pos[k] * ldo + c]; HX[gid] = hx; }      // the gauge rows gathered on the way
-    else hx = HX[gid];
-    const double ha = hx - mean[obs_pos[k]], dz = Zp[gid] - hx;
-    const size_t o = (size_t)k * 2 * Mt + c;
-    Bc[o] = ha; Bc[o + Mt] = dz;
-    if (dinv_diag) { const double d = dinv_diag[k]; Y[o] = d * ha; Y[o + Mt] = d * dz; }
+    const int k = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+    if (k >= m) return;                                           // (warp-uniform)
+    const size_t r = (size_t)k * Mt;
+    const bool miss = gauge_row_missing(Zp + r, Mt);
+    if (miss && !dinv_diag && lane == 0) *info = kInfoMissingObs;
+    const bool zero = miss && dinv_diag;
+    const int pos = obs_pos[k];
+    const double mu = mean[pos], d = dinv_diag ? dinv_diag[k] : 0.0;
+    for (int c = lane; c < Mt; c += 32) {
+        double hx;
+        if (O) { hx = O[(size_t)pos * ldo + c]; HX[r + c] = hx; }     // the gauge rows gathered on the way
+        else hx = HX[r + c];
+        const double ha = zero ? 0.0 : hx - mu, dz = zero ? 0.0 : Zp[r + c] - hx;
+        const size_t o = (size_t)k * 2 * Mt + c;
+        Bc[o] = ha; Bc[o + Mt] = dz;
+        if (dinv_diag) { Y[o] = d * ha; Y[o + Mt] = d * dz; }
+    }
 }
 
 // (sum of the split-K partials of C) -> A = C0 + shift*I, B = C1, then (C0 + shift I) Z = C1 by Cholesky.
@@ -594,7 +628,8 @@ constexpr int SS_OFF_INVD = SS_OFF_BS + 64 * 9;            // invd [64]
 constexpr int SS_OFF_Z = SS_OFF_INVD + 64;                 // sZ   [64][72]
 constexpr int SS_OFF_D = SS_OFF_Z + 64 * SS_LDZ;           // sd   [64]
 constexpr int SS_OFF_LINV = SS_OFF_D + SS_KT;              // Linv [8][8][9] inverted diagonal blocks of the factor
-constexpr int SS_SMEM = (SS_OFF_LINV + 8 * 72) * 8;        // 223,744 bytes
+constexpr int SS_OFF_MISS = SS_OFF_LINV + 8 * 72;          // miss [4][2] 16-bit masks of missing rows (see load_tile)
+constexpr int SS_SMEM = (SS_OFF_MISS + 2) * 8;             // 223,760 bytes
 
 template <int NC>
 __global__ void __launch_bounds__(256, 1)
@@ -616,6 +651,12 @@ enkf_small_system_kernel(double* __restrict__ HX, const double* __restrict__ O, 
     double* sZ = ss + SS_OFF_Z;
     double* sd = ss + SS_OFF_D;
     double* Linv = ss + SS_OFF_LINV;
+    unsigned short* miss = reinterpret_cast<unsigned short*>(ss + SS_OFF_MISS);
+    // bit u: tile row 4u + q is a missing gauge (a NaN in either half of the row); its weight D^-1_k is read as 0
+    auto missing_rows = [&](int q) {
+        const unsigned w = reinterpret_cast<const unsigned*>(miss)[q];
+        return (w | (w >> 16)) & 0xffffu;
+    };
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int g = lane >> 2, t = lane & 3;
     const int mc = (((m + NC - 1) / NC) + 3) & ~3;                 // gauges per CTA
@@ -632,7 +673,10 @@ enkf_small_system_kernel(double* __restrict__ HX, const double* __restrict__ O, 
     stamp(0);
 
     // [HA | dz] of the gauges kt .. kt+63 -> sB (zero rows beyond k_hi), D^-1 -> sd; every load of a thread's
-    // elements is in flight before the first use
+    // elements is in flight before the first use.  A missing gauge (gauge_row_missing): its NaN observations become
+    // dz = 0 here, and the warp holding each half of the row (32 members) flags it with a ballot: one 16-bit mask per
+    // (row group tid / 64, half), rows 4u + tid / 64 -- no zeroing pass and no barrier beyond the one after the load;
+    // the product and W phases read the weight of a flagged row as 0.
     auto load_tile = [&](int kt) {
         const int c = tid & 63;
         int pos[16];
@@ -642,6 +686,7 @@ enkf_small_system_kernel(double* __restrict__ HX, const double* __restrict__ O, 
             pos[u] = k < k_hi ? __ldg(obs_pos + k) : -1;
         }
         double hx[16], zp[16], mu[16];
+        unsigned nan_rows = 0;
 #pragma unroll
         for (int u = 0; u < 16; ++u) {
             const int k = kt + (tid >> 6) + 4 * u;
@@ -664,10 +709,14 @@ enkf_small_system_kernel(double* __restrict__ HX, const double* __restrict__ O, 
         for (int u = 0; u < 16; ++u) {
             const int kk = (tid >> 6) + 4 * u, k = kt + kk;
             const bool on = pos[u] >= 0 && c < Mt;
+            const bool nan = obs_missing(zp[u]);                   // (zp = 0 off the matrix)
+            const unsigned any = __ballot_sync(0xffffffffu, nan);
             if (on && O) HX[(size_t)k * Mt + c] = hx[u];
             sB[kk * SS_LDB + c] = hx[u] - mu[u];
-            sB[kk * SS_LDB + 64 + c] = zp[u] - hx[u];
+            sB[kk * SS_LDB + 64 + c] = nan ? 0.0 : zp[u] - hx[u];
+            nan_rows |= (any != 0u ? 1u : 0u) << u;
         }
+        if (lane == 0) miss[warp] = (unsigned short)nan_rows;       // miss[2 (tid / 64) + half]
         if (tid < SS_KT) sd[tid] = dk;
     };
 
@@ -683,9 +732,10 @@ enkf_small_system_kernel(double* __restrict__ HX, const double* __restrict__ O, 
         load_tile(kt);
         __syncthreads();
         const int nk = min(SS_KT, (max(k_hi - kt, 0) + 3) & ~3);
+        const unsigned out_t = missing_rows(t);                   // rows kk + t: bit kk / 4
         for (int kk = 0; kk < nk; kk += 4) {
             const double* row = sB + (kk + t) * SS_LDB;
-            const double d = sd[kk + t];
+            const double d = (out_t >> (kk >> 2)) & 1u ? 0.0 : sd[kk + t];
             double a[2], b[8];
 #pragma unroll
             for (int i = 0; i < 2; ++i) a[i] = d * row[wm + 8 * i + g];
@@ -796,11 +846,12 @@ enkf_small_system_kernel(double* __restrict__ HX, const double* __restrict__ O, 
         const int k = kt + 8 * warp + g;
         if (k < k_hi) {
             const double d = sd[8 * warp + g];
+            const bool out = (missing_rows(g & 3) >> (2 * warp + (g >> 2))) & 1u;   // W = 0.0 exactly, not -0.0
 #pragma unroll
             for (int j = 0; j < 8; ++j) {
                 const int col = 8 * j + 2 * t;
-                if (col < Mt) W[(size_t)k * Mt + col] = d * (hrow[64 + col] - w[j][0]);
-                if (col + 1 < Mt) W[(size_t)k * Mt + col + 1] = d * (hrow[64 + col + 1] - w[j][1]);
+                if (col < Mt) W[(size_t)k * Mt + col] = out ? 0.0 : d * (hrow[64 + col] - w[j][0]);
+                if (col + 1 < Mt) W[(size_t)k * Mt + col + 1] = out ? 0.0 : d * (hrow[64 + col + 1] - w[j][1]);
             }
         }
     }
@@ -1526,9 +1577,9 @@ cudaError_t launch_dgemm_splitk(int transA, int transB, int M, int N, int K, con
 
 cudaError_t launch_innovation_cat(double* HX, const double* O, int ldo, const double* Zp, const double* mean,
                                   const int32_t* obs_pos, const double* dinv_diag, int m, int Mt, double* Bc, double* Y,
-                                  cudaStream_t st)
+                                  int* info, cudaStream_t st)
 {
-    innovation_cat_kernel<<<nblk((long long)m * Mt, 256), 256, 0, st>>>(HX, O, ldo, Zp, mean, obs_pos, dinv_diag, m, Mt, Bc, Y);
+    innovation_cat_kernel<<<nblk(m, 8), 256, 0, st>>>(HX, O, ldo, Zp, mean, obs_pos, dinv_diag, m, Mt, Bc, Y, info);
     count_launch();
     return cudaGetLastError();
 }
@@ -1627,10 +1678,10 @@ cudaError_t launch_enkf_stats(const double* X, int ld, int M, int64_t n, double 
     return cudaGetLastError();
 }
 
-cudaError_t launch_innovation(const double* HX, const double* Zp, const double* mean_obs, int m, int M, double* HA,
-                              double* dz, cudaStream_t st)
+cudaError_t launch_innovation(const double* HX, const double* Zp, const double* mean_obs, int m, int M, bool diag_R,
+                              double* HA, double* dz, int* info, cudaStream_t st)
 {
-    innovation_kernel<<<nblk((long long)m * M, 256), 256, 0, st>>>(HX, Zp, mean_obs, m, M, HA, dz);
+    innovation_kernel<<<nblk(m, 8), 256, 0, st>>>(HX, Zp, mean_obs, m, M, diag_R ? 1 : 0, HA, dz, info);
     count_launch();
     return cudaGetLastError();
 }

@@ -231,10 +231,14 @@ cudaError_t launch_dgemm(int transA, int transB, int M, int N, int K, double alp
                          const double* B, int ldb, double beta, double* C, int ldc, cudaStream_t st);
 cudaError_t launch_dgemm_splitk(int transA, int transB, int M, int N, int K, const double* A, int lda, const double* B,
                                 int ldb, double* Cpart, int ldc, int nsplit, long long pstride, cudaStream_t st);
+// A gauge whose observation row holds a NaN is missing at that update (txh_da.cu: gauge_row_missing).  The solve
+// leaves it out with a diagonal D; with a dense one it writes this value to the info word instead, which txh_check
+// reports.  It lies outside the pivots the other solves write there (1..m Cholesky, -1..-m Gauss-Jordan).
+constexpr int kInfoMissingObs = -0x7fffffff - 1;
 // O != nullptr: HX is gathered from the gauge rows of O on the way (and written out)
 cudaError_t launch_innovation_cat(double* HX, const double* O, int ldo, const double* Zp, const double* mean,
                                   const int32_t* obs_pos, const double* dinv_diag, int m, int Mt, double* Bc, double* Y,
-                                  cudaStream_t st);
+                                  int* info, cudaStream_t st);
 cudaError_t launch_chol_solve_small(const double* Cpart, int nsplit, long long pstride, int Mt, double shift, double* Z,
                                     int* info, cudaStream_t st);
 cudaError_t launch_enkf_small_system(double* HX, const double* O, int ldo, const double* Zp, const double* mean,
@@ -247,8 +251,9 @@ cudaError_t launch_woodbury_assemble(const double* Cpart, int nsplit, long long 
                                      double* C1, cudaStream_t st);
 cudaError_t launch_enkf_stats(const double* X, int ld, int M, int64_t n, double scale, const int32_t* gauge_of_pos,
                               double* rowsum, double* HX, cudaStream_t st);
-cudaError_t launch_innovation(const double* HX, const double* Zp, const double* mean_obs, int m, int M, double* HA,
-                              double* dz, cudaStream_t st);
+// diag_R: R (and D) diagonal, a missing gauge gets zero rows of HA and dz; otherwise it is reported through *info
+cudaError_t launch_innovation(const double* HX, const double* Zp, const double* mean_obs, int m, int M, bool diag_R,
+                              double* HA, double* dz, int* info, cudaStream_t st);
 cudaError_t launch_innov_cov_finish(double* S, const double* qs, const double* R, int m, double scale, cudaStream_t st);
 cudaError_t launch_spd_solve(double* S, double* B, int m, int k, int* info, cudaStream_t st);
 cudaError_t launch_inverse(double* A, double* W, int m, int* info, cudaStream_t st);

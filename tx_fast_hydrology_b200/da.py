@@ -71,6 +71,19 @@ class _MeasurementTable:
         self._meas_values = np.ascontiguousarray(frame.values, dtype=np.float64)
 
 
+def interpolate_gappy(x, xp, fp):
+    """`interpolate_sample` (linear) of a table with gaps: NaN entries of `fp` are missing values.  Entry j of the
+    result is NaN when a row with a NaN in column j has non-zero weight at `x`, else the interpolation of the rows with
+    weight, bitwise as `interpolate_sample` gives it for a table without NaN.  (`interpolate_sample` itself forms
+    (1 - frac) fp[ix-1] + frac fp[ix], so a NaN in the previous row would reach even the exact time of the next one
+    through 0 * NaN.)"""
+    fp = np.asarray(fp, dtype=np.float64)
+    gap = np.isnan(fp)
+    out = interpolate_sample(x, xp, np.where(gap, 0.0, fp))
+    out[interpolate_sample(x, xp, gap.astype(np.float64)) > 0] = np.nan
+    return out
+
+
 class KalmanFilter(_MeasurementTable, BaseCallback):
     def __init__(self, model, measurements, Q_cov, R_cov, P_t_init):
         import torch
@@ -327,11 +340,18 @@ class EnsembleKalmanFilter(_MeasurementTable, BaseCallback):
         self._torch = torch
         self.model = model
         self.reach_indices, perm = _gauge_setup(model, measurements)
-        self.measurements = measurements.iloc[:, perm]
-        self.num_measurements = m = self.measurements.shape[1]
+        m = measurements.shape[1]
         if np.shape(R_cov) != (m, m):
             raise ValueError(f'`R_cov` must be ({m}, {m}), got {np.shape(R_cov)}')
         self.reach_indices = np.ascontiguousarray(self.reach_indices, dtype=np.int64)
+        Rp = np.asarray(R_cov, dtype=np.float64)[perm, :][:, perm]
+        q = np.broadcast_to(np.asarray(Q_diag, dtype=np.float64), (model.n,))
+        # D = R + diag(Q[s,s]) never changes.  Diagonal, it lets an update leave out a gauge with a missing (NaN)
+        # observation exactly; dense, it does not, so a frame with gaps is refused here, before any device work.
+        D = Rp + np.diag(q[self.reach_indices])
+        self._dense_D = np.count_nonzero(D - np.diag(np.diagonal(D))) != 0
+        self.measurements = measurements.iloc[:, perm]
+        self.num_measurements = m
         self.every = every
         self.group = group
         self.rank, self.world = 0, 1
@@ -347,8 +367,6 @@ class EnsembleKalmanFilter(_MeasurementTable, BaseCallback):
             # first solve, after the assimilation loop has already routed a window
             raise ValueError(f'an ensemble Kalman filter needs at least 2 members in all, got {self.Mtot} '
                              f'({self.M} per rank x {self.world} ranks)')
-        Rp =np.asarray(R_cov, dtype=np.float64)[perm, :][:, perm]
-        q = np.broadcast_to(np.asarray(Q_diag, dtype=np.float64), (model.n,))
         self._R = torch.as_tensor(np.ascontiguousarray(Rp), device='cuda')
         self._qs = torch.as_tensor(np.ascontiguousarray(q[self.reach_indices]), device='cuda')
         self._noise = None
@@ -362,10 +380,9 @@ class EnsembleKalmanFilter(_MeasurementTable, BaseCallback):
         self._HX = torch.empty((m, self.M), **f64)
         self._HXall = torch.empty((m, Mt), **f64) if self.world > 1 else self._HX
         self._work = torch.empty(model.network.enkf_work_size(m, Mt), **f64)
-        # D = R + diag(Q[s,s]) never changes: its inverse (diagonal or dense) lets the update solve in
-        # ensemble space when the ensemble is smaller than the gauge network
-        D = Rp + np.diag(q[self.reach_indices])
-        if np.count_nonzero(D - np.diag(np.diagonal(D))) == 0:
+        # the inverse of D (diagonal or dense) lets the update solve in ensemble space when the ensemble is smaller
+        # than the gauge network
+        if not self._dense_D:
             self._Dinv, self._dinv_kind = torch.as_tensor(1.0 / np.diagonal(D), device='cuda').contiguous(), 1
         else:
             self._Dinv, self._dinv_kind = inverse(torch.as_tensor(np.ascontiguousarray(D), device='cuda').clone()), 2
@@ -432,6 +449,13 @@ class EnsembleKalmanFilter(_MeasurementTable, BaseCallback):
         self._sym = None
         self.update_path = 'allgather'
 
+    @_MeasurementTable.measurements.setter
+    def measurements(self, frame):
+        if getattr(self, '_dense_D', False) and np.isnan(np.asarray(frame.values, dtype=np.float64)).any():
+            raise ValueError('the measurements hold missing values (NaN): an ensemble update leaves out a missing gauge '
+                             'only when the observation covariance R_cov is diagonal')
+        _MeasurementTable.measurements.fset(self, frame)
+
     @property
     def latest_timestamp(self):
         return self.measurements.index[-1]
@@ -451,9 +475,11 @@ class EnsembleKalmanFilter(_MeasurementTable, BaseCallback):
         return self.filter() if self._due() else None
 
     def perturbed_observations(self, datetime):
-        """[m][Mtot] per-member observations at `datetime` (interpolated measurements + supplied noise)."""
+        """[m][Mtot] per-member observations at `datetime` (interpolated measurements + supplied noise).  A gauge
+        whose measurement is missing (NaN) at a table row with weight at `datetime` is NaN in every member: the update
+        leaves it out (interpolate_gappy)."""
         x = float(datetime.value)
-        Z = interpolate_sample(x, self._meas_times, self._meas_values)
+        Z = interpolate_gappy(x, self._meas_times, self._meas_values)
         Zp = np.repeat(Z[:, None], self.Mtot, axis=1)
         if self._noise is not None:
             flat = self._noise.reshape(self._noise.shape[0], -1)

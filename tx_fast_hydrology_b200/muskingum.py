@@ -488,7 +488,11 @@ class Muskingum:
         smoother, `smoothed` shaped like `rec`, as (rec, smoothed) or (rec, prior, smoothed): slot j (after step
         s = (j+1) record_every) conditioned on every update of the call after s up to s + smooth_lag, from the
         transforms the updates solved (txh_enks_smooth; DESIGN.md §4.4).  `rec` keeps the filtered hydrographs.  A
-        lag of at least `nsteps` gives the fixed-interval smoother.  Not for a member-sharded filter."""
+        lag of at least `nsteps` gives the fixed-interval smoother.  Not for a member-sharded filter.
+        Missing observations: a gauge whose row `observations[k][g]` holds a NaN (in any member) is left out of
+        update k -- the update is that of a filter without the gauge, its W row is 0 -- when the filter's D = R + Q[s,s]
+        is diagonal; with every gauge missing the posterior is the forecast.  With a dense R, `observations` holding a
+        NaN raise ValueError before any device work (DESIGN.md §4.4)."""
         if smooth_lag is not None:
             if isinstance(smooth_lag, bool) or not isinstance(smooth_lag, (int, np.integer)) or smooth_lag < 0:
                 raise ValueError(f'`smooth_lag` must be a non-negative integer number of steps, got {smooth_lag!r}')
@@ -498,12 +502,25 @@ class Muskingum:
                 raise ValueError('`smooth_lag` is not available for a member-sharded filter (smoothing one rank\'s '
                                  'members needs every rank\'s)')
         ridx = None if record_reaches is None else self._record_reaches(record_reaches, record_every, nsteps)
+        torch = _torch()
+        nwin = nsteps // every
+        if torch.is_tensor(observations) or isinstance(observations, np.ndarray):
+            want = (enkf.num_measurements, enkf.Mtot)
+            if observations.ndim != 3 or observations.shape[0] < nwin or tuple(observations.shape[1:]) != want:
+                raise ValueError(f'`observations` must be [>= {nwin}][{want[0]}][{want[1]}], got {tuple(observations.shape)}')
+        if enkf._dinv_kind != 1 and nwin:
+            # only a diagonal D lets an update leave out a missing gauge exactly (EnsembleKalmanFilter refuses a
+            # measurement frame with gaps for the same reason); refused before any device work
+            obs = observations[:nwin]
+            if (bool(torch.isnan(obs).any()) if torch.is_tensor(obs) else
+                    any(bool(torch.isnan(torch.as_tensor(o)).any()) for o in obs)):
+                raise ValueError('`observations` hold missing values (NaN): an ensemble update leaves out a missing '
+                                 'gauge only when the observation covariance R_cov is diagonal')
         torch = self._ensure_device()
         self._sync_coeffs()
         d, net, M = self._dev, self.network, self.members
         step_ns = int(self.timedelta.value)
         t = int(self.datetime.value)
-        nwin = nsteps // every
         rec = prior = None
         if ridx is not None:
             record_every = int(record_every)
@@ -520,10 +537,6 @@ class Muskingum:
             if T_hist is not None:
                 out += (net.enks_smooth(M, nwin, every, T_hist, rec, record_every, smooth_lag, torch.empty_like(rec)),)
             return out if len(out) > 1 else rec
-        if torch.is_tensor(observations) or isinstance(observations, np.ndarray):
-            want = (enkf.num_measurements, enkf.Mtot)
-            if observations.ndim != 3 or observations.shape[0] < nwin or tuple(observations.shape[1:]) != want:
-                raise ValueError(f'`observations` must be [>= {nwin}][{want[0]}][{want[1]}], got {tuple(observations.shape)}')
         if (enkf.world == 1 and torch.is_tensor(observations) and observations.is_cuda and observations.is_contiguous()
                 and observations.shape[0] >= nwin and observations.dtype == torch.float64):
             # one call: the loop below, in the library (txh_run_assimilating)
