@@ -443,6 +443,9 @@ int run_window(txh_net* net, double* O, double* I, int64_t M, const double* F, c
     const int64_t spl_max = std::min<int64_t>(64, std::max<int64_t>(16, (int64_t)((size_t(64) << 20) / (slot_row * sizeof(double)))));
     int64_t spl = std::min<int64_t>(spl_max, nsteps);
     while (spl > 1 && slot_row * spl * sizeof(double) > (size_t(1) << 30)) --spl;
+    // the kernel addresses the ring cells of a whole launch by 32-bit byte offsets (txh_window.cu: InStream): one step
+    // is below 4 GiB (window_fit) and several stay below 1 GiB (above), so this holds; it must keep holding
+    if (slot_row * spl * sizeof(double) >= (size_t(1) << 32)) return fail(TXH_E_INVALID, "window ring beyond 32-bit offsets");
     // every cell starts EMPTY (all bits set); consumers put EMPTY back, so a finished launch leaves the whole
     // ring EMPTY again whatever row stride the next launch lays over it
     int rc;

@@ -79,14 +79,14 @@ constexpr uint32_t kIdMask = 0x3fffffffu;
 
 // Hand-over protocol (EMPTY, txh_device.cuh): the consumer polls the 16 bytes of its own two member columns until
 // neither is EMPTY.  No flags, no fences: a lane only ever depends on the cell the same lane of the producer wrote.
-// Polls `cell` (this lane's 16 bytes of a ring row) until it is full; `v` is what an earlier read saw.
-// Returns false when the launch is being abandoned (watchdog / poisoned handle).  (Moving the polling loop into a
-// function of its own to shrink the dozen walks that inline it costs 40 us per launch: the call spills the walk's
-// registers.)
-__device__ __forceinline__ bool wait_cell(const WinArgs& a, const double* cell, bool active, double2& v, int lane)
+// The fast path of a consumer is one warp vote on what it already read (cell_ready); only when that fails does it poll
+// `cell` (this lane's 16 bytes of a ring row) until it is full; `v` is what the earlier read saw.  Returns false when
+// the launch is being abandoned (watchdog / poisoned handle).  (Moving the polling loop into a function of its own to
+// shrink the dozen walks that inline it costs 40 us per launch: the call spills the walk's registers.)
+__device__ __forceinline__ bool cell_ready(double2 v, unsigned dead) { return __all_sync(0xffffffffu, cell_full(v) || dead != 0u); }
+__device__ __forceinline__ bool poll_cell(const WinArgs& a, const double* cell, double2& v, int lane)
 {
-    bool ok = !active || cell_full(v);
-    if (__all_sync(0xffffffffu, ok)) return true;
+    bool ok = cell_full(v);
     unsigned spins = 0, nap = (unsigned)a.nap_min;
     unsigned long long t0 = 0;
     for (;;) {
@@ -104,44 +104,46 @@ __device__ __forceinline__ bool wait_cell(const WinArgs& a, const double* cell, 
 }
 
 // Rows handed over by other tasks, consumed in a fixed order every step: a continuous stream (step, index)
-// prefetched D rows ahead through a shared-memory ring, across step boundaries.  One cp.async group per row.
-// A prefetch that came too early sees EMPTY and the consumer falls back to polling the cell itself.
-// The list holds byte offsets of the slots inside one step of the ring.
+// prefetched D rows ahead through a shared-memory ring of D cells, across step boundaries.  One cp.async group per
+// position, empty past the end of the stream, so exactly D groups are in flight at every consume and the row read
+// leaves its ring cell to the row D positions ahead.  A prefetch that came too early sees EMPTY and the consumer polls
+// the cell itself.  Every step consumes the same nL rows, so all offsets are relative to the ring step being consumed
+// (`ringS`): the consumer's is in its input word (stream_word), the producer's in the issue list, which the task load
+// fills with the offset of position k + D for the consume at position k (ahead by r steps: + r * step_bytes; past the
+// last step of the launch: ~0).  Every offset stays below the size of the launch's ring, which run_window keeps below
+// 4 GiB (one step: window_fit; several: at most 1 GiB) and checks.
 struct InStream {
-    int in_flight;             // rows issued and not yet consumed
-    int pi, ci;                // index of the next row to issue / consume within its step
-    int psteps;                // steps left to issue (including the current one)
-    unsigned slot_i, slot_c;   // byte offsets of the ring cells of the next issue / next consume
-    char* pbase;               // this lane's columns of the ring step being issued / consumed
-    char* cbase;
-    bool dead;                 // the launch is being abandoned: stop waiting
+    unsigned cell;             // shared address of the ring cell of the next consume (and of the issue after it)
+    unsigned pl;               // shared address of the next issue-list entry (reset to the list every step)
+    unsigned plim;             // issue-list offsets below this lie in a step of the launch
+    unsigned dead;             // not 0: the launch is being abandoned, stop waiting
 };
 
-template <int D>
-__device__ __forceinline__ void stream_issue(InStream& st, const WinArgs& a, unsigned ring_sa, unsigned list_sa, int nL,
-                                             size_t step_bytes, bool active)
-{
-    if (active) cp_async16(ring_sa + st.slot_i, st.pbase + lds_u32(list_sa + 4u * st.pi));
-    cp_async_commit();
-    st.slot_i = st.slot_i + 512u == D * 512u ? 0u : st.slot_i + 512u;
-    ++st.in_flight;
-    if (++st.pi == nL) { st.pi = 0; --st.psteps; st.pbase += step_bytes; }
-}
+// A stream input word after the task load: WIN_SLOT | (byte offset of the slot in a ring step) >> 4
+__device__ __forceinline__ uint32_t stream_word(uint32_t off) { return WIN_SLOT | (off >> 4); }
+__device__ __forceinline__ uint32_t stream_off(uint32_t w) { return w << 4; }
 
 template <int D>
-__device__ __forceinline__ double2 stream_next(InStream& st, const WinArgs& a, unsigned ring_sa, unsigned list_sa, int nL,
-                                               size_t step_bytes, bool active, int lane)
+__device__ __forceinline__ void stream_issue(InStream& st, unsigned ring_sa, const char* ringS, uint32_t off, bool valid)
 {
-    if (st.in_flight >= D) cp_async_wait_group<D - 1>();                // the oldest of D rows in flight
-    else cp_async_wait_all();
-    double2 v = lds_row(ring_sa + st.slot_c);
-    double* cell = reinterpret_cast<double*>(st.cbase + lds_u32(list_sa + 4u * st.ci));
-    if (!st.dead && !wait_cell(a, cell, active, v, lane)) st.dead = true;
-    if (active) st_row(cell, empty_row());
-    st.slot_c = st.slot_c + 512u == D * 512u ? 0u : st.slot_c + 512u;
-    --st.in_flight;
-    if (++st.ci == nL) { st.ci = 0; st.cbase += step_bytes; }
-    if (st.psteps > 0) stream_issue<D>(st, a, ring_sa, list_sa, nL, step_bytes, active);
+    if (valid) cp_async16(st.cell, ringS + off);
+    cp_async_commit();
+    st.cell = st.cell + 512u == ring_sa + D * 512u ? ring_sa : st.cell + 512u;
+}
+
+// the row of input word w: consume it, put EMPTY back, issue the position D ahead into the cell it leaves
+template <int D>
+__device__ __forceinline__ double2 stream_next(InStream& st, const WinArgs& a, unsigned ring_sa, char* ringS, uint32_t w,
+                                               int lane)
+{
+    cp_async_wait_group<D - 1>();                                     // the oldest of the D positions in flight
+    double2 v = lds_row(st.cell);
+    double* cell = reinterpret_cast<double*>(ringS + stream_off(w));
+    if (!cell_ready(v, st.dead) && !poll_cell(a, cell, v, lane)) st.dead = 1u;
+    const uint32_t pe = lds_u32(st.pl);                               // (read after the polling loop: not live across it)
+    st_row(cell, empty_row());
+    st.pl += 4u;
+    stream_issue<D>(st, ring_sa, ringS, pe, pe < st.plim);
     return v;
 }
 
@@ -206,9 +208,9 @@ __device__ __forceinline__ double2 forcing_q(const FCtx& c, double g0, double g1
 // per-task context
 struct Tk {
     unsigned sP, sScr, sIn, sRec, sCum, sCumC, sWords, sList;
-    int len, n_in, nL, col, lane, begin, ld;
+    int len, n_in, col, lane, begin, ld;
     unsigned ldb;              // bytes of a ring row (ld doubles; a ring step stays below 4 GiB, see window_fit)
-    bool active;
+    bool active;               // col < ld; an inactive lane aliases lane 0's columns (ccol), so every store of its own must test this
     double* Ig;
     double* Og;
     size_t step_bytes;
@@ -262,7 +264,7 @@ __device__ __forceinline__ void pocket_step(const WinArgs& a, const Tk& tk, InSt
             for (uint32_t k = (h >> 6) & 0x1ffffffu; k > 0; --k) {
                 const uint32_t w = lds_u32(aW);
                 aW += 4u;
-                const double2 v = (w & WIN_SLOT) ? stream_next<IR>(ist, a, tk.sIn, tk.sList, tk.nL, tk.step_bytes, tk.active, tk.lane)
+                const double2 v = (w & WIN_SLOT) ? stream_next<IR>(ist, a, tk.sIn, ringS, w, tk.lane)
                                                  : lds_row(tk.sScr + (w << 9));
                 inflow.x += v.x; inflow.y += v.y;
             }
@@ -317,7 +319,7 @@ template <bool LAST, bool HAS_F, bool HAS_W, int SR, bool REC>
 __device__ __forceinline__ void segment_step(const WinArgs& a, const Tk& tk, InStream& ist, const FCtx& fc, char* ringS,
                                              int out_slot, unsigned long long* trs, int rj)
 {
-    unsigned aRec = tk.sRec, aP = tk.sP;
+    unsigned aRec = tk.sRec, aP = tk.sP, aW = tk.sWords + 4u * tk.n_in;   // the side words follow the entering ones
     double* ig = tk.Ig;
     double* og = tk.Og;
     double2 B = make_double2(0.0, 0.0);
@@ -329,7 +331,8 @@ __device__ __forceinline__ void segment_step(const WinArgs& a, const Tk& tk, InS
         double2 inflow = (h & HDR_ACC) ? B : make_double2(0.0, 0.0);   // side_k + B_{k-1}
         double2 side = make_double2(0.0, 0.0);
         for (uint32_t k = (h >> 6) & 0x1fffu; k > 0; --k) {
-            const double2 v = stream_next<SR>(ist, a, tk.sScr, tk.sList, tk.nL, tk.step_bytes, tk.active, tk.lane);
+            const double2 v = stream_next<SR>(ist, a, tk.sScr, ringS, lds_u32(aW), tk.lane);
+            aW += 4u;
             side.x += v.x; side.y += v.y;
         }
         inflow.x += side.x; inflow.y += side.y;
@@ -354,10 +357,10 @@ __device__ __forceinline__ void segment_step(const WinArgs& a, const Tk& tk, InS
     // hop
     double2 oin = make_double2(0.0, 0.0);
     for (int k = 0; k < tk.n_in; ++k) {
-        double* cell = reinterpret_cast<double*>(ringS + (size_t)(lds_u32(tk.sWords + 4u * k) & kIdMask) * tk.ld * sizeof(double));
-        double2 v = tk.active ? ld_relaxed_row(cell) : make_double2(0.0, 0.0);
-        if (!ist.dead && !wait_cell(a, cell, tk.active, v, tk.lane)) ist.dead = true;
-        if (tk.active) st_row(cell, empty_row());
+        double* cell = reinterpret_cast<double*>(ringS + stream_off(lds_u32(tk.sWords + 4u * k)));
+        double2 v = ld_relaxed_row(cell);
+        if (!cell_ready(v, ist.dead) && !poll_cell(a, cell, v, tk.lane)) ist.dead = 1u;
+        st_row(cell, empty_row());
         oin.x += v.x; oin.y += v.y;
     }
     const double Al = lds_f64(tk.sCum + 8u * (tk.len - 1));
@@ -578,7 +581,11 @@ route_window_kernel(const WinArgs a)
     auto stage_T = [&]() {
         griddep_wait();
         const int nw = blockDim.x >> 5;
-        for (int e = warp * 32 + lane; e < 64 * 64; e += nw * 32) {
+        // the thread index is read here, not formed from `warp` and `lane`: ptxas otherwise computes the bounds of the
+        // first elements at kernel entry and holds them across the task loop (a spill in the UPD + REC instantiation)
+        unsigned tid;
+        asm volatile("mov.u32 %0, %%tid.x;" : "=r"(tid));
+        for (int e = (int)tid; e < 64 * 64; e += nw * 32) {
             const int k = e >> 6, c = e & 63;
             sts_f64(sT + t_swz(k, c), (k < a.M && c < a.M) ? __ldcg(a.upT + (size_t)k * a.M + c) : 0.0);
         }
@@ -606,7 +613,9 @@ route_window_kernel(const WinArgs a)
         const int len = td.len;
         const int col = mb * kMemberBlock + lane * 2;
         const bool active = col < ld;
-        const int ccol = active ? col : 0;
+        // a lane past the last member column shadows lane 0 of its warp: the same ring cells, prefetched, polled and put
+        // back EMPTY with the same values (after the vote, so never before lane 0 has its row), no stores of its own
+        const int ccol = active ? col : mb * kMemberBlock;
         tk.len = len; tk.n_in = td.n_in; tk.col = col; tk.active = active; tk.begin = td.begin;
         tk.Og = a.O + (size_t)td.begin * ld + ccol;
         tk.Ig = a.I + (size_t)td.begin * ld + ccol;
@@ -705,18 +714,34 @@ route_window_kernel(const WinArgs a)
             __syncwarp();
             if (REC && (a.rec_prior || a.rec_post)) record_posterior(a, tk.sRec, sT, task, td.begin, len, lane);
         }
-        // rows of other tasks consumed through the input ring, in consumption order: byte offsets of their slots
+        // rows of other tasks consumed through the input ring (InStream): nL per step; every slot word becomes the byte
+        // offset of its slot (stream_word), and the issue list gets, for the consume at position q - D, the offset of
+        // position q (r steps ahead of that consume)
+        const bool seg = td.kind == WTASK_SEG;
+        const int D = seg ? SR : IR;
         int nL = 0;
         for (int base = 0; base < td.n_words; base += 32) {
             const int i = base + lane;
             const uint32_t w = i < td.n_words ? lds_u32(tk.sWords + 4u * i) : 0u;
+            nL += __popc(__ballot_sync(0xffffffffu, (w & WIN_SLOT) != 0u && i >= td.n_in));
+        }
+        for (int base = 0, q0 = 0; base < td.n_words; base += 32) {
+            const int i = base + lane;
+            const uint32_t w = i < td.n_words ? lds_u32(tk.sWords + 4u * i) : 0u;
             const bool is = (w & WIN_SLOT) != 0u && i >= td.n_in;
             const unsigned m = __ballot_sync(0xffffffffu, is);
-            if (is) sts_u32(tk.sList + 4u * (nL + __popc(m & ((1u << lane) - 1u))), (w & kIdMask) * (unsigned)(ld * sizeof(double)));
-            nL += __popc(m);
+            if (w & WIN_SLOT) {
+                const uint32_t off = (w & kIdMask) * tk.ldb;
+                sts_u32(tk.sWords + 4u * i, stream_word(off));
+                if (is) {
+                    int j = q0 + __popc(m & ((1u << lane) - 1u)) - D, r = 0;
+                    while (j < 0) { j += nL; ++r; }
+                    sts_u32(tk.sList + 4u * j, r < a.nsteps ? off + (uint32_t)r * (uint32_t)tk.step_bytes : ~0u);
+                }
+            }
+            q0 += __popc(m);
         }
         __syncwarp();
-        tk.nL = nL;
         int cur_r0 = -1, cur_r1 = -1;
         if (tr && lane == 0) tr[1] = globaltimer_ns();
         // per-step forcing weights of this lane's two members: (w0*mul[r0][m], w1*mul[r1][m]), muskingum.py:528-531
@@ -739,21 +764,32 @@ route_window_kernel(const WinArgs a)
             return c;
         };
         FCtx fc_next = load_fctx(0);
-        const bool seg = td.kind == WTASK_SEG;
         const unsigned ring_sa = seg ? tk.sScr : tk.sIn;
+        char* const ring0 = reinterpret_cast<char*>(a.ring + ccol);
         InStream ist;
-        ist.in_flight = 0; ist.pi = ist.ci = 0; ist.slot_i = ist.slot_c = 0u; ist.dead = false;
-        ist.psteps = nL > 0 ? a.nsteps : 0;
-        ist.pbase = reinterpret_cast<char*>(a.ring + ccol);
-        ist.cbase = ist.pbase;
-        for (int j = 0; j < (seg ? SR : IR) && ist.psteps > 0; ++j) {
-            if (seg) stream_issue<SR>(ist, a, ring_sa, tk.sList, nL, tk.step_bytes, active);
-            else stream_issue<IR>(ist, a, ring_sa, tk.sList, nL, tk.step_bytes, active);
+        ist.cell = ring_sa; ist.dead = 0u;
+        if (nL > 0) {
+            // the first D positions: the slot words in order, round after round (one ring step further each round)
+            const unsigned w0 = tk.sWords + 4u * td.n_in, w1 = tk.sWords + 4u * td.n_words;
+            size_t soff = 0;
+            unsigned aw = w0;
+            for (int j = 0, r = 0; j < D;) {
+                const uint32_t w = lds_u32(aw);
+                if (w & WIN_SLOT) {
+                    if (seg) stream_issue<SR>(ist, ring_sa, ring0 + soff, stream_off(w), r < a.nsteps);
+                    else stream_issue<IR>(ist, ring_sa, ring0 + soff, stream_off(w), r < a.nsteps);
+                    ++j;
+                }
+                aw += 4;
+                if (aw == w1) { aw = w0; soff += tk.step_bytes; ++r; }
+            }
         }
 
         for (int s = 0; s < a.nsteps; ++s) {
             const bool last = s + 1 == a.nsteps;                   // outflows and inflows go to global memory
-            char* ringS = reinterpret_cast<char*>(a.ring + ccol) + (size_t)s * tk.step_bytes;
+            char* ringS = ring0 + (size_t)s * tk.step_bytes;
+            ist.pl = tk.sList;
+            ist.plim = (uint32_t)((size_t)(a.nsteps - s) * tk.step_bytes);
             const FCtx fc = fc_next;
             int rj = -1;                                          // index of this step in rec_out, if it is recorded
             if (REC) {
@@ -786,7 +822,7 @@ route_window_kernel(const WinArgs a)
                 if (last) segment_step<true, HAS_F, HAS_W, SR, REC>(a, tk, ist, fc, ringS, td.out_slot, trs, rj);
                 else segment_step<false, HAS_F, HAS_W, SR, REC>(a, tk, ist, fc, ringS, td.out_slot, trs, rj);
             }
-            if (ist.dead) break;
+            if (ist.dead != 0u) break;
         }
         cp_async_wait_all();
         if (tr && lane == 0) {
