@@ -267,6 +267,22 @@ int txh_get_route_timings(txh_net* net, double* ms_out, int64_t capacity, int64_
  * the transforms of a call survive it (txh_enks_smooth).  A call whose (nsteps / every) * M * M exceeds
  * capacity_doubles fails with TXH_E_INVALID before any device work.  NULL switches it off. */
 int txh_set_transform_history(txh_net* net, double* T_hist_dev, int64_t capacity_doubles);
+/* The form of the ensemble update every later txh_enkf_solve and txh_run_assimilating(_rec) on the handle solves:
+ *   kind 0 (default): the stochastic (perturbed-observation) EnKF, the solve as described at txh_enkf_solve;
+ *   kind 1: the square-root ETKF (Hunt et al. 2007).  The solve must be given identical observation columns,
+ *     Zp[g][c] = z[g] (no perturbations); it then leaves T = wbar 1^T - I + G with G = (Mtot-1) (C0 + (Mtot-1) I)^-1
+ *     (SPD, spectrum in (0, 1], G 1 = 1) and row means Wbar of W, and is followed by one more launch that rewrites
+ *     T <- wbar 1^T + (1 - rtpp) (G^1/2 - I) and W[g][c] <- Wbar[g], in place.  Mtot <= 64.
+ *   rtpp in [0, 1): relaxation to prior perturbations (Zhang et al. 2004).  With kind 0 and rtpp > 0, every row of T
+ *     and of W becomes mean + (1 - rtpp) (row - mean): the posterior anomalies of every reach are (1 - rtpp) times
+ *     the stochastic filter's plus rtpp times the prior's, and the mean is the stochastic filter's.
+ * Every consumer of T and W (txh_enkf_apply(_peers), the routing launch that applies an owed update, the recorded
+ * rows, the transform history, txh_enks_smooth -- with ETKF transforms the ETKS) reads the final form.  Missing gauges
+ * carry over: with every gauge missing T' = 0 and W' = 0.  kind 0 with rtpp 0 adds no launch and changes no bit.
+ * TXH_E_INVALID for another kind or an rtpp outside [0, 1) (the handle keeps its setting), and -- before any device
+ * work -- for a solve or assimilating run with kind 1 and more than 64 members in all.  An ETKF eigensolve that does
+ * not converge (20 Jacobi sweeps) is reported by txh_check. */
+int txh_set_enkf_transform(txh_net* net, int kind /* 0 stochastic, 1 ETKF */, double rtpp /* [0, 1) */);
 
 /* ---- ensemble Kalman smoother of recorded hydrographs ----------------------------------------------------------------
  * Fixed-lag EnKS of the slots txh_run_assimilating_rec recorded, from the transforms it kept (txh_set_transform_history):
@@ -333,7 +349,8 @@ int txh_kfb_filter(txh_kfb* b, const uint8_t* active_host, const double* z_host,
 /* Synchronise `stream` and report a poisoned launch (TXH_E_WATCHDOG), an innovation covariance that was
  * not positive definite in an earlier txh_enkf_solve (TXH_E_INVALID), a missing (NaN) observation given to an earlier
  * txh_enkf_solve or txh_run_assimilating(_rec) with a non-diagonal observation covariance (dinv_kind 0 or 2;
- * TXH_E_INVALID, "missing observation ... non-diagonal observation covariance"), or a CUDA fault.  The report clears
+ * TXH_E_INVALID, "missing observation ... non-diagonal observation covariance"), a square-root (ETKF) transform whose
+ * eigensolve did not converge (TXH_E_INVALID, "square-root (ETKF) transform did not converge"), or a CUDA fault.  The report clears
  * the record: the next solve on the handle is unaffected. */
 int txh_check(txh_net* net, void* stream);
 

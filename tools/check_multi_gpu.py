@@ -7,7 +7,9 @@ Every rank routes its M members of a synthetic network for a few hourly windows 
 (row sums all-reduced and gauge rows all-gathered over NCCL; the transform reads the other shards' state rows in
 place over NVLink -- TXH_MEMBER_UPDATE=peers, the default -- or after an NCCL all-gather -- =allgather); rank 0
 also runs all N*M members unsharded and compares the gathered shards with it (FP64, element-wise relative error
-<= 1e-9 with the forecast-scale floor of tests/parity.py).  Both update paths are run."""
+<= 1e-9 with the forecast-scale floor of tests/parity.py).  Both update paths are run, with the stochastic filter
+and, from two GPUs on, with the square-root filter (method='etkf', rtpp 0.3, the same observation in every member):
+every rank post-processes the same Mtot x Mtot system."""
 import os
 import sys
 
@@ -47,29 +49,33 @@ def main():
     mdf = pd.DataFrame(meas, index=idx, columns=[d0["reach_ids"][j] for j in gidx])
     R = 1e-2 * np.eye(m)
     q = rng.uniform(0.5, 2.0, size=n)
-    Zp = np.ascontiguousarray(meas[:, :, None] + 0.1 * rng.standard_normal((nwin, m, Mt)))
+    Zp = {"stochastic": np.ascontiguousarray(meas[:, :, None] + 0.1 * rng.standard_normal((nwin, m, Mt))),
+          "etkf": np.ascontiguousarray(np.repeat(meas[:, :, None], Mt, axis=2))}
 
     from parity import relerr
 
-    def run(cols, group):
+    def run(cols, group, method):
         d = dict(d0); d["o_t"] = np.ascontiguousarray(o_all[:, cols])
         mdl = Muskingum(d, members=len(cols))
-        enkf = EnsembleKalmanFilter(mdl, mdf, q, R, group=group)
+        enkf = EnsembleKalmanFilter(mdl, mdf, q, R, group=group, method=method, rtpp=0.3 if method == "etkf" else 0.0)
         path = enkf.update_path
         f = mdl.make_forcing(times_ns=times, table=table, member_mul=np.ascontiguousarray(mul_all[:, cols]))
-        mdl.run_assimilating(f, every * nwin, enkf, every, torch.as_tensor(Zp[:, :, :enkf.Mtot], device="cuda"))
+        mdl.run_assimilating(f, every * nwin, enkf, every, torch.as_tensor(Zp[method][:, :, :enkf.Mtot], device="cuda"))
         mdl.network.check()
         enkf.release_peers()                                         # collective on the peer-read path
         return mdl.o_t_next.reshape(n, -1), mdl.i_t_next.reshape(n, -1), path
 
     ok = True
     cols = list(range(rank * M, (rank + 1) * M))
-    o_ref = i_ref = None
-    if rank == 0:
-        o_ref, i_ref, _ = run(list(range(Mt)), singles[0])          # the whole ensemble on one GPU
-    for want in ("peers", "allgather"):
+    methods = ["stochastic"] + (["etkf"] if world >= 2 else [])
+    if world < 2 and rank == 0:
+        print("multi-GPU check: the ETKF case needs two GPUs: skipped", flush=True)
+    for method, want in [(a, b) for a in methods for b in ("peers", "allgather")]:
+        o_ref = i_ref = None
+        if rank == 0:
+            o_ref, i_ref, _ = run(list(range(Mt)), singles[0], method)   # the whole ensemble on one GPU
         os.environ["TXH_MEMBER_UPDATE"] = want
-        o_loc, i_loc, path = run(cols, None)                         # sharded: default group = all ranks
+        o_loc, i_loc, path = run(cols, None, method)                 # sharded: default group = all ranks
         parts = [torch.empty((n, 2 * M), dtype=torch.float64, device="cuda") for _ in range(world)] if rank == 0 else None
         mine = torch.as_tensor(np.concatenate([o_loc, i_loc], axis=1), device="cuda")
         dist.gather(mine, parts, dst=0)
@@ -82,7 +88,7 @@ def main():
             eo, ei = relerr(o_sh, o_ref, scale=so), relerr(i_sh, i_ref, scale=si)
             good = eo <= 1e-9 and ei <= 1e-9 and path == want
             ok = ok and good
-            print(f"multi-GPU check: world={world} members={Mt} n={n} update_path={path} (asked {want})  "
+            print(f"multi-GPU check: {method} world={world} members={Mt} n={n} update_path={path} (asked {want})  "
                   f"max rel err o={eo:.2e} i={ei:.2e}  {'OK' if good else 'FAIL'}", flush=True)
         dist.barrier()
     flag = torch.tensor([1.0 if ok else 0.0], device="cuda")

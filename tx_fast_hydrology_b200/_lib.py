@@ -80,6 +80,7 @@ SIGNATURES = {
                                                 c_vp, c_vp, c_i64, c_vp, p_i64, c_i64, c_i64, c_vp, c_vp, c_vp]),
     "txh_get_route_timings": (ctypes.c_int, [c_vp, p_f64, c_i64, p_i64]),
     "txh_set_transform_history": (ctypes.c_int, [c_vp, c_vp, c_i64]),
+    "txh_set_enkf_transform": (ctypes.c_int, [c_vp, ctypes.c_int, c_f64]),
     "txh_enks_work_size": (c_i64, [c_i64, c_i64]),
     "txh_enks_smooth": (ctypes.c_int, [c_i64, c_i64, c_i64, c_vp, c_i64, c_i64, c_i64, c_i64, c_vp, c_vp, c_vp, c_vp]),
     "txh_dgemm": (ctypes.c_int, [ctypes.c_int, ctypes.c_int, c_i64, c_i64, c_i64, c_f64, c_vp, c_i64, c_vp, c_i64,

@@ -143,6 +143,8 @@ struct txh_net {
     double stats_scale = 1.0;
     double* T_hist = nullptr;           // txh_set_transform_history: update k of a run_assimilating call solves into
     int64_t T_hist_cap = 0;             // T_hist + k*M*M (capacity in doubles)
+    int enkf_kind = 0;                  // txh_set_enkf_transform: 0 stochastic, 1 ETKF (square root)
+    double enkf_rtpp = 0.0;             // relaxation to prior perturbations, [0, 1)
     std::vector<std::pair<cudaEvent_t, cudaEvent_t>> route_events;   // txh_run_assimilating(time_every > 0)
 };
 
@@ -268,6 +270,9 @@ int report_status(txh_net* net, cudaStream_t st)
     if (info == kInfoMissingObs)
         return fail(TXH_E_INVALID, "a missing observation (NaN) with a non-diagonal observation covariance: an ensemble "
                                    "update can leave out a gauge only when R is diagonal");
+    if (info == kInfoEtkfNoConvergence)
+        return fail(TXH_E_INVALID, "the square-root (ETKF) transform did not converge: the Jacobi eigensolve of the "
+                                   "ensemble-space matrix stopped at its sweep limit (a non-finite T or W?)");
     if (info > 0)
         return fail(TXH_E_INVALID, "an ensemble innovation covariance was not positive definite (Cholesky pivot " +
                                    std::to_string(info) + ")");
@@ -1288,6 +1293,23 @@ int64_t txh_enkf_work_size(int64_t m, int64_t Mtot)
 }  // extern "C"
 
 namespace {
+// the transform set on the handle (txh_set_enkf_transform) for an ensemble of Mtot members
+int check_enkf_transform(const txh_net* net, int64_t Mtot)
+{
+    if (net->enkf_kind == 1 && Mtot > 64)
+        return fail(TXH_E_INVALID, "the square-root (ETKF) transform takes at most 64 members in all, got " +
+                                   std::to_string(Mtot));
+    return TXH_OK;
+}
+
+// what every solve path ends with: the square-root or relaxed form of (T, W), in place; the default adds no launch
+int transform_post(txh_net* net, int64_t m, int64_t Mtot, double* W, double* T, cudaStream_t st)
+{
+    if (net->enkf_kind == 0 && net->enkf_rtpp == 0.0) return TXH_OK;
+    CU(launch_enkf_transform_post(T, W, (int)Mtot, (int)m, net->enkf_kind, net->enkf_rtpp, info_word(net), st));
+    return TXH_OK;
+}
+
 // txh_enkf_solve; with O_gather the gauge rows HX are gathered from the state (unsharded ensemble, ld = row stride of
 // Mtot members) inside the first kernel instead of by a launch of their own
 int enkf_solve_impl(txh_net* net, int64_t m, int64_t Mtot, double* HX, const double* O_gather, const double* Zp,
@@ -1298,6 +1320,7 @@ int enkf_solve_impl(txh_net* net, int64_t m, int64_t Mtot, double* HX, const dou
         return fail(TXH_E_INVALID, "bad argument");
     if (dinv_kind < 0 || dinv_kind > 2 || (dinv_kind != 0 && !Dinv)) return fail(TXH_E_INVALID, "bad D^-1 argument");
     int rc;
+    if ((rc = check_enkf_transform(net, Mtot))) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     if ((rc = ensure_device(net))) return rc;
     int32_t* d_pos = nullptr;
@@ -1310,7 +1333,7 @@ int enkf_solve_impl(txh_net* net, int64_t m, int64_t Mtot, double* HX, const dou
             // one cluster launch: gather, split-K product, reduction, Cholesky solve and W (txh_da.cu)
             CU(launch_enkf_small_system(HX, O_gather, (int)txh_row_stride(Mtot), Zp, mean, d_pos, Dinv, (int)m, Mt,
                                         (double)(Mtot - 1), T, W, info_word(net), st));
-            return TXH_OK;
+            return transform_post(net, m, Mtot, W, T, st);
         }
         double* Bc = work;                                  // [m][2Mt] = [HA | dz]
         double* Y = Bc + 2 * m * Mtot;                      // [m][2Mt] = D^-1 Bc
@@ -1344,7 +1367,7 @@ int enkf_solve_impl(txh_net* net, int64_t m, int64_t Mtot, double* HX, const dou
                         T, (int)Mtot, st));
     }
     // asynchronous: a failed factorisation leaves a non-zero info word that txh_check reports
-    return TXH_OK;
+    return transform_post(net, m, Mtot, W, T, st);
 }
 }  // namespace
 
@@ -1438,6 +1461,8 @@ int txh_run_assimilating_rec(txh_net* net, double* O, double* I, int64_t M, cons
         return fail(TXH_E_INVALID, "bad recording arguments");
     if (net->T_hist && (nsteps / every) * M * M > net->T_hist_cap)
         return fail(TXH_E_INVALID, "the transform history holds fewer than nsteps / every transforms of M x M");
+    int rc;
+    if ((rc = check_enkf_transform(net, M))) return rc;
     // segments: nwin windows of `every` steps, each followed by an update, then the remaining steps
     const int64_t nwin = nsteps / every, nseg = nwin + (nsteps > nwin * every ? 1 : 0);
     auto seg_steps = [&](int64_t k) { return k < nwin ? every : nsteps - nwin * every; };
@@ -1445,7 +1470,6 @@ int txh_run_assimilating_rec(txh_net* net, double* O, double* I, int64_t M, cons
     if (nwin > 0 && every > (1 << 24)) return fail(TXH_E_INVALID, "nsteps out of range");
     if (fo && fo->net != net) return fail(TXH_E_INVALID, "forcing belongs to another network");
     if (fo && fo->d_W && fo->M != M) return fail(TXH_E_INVALID, "forcing member multipliers do not match M");
-    int rc;
     if ((rc = check_M(M))) return rc;
     const bool rec = rec_count > 0;
     if (rec) {
@@ -1535,6 +1559,15 @@ int txh_set_transform_history(txh_net* net, double* T_hist, int64_t capacity)
     if (!net) return fail(TXH_E_INVALID, "null argument");
     if (T_hist && capacity < 0) return fail(TXH_E_INVALID, "negative transform history capacity");
     net->T_hist = T_hist; net->T_hist_cap = T_hist ? capacity : 0;
+    return TXH_OK;
+}
+
+int txh_set_enkf_transform(txh_net* net, int kind, double rtpp)
+{
+    if (!net) return fail(TXH_E_INVALID, "null argument");
+    if (kind != 0 && kind != 1) return fail(TXH_E_INVALID, "ensemble transform kind must be 0 (stochastic) or 1 (ETKF)");
+    if (!(rtpp >= 0.0 && rtpp < 1.0)) return fail(TXH_E_INVALID, "relaxation to prior perturbations must lie in [0, 1)");
+    net->enkf_kind = kind; net->enkf_rtpp = rtpp;
     return TXH_OK;
 }
 

@@ -1536,6 +1536,167 @@ enks_apply_kernel(const double* __restrict__ rec, double* __restrict__ out, cons
     }
 }
 
+// ---- the square-root (ETKF) and relaxed (RTPP) forms of a solved transform -----------------------------------------
+// A solve run with identical observation columns leaves T = wbar 1^T - I + G, G = (M-1) (C0 + (M-1) I)^-1 SPD with
+// G 1 = 1, and W with row means Wbar = D^-1 (dzbar - HA wbar).  In place:
+//   ETKF  T <- wbar 1^T + (1 - rho) (G^1/2 - I),       W <- Wbar 1^T
+//   RTPP  T <- wbar 1^T + (1 - rho) (T - wbar 1^T),    W <- Wbar 1^T + (1 - rho) (W - Wbar 1^T)
+// (row means throughout).  Every consumer of (T, W) then applies the new update unchanged.
+
+// Rows of Mt entries, one per warp, the nT rows of T then the m rows of W: x <- mean + f (x - mean); f = 0 writes the
+// mean.
+__device__ __forceinline__ void relax_rows(double* __restrict__ T, int nT, double* __restrict__ W, int m, int Mt,
+                                           double f, int warp0, int nwarps)
+{
+    const int lane = threadIdx.x & 31;
+    for (int r = warp0; r < nT + m; r += nwarps) {
+        double* row = r < nT ? T + (size_t)r * Mt : W + (size_t)(r - nT) * Mt;
+        double s = 0.0;
+        for (int c = lane; c < Mt; c += 32) s += row[c];
+        for (int o = 16; o; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+        const double mu = s / (double)Mt;
+        for (int c = lane; c < Mt; c += 32) row[c] = mu + f * (row[c] - mu);
+    }
+}
+
+__global__ void __launch_bounds__(256)
+enkf_rtpp_kernel(double* __restrict__ T, double* __restrict__ W, int Mt, int m, double keep)
+{
+    relax_rows(T, Mt, W, m, Mt, keep, blockIdx.x * 8 + (threadIdx.x >> 5), gridDim.x * 8);
+}
+
+// ETKF, Mt <= 64, one CTA of 1024 threads.  G = T - wbar 1^T + I is symmetrised and diagonalised by cyclic two-sided
+// Jacobi in the round-robin (Brent-Luk) order: a round is N/2 disjoint rotations (N = Mt rounded up to even, an odd Mt
+// padded with a decoupled identity row and column), and thread (P, Q) applies rotations P and Q to its 2 x 2 block of G
+// (G <- J^T G J) and of V (V <- V J).  Clustered eigenvalues -- G has at least Mt - m of them equal to 1, and G = I with
+// every gauge missing -- are where Jacobi stays accurate.  Sweeps of N - 1 rounds until off(G) <= kEtkfOffTol ||G||_F;
+// kEtkfSweeps sweeps without that write kInfoEtkfNoConvergence to the info word.  Then S = V diag(sqrt(max(lambda, 0)))
+// V^T, and T, W as above.
+constexpr int ET_LD = 65;                               // row stride of G and V in shared memory
+constexpr int kEtkfSweeps = 20;
+constexpr double kEtkfOffTol = 1e-14;
+constexpr size_t ET_SMEM = sizeof(double) * (2 * 64 * ET_LD + 64 + 2 * 32 + 2 * 32);
+
+__global__ void __launch_bounds__(1024, 1)
+enkf_transform_post_kernel(double* __restrict__ T, double* __restrict__ W, int Mt, int m, double keep, int* info)
+{
+    // the next routing launch (programmatic dependent launch) may load its first tasks while this CTA runs; it waits for
+    // this grid to complete before it reads T
+    griddep_launch_dependents();
+    extern __shared__ double et_sm[];
+    double* G = et_sm;                                   // [64][ET_LD]
+    double* V = G + 64 * ET_LD;                          // [64][ET_LD]
+    double* wbar = V + 64 * ET_LD;                       // [64]
+    double* rc = wbar + 64;                              // [32] cosines
+    double* rs = rc + 32;                                // [32] sines
+    double* red = rs + 32;                               // [2][32] warp partials of off(G)^2, ||G||_F^2
+    __shared__ int pp[32], pq[32];
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int N = (Mt + 1) & ~1, h = N >> 1;
+    // row means of T and G = T - wbar 1^T + I (the pad: identity)
+    for (int j = warp; j < N; j += 32) {
+        double s = 0.0;
+        if (j < Mt)
+            for (int c = lane; c < Mt; c += 32) s += T[(size_t)j * Mt + c];
+        for (int o = 16; o; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+        const double mu = s / (double)Mt;
+        if (lane == 0) wbar[j] = j < Mt ? mu : 0.0;
+        for (int c = lane; c < N; c += 32) {
+            G[j * ET_LD + c] = (j < Mt && c < Mt ? T[(size_t)j * Mt + c] - mu : 0.0) + (j == c ? 1.0 : 0.0);
+            V[j * ET_LD + c] = j == c ? 1.0 : 0.0;
+        }
+    }
+    __syncthreads();
+    // symmetrise: (G + G^T) / 2
+    for (int e = tid; e < N * N; e += blockDim.x) {
+        const int j = e / N, c = e - j * N;
+        if (j < c) { const double a = 0.5 * (G[j * ET_LD + c] + G[c * ET_LD + j]); G[j * ET_LD + c] = a; G[c * ET_LD + j] = a; }
+    }
+    __syncthreads();
+    // W <- Wbar 1^T: the ETKF mean weights (independent of the eigenproblem)
+    relax_rows(T, 0, W, m, Mt, 0.0, warp, 32);
+    // thread (P, Q) of the h x h blocks
+    const bool act = tid < h * h;
+    const int P = act ? tid / h : 0, Q = act ? tid - P * h : 0;
+    bool converged = false;
+    for (int sweep = 0; sweep <= kEtkfSweeps && !converged; ++sweep) {
+        // off(G)^2 and ||G||_F^2 over the blocks of the current pairing (any pairing tiles G)
+        double off2 = 0.0, fro2 = 0.0;
+        for (int e = tid; e < N * N; e += blockDim.x) {
+            const int j = e / N, c = e - j * N;
+            const double g = G[j * ET_LD + c];
+            fro2 += g * g;
+            if (j != c) off2 += g * g;
+        }
+        for (int o = 16; o; o >>= 1) {
+            off2 += __shfl_xor_sync(0xffffffffu, off2, o);
+            fro2 += __shfl_xor_sync(0xffffffffu, fro2, o);
+        }
+        if (lane == 0) { red[warp] = off2; red[32 + warp] = fro2; }
+        __syncthreads();
+        off2 = 0.0; fro2 = 0.0;
+        for (int w = 0; w < 32; ++w) { off2 += red[w]; fro2 += red[32 + w]; }
+        converged = off2 <= kEtkfOffTol * kEtkfOffTol * fro2;
+        __syncthreads();                                  // red is rewritten by the next sweep
+        if (converged || sweep == kEtkfSweeps) break;
+        for (int r = 0; r < N - 1; ++r) {
+            // pairs of round r (circle method: player N-1 fixed, the others turn) and their rotations
+            if (tid < h) {
+                int p, q;
+                if (tid == 0) { p = r; q = N - 1; }
+                else { p = (r + tid) % (N - 1); q = (r - tid + N - 1) % (N - 1); }
+                if (p > q) { const int t = p; p = q; q = t; }
+                const double gpq = G[p * ET_LD + q], gpp = G[p * ET_LD + p], gqq = G[q * ET_LD + q];
+                double c = 1.0, s = 0.0;
+                if (gpq != 0.0) {
+                    const double tau = (gqq - gpp) / (2.0 * gpq);
+                    const double t = (tau >= 0.0 ? 1.0 : -1.0) / (fabs(tau) + hypot(1.0, tau));   // no overflow at |tau| >> 1
+                    c = rsqrt(1.0 + t * t);
+                    s = t * c;
+                }
+                pp[tid] = p; pq[tid] = q; rc[tid] = c; rs[tid] = s;
+            }
+            __syncthreads();
+            if (act) {
+                const int p1 = pp[P], q1 = pq[P], p2 = pp[Q], q2 = pq[Q];
+                const double c1 = rc[P], s1 = rs[P], c2 = rc[Q], s2 = rs[Q];
+                const double a = G[p1 * ET_LD + p2], b = G[p1 * ET_LD + q2];
+                const double d = G[q1 * ET_LD + p2], e = G[q1 * ET_LD + q2];
+                // J^T B J with J = [c s; -s c] on (p, q)
+                const double u0 = c1 * a - s1 * d, u1 = c1 * b - s1 * e;      // rows of J1^T B
+                const double v0 = s1 * a + c1 * d, v1 = s1 * b + c1 * e;
+                double np = c2 * u0 - s2 * u1, nb = s2 * u0 + c2 * u1;
+                double nd = c2 * v0 - s2 * v1, ne = s2 * v0 + c2 * v1;
+                if (P == Q && s1 != 0.0) { nb = 0.0; nd = 0.0; }             // the annihilated pair
+                G[p1 * ET_LD + p2] = np; G[p1 * ET_LD + q2] = nb;
+                G[q1 * ET_LD + p2] = nd; G[q1 * ET_LD + q2] = ne;
+                // V <- V J: rows (p1, q1), columns (p2, q2)
+                const double va = V[p1 * ET_LD + p2], vb = V[p1 * ET_LD + q2];
+                const double vd = V[q1 * ET_LD + p2], ve = V[q1 * ET_LD + q2];
+                V[p1 * ET_LD + p2] = c2 * va - s2 * vb; V[p1 * ET_LD + q2] = s2 * va + c2 * vb;
+                V[q1 * ET_LD + p2] = c2 * vd - s2 * ve; V[q1 * ET_LD + q2] = s2 * vd + c2 * ve;
+            }
+            __syncthreads();
+        }
+    }
+    if (!converged && tid == 0) atomicCAS(info, 0, kInfoEtkfNoConvergence);
+    // U = V diag(sqrt(max(lambda, 0))) into G (its diagonal read first), then S = U V^T and the new T
+    double* lam = rc;                                    // reuse: [64] fits rc + rs
+    for (int j = tid; j < N; j += blockDim.x) lam[j] = sqrt(fmax(G[j * ET_LD + j], 0.0));
+    __syncthreads();
+    for (int e = tid; e < N * N; e += blockDim.x) {
+        const int j = e / N, k = e - j * N;
+        G[j * ET_LD + k] = V[j * ET_LD + k] * lam[k];
+    }
+    __syncthreads();
+    for (int e = tid; e < Mt * Mt; e += blockDim.x) {
+        const int j = e / Mt, c = e - j * Mt;
+        double s = 0.0;
+        for (int k = 0; k < N; ++k) s = fma(G[j * ET_LD + k], V[c * ET_LD + k], s);
+        T[(size_t)j * Mt + c] = wbar[j] + keep * (s - (j == c ? 1.0 : 0.0));
+    }
+}
+
 }  // namespace
 
 cudaError_t launch_dgemm(int transA, int transB, int M, int N, int K, double alpha, const double* A, int lda,
@@ -1801,6 +1962,25 @@ cudaError_t launch_inflow_gain(const int32_t* inner, int64_t n_inner, const int3
 {
     if (n_inner == 0) return cudaSuccess;
     inflow_gain_kernel<<<nblk(n_inner * (ld >> 1), 256), 256, 0, st>>>(inner, n_inner, up_off, up_pos, G, I, ld);
+    count_launch();
+    return cudaGetLastError();
+}
+
+// Launched without the programmatic-dependent-launch attribute: the solve in front of it has completed and its T, W
+// are visible by plain stream order.  The next routing launch, which does carry the attribute, waits for this grid
+// (griddep_wait) before it stages T.
+cudaError_t launch_enkf_transform_post(double* T, double* W, int Mt, int m, int kind, double rtpp, int* info,
+                                       cudaStream_t st)
+{
+    if (kind == 1) {
+        if (Mt > 64 || Mt < 1) return cudaErrorInvalidValue;
+        cudaError_t e = cudaFuncSetAttribute(enkf_transform_post_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                             (int)ET_SMEM);
+        if (e != cudaSuccess) return e;
+        enkf_transform_post_kernel<<<1, 1024, ET_SMEM, st>>>(T, W, Mt, m, 1.0 - rtpp, info);
+    } else {
+        enkf_rtpp_kernel<<<nblk((long long)Mt + m, 8), 256, 0, st>>>(T, W, Mt, m, 1.0 - rtpp);
+    }
     count_launch();
     return cudaGetLastError();
 }

@@ -274,6 +274,11 @@ cudaError_t launch_inflow_rebuild(const int4* rec, int64_t n_inner, const int32_
 cudaError_t launch_enkf_record(const double* O, int ld, int M, const double* mean, const double* T,
                                const int32_t* gauge_of_pos, const double* qs, const double* W, const int32_t* rec_pos,
                                int rec_count, double* prior_out, double* post_out, cudaStream_t st);
+// The square-root (kind 1, ETKF, Mt <= 64) or relaxed (kind 0, rtpp > 0) form of a solved (T, W), in place; an ETKF
+// eigensolve that does not converge writes kInfoEtkfNoConvergence to *info
+constexpr int kInfoEtkfNoConvergence = -0x7fffffff;
+cudaError_t launch_enkf_transform_post(double* T, double* W, int Mt, int m, int kind, double rtpp, int* info,
+                                       cudaStream_t st);
 // txh_enks_smooth (arguments checked by the caller): cumulative transforms, then one pass over rec
 cudaError_t launch_enks_smooth(int M, int nupd, long long every, const double* T_hist, long long nslots, long long rec_count,
                                long long rec_every, long long lag, const double* rec, double* out, double* work,

@@ -16,6 +16,7 @@ member-batched forecast plus a diagonal Q (SURVEY.md section 8c).  Members may b
 sharded over ranks; the statistics are then combined with torch.distributed
 collectives (NCCL over NVLink) between the three device phases.
 """
+import contextlib
 import copy
 import datetime as _dt
 import logging
@@ -327,16 +328,35 @@ class EnsembleKalmanFilter(_MeasurementTable, BaseCallback):
     Q_diag       : scalar or [n] diagonal of the model-noise covariance
     R_cov        : [m][m] observation-noise covariance
     obs_noise    : optional [len(measurements)][m][M_total] perturbations added to the interpolated
-                   measurements per member (supplied as data so CPU and GPU consume identical numbers);
-                   zeros if omitted (deterministic ensemble update)
+                   measurements per member (supplied as data so CPU and GPU consume identical numbers).
+                   The stochastic filter needs them, drawn with covariance R_cov: without them every
+                   member sees the same observations and the update shrinks the ensemble spread below the
+                   Kalman posterior's at every update.  `method='etkf'` needs no perturbations and takes none.
     every        : pd.Timedelta cadence (e.g. hourly); None = every step as the reference (da.py:56-61)
     group        : torch.distributed process group when members are sharded over ranks (this rank
                    holds columns [rank*M, (rank+1)*M) of the global ensemble); None = the default group
                    if torch.distributed is initialised; False = never sharded (independent ensembles)
+    method       : 'stochastic' (perturbed-observation EnKF) or 'etkf' (the deterministic square-root
+                   filter of Hunt et al. 2007: the posterior ensemble has exactly the Kalman posterior
+                   covariance of the ensemble's; at most 64 members in all)
+    rtpp         : relaxation to prior perturbations in [0, 1) (Zhang et al. 2004): the posterior
+                   anomalies become (1 - rtpp) x the filter's + rtpp x the forecast's; the mean is the filter's
     """
 
-    def __init__(self, model, measurements, Q_diag, R_cov, obs_noise=None, every=None, group=None):
+    METHODS = ('stochastic', 'etkf')
+
+    def __init__(self, model, measurements, Q_diag, R_cov, obs_noise=None, every=None, group=None,
+                 method='stochastic', rtpp=0.0):
         import torch
+        if method not in self.METHODS:
+            raise ValueError(f'`method` must be one of {self.METHODS}, got {method!r}')
+        if isinstance(rtpp, bool) or not isinstance(rtpp, (int, float, np.integer, np.floating)) \
+                or not 0.0 <= float(rtpp) < 1.0:
+            raise ValueError(f'`rtpp` must be a number in [0, 1), got {rtpp!r}')
+        if method == 'etkf' and obs_noise is not None:
+            raise ValueError("`method='etkf'` is deterministic: it takes no `obs_noise` (every member sees the "
+                             "same observations)")
+        self.method, self.rtpp = method, float(rtpp)
         self._torch = torch
         self.model = model
         self.reach_indices, perm = _gauge_setup(model, measurements)
@@ -366,6 +386,10 @@ class EnsembleKalmanFilter(_MeasurementTable, BaseCallback):
             # the sample covariance divides by Mtot - 1: refused here, before any device work, rather than by the
             # first solve, after the assimilation loop has already routed a window
             raise ValueError(f'an ensemble Kalman filter needs at least 2 members in all, got {self.Mtot} '
+                             f'({self.M} per rank x {self.world} ranks)')
+        if method == 'etkf' and self.Mtot > 64:
+            # the square root is an eigensolve of one Mtot x Mtot matrix in one CTA's shared memory
+            raise ValueError(f"`method='etkf'` takes at most 64 members in all, got {self.Mtot} "
                              f'({self.M} per rank x {self.world} ranks)')
         self._R = torch.as_tensor(np.ascontiguousarray(Rp), device='cuda')
         self._qs = torch.as_tensor(np.ascontiguousarray(q[self.reach_indices]), device='cuda')
@@ -489,9 +513,23 @@ class EnsembleKalmanFilter(_MeasurementTable, BaseCallback):
     def stats_scale(self):
         return 1.0 / self.Mtot if self.world == 1 else 1.0
 
+    @contextlib.contextmanager
+    def transform_on(self, net):
+        """Inside the block the network's solves produce this filter's form of the update (`method`, `rtpp`);
+        after it, the handle is back at the default.  The default filter touches nothing."""
+        if self.method == 'stochastic' and self.rtpp == 0.0:
+            yield
+            return
+        net.set_enkf_transform(self.method, self.rtpp)
+        try:
+            yield
+        finally:
+            net.set_enkf_transform()
+
     def filter(self, Zp_dev=None, stats_fresh=False):
         """One ensemble update on the device.  `Zp_dev` ([m][Mtot] CUDA tensor) overrides the
-        interpolated observations (used by the fast path that pre-stages them).  `stats_fresh`: the row
+        interpolated observations (used by the fast path that pre-stages them); for `method='etkf'` its member
+        columns must be identical.  `stats_fresh`: the row
         sums of the forecast are already in `self._rowsum` (written by the routing launch)."""
         torch = self._torch
         mdl = self.model
@@ -517,8 +555,9 @@ class EnsembleKalmanFilter(_MeasurementTable, BaseCallback):
             # rank has left the previous update, i.e. nobody reads the buffer this update is about to overwrite.
             cur, nxt = self._sym[self._cur], self._sym[self._cur ^ 1]
             mean, self._HXall = combine_statistics(self._rowsum, self._HX, Mt, group=self.group)
-            net.enkf_solve(m, Mt, self._HXall, Zp_dev, mean, self.reach_indices, self._qs, self._R, self._work,
-                           self._W, self._T, self._Dinv, self._dinv_kind)
+            with self.transform_on(net):
+                net.enkf_solve(m, Mt, self._HXall, Zp_dev, mean, self.reach_indices, self._qs, self._R, self._work,
+                               self._W, self._T, self._Dinv, self._dinv_kind)
             net.enkf_apply_peers(cur[0], nxt[0], I, M, cur[1], Mt, self.rank * M, mean, self._T, self.reach_indices,
                                  self._qs, self._W, self._G)
             mdl._dev['O'] = nxt[0]
@@ -536,8 +575,9 @@ class EnsembleKalmanFilter(_MeasurementTable, BaseCallback):
                 self._Xall = torch.empty((self.world, mdl.n, ld), dtype=torch.float64, device='cuda')
             gather = dist.all_gather_into_tensor(self._Xall, O, group=self.group, async_op=True)
             Xall, ldx, xstride = self._Xall, ld, mdl.n * ld
-        net.enkf_solve(m, Mt, self._HXall, Zp_dev, mean, self.reach_indices, self._qs, self._R, self._work,
-                       self._W, self._T, self._Dinv, self._dinv_kind)
+        with self.transform_on(net):
+            net.enkf_solve(m, Mt, self._HXall, Zp_dev, mean, self.reach_indices, self._qs, self._R, self._work,
+                           self._W, self._T, self._Dinv, self._dinv_kind)
         if gather is not None:
             gather.wait()
         net.enkf_apply(O, I, M, Xall, ldx, Mt, self.rank * M, mean, self._T, self.reach_indices, self._qs,

@@ -492,7 +492,10 @@ class Muskingum:
         Missing observations: a gauge whose row `observations[k][g]` holds a NaN (in any member) is left out of
         update k -- the update is that of a filter without the gauge, its W row is 0 -- when the filter's D = R + Q[s,s]
         is diagonal; with every gauge missing the posterior is the forecast.  With a dense R, `observations` holding a
-        NaN raise ValueError before any device work (DESIGN.md §4.4)."""
+        NaN raise ValueError before any device work (DESIGN.md §4.4).
+        The update is the filter's `method` with its `rtpp`.  An `'etkf'` filter needs the same observation in
+        every member: a row of `observations[k]` without a NaN whose member columns differ raises ValueError before
+        any device work."""
         if smooth_lag is not None:
             if isinstance(smooth_lag, bool) or not isinstance(smooth_lag, (int, np.integer)) or smooth_lag < 0:
                 raise ValueError(f'`smooth_lag` must be a non-negative integer number of steps, got {smooth_lag!r}')
@@ -516,6 +519,14 @@ class Muskingum:
                     any(bool(torch.isnan(torch.as_tensor(o)).any()) for o in obs)):
                 raise ValueError('`observations` hold missing values (NaN): an ensemble update leaves out a missing '
                                  'gauge only when the observation covariance R_cov is diagonal')
+        if getattr(enkf, 'method', 'stochastic') == 'etkf' and nwin:
+            # the square-root update is derived for one observation seen by every member (a NaN row: missing gauge)
+            whole = torch.is_tensor(observations) or isinstance(observations, np.ndarray)
+            for o in ([observations[:nwin]] if whole else observations[:nwin]):
+                o = torch.as_tensor(o)
+                if bool(((o != o[..., :1]).any(dim=-1) & ~torch.isnan(o).any(dim=-1)).any()):
+                    raise ValueError("`observations` differ between members on a gauge row without NaN: "
+                                     "`method='etkf'` needs the same observation in every member (no perturbations)")
         torch = self._ensure_device()
         self._sync_coeffs()
         d, net, M = self._dev, self.network, self.members
@@ -543,11 +554,12 @@ class Muskingum:
             if T_hist is not None:
                 net.set_transform_history(T_hist)
             try:
-                net.run_assimilating(d['O'], d['I'], M, forcing, t, step_ns, nsteps, every, enkf.reach_indices,
-                                     observations, enkf._qs, enkf._R, enkf._Dinv, enkf._dinv_kind, enkf._rowsum,
-                                     enkf._HX, enkf._work, enkf._W, enkf._T, enkf._G,
-                                     time_every=8 if timers is not None else 0, obs_ready=observations_ready,
-                                     rec_reach=ridx, rec_every=record_every, rec_out=rec, prior_out=prior)
+                with enkf.transform_on(net):
+                    net.run_assimilating(d['O'], d['I'], M, forcing, t, step_ns, nsteps, every, enkf.reach_indices,
+                                         observations, enkf._qs, enkf._R, enkf._Dinv, enkf._dinv_kind, enkf._rowsum,
+                                         enkf._HX, enkf._work, enkf._W, enkf._T, enkf._G,
+                                         time_every=8 if timers is not None else 0, obs_ready=observations_ready,
+                                         rec_reach=ridx, rec_every=record_every, rec_out=rec, prior_out=prior)
             finally:
                 if T_hist is not None:
                     net.set_transform_history(None)

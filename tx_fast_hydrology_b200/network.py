@@ -339,6 +339,17 @@ class RiverNetwork:
         L.check(self._lib.txh_set_transform_history(self.handle, _cuda_ptr(T_hist) if T_hist is not None else None,
                                                     T_hist.numel() if T_hist is not None else 0))
 
+    ENKF_METHODS = ("stochastic", "etkf")
+
+    def set_enkf_transform(self, method="stochastic", rtpp=0.0):
+        """`txh_set_enkf_transform`: the form of the ensemble update every later `enkf_solve` and `run_assimilating`
+        on the handle solves -- "stochastic" (perturbed observations, the default) or "etkf" (square root, needs
+        identical observation columns, at most 64 members in all) -- and the relaxation to prior perturbations
+        `rtpp` in [0, 1)."""
+        if method not in self.ENKF_METHODS:
+            raise ValueError(f"set_enkf_transform: `method` must be one of {self.ENKF_METHODS}, got {method!r}")
+        L.check(self._lib.txh_set_enkf_transform(self.handle, self.ENKF_METHODS.index(method), float(rtpp)))
+
     @staticmethod
     def enks_work_size(M, nupd):
         return int(L.load().txh_enks_work_size(int(M), int(nupd)))
