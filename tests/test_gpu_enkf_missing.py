@@ -11,10 +11,11 @@ import pytest
 
 import enkf_reference as E
 import enkf_missing_reference as X
+from assim_case import (torch_cuda, fnet, _kernels, _expect, _dev, _f64, _solve_dev, _solve_kernels,  # noqa: F401
+                        _loop_kernels, _state, LOOP_CASES, loop_params, make_case, run_device, reference_loop,
+                        update_masked)
 from enks_oracle import smooth_transforms
-from parity import relerr, normerr, enkf_tolerance
-from test_gpu_enkf_paths import (torch_cuda, fnet, _kernels, _expect, _dev, _f64, _solve_dev,  # noqa: F401
-                                 _solve_kernels, _loop_kernels, _state, LOOP_CASES, RTOL)
+from parity import relerr, normerr
 
 pytestmark = pytest.mark.gpu
 
@@ -196,94 +197,14 @@ def outage(endnodes, gidx, nwin, seed):
     return miss, (last, one)
 
 
-def _outage_loop(torch, oracle, monkeypatch, n, M, m, seed, every, nwin, rest, kernel, in_library, lag=None):
-    """test_gpu_enkf_paths.py:_loop_case with the outage pattern planted in the observations and the masked update in
-    the extended-precision loop.  Returns the device run, the reference hydrographs and priors with their error scales,
-    the tolerance, the reference transforms and the outage pattern."""
-    if kernel is not None:
-        monkeypatch.setenv("TXH_ROUTE_KERNEL", kernel)
-    else:
-        monkeypatch.delenv("TXH_ROUTE_KERNEL", raising=False)
-    from tx_fast_hydrology_b200 import synthetic as S
-    from tx_fast_hydrology_b200.muskingum import Muskingum
-    from tx_fast_hydrology_b200.da import EnsembleKalmanFilter
-    nsteps = every * nwin + rest
-    net_d = S.make_network(n, seed)
-    prm = S.make_params(n, seed, well_posed=True)
-    rng = np.random.default_rng(seed)
-    o0 = prm["o_t"][:, None] * rng.uniform(0.5, 1.5, size=(n, M))
-    d = S.model_dict(net_d, prm, dt_s=300.0)
-    d["o_t"] = o0
-    mdl = Muskingum(d, members=M)
-    t0 = int(mdl.datetime.value)
-    times, table = S.make_forcing(n, nsteps, 300.0, seed, t0_ns=t0, rows_every=4)
-    mul = S.make_member_multipliers(times.size, M, seed)
-    gidx = E.gauge_set(net_d["endnodes"], m, seed)
-    mt = t0 + (np.arange(nwin, dtype=np.int64) + 1) * int(every * 300e9)
-    meas = rng.uniform(0.5, 8.0, size=(nwin, m))
-    mdf = pd.DataFrame(meas, index=pd.DatetimeIndex(pd.to_datetime(mt, unit="ns", utc=True)).as_unit("ns"),
-                       columns=[d["reach_ids"][j] for j in gidx])
-    R = 1e-2 * np.eye(m)
-    q = rng.uniform(0.5, 2.0, size=n)
-    enkf = EnsembleKalmanFilter(mdl, mdf, q, R)
-    Zp = meas[:, :, None] + 0.1 * rng.standard_normal((nwin, m, M))
-    miss, (k1, g1) = outage(net_d["endnodes"], gidx, nwin, seed)
+def _outage_case(n, M, m, seed, every, nwin, rest):
+    """A loop case with the outage pattern planted in its observations, and the pattern."""
+    c = make_case(n, M, m, seed, every, nwin, rest, gauges="reference")
+    miss, (k1, g1) = outage(c["net"]["endnodes"], c["gidx"], nwin, seed)
     for k in range(nwin):
-        Zp[k][miss[k]] = np.nan
-    Zp[k1, g1, M - 1] = np.nan
-    f = mdl.make_forcing(times_ns=times, table=table, member_mul=mul)
-    ung = np.setdiff1d(np.arange(n), gidx)
-    reaches = rng.permutation(np.concatenate([gidx[:max(3, m // 2)], rng.choice(ung, size=40, replace=False)]))
-    Zd = torch.as_tensor(np.ascontiguousarray(Zp), device="cuda")
-    out = {}
-
-    def run():
-        out["r"] = mdl.run_assimilating(f, nsteps, enkf, every, Zd if in_library else list(Zd), record_reaches=reaches,
-                                        record_prior=True, smooth_lag=lag)
-    names = _kernels(torch, run)
-    mdl.network.check()
-    res = [x.cpu().numpy() for x in out["r"]]
-    ind = oracle.compute_indegree(net_d["startnodes"], net_d["endnodes"])
-    al, be, ch, ga = oracle.compute_coeffs(prm["K"], prm["X"], 300.0)
-    onet = {"startnodes": net_d["startnodes"], "endnodes": net_d["endnodes"], "indegree": ind,
-            "alpha": al, "beta": be, "chi": ch, "gamma": ga}
-    o = np.ascontiguousarray(o0.T)
-    i = np.stack([oracle.init_states(net_d["startnodes"], net_d["endnodes"], x) for x in o])
-    hyd = np.empty((nsteps, reaches.size, M))
-    pri = np.empty((nwin, reaches.size, M))
-    # error scales as in test_gpu_enkf_paths.py:_loop_case
-    om = np.zeros_like(o); im = np.zeros_like(i)
-    anet = dict(onet, alpha=np.abs(al), beta=np.abs(be), chi=np.abs(ch), gamma=np.zeros(n))
-    zero = np.zeros_like(table)
-    sc = np.empty_like(hyd)
-    sc_pri = np.empty_like(pri)
-    tol, Ts = RTOL, []
-    for s in range(1, nsteps + 1):
-        t = float(t0 + (s - 1) * 300e9)
-        oracle.run_members(onet, o, i, 1, times.astype(np.float64), table, t, 300e9, wmul=mul)
-        oracle.run_members(anet, om, im, 1, times.astype(np.float64), zero, t, 300e9)
-        hyd[s - 1] = o[:, reaches].T
-        sc[s - 1] = om[:, reaches].T
-        if s % every == 0 and s // every <= nwin:
-            k = s // every - 1
-            pri[k] = o[:, reaches].T
-            sc_pri[k] = om[:, reaches].T
-            O, I = o.T, i.T
-            keep = ~X.missing_rows(Zp[k])
-            if keep.any():
-                tol = max(tol, enkf_tolerance(O, gidx[keep], q, R[np.ix_(keep, keep)]))
-            mean = np.asarray(np.asarray(O, dtype=E.LD).sum(axis=1) / M, dtype=np.float64)
-            T, W, _, _ = X.solve_masked(O[gidx], Zp[k], mean[gidx], q[gidx], R)
-            Ts.append(_f64(T))
-            Op, Ip = E.apply_ref(O, I, mean, T, W, gidx, q[gidx], net_d["endnodes"])
-            Op, Ip = _f64(Op), _f64(Ip)
-            om = np.ascontiguousarray(np.maximum(np.abs(Op), np.abs(O)).T)
-            im = np.ascontiguousarray(np.maximum(np.abs(Ip), np.abs(I)).T)
-            o = np.ascontiguousarray(Op.T); i = np.ascontiguousarray(Ip.T)
-            hyd[s - 1] = o[:, reaches].T
-            sc[s - 1] = om[:, reaches].T
-    return dict(names=names, res=res, final=mdl.o_t_next[reaches], hyd=hyd, pri=pri, sc=sc, sc_pri=sc_pri, tol=tol,
-                Ts=Ts, miss=miss)
+        c["Zp"][k][miss[k]] = np.nan
+    c["Zp"][k1, g1, M - 1] = np.nan
+    return c, miss
 
 
 MISSING_LOOP_CASES = [c for c in LOOP_CASES
@@ -291,32 +212,25 @@ MISSING_LOOP_CASES = [c for c in LOOP_CASES
                       or (c[7] == "lane" and c[1] == 16) or c[7] == "dataflow"]
 
 
-def _missing_loop_params():
-    out = []
-    for c in MISSING_LOOP_CASES:
-        out.append(pytest.param(*c[:8], True, id=f"M{c[1]}-m{c[2]}-{c[7] or 'default'}-lib"))
-        if c[8]:
-            out.append(pytest.param(*c[:8], False, id=f"M{c[1]}-m{c[2]}-{c[7] or 'default'}-py"))
-    return out
-
-
-@pytest.mark.parametrize("n,M,m,seed,every,nwin,rest,kernel,in_library", _missing_loop_params())
+@pytest.mark.parametrize("n,M,m,seed,every,nwin,rest,kernel,in_library", loop_params(MISSING_LOOP_CASES))
 def test_assimilation_loop_with_outages(torch_cuda, oracle, monkeypatch, record_property, n, M, m, seed, every, nwin,
                                         rest, kernel, in_library):
     """Hydrographs, priors and final state of an outage run against the masked extended-precision loop, at the
     tolerance and error scale of test_gpu_enkf_paths.py; at the update with every gauge missing the recorded posterior
     equals the prior element-wise.  (Without the masking the run comes out all NaN.)"""
-    r = _outage_loop(torch_cuda, oracle, monkeypatch, n, M, m, seed, every, nwin, rest, kernel, in_library)
-    _expect(r["names"], _loop_kernels(M, m, kernel, in_library))
-    rec, prior = r["res"]
+    c, miss = _outage_case(n, M, m, seed, every, nwin, rest)
+    d = run_device(c, in_library, monkeypatch=monkeypatch, kernel=kernel)
+    r = reference_loop(oracle, c, update_masked)
+    _expect(d["names"], _loop_kernels(M, m, kernel, in_library))
+    rec, prior = d["res"]
     assert not np.isnan(rec).any() and not np.isnan(prior).any()
     e_pri, e_rec = relerr(prior, r["pri"], scale=r["sc_pri"]), relerr(rec, r["hyd"], scale=r["sc"])
     record_property("rec_ratio", e_rec / r["tol"])
     assert e_pri < r["tol"], f"priors: {e_pri:.2e}, bound {r['tol']:.2e}"
     assert e_rec < r["tol"], f"hydrographs: {e_rec:.2e}, bound {r['tol']:.2e}"
     nsteps = every * nwin + rest
-    assert relerr(r["final"], r["hyd"][nsteps - 1], scale=r["sc"][nsteps - 1]) < r["tol"]
-    assert r["miss"][1].all()
+    assert relerr(d["final"], r["hyd"][nsteps - 1], scale=r["sc"][nsteps - 1]) < r["tol"]
+    assert miss[1].all()
     assert np.array_equal(rec[2 * every - 1], prior[1]), "the update with every gauge missing changed the state"
 
 
@@ -326,9 +240,10 @@ def test_smoother_on_an_outage_run(torch_cuda, oracle, monkeypatch, in_library):
     reference hydrographs with the masked reference transforms."""
     n, M, m, seed, every, nwin, rest = 2500, 64, 120, 81, 6, 3, 0
     lag = every + 2
-    r = _outage_loop(torch_cuda, oracle, monkeypatch, n, M, m, seed, every, nwin, rest, None, in_library, lag=lag)
-    rec, prior, sm = r["res"]
-    want = smooth_transforms(r["hyd"], np.stack(r["Ts"]), nwin, every, 1, lag)
+    c, _ = _outage_case(n, M, m, seed, every, nwin, rest)
+    rec, prior, sm = run_device(c, in_library, monkeypatch=monkeypatch, lag=lag)["res"]
+    r = reference_loop(oracle, c, update_masked)
+    want = smooth_transforms(r["hyd"], np.stack(r["kept"]), nwin, every, 1, lag)
     sc = np.maximum(np.maximum(np.abs(want), r["sc"]), np.abs(rec))
     assert not np.isnan(sm).any()
     assert relerr(sm, want, scale=sc) < r["tol"] * (nwin + 1)

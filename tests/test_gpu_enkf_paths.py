@@ -20,94 +20,15 @@ import pandas as pd
 import pytest
 
 import enkf_reference as E
-from parity import relerr, normerr, enkf_tolerance
+from assim_case import (torch_cuda, fnet, _kernels, _expect, _dev, _f64, _sched, _state, SENTINEL,  # noqa: F401
+                        _solve_kernels, _solve_dev, _loop_kernels, LOOP_CASES, loop_params, make_case, run_device,
+                        reference_loop, update_ref)
+from parity import relerr, normerr
 
 pytestmark = pytest.mark.gpu
 
-SENTINEL = 1e6
-RTOL = 1e-9
-
-
-@pytest.fixture(scope="module")
-def torch_cuda():
-    import torch
-    assert torch.cuda.is_available(), "GPU tests need a CUDA device (no CPU fallback exists)"
-    return torch
-
-
-@pytest.fixture(scope="module")
-def fnet(torch_cuda):
-    """The network of the shared forecast (tests/enkf_reference.py) and its reach -> schedule position map."""
-    from tx_fast_hydrology_b200.network import RiverNetwork
-    fc = E.forecast()
-    net = RiverNetwork(fc["endnodes"])
-    n = net.n
-    net.set_coeffs(np.zeros(n), np.zeros(n), np.zeros(n), np.zeros(n))
-    return net, net.schedule()["pos_of_reach"], fc
-
-
-def _kernels(torch, fn):
-    """Run `fn` under the profiler; the names of the CUDA kernels it launched, in one string."""
-    from torch.profiler import profile, ProfilerActivity
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        fn()
-        torch.cuda.synchronize()
-    return " ".join(e.name for e in prof.events())
-
-
-def _expect(names, want, absent=()):
-    for k in want:
-        assert k in names, f"{k} did not run (kernels: {sorted(set(names.split()))[:40]})"
-    for k in absent:
-        assert k not in names, f"{k} ran, but this case is meant to take another path"
-
-
-def _dev(torch, a):
-    return torch.as_tensor(np.ascontiguousarray(a, dtype=np.float64), device="cuda")
-
-
-def _sched(vec, pos):
-    out = np.empty_like(vec)
-    out[pos] = vec
-    return out
-
-
-def _f64(a):
-    return np.asarray(a, dtype=np.float64)
-
 
 # ---- (a) the solve --------------------------------------------------------------------------------------------
-def _solve_kernels(M, m, dinv_kind, path):
-    if path == "cluster":
-        return ["enkf_small_system_kernel"], ["innovation_cat_kernel", "spd_solve_kernel", "chol_panel_kernel"]
-    if path == "woodbury":
-        mt = 64 if M <= 64 else (96 if M <= 96 else 128)
-        return ["innovation_cat_kernel", "dgemm_kernel", f"chol_solve_blocked_kernel<{mt}>"], \
-               ["enkf_small_system_kernel", "woodbury_assemble_kernel"]
-    if path == "woodbury_big":
-        return ["innovation_cat_kernel", "woodbury_assemble_kernel", "chol_panel_kernel"], \
-               ["enkf_small_system_kernel", "chol_solve_blocked_kernel"]
-    return ["innov_cov_finish_kernel", "spd_solve_kernel" if m <= 48 else "chol_panel_kernel"], \
-           ["enkf_small_system_kernel", "innovation_cat_kernel"]
-
-
-def _solve_dev(torch, net, pos, inp, M, dinv_kind, R=None):
-    m = inp["HX"].shape[0]
-    R = inp["R"] if R is None else R
-    D = np.diag(inp["qs"]) + R
-    Dinv = None if dinv_kind == 0 else _dev(torch, 1.0 / np.diagonal(D) if dinv_kind == 1 else np.linalg.inv(D))
-    args = dict(HX=_dev(torch, inp["HX"]), Zp=_dev(torch, inp["Zp"]), mean=_dev(torch, _sched(inp["mean_all"], pos)),
-                qs=_dev(torch, inp["qs"]), R=_dev(torch, R), Dinv=Dinv,
-                work=torch.empty(net.enkf_work_size(m, M), dtype=torch.float64, device="cuda"),
-                W=torch.full((m, M), np.nan, dtype=torch.float64, device="cuda"),
-                T=torch.full((M, M), np.nan, dtype=torch.float64, device="cuda"))
-
-    def run():
-        net.enkf_solve(m, M, args["HX"], args["Zp"], args["mean"], inp["gauges"], args["qs"], args["R"], args["work"],
-                       args["W"], args["T"], args["Dinv"], dinv_kind)
-    return run, args
-
-
 @pytest.mark.parametrize("M,m,dense_R,dinv_kind,path", E.SOLVE_CASES)
 def test_solve_paths_vs_reference(torch_cuda, fnet, record_property, M, m, dense_R, dinv_kind, path):
     """T and W of RiverNetwork.enkf_solve against the longdouble reference, max-norm relative error within
@@ -159,15 +80,6 @@ def _apply_setup(Mtot):
     inp = E.solve_inputs(Mtot, APPLY_GAUGES, E.case_seed(Mtot, APPLY_GAUGES))
     T, W, _ = E.solve_ref(inp["HX"], inp["Zp"], inp["mean"], inp["qs"], inp["R"])
     return fc, inp, _f64(T), _f64(W)
-
-
-def _state(torch, net, x, M):
-    """alloc_state(M) holding x [n][M] (reach order), its pad column (odd M) set to the sentinel."""
-    X = net.alloc_state(M)
-    net.pack_host(np.ascontiguousarray(x), M, X)
-    if X.shape[1] > M:
-        X[:, M:] = SENTINEL
-    return X
 
 
 @pytest.mark.parametrize("M", APPLY_M)
@@ -244,147 +156,19 @@ def test_sharded_apply_on_one_gpu(torch_cuda, fnet, world, Mloc):
 
 
 # ---- (c) the assimilation loop against the oracle, step by step ------------------------------------------------
-def _loop_case(torch, oracle, monkeypatch, n, M, m, seed, every, nwin, rest, kernel, in_library):
-    """test_gpu_record.py:_assim_case with the routing kernel chosen by TXH_ROUTE_KERNEL (set before the model's
-    device state exists) and the kernels of the run returned."""
-    if kernel is not None:
-        monkeypatch.setenv("TXH_ROUTE_KERNEL", kernel)
-    else:
-        monkeypatch.delenv("TXH_ROUTE_KERNEL", raising=False)
-    from tx_fast_hydrology_b200 import synthetic as S
-    from tx_fast_hydrology_b200.muskingum import Muskingum
-    from tx_fast_hydrology_b200.da import EnsembleKalmanFilter
-    nsteps = every * nwin + rest
-    net_d = S.make_network(n, seed)
-    prm = S.make_params(n, seed, well_posed=True)
-    rng = np.random.default_rng(seed)
-    o0 = prm["o_t"][:, None] * rng.uniform(0.5, 1.5, size=(n, M))
-    d = S.model_dict(net_d, prm, dt_s=300.0)
-    d["o_t"] = o0
-    mdl = Muskingum(d, members=M)
-    t0 = int(mdl.datetime.value)
-    times, table = S.make_forcing(n, nsteps, 300.0, seed, t0_ns=t0, rows_every=4)
-    mul = S.make_member_multipliers(times.size, M, seed)
-    gidx = E.gauge_set(net_d["endnodes"], m, seed)
-    mt = t0 + (np.arange(nwin, dtype=np.int64) + 1) * int(every * 300e9)
-    meas = rng.uniform(0.5, 8.0, size=(nwin, m))
-    mdf = pd.DataFrame(meas, index=pd.DatetimeIndex(pd.to_datetime(mt, unit="ns", utc=True)).as_unit("ns"),
-                       columns=[d["reach_ids"][j] for j in gidx])
-    R = 1e-2 * np.eye(m)
-    q = rng.uniform(0.5, 2.0, size=n)
-    enkf = EnsembleKalmanFilter(mdl, mdf, q, R)
-    Zp = meas[:, :, None] + 0.1 * rng.standard_normal((nwin, m, M))
-    f = mdl.make_forcing(times_ns=times, table=table, member_mul=mul)
-    ung = np.setdiff1d(np.arange(n), gidx)
-    reaches = rng.permutation(np.concatenate([gidx[:max(3, m // 2)], rng.choice(ung, size=40, replace=False)]))
-    Zd = torch.as_tensor(np.ascontiguousarray(Zp), device="cuda")
-    out = {}
-
-    def run():
-        out["r"] = mdl.run_assimilating(f, nsteps, enkf, every, Zd if in_library else list(Zd), record_reaches=reaches,
-                                        record_prior=True)
-    names = _kernels(torch, run)
-    mdl.network.check()
-    rec, prior = out["r"]
-    ind = oracle.compute_indegree(net_d["startnodes"], net_d["endnodes"])
-    al, be, ch, ga = oracle.compute_coeffs(prm["K"], prm["X"], 300.0)
-    onet = {"startnodes": net_d["startnodes"], "endnodes": net_d["endnodes"], "indegree": ind,
-            "alpha": al, "beta": be, "chi": ch, "gamma": ga}
-    o = np.ascontiguousarray(o0.T)
-    i = np.stack([oracle.init_states(net_d["startnodes"], net_d["endnodes"], x) for x in o])
-    hyd = np.empty((nsteps, reaches.size, M))
-    pri = np.empty((nwin, reaches.size, M))
-    # Error scales.  An update forms o + gain; where the gain cancels most of the forecast (here down to 1e-6 of it)
-    # no FP64 implementation holds the posterior to 1e-9 of its own size, only to 1e-9 of the forecast
-    # (parity.relerr).  Routing is linear, so that absolute error travels on with the state: e' = A e, and
-    # |A e| <= |A| |e|.  The scale of every later step is therefore max(|post|, |forecast|) routed with the absolute
-    # values of the coefficients and no forcing (om, im), and the value's own size where that is larger.  (Measured
-    # on these cases: the FP64 oracle's update, against the extended-precision one, stays within 4e-12 of this scale
-    # and exceeds 1e-9 of |value| by up to 20x a few steps after an update.)
-    om = np.zeros_like(o); im = np.zeros_like(i)
-    anet = dict(onet, alpha=np.abs(al), beta=np.abs(be), chi=np.abs(ch), gamma=np.zeros(n))
-    zero = np.zeros_like(table)
-    sc = np.empty_like(hyd)
-    sc_pri = np.empty_like(pri)
-    tol, oracle_err = RTOL, 0.0
-    for s in range(1, nsteps + 1):
-        t = float(t0 + (s - 1) * 300e9)
-        oracle.run_members(onet, o, i, 1, times.astype(np.float64), table, t, 300e9, wmul=mul)
-        oracle.run_members(anet, om, im, 1, times.astype(np.float64), zero, t, 300e9)
-        hyd[s - 1] = o[:, reaches].T
-        sc[s - 1] = om[:, reaches].T
-        if s % every == 0 and s // every <= nwin:
-            k = s // every - 1
-            pri[k] = o[:, reaches].T
-            sc_pri[k] = om[:, reaches].T
-            tol = max(tol, enkf_tolerance(o.T, gidx, q, R))
-            # the update in extended precision (the routing between updates is exact enough in FP64); the FP64
-            # oracle's explicit-inverse update is kept for comparison only
-            O, I = o.T, i.T
-            mean = np.asarray(np.asarray(O, dtype=E.LD).sum(axis=1) / M, dtype=np.float64)
-            T, W, _ = E.solve_ref(O[gidx], Zp[k], mean[gidx], q[gidx], R)
-            Op, Ip = E.apply_ref(O, I, mean, T, W, gidx, q[gidx], net_d["endnodes"])
-            Op, Ip = _f64(Op), _f64(Ip)
-            Oo, _, _ = oracle.enkf_update(onet, O, I, gidx, Zp[k], q, R)
-            oracle_err = max(oracle_err, relerr(Oo, Op, scale=np.abs(O)))
-            om = np.ascontiguousarray(np.maximum(np.abs(Op), np.abs(O)).T)
-            im = np.ascontiguousarray(np.maximum(np.abs(Ip), np.abs(I)).T)
-            o = np.ascontiguousarray(Op.T); i = np.ascontiguousarray(Ip.T)
-            hyd[s - 1] = o[:, reaches].T
-            sc[s - 1] = om[:, reaches].T
-    return names, rec.cpu().numpy(), prior.cpu().numpy(), mdl.o_t_next[reaches], hyd, pri, sc, sc_pri, tol, oracle_err
-
-
-def _loop_kernels(M, m, kernel, in_library):
-    ld = M + (M & 1)
-    solve = ["enkf_small_system_kernel"] if (M < m and M <= 64) else \
-            ["chol_solve_blocked_kernel<128>"] if M < m and M <= 128 else ["woodbury_assemble_kernel"]
-    route = {"lane": "route_lane_kernel", "dataflow": "route_dataflow_kernel"}.get(kernel, "route_window_kernel")
-    want = [route] + solve
-    if ld > 64:
-        return want + ["enkf_update_kernel", "apply_gain_kernel"] + (["enkf_record_kernel"] if in_library else [])
-    if kernel in ("lane", "dataflow"):
-        # the row sums: enkf_stats after the routing launch
-        return want + ["enkf_stats_kernel", "enkf_update64_kernel"] + (
-            ["enkf_record_kernel", "inflow_rebuild_kernel"] if in_library else ["inflow_gain_kernel"])
-    if in_library:                                     # the next window applies the update and records its rows
-        return want + ["route_window_kernel<true, true, true, true>"]
-    return want + ["enkf_update64_kernel"]
-
-
-LOOP_CASES = [  # n, M, m, seed, every, nwin, rest, route kernel, also with the Python loop
-    (2500, 64, 120, 81, 6, 3, 0, None, True),       # cluster kernel + UPD window + record_posterior at M = 64
-    (2500, 63, 90, 82, 6, 3, 0, None, False),       # pad column on the TMA bulk path (ld = 64)
-    (2500, 33, 70, 83, 6, 3, 4, None, True),        # odd M on cp.async; the remainder launch applies the last update
-    (2000, 5, 12, 84, 6, 3, 0, None, False),        # smallest window-kernel ensemble; most cluster CTAs empty
-    (2000, 2, 6, 85, 6, 3, 0, "lane", True),        # lane kernel + stand-alone update + enkf_record_kernel
-    (2000, 3, 8, 86, 6, 3, 2, "lane", False),
-    (2000, 16, 40, 87, 12, 3, 0, "lane", True),     # lane kernel at its largest M, hourly updates
-    (2000, 40, 60, 88, 6, 3, 0, "dataflow", True),  # stand-alone update after the dataflow kernel
-    (2500, 97, 200, 89, 6, 3, 0, None, True),       # partial Cholesky panel (chol<128>)
-    (2500, 129, 300, 90, 6, 3, 3, None, False),     # three member blocks with a pad; M > 128 solve
-    (4000, 64, 1100, 91, 6, 3, 0, None, False),     # cluster kernel with more than one gauge tile per CTA
-]
-
-
-def _loop_params():
-    out = []
-    for c in LOOP_CASES:
-        out.append(pytest.param(*c[:8], True, id=f"M{c[1]}-m{c[2]}-{c[7] or 'default'}-lib"))
-        if c[8]:
-            out.append(pytest.param(*c[:8], False, id=f"M{c[1]}-m{c[2]}-{c[7] or 'default'}-py"))
-    return out
-
-
-@pytest.mark.parametrize("n,M,m,seed,every,nwin,rest,kernel,in_library", _loop_params())
+@pytest.mark.parametrize("n,M,m,seed,every,nwin,rest,kernel,in_library", loop_params(LOOP_CASES))
 def test_assimilation_loop_paths_vs_oracle(torch_cuda, oracle, monkeypatch, record_property, n, M, m, seed, every,
                                            nwin, rest, kernel, in_library):
     """run_assimilating with record_reaches and record_prior: hydrographs (forecast, posterior at update steps),
     priors and final state against the oracle's routing and the extended-precision update, with the tolerance of
-    test_gpu_record.py (1e-9, or 64 eps cond(S) after an update) relative to the error scale of _loop_case."""
-    names, rec, prior, final, hyd, pri, sc, sc_pri, tol, oracle_err = _loop_case(
-        torch_cuda, oracle, monkeypatch, n, M, m, seed, every, nwin, rest, kernel, in_library)
-    _expect(names, _loop_kernels(M, m, kernel, in_library))
+    test_gpu_record.py (1e-9, or 64 eps cond(S) after an update) relative to the error scale of
+    assim_case.reference_loop."""
+    c = make_case(n, M, m, seed, every, nwin, rest, gauges="reference")
+    d = run_device(c, in_library, monkeypatch=monkeypatch, kernel=kernel)
+    r = reference_loop(oracle, c, update_ref)
+    _expect(d["names"], _loop_kernels(M, m, kernel, in_library))
+    (rec, prior), final = d["res"], d["final"]
+    hyd, pri, sc, sc_pri, tol, oracle_err = r["hyd"], r["pri"], r["sc"], r["sc_pri"], r["tol"], max(r["kept"])
     nsteps = every * nwin + rest
     assert rec.shape == hyd.shape and prior.shape == pri.shape
     assert not np.isnan(rec).any() and not np.isnan(prior).any()

@@ -9,6 +9,8 @@ Tolerances: T' and W' against the reference at etkf_reference.case's bounds -- t
 enkf_reference.solve_tolerance (64 eps cond), for T' of the ETKF amplified by M / (2 sqrt(lambda_min(G))), the
 conditioning of the matrix square root, plus the Jacobi stop (1e-14 ||G||_F).  The loops use the tolerance of
 test_gpu_enkf_paths.py times the same amplification of the worst update."""
+import functools
+
 import numpy as np
 import pandas as pd
 import pytest
@@ -16,10 +18,10 @@ import pytest
 import enkf_reference as E
 import enkf_missing_reference as X
 import etkf_reference as K
+from assim_case import (torch_cuda, fnet, _kernels, _expect, _f64, _solve_dev, _solve_kernels,  # noqa: F401
+                        make_case, run_device, reference_loop, update_etkf)
 from enks_oracle import smooth_transforms
-from parity import relerr, normerr, enkf_tolerance
-from test_gpu_enkf_paths import (torch_cuda, fnet, _kernels, _expect, _dev, _f64, _solve_dev,  # noqa: F401
-                                 _solve_kernels, RTOL)
+from parity import relerr, normerr
 
 pytestmark = pytest.mark.gpu
 
@@ -213,98 +215,15 @@ def test_refusals(torch_cuda):
 
 
 # ---- (c) the loops and the smoother ----------------------------------------------------------------------------------
-def _etkf_loop(torch, oracle, monkeypatch, n, M, m, seed, every, nwin, rest, kernel, in_library, rho=0.0, lag=None,
-               outage=True):
-    """An ETKF run (identical observation columns; an outlet gauge missing at every update and every gauge at update
-    1 when `outage`) on the device, and the same run in extended precision: the oracle's routing and the reference's
-    T', W' applied by enkf_reference.apply_ref.  Returns the device results, the reference hydrographs, their error
-    scales (test_gpu_enkf_paths.py:_loop_case), the tolerance and the reference transforms."""
-    if kernel is not None:
-        monkeypatch.setenv("TXH_ROUTE_KERNEL", kernel)
-    else:
-        monkeypatch.delenv("TXH_ROUTE_KERNEL", raising=False)
-    from tx_fast_hydrology_b200 import synthetic as S
-    from tx_fast_hydrology_b200.muskingum import Muskingum
-    from tx_fast_hydrology_b200.da import EnsembleKalmanFilter
-    nsteps = every * nwin + rest
-    net_d = S.make_network(n, seed)
-    prm = S.make_params(n, seed, well_posed=True)
-    rng = np.random.default_rng(seed)
-    o0 = prm["o_t"][:, None] * rng.uniform(0.5, 1.5, size=(n, M))
-    d = S.model_dict(net_d, prm, dt_s=300.0)
-    d["o_t"] = o0
-    mdl = Muskingum(d, members=M)
-    t0 = int(mdl.datetime.value)
-    times, table = S.make_forcing(n, nsteps, 300.0, seed, t0_ns=t0, rows_every=4)
-    mul = S.make_member_multipliers(times.size, M, seed)
-    gidx = E.gauge_set(net_d["endnodes"], m, seed)
-    mt = t0 + (np.arange(nwin, dtype=np.int64) + 1) * int(every * 300e9)
-    meas = rng.uniform(0.5, 8.0, size=(nwin, m))
-    mdf = pd.DataFrame(meas, index=pd.DatetimeIndex(pd.to_datetime(mt, unit="ns", utc=True)).as_unit("ns"),
-                       columns=[d["reach_ids"][j] for j in gidx])
-    R = 1e-2 * np.eye(m)
-    q = rng.uniform(0.5, 2.0, size=n)
-    enkf = EnsembleKalmanFilter(mdl, mdf, q, R, method="etkf", rtpp=rho)
-    Zp = np.repeat(meas[:, :, None], M, axis=2)
-    if outage:
-        end = np.asarray(net_d["endnodes"])
-        Zp[:, np.flatnonzero(end[gidx] == gidx)[0]] = np.nan
-        if nwin > 1:
-            Zp[1] = np.nan
-    f = mdl.make_forcing(times_ns=times, table=table, member_mul=mul)
-    ung = np.setdiff1d(np.arange(n), gidx)
-    reaches = rng.permutation(np.concatenate([gidx[:max(3, m // 2)], rng.choice(ung, size=40, replace=False)]))
-    Zd = torch.as_tensor(np.ascontiguousarray(Zp), device="cuda")
-    out = {}
-
-    def run():
-        out["r"] = mdl.run_assimilating(f, nsteps, enkf, every, Zd if in_library else list(Zd), record_reaches=reaches,
-                                        record_prior=True, smooth_lag=lag)
-    names = _kernels(torch, run)
-    mdl.network.check()
-    res = [x.cpu().numpy() for x in out["r"]]
-    ind = oracle.compute_indegree(net_d["startnodes"], net_d["endnodes"])
-    al, be, ch, ga = oracle.compute_coeffs(prm["K"], prm["X"], 300.0)
-    onet = {"startnodes": net_d["startnodes"], "endnodes": net_d["endnodes"], "indegree": ind,
-            "alpha": al, "beta": be, "chi": ch, "gamma": ga}
-    o = np.ascontiguousarray(o0.T)
-    i = np.stack([oracle.init_states(net_d["startnodes"], net_d["endnodes"], x) for x in o])
-    hyd = np.empty((nsteps, reaches.size, M))
-    pri = np.empty((nwin, reaches.size, M))
-    om = np.zeros_like(o); im = np.zeros_like(i)
-    anet = dict(onet, alpha=np.abs(al), beta=np.abs(be), chi=np.abs(ch), gamma=np.zeros(n))
-    zero = np.zeros_like(table)
-    sc = np.empty_like(hyd)
-    sc_pri = np.empty_like(pri)
-    tol, amp, Ts = RTOL, 1.0, []
-    for s in range(1, nsteps + 1):
-        t = float(t0 + (s - 1) * 300e9)
-        oracle.run_members(onet, o, i, 1, times.astype(np.float64), table, t, 300e9, wmul=mul)
-        oracle.run_members(anet, om, im, 1, times.astype(np.float64), zero, t, 300e9)
-        hyd[s - 1] = o[:, reaches].T
-        sc[s - 1] = om[:, reaches].T
-        if s % every == 0 and s // every <= nwin:
-            k = s // every - 1
-            pri[k] = o[:, reaches].T
-            sc_pri[k] = om[:, reaches].T
-            O, I = o.T, i.T
-            keep = ~X.missing_rows(Zp[k])
-            if keep.any():
-                tol = max(tol, enkf_tolerance(O, gidx[keep], q, R[np.ix_(keep, keep)]))
-            mean = np.asarray(np.asarray(O, dtype=E.LD).sum(axis=1) / M, dtype=np.float64)
-            T, W, _, _ = X.solve_masked(O[gidx], Zp[k], mean[gidx], q[gidx], R)
-            amp = max(amp, M / (2.0 * np.sqrt(K.lambda_min(T))))
-            Tp, Wp = K.etkf_post(T, W, rho)
-            Ts.append(_f64(Tp))
-            Op, Ip = E.apply_ref(O, I, mean, Tp, Wp, gidx, q[gidx], net_d["endnodes"])
-            Op, Ip = _f64(Op), _f64(Ip)
-            om = np.ascontiguousarray(np.maximum(np.abs(Op), np.abs(O)).T)
-            im = np.ascontiguousarray(np.maximum(np.abs(Ip), np.abs(I)).T)
-            o = np.ascontiguousarray(Op.T); i = np.ascontiguousarray(Ip.T)
-            hyd[s - 1] = o[:, reaches].T
-            sc[s - 1] = om[:, reaches].T
-    return dict(names=names, res=res, final=mdl.o_t_next[reaches], hyd=hyd, pri=pri, sc=sc, sc_pri=sc_pri,
-                tol=tol * amp, Ts=Ts)
+def _etkf_case(n, M, m, seed, every, nwin, rest):
+    """A loop case for the ETKF: identical observation columns, an outlet gauge missing at every update and every gauge
+    missing at update 1."""
+    c = make_case(n, M, m, seed, every, nwin, rest, gauges="reference", observations="identical")
+    end = np.asarray(c["net"]["endnodes"])
+    c["Zp"][:, np.flatnonzero(end[c["gidx"]] == c["gidx"])[0]] = np.nan
+    if nwin > 1:
+        c["Zp"][1] = np.nan
+    return c
 
 
 ETKF_LOOPS = [  # n, M, m, seed, every, nwin, rest, route kernel, in the library
@@ -323,30 +242,35 @@ def test_etkf_assimilation_loop_vs_reference(torch_cuda, oracle, monkeypatch, re
                                              nwin, rest, kernel, in_library, rho):
     """Hydrographs, priors and final state of an ETKF run (with an outage) against the extended-precision loop; the
     post kernel runs once per update; the update with every gauge missing leaves the state as it was."""
-    r = _etkf_loop(torch_cuda, oracle, monkeypatch, n, M, m, seed, every, nwin, rest, kernel, in_library, rho=rho)
-    assert r["names"].count(POST + "(") == nwin
+    c = _etkf_case(n, M, m, seed, every, nwin, rest)
+    d = run_device(c, in_library, monkeypatch=monkeypatch, kernel=kernel, method="etkf", rtpp=rho)
+    r = reference_loop(oracle, c, functools.partial(update_etkf, rho=rho))
+    assert d["names"].count(POST + "(") == nwin
     if kernel is None and in_library:
-        _expect(r["names"], [FUSED])                                                  # applied by the next window
+        _expect(d["names"], [FUSED])                                                  # applied by the next window
     elif kernel is not None:
-        _expect(r["names"], ["enkf_update64_kernel"])                                 # the stand-alone kernels
-    rec, prior = r["res"]
+        _expect(d["names"], ["enkf_update64_kernel"])                                 # the stand-alone kernels
+    rec, prior = d["res"]
     e_pri, e_rec = relerr(prior, r["pri"], scale=r["sc_pri"]), relerr(rec, r["hyd"], scale=r["sc"])
     record_property("rec_ratio", e_rec / r["tol"])
     assert e_pri < r["tol"], f"priors: {e_pri:.2e}, bound {r['tol']:.2e}"
     assert e_rec < r["tol"], f"hydrographs: {e_rec:.2e}, bound {r['tol']:.2e}"
     nsteps = every * nwin + rest
-    assert relerr(r["final"], r["hyd"][nsteps - 1], scale=r["sc"][nsteps - 1]) < r["tol"]
+    assert relerr(d["final"], r["hyd"][nsteps - 1], scale=r["sc"][nsteps - 1]) < r["tol"]
     assert np.array_equal(rec[2 * every - 1], prior[1]), "the update with every gauge missing changed the state"
 
 
 def test_fused_load_matches_standalone_apply(torch_cuda, oracle, monkeypatch):
     """The same ETKF run with the update applied by the next window launch and by the stand-alone kernels (dataflow
     routing): the hydrographs agree to the loop tolerance."""
-    a = _etkf_loop(torch_cuda, oracle, monkeypatch, 2000, 40, 60, 88, 6, 3, 0, None, True, rho=0.2)
-    b = _etkf_loop(torch_cuda, oracle, monkeypatch, 2000, 40, 60, 88, 6, 3, 0, "dataflow", True, rho=0.2)
+    c = _etkf_case(2000, 40, 60, 88, 6, 3, 0)
+    a = run_device(c, True, monkeypatch=monkeypatch, method="etkf", rtpp=0.2)
+    r = reference_loop(oracle, c, functools.partial(update_etkf, rho=0.2))
+    b = run_device(_etkf_case(2000, 40, 60, 88, 6, 3, 0), True, monkeypatch=monkeypatch, kernel="dataflow",
+                   method="etkf", rtpp=0.2)
     _expect(a["names"], [FUSED])
     _expect(b["names"], ["route_dataflow_kernel", "enkf_update64_kernel"])
-    assert relerr(a["res"][0], b["res"][0], scale=a["sc"]) < a["tol"]
+    assert relerr(a["res"][0], b["res"][0], scale=r["sc"]) < r["tol"]
 
 
 @pytest.mark.parametrize("in_library", [True, False])
@@ -355,9 +279,10 @@ def test_smoother_on_an_etkf_run(torch_cuda, oracle, monkeypatch, in_library):
     reference ETKF transforms."""
     n, M, m, seed, every, nwin, rest = 2500, 64, 120, 81, 6, 3, 0
     lag = every + 2
-    r = _etkf_loop(torch_cuda, oracle, monkeypatch, n, M, m, seed, every, nwin, rest, None, in_library, lag=lag)
-    rec, prior, sm = r["res"]
-    want = smooth_transforms(r["hyd"], np.stack(r["Ts"]), nwin, every, 1, lag)
+    c = _etkf_case(n, M, m, seed, every, nwin, rest)
+    rec, prior, sm = run_device(c, in_library, monkeypatch=monkeypatch, lag=lag, method="etkf")["res"]
+    r = reference_loop(oracle, c, update_etkf)
+    want = smooth_transforms(r["hyd"], np.stack(r["kept"]), nwin, every, 1, lag)
     sc = np.maximum(np.maximum(np.abs(want), r["sc"]), np.abs(rec))
     assert np.isfinite(sm).all()
     assert relerr(sm, want, scale=sc) < r["tol"] * (nwin + 1)

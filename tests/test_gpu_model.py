@@ -8,6 +8,7 @@ import pandas as pd
 import pytest
 
 pytestmark = pytest.mark.gpu
+HERE = os.path.dirname(os.path.abspath(__file__))
 RTOL = 1e-9
 # Dense filter / smoother quantities are held to the same 1e-9 as the states.  Measured on B200 against the
 # reference goldens (tests/perf/kf_error_budget.py, profiles/r02_kf_error_budget.json): gains 6e-16, P 2.4e-16,
@@ -18,6 +19,7 @@ SMOOTH_X_TOL = RTOL
 SMOOTH_P_TOL = RTOL
 
 
+from assim_case import make_case, model, oracle_start
 from parity import relerr, normerr, enkf_tolerance        # element-wise with a floor / max-norm (dense matrices)
 
 
@@ -337,35 +339,10 @@ def _run_assimilating_case(oracle, n, M, m, seed, in_library, every=6, nwin=3, r
     """`nwin` windows of `every` routing steps + one EnKF update each, then `rest` more routing steps, on the device
     (through the Python API) and on the CPU oracle; returns what the assertions need."""
     import torch
-    from tx_fast_hydrology_b200 import synthetic as S
-    from tx_fast_hydrology_b200.muskingum import Muskingum
-    from tx_fast_hydrology_b200.da import EnsembleKalmanFilter
-    nsteps = every * nwin + rest
-    net_d = S.make_network(n, seed)
-    prm = S.make_params(n, seed, well_posed=True)
-    rng = np.random.default_rng(seed)
-    o0 = prm["o_t"][:, None] * rng.uniform(0.5, 1.5, size=(n, M))
-    d = S.model_dict(net_d, prm, dt_s=300.0)
-    d["o_t"] = o0
-    mdl = Muskingum(d, members=M)
-    t0 = int(mdl.datetime.value)
-    times, table = S.make_forcing(n, nsteps, 300.0, seed, t0_ns=t0, rows_every=4)
-    mul = S.make_member_multipliers(times.size, M, seed)
-    if gidx is None:
-        gidx = S.make_gauges(net_d["endnodes"], m, seed=seed)
-    gidx = np.asarray(gidx, dtype=np.int64)
-    m = gidx.size
-    mt = t0 + (np.arange(nwin, dtype=np.int64) + 1) * int(every * 300e9)
-    meas = rng.uniform(0.5, 8.0, size=(nwin, m))
-    mdf = frame(mt, meas, [d["reach_ids"][j] for j in gidx])
-    R = 1e-2 * np.eye(m)
-    if dense_R:                                                   # correlated observation errors: SPD, not diagonal
-        Bm = rng.standard_normal((m, m))
-        R = 1e-2 * (np.eye(m) + 0.5 * (Bm @ Bm.T) / m)
-    q = rng.uniform(0.5, 2.0, size=n)
-    enkf = EnsembleKalmanFilter(mdl, mdf, q, R)
-    Zp = meas[:, :, None] + 0.1 * rng.standard_normal((nwin, m, M))
-    f = mdl.make_forcing(times_ns=times, table=table, member_mul=mul)
+    c = make_case(n, M, m, seed, every, nwin, rest, gauges="synthetic" if gidx is None else gidx, dense_R=dense_R,
+                  extra_reaches=None)
+    mdl, enkf, f = model(c)
+    nsteps, t0, Zp, gidx, q, R = c["nsteps"], c["t0"], c["Zp"], c["gidx"], c["q"], c["R"]
     # the observations travel on a side stream; the first update waits for the event, the first window does not
     Zh = torch.from_numpy(np.ascontiguousarray(Zp)).pin_memory()
     Zd = torch.empty(Zh.shape, dtype=torch.float64, device="cuda")
@@ -376,12 +353,8 @@ def _run_assimilating_case(oracle, n, M, m, seed, in_library, every=6, nwin=3, r
     mdl.run_assimilating(f, nsteps, enkf, every, Zd if in_library else list(Zd), observations_ready=ready)
     mdl.network.check()
     assert enkf.n_updates == nwin and mdl.datetime.value == t0 + int(nsteps * 300e9)
-    ind = oracle.compute_indegree(net_d["startnodes"], net_d["endnodes"])
-    al, be, ch, ga = oracle.compute_coeffs(prm["K"], prm["X"], 300.0)
-    onet = {"startnodes": net_d["startnodes"], "endnodes": net_d["endnodes"], "indegree": ind,
-            "alpha": al, "beta": be, "chi": ch, "gamma": ga}
-    o = np.ascontiguousarray(o0.T)
-    i = np.stack([oracle.init_states(net_d["startnodes"], net_d["endnodes"], x) for x in o])
+    onet, o, i = oracle_start(oracle, c)
+    times, table, mul = c["times"], c["table"], c["mul"]
     t = float(t0)
     tol = RTOL
     so, si = np.zeros((n, M)), np.zeros((n, M))                   # magnitudes of the forecasts the updates started from
@@ -469,29 +442,14 @@ def test_run_assimilating_variants_agree():
     import tempfile
     code = (
         "import sys, numpy as np, torch\n"
-        "sys.path.insert(0, %r)\n"
-        "from tx_fast_hydrology_b200 import synthetic as S\n"
-        "from tx_fast_hydrology_b200.muskingum import Muskingum\n"
-        "from tx_fast_hydrology_b200.da import EnsembleKalmanFilter\n"
-        "import pandas as pd\n"
-        "n, M, m, seed, every, nwin = 2500, 64, 40, 21, 6, 4\n"
-        "net = S.make_network(n, seed); prm = S.make_params(n, seed, well_posed=True)\n"
-        "rng = np.random.default_rng(seed)\n"
-        "d = S.model_dict(net, prm, dt_s=300.0); d['o_t'] = prm['o_t'][:, None] * rng.uniform(0.5, 1.5, size=(n, M))\n"
-        "mdl = Muskingum(d, members=M); t0 = int(mdl.datetime.value)\n"
-        "times, table = S.make_forcing(n, every * nwin, 300.0, seed, t0_ns=t0, rows_every=4)\n"
-        "mul = S.make_member_multipliers(times.size, M, seed)\n"
-        "g = S.make_gauges(net['endnodes'], m, seed=seed)\n"
-        "mt = t0 + (np.arange(nwin, dtype=np.int64) + 1) * int(every * 300e9)\n"
-        "meas = rng.uniform(0.5, 8.0, size=(nwin, m))\n"
-        "idx = pd.DatetimeIndex(pd.to_datetime(mt, unit='ns', utc=True)).as_unit('ns')\n"
-        "mdf = pd.DataFrame(meas, index=idx, columns=[d['reach_ids'][j] for j in g])\n"
-        "enkf = EnsembleKalmanFilter(mdl, mdf, rng.uniform(0.5, 2.0, size=n), 1e-2 * np.eye(m))\n"
-        "Zp = torch.as_tensor(meas[:, :, None] + 0.1 * rng.standard_normal((nwin, m, M)), device='cuda')\n"
-        "f = mdl.make_forcing(times_ns=times, table=table, member_mul=mul)\n"
-        "mdl.run_assimilating(f, every * nwin, enkf, every, Zp)\n"
+        "sys.path.insert(0, %r); sys.path.insert(0, %r)\n"
+        "from assim_case import make_case, model\n"
+        "c = make_case(2500, 64, 40, 21, 6, 4, 0, gauges='synthetic', extra_reaches=None)\n"
+        "mdl, enkf, f = model(c)\n"
+        "Zp = torch.as_tensor(c['Zp'], device='cuda')\n"
+        "mdl.run_assimilating(f, c['nsteps'], enkf, 6, Zp)\n"
         "mdl.network.check()\n"
-        "np.savez(sys.argv[1], o=mdl.o_t_next, i=mdl.i_t_next)\n") % os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+        "np.savez(sys.argv[1], o=mdl.o_t_next, i=mdl.i_t_next)\n") % (os.path.dirname(HERE), HERE)
     out = {}
     with tempfile.TemporaryDirectory() as tmp:
         for name, env in (("fused", {}), ("plain", {"TXH_ENKF_FUSED": "0", "TXH_ENKF_FUSE_LOAD": "0", "TXH_PDL": "0"})):

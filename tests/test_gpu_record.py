@@ -12,15 +12,10 @@ import pytest
 pytestmark = pytest.mark.gpu
 
 RTOL = 1e-9
+HERE = os.path.dirname(os.path.abspath(__file__))
 
-from parity import relerr, normerr, enkf_tolerance        # noqa: E402
-
-
-@pytest.fixture(scope="module")
-def torch_cuda():
-    import torch
-    assert torch.cuda.is_available(), "GPU tests need a CUDA device (no CPU fallback exists)"
-    return torch
+from assim_case import torch_cuda, make_case, model, run_device, reference_loop, update_fp64  # noqa: E402, F401
+from parity import relerr, normerr        # noqa: E402
 
 
 def _upload(net, o, i, M):
@@ -145,68 +140,6 @@ def test_recording_leaves_route_state_alone(torch_cuda, monkeypatch, M):
     assert (out[0][0] == out[1][0]).all() and (out[0][1] == out[1][1]).all()
 
 
-def _assim_case(oracle, n, M, m, seed, in_library, every, nwin, rest=0, dense_R=False, record_every=1, reaches=None):
-    """_run_assimilating_case of test_gpu_model.py with recording: returns the device's (rec, prior, final state) and
-    the oracle's hydrographs at every step (posterior at update steps), its priors and tolerances."""
-    import torch
-    from tx_fast_hydrology_b200 import synthetic as S
-    from tx_fast_hydrology_b200.muskingum import Muskingum
-    from tx_fast_hydrology_b200.da import EnsembleKalmanFilter
-    nsteps = every * nwin + rest
-    net_d = S.make_network(n, seed)
-    prm = S.make_params(n, seed, well_posed=True)
-    rng = np.random.default_rng(seed)
-    o0 = prm["o_t"][:, None] * rng.uniform(0.5, 1.5, size=(n, M))
-    d = S.model_dict(net_d, prm, dt_s=300.0)
-    d["o_t"] = o0
-    mdl = Muskingum(d, members=M)
-    t0 = int(mdl.datetime.value)
-    times, table = S.make_forcing(n, nsteps, 300.0, seed, t0_ns=t0, rows_every=4)
-    mul = S.make_member_multipliers(times.size, M, seed)
-    gidx = np.asarray(S.make_gauges(net_d["endnodes"], m, seed=seed), dtype=np.int64)
-    m = gidx.size
-    mt = t0 + (np.arange(nwin, dtype=np.int64) + 1) * int(every * 300e9)
-    meas = rng.uniform(0.5, 8.0, size=(nwin, m))
-    mdf = pd.DataFrame(meas, index=pd.DatetimeIndex(pd.to_datetime(mt, unit="ns", utc=True)).as_unit("ns"),
-                       columns=[d["reach_ids"][j] for j in gidx])
-    R = 1e-2 * np.eye(m)
-    if dense_R:
-        Bm = rng.standard_normal((m, m))
-        R = 1e-2 * (np.eye(m) + 0.5 * (Bm @ Bm.T) / m)
-    q = rng.uniform(0.5, 2.0, size=n)
-    enkf = EnsembleKalmanFilter(mdl, mdf, q, R)
-    Zp = meas[:, :, None] + 0.1 * rng.standard_normal((nwin, m, M))
-    f = mdl.make_forcing(times_ns=times, table=table, member_mul=mul)
-    if reaches is None:                      # gauged and ungauged reaches, in no particular order
-        ung = np.setdiff1d(np.arange(n), gidx)
-        reaches = rng.permutation(np.concatenate([gidx[:max(3, m // 2)], rng.choice(ung, size=60, replace=False)]))
-    Zd = torch.as_tensor(np.ascontiguousarray(Zp), device="cuda")
-    rec, prior = mdl.run_assimilating(f, nsteps, enkf, every, Zd if in_library else list(Zd), record_reaches=reaches,
-                                      record_every=record_every, record_prior=True)
-    mdl.network.check()
-    ind = oracle.compute_indegree(net_d["startnodes"], net_d["endnodes"])
-    al, be, ch, ga = oracle.compute_coeffs(prm["K"], prm["X"], 300.0)
-    onet = {"startnodes": net_d["startnodes"], "endnodes": net_d["endnodes"], "indegree": ind,
-            "alpha": al, "beta": be, "chi": ch, "gamma": ga}
-    o = np.ascontiguousarray(o0.T)
-    i = np.stack([oracle.init_states(net_d["startnodes"], net_d["endnodes"], x) for x in o])
-    hyd = np.empty((nsteps, reaches.size, M))
-    pri = np.empty((nwin, reaches.size, M))
-    tol = RTOL
-    for s in range(1, nsteps + 1):
-        oracle.run_members(onet, o, i, 1, times.astype(np.float64), table, float(t0 + (s - 1) * 300e9), 300e9, wmul=mul)
-        hyd[s - 1] = o[:, reaches].T
-        if s % every == 0 and s // every <= nwin:
-            k = s // every - 1
-            pri[k] = o[:, reaches].T
-            tol = max(tol, enkf_tolerance(o.T, gidx, q, R))
-            Op, Ip, _ = oracle.enkf_update(onet, o.T, i.T, gidx, Zp[k], q, R)
-            o = np.ascontiguousarray(Op.T); i = np.ascontiguousarray(Ip.T)
-            hyd[s - 1] = o[:, reaches].T
-    sel = np.arange(record_every, nsteps + 1, record_every) - 1
-    return rec.cpu().numpy(), prior.cpu().numpy(), mdl.o_t_next[reaches], hyd[sel], pri, tol, sel
-
-
 @pytest.mark.parametrize("n,M,m,seed,every,nwin,rest,record_every,dense_R", [
     (2000, 64, 50, 51, 6, 3, 0, 1, False),
     (1200, 20, 30, 52, 6, 3, 4, 4, False),       # 4 does not divide 6; remainder steps
@@ -218,8 +151,11 @@ def test_run_assimilating_recording_vs_oracle(oracle, n, M, m, seed, every, nwin
                                               in_library):
     """rec = the forecast at non-update steps and the posterior at update steps; prior = the forecast every update
     started from; the last slot is the final state when record_every divides nsteps."""
-    rec, prior, final, want, pri, tol, sel = _assim_case(oracle, n, M, m, seed, in_library, every, nwin, rest, dense_R,
-                                                         record_every)
+    c = make_case(n, M, m, seed, every, nwin, rest, gauges="synthetic", dense_R=dense_R, extra_reaches=60)
+    d = run_device(c, in_library, record_every=record_every)
+    r = reference_loop(oracle, c, update_fp64, record_every=record_every)
+    (rec, prior), final = d["res"], d["final"]
+    want, pri, tol, sel = r["hyd"], r["pri"], r["tol"], r["sel"]
     assert rec.shape == want.shape and prior.shape == pri.shape
     assert relerr(prior, pri) < tol
     assert relerr(rec, want, scale=_update_scale(want, pri, sel, every)) < tol
@@ -239,25 +175,12 @@ def _update_scale(want, pri, sel, every):
 def test_run_assimilating_recording_leaves_state_alone():
     """run_assimilating with and without recording end in the bit-identical state (in-library loop, M = 64)."""
     import torch
-    from tx_fast_hydrology_b200 import synthetic as S
-    from tx_fast_hydrology_b200.muskingum import Muskingum
-    from tx_fast_hydrology_b200.da import EnsembleKalmanFilter
     n, M, m, seed, every, nwin = 2500, 64, 40, 56, 6, 3
     out = []
     for record in (False, True):
-        net = S.make_network(n, seed); prm = S.make_params(n, seed, well_posed=True)
-        rng = np.random.default_rng(seed)
-        d = S.model_dict(net, prm, dt_s=300.0); d["o_t"] = prm["o_t"][:, None] * rng.uniform(0.5, 1.5, size=(n, M))
-        mdl = Muskingum(d, members=M); t0 = int(mdl.datetime.value)
-        times, table = S.make_forcing(n, every * nwin, 300.0, seed, t0_ns=t0, rows_every=4)
-        g = S.make_gauges(net["endnodes"], m, seed=seed)
-        mt = t0 + (np.arange(nwin, dtype=np.int64) + 1) * int(every * 300e9)
-        meas = rng.uniform(0.5, 8.0, size=(nwin, m))
-        mdf = pd.DataFrame(meas, index=pd.DatetimeIndex(pd.to_datetime(mt, unit="ns", utc=True)).as_unit("ns"),
-                           columns=[d["reach_ids"][j] for j in g])
-        enkf = EnsembleKalmanFilter(mdl, mdf, rng.uniform(0.5, 2.0, size=n), 1e-2 * np.eye(m))
-        Zp = torch.as_tensor(meas[:, :, None] + 0.1 * rng.standard_normal((nwin, m, M)), device="cuda")
-        f = mdl.make_forcing(times_ns=times, table=table, member_mul=S.make_member_multipliers(times.size, M, seed))
+        c = make_case(n, M, m, seed, every, nwin, 0, gauges="synthetic", extra_reaches=None)
+        mdl, enkf, f = model(c)
+        Zp = torch.as_tensor(c["Zp"], device="cuda")
         r = mdl.run_assimilating(f, every * nwin, enkf, every, Zp,
                                  record_reaches=np.arange(0, n, 7) if record else None, record_prior=record)
         assert (r is None) == (not record)
@@ -272,23 +195,14 @@ def test_run_assimilating_recording_refuses_multipliers_for_another_M():
     import torch
     from tx_fast_hydrology_b200 import synthetic as S
     from tx_fast_hydrology_b200._lib import TxhError
-    from tx_fast_hydrology_b200.muskingum import Muskingum
-    from tx_fast_hydrology_b200.da import EnsembleKalmanFilter
     n, M, m, seed, every, nwin = 1500, 16, 20, 57, 6, 2
-    net = S.make_network(n, seed); prm = S.make_params(n, seed, well_posed=True)
-    rng = np.random.default_rng(seed)
-    d = S.model_dict(net, prm, dt_s=300.0); d["o_t"] = prm["o_t"][:, None] * rng.uniform(0.5, 1.5, size=(n, M))
-    mdl = Muskingum(d, members=M); t0 = mdl.datetime
-    times, table = S.make_forcing(n, every * nwin, 300.0, seed, t0_ns=int(t0.value), rows_every=4)
-    g = S.make_gauges(net["endnodes"], m, seed=seed)
-    mt = int(t0.value) + (np.arange(nwin, dtype=np.int64) + 1) * int(every * 300e9)
-    meas = rng.uniform(0.5, 8.0, size=(nwin, m))
-    mdf = pd.DataFrame(meas, index=pd.DatetimeIndex(pd.to_datetime(mt, unit="ns", utc=True)).as_unit("ns"),
-                       columns=[d["reach_ids"][j] for j in g])
-    enkf = EnsembleKalmanFilter(mdl, mdf, rng.uniform(0.5, 2.0, size=n), 1e-2 * np.eye(m))
-    Zp = torch.as_tensor(meas[:, :, None] + 0.1 * rng.standard_normal((nwin, m, M)), device="cuda")
+    c = make_case(n, M, m, seed, every, nwin, 0, gauges="synthetic", extra_reaches=None)
+    mdl, enkf, _ = model(c)
+    t0 = mdl.datetime
+    Zp = torch.as_tensor(c["Zp"], device="cuda")
     # multipliers of M + 3 members: a run that went ahead would read them inside the table, with the wrong stride
-    f = mdl.make_forcing(times_ns=times, table=table, member_mul=S.make_member_multipliers(times.size, M + 3, seed))
+    f = mdl.make_forcing(times_ns=c["times"], table=c["table"],
+                         member_mul=S.make_member_multipliers(c["times"].size, M + 3, seed))
     O, I = mdl.device_state
     O0, I0 = O.clone(), I.clone()
     for record in (None, np.arange(0, n, 7)):
@@ -308,32 +222,17 @@ def test_run_assimilating_recording_variants_agree():
     import tempfile
     code = (
         "import sys, numpy as np, torch\n"
-        "sys.path.insert(0, %r)\n"
-        "from tx_fast_hydrology_b200 import synthetic as S\n"
-        "from tx_fast_hydrology_b200.muskingum import Muskingum\n"
-        "from tx_fast_hydrology_b200.da import EnsembleKalmanFilter\n"
-        "import pandas as pd\n"
-        "n, M, m, seed, every, nwin = 2500, 64, 40, 57, 6, 4\n"
-        "net = S.make_network(n, seed); prm = S.make_params(n, seed, well_posed=True)\n"
-        "rng = np.random.default_rng(seed)\n"
-        "d = S.model_dict(net, prm, dt_s=300.0); d['o_t'] = prm['o_t'][:, None] * rng.uniform(0.5, 1.5, size=(n, M))\n"
-        "mdl = Muskingum(d, members=M); t0 = int(mdl.datetime.value)\n"
-        "times, table = S.make_forcing(n, every * nwin + 3, 300.0, seed, t0_ns=t0, rows_every=4)\n"
-        "mul = S.make_member_multipliers(times.size, M, seed)\n"
-        "g = S.make_gauges(net['endnodes'], m, seed=seed)\n"
-        "mt = t0 + (np.arange(nwin, dtype=np.int64) + 1) * int(every * 300e9)\n"
-        "meas = rng.uniform(0.5, 8.0, size=(nwin, m))\n"
-        "idx = pd.DatetimeIndex(pd.to_datetime(mt, unit='ns', utc=True)).as_unit('ns')\n"
-        "mdf = pd.DataFrame(meas, index=idx, columns=[d['reach_ids'][j] for j in g])\n"
-        "enkf = EnsembleKalmanFilter(mdl, mdf, rng.uniform(0.5, 2.0, size=n), 1e-2 * np.eye(m))\n"
-        "Zp = torch.as_tensor(meas[:, :, None] + 0.1 * rng.standard_normal((nwin, m, M)), device='cuda')\n"
-        "f = mdl.make_forcing(times_ns=times, table=table, member_mul=mul)\n"
-        "r = np.concatenate([g[:10], np.arange(1, n, 37)])\n"
-        "rec, pri = mdl.run_assimilating(f, every * nwin + 3, enkf, every, Zp, record_reaches=np.unique(r),\n"
-        "                                record_every=2, record_prior=True)\n"
+        "sys.path.insert(0, %r); sys.path.insert(0, %r)\n"
+        "from assim_case import make_case, model\n"
+        "c = make_case(2500, 64, 40, 57, 6, 4, 3, gauges='synthetic', extra_reaches=None)\n"
+        "mdl, enkf, f = model(c)\n"
+        "Zp = torch.as_tensor(c['Zp'], device='cuda')\n"
+        "r = np.concatenate([c['gidx'][:10], np.arange(1, c['n'], 37)])\n"
+        "rec, pri = mdl.run_assimilating(f, c['nsteps'], enkf, 6, Zp, record_reaches=np.unique(r), record_every=2,\n"
+        "                                record_prior=True)\n"
         "mdl.network.check()\n"
         "np.savez(sys.argv[1], rec=rec.cpu().numpy(), pri=pri.cpu().numpy())\n"
-    ) % os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    ) % (os.path.dirname(HERE), HERE)
     out = {}
     with tempfile.TemporaryDirectory() as tmp:
         for name, env in (("fused", {}), ("plain", {"TXH_ENKF_FUSED": "0", "TXH_ENKF_FUSE_LOAD": "0", "TXH_PDL": "0"})):

@@ -7,92 +7,18 @@ error, and a smoothed slot has been through several of them."""
 import os
 
 import numpy as np
-import pandas as pd
 import pytest
 
 pytestmark = pytest.mark.gpu
 
-RTOL = 1e-9
-
-from parity import relerr, normerr, enkf_tolerance        # noqa: E402
+from assim_case import make_case, model, run_device, reference_loop, update_fp64  # noqa: E402
+from parity import relerr, normerr                        # noqa: E402
 from enks_oracle import enks_gain, smooth_transforms      # noqa: E402
 
 
-def _model(n, M, m, seed, every, nwin, rest, dense_R=False):
-    """The assimilation case of test_gpu_record.py: a model, its filter, forcing and per-member observations."""
-    from tx_fast_hydrology_b200 import synthetic as S
-    from tx_fast_hydrology_b200.muskingum import Muskingum
-    from tx_fast_hydrology_b200.da import EnsembleKalmanFilter
-    nsteps = every * nwin + rest
-    net_d = S.make_network(n, seed)
-    prm = S.make_params(n, seed, well_posed=True)
-    rng = np.random.default_rng(seed)
-    o0 = prm["o_t"][:, None] * rng.uniform(0.5, 1.5, size=(n, M))
-    d = S.model_dict(net_d, prm, dt_s=300.0)
-    d["o_t"] = o0
-    mdl = Muskingum(d, members=M)
-    t0 = int(mdl.datetime.value)
-    times, table = S.make_forcing(n, nsteps, 300.0, seed, t0_ns=t0, rows_every=4)
-    mul = S.make_member_multipliers(times.size, M, seed)
-    gidx = np.asarray(S.make_gauges(net_d["endnodes"], m, seed=seed), dtype=np.int64)
-    m = gidx.size
-    mt = t0 + (np.arange(nwin, dtype=np.int64) + 1) * int(every * 300e9)
-    meas = rng.uniform(0.5, 8.0, size=(nwin, m))
-    mdf = pd.DataFrame(meas, index=pd.DatetimeIndex(pd.to_datetime(mt, unit="ns", utc=True)).as_unit("ns"),
-                       columns=[d["reach_ids"][j] for j in gidx])
-    R = 1e-2 * np.eye(m)
-    if dense_R:
-        Bm = rng.standard_normal((m, m))
-        R = 1e-2 * (np.eye(m) + 0.5 * (Bm @ Bm.T) / m)
-    q = rng.uniform(0.5, 2.0, size=n)
-    enkf = EnsembleKalmanFilter(mdl, mdf, q, R)
-    Zp = meas[:, :, None] + 0.1 * rng.standard_normal((nwin, m, M))
-    f = mdl.make_forcing(times_ns=times, table=table, member_mul=mul)
-    ung = np.setdiff1d(np.arange(n), gidx)
-    reaches = rng.permutation(np.concatenate([gidx[:max(3, m // 2)], rng.choice(ung, size=60, replace=False)]))
-    return dict(mdl=mdl, enkf=enkf, f=f, Zp=Zp, q=q, R=R, gidx=gidx, reaches=reaches, net_d=net_d, prm=prm, o0=o0,
-                t0=t0, times=times, table=table, mul=mul, nsteps=nsteps)
-
-
-def _device(c, every, in_library, record_every, lag):
-    import torch
-    Zd = torch.as_tensor(np.ascontiguousarray(c["Zp"]), device="cuda")
-    out = c["mdl"].run_assimilating(c["f"], c["nsteps"], c["enkf"], every, Zd if in_library else list(Zd),
-                                    record_reaches=c["reaches"], record_every=record_every, record_prior=True,
-                                    smooth_lag=lag)
-    c["mdl"].network.check()
-    return tuple(x.cpu().numpy() for x in out)
-
-
-def _oracle(oracle, c, every, nwin, record_every):
-    """The filter of the oracle with the recorded slots (posterior at update steps) and, per update, what the smoother
-    needs: its forecast anomalies at the gauges, innovations and innovation covariance."""
-    net_d, prm = c["net_d"], c["prm"]
-    ind = oracle.compute_indegree(net_d["startnodes"], net_d["endnodes"])
-    al, be, ch, ga = oracle.compute_coeffs(prm["K"], prm["X"], 300.0)
-    onet = {"startnodes": net_d["startnodes"], "endnodes": net_d["endnodes"], "indegree": ind,
-            "alpha": al, "beta": be, "chi": ch, "gamma": ga}
-    o = np.ascontiguousarray(c["o0"].T)
-    i = np.stack([oracle.init_states(net_d["startnodes"], net_d["endnodes"], x) for x in o])
-    gidx, q, R, reaches = c["gidx"], c["q"], c["R"], c["reaches"]
-    M = o.shape[0]
-    slots, upd, tols, pri = [], [], [], []
-    for s in range(1, c["nsteps"] + 1):
-        oracle.run_members(onet, o, i, 1, c["times"].astype(np.float64), c["table"], float(c["t0"] + (s - 1) * 300e9),
-                           300e9, wmul=c["mul"])
-        if s % every == 0 and s // every <= nwin:
-            k = s // every - 1
-            X = o.T
-            HA = X[gidx] - X[gidx].mean(axis=1, keepdims=True)
-            dz = c["Zp"][k] - X[gidx]
-            upd.append((HA, dz, HA @ HA.T / (M - 1) + np.diag(q[gidx]) + R))
-            tols.append(enkf_tolerance(X, gidx, q, R))
-            pri.append(X[reaches].copy())
-            Op, Ip, _ = oracle.enkf_update(onet, X, i.T, gidx, c["Zp"][k], q, R)
-            o = np.ascontiguousarray(Op.T); i = np.ascontiguousarray(Ip.T)
-        if s % record_every == 0:
-            slots.append(o[:, reaches].T.copy())
-    return np.stack(slots), upd, tols, np.stack(pri)
+def _case(n, M, m, seed, every, nwin, rest, dense_R=False):
+    """The assimilation case of test_gpu_record.py."""
+    return make_case(n, M, m, seed, every, nwin, rest, gauges="synthetic", dense_R=dense_R, extra_reaches=60)
 
 
 def _smoothed_oracle(slots, upd, every, record_every, lag):
@@ -130,11 +56,13 @@ def test_smoothed_hydrographs_vs_oracle(oracle, n, M, m, seed, every, nwin, rest
     nsteps = every * nwin + rest
     ref = None
     for lag in (0, 3, every + 2, 2 * every, nsteps + 5):
-        c = _model(n, M, m, seed, every, nwin, rest, dense_R)
-        rec, prior, sm = _device(c, every, in_library, record_every, lag)
+        c = _case(n, M, m, seed, every, nwin, rest, dense_R)
+        rec, prior, sm = run_device(c, in_library, record_every=record_every, lag=lag)["res"]
         if ref is None:
-            ref = _oracle(oracle, c, every, nwin, record_every)
-        slots, upd, tols, pri = ref
+            # the oracle's filter with the recorded slots (posterior at update steps) and, per update, what the
+            # smoother needs
+            ref = reference_loop(oracle, c, update_fp64, record_every=record_every)
+        slots, upd, tols, pri = ref["hyd"], ref["kept"], ref["tols"], ref["pri"]
         want = _smoothed_oracle(slots, upd, every, record_every, lag)
         tol = sum(tols)
         assert sm.shape == rec.shape == want.shape
@@ -152,23 +80,18 @@ def test_smoothing_leaves_the_filter_alone():
     for in_library in (True, False):
         out = []
         for lag in (None, 7):
-            c = _model(1500, 64, 40, 61, 6, 3, 2)
-            import torch
-            Zd = torch.as_tensor(np.ascontiguousarray(c["Zp"]), device="cuda")
-            r = c["mdl"].run_assimilating(c["f"], c["nsteps"], c["enkf"], 6, Zd if in_library else list(Zd),
-                                          record_reaches=c["reaches"], record_prior=True, smooth_lag=lag)
-            c["mdl"].network.check()
+            d = run_device(_case(1500, 64, 40, 61, 6, 3, 2), in_library, lag=lag)
+            r = d["res"]
             assert len(r) == (2 if lag is None else 3)
-            out.append((r[0].cpu().numpy(), r[1].cpu().numpy(), c["mdl"].o_t_next, c["mdl"].i_t_next,
-                        c["enkf"]._T.cpu().numpy()))
+            out.append((r[0], r[1], d["mdl"].o_t_next, d["mdl"].i_t_next, d["enkf"]._T.cpu().numpy()))
         for a, b in zip(*out):
             assert (a == b).all()
 
 
 @pytest.mark.parametrize("lag", [4, 100])
 def test_in_library_and_python_loop_agree(lag):
-    a = _device(_model(1500, 64, 40, 62, 6, 3, 2), 6, True, 2, lag)
-    b = _device(_model(1500, 64, 40, 62, 6, 3, 2), 6, False, 2, lag)
+    a = run_device(_case(1500, 64, 40, 62, 6, 3, 2), True, record_every=2, lag=lag)["res"]
+    b = run_device(_case(1500, 64, 40, 62, 6, 3, 2), False, record_every=2, lag=lag)["res"]
     assert normerr(a[2], b[2]) < 1e-10
     assert normerr(a[0], b[0]) < 1e-10
 
@@ -180,36 +103,36 @@ def test_transform_history_adds_no_launch():
     lib = _lib.load()
     counts, T_last = [], None
     for hist in (False, True):
-        c = _model(1500, 64, 40, 63, 6, 4, 3)
-        mdl = c["mdl"]
+        c = _case(1500, 64, 40, 63, 6, 4, 3)
+        mdl, enkf, f = model(c)
         Zd = torch.as_tensor(np.ascontiguousarray(c["Zp"]), device="cuda")
         mdl._ensure_device()
         T_hist = torch.empty((4, 64, 64), dtype=torch.float64, device="cuda")
         if hist:
             mdl.network.set_transform_history(T_hist)
         n0 = lib.txh_launch_count()
-        mdl.run_assimilating(c["f"], c["nsteps"], c["enkf"], 6, Zd, record_reaches=c["reaches"], record_prior=True)
+        mdl.run_assimilating(f, c["nsteps"], enkf, 6, Zd, record_reaches=c["reaches"], record_prior=True)
         counts.append(lib.txh_launch_count() - n0)
         mdl.network.set_transform_history(None)
         mdl.network.check()
         if hist:                                   # the last update's transform went to the history
             assert (T_hist[3] == T_last).all()
         else:
-            T_last = c["enkf"]._T.clone()
+            T_last = enkf._T.clone()
     assert counts[0] == counts[1]
 
 
 def test_transform_history_capacity_is_checked():
     import torch
     from tx_fast_hydrology_b200._lib import TxhError
-    c = _model(800, 16, 20, 64, 5, 3, 0)
-    mdl = c["mdl"]
+    c = _case(800, 16, 20, 64, 5, 3, 0)
+    mdl, enkf, f = model(c)
     mdl._ensure_device()
     mdl.network.set_transform_history(torch.empty((2, 16, 16), dtype=torch.float64, device="cuda"))
     Zd = torch.as_tensor(np.ascontiguousarray(c["Zp"]), device="cuda")
     O0 = mdl.o_t_next.copy()
     with pytest.raises(TxhError, match="transform history"):
-        mdl.run_assimilating(c["f"], c["nsteps"], c["enkf"], 5, Zd)
+        mdl.run_assimilating(f, c["nsteps"], enkf, 5, Zd)
     mdl.network.set_transform_history(None)
     assert (mdl.o_t_next == O0).all()                     # refused before any device work
 
@@ -224,9 +147,9 @@ def test_fused_and_plain_paths_agree():
     code = (
         "import sys, numpy as np\n"
         "sys.path.insert(0, %r); sys.path.insert(0, %r)\n"
-        "from test_gpu_smooth import _model, _device\n"
-        "c = _model(2500, 64, 40, 65, 6, 4, 3)\n"
-        "rec, pri, sm = _device(c, 6, True, 2, 13)\n"
+        "from assim_case import make_case, run_device\n"
+        "c = make_case(2500, 64, 40, 65, 6, 4, 3, gauges='synthetic', extra_reaches=60)\n"
+        "rec, pri, sm = run_device(c, True, record_every=2, lag=13)['res']\n"
         "np.savez(sys.argv[1], rec=rec, sm=sm)\n"
     ) % (os.path.dirname(here), here)
     out = {}
