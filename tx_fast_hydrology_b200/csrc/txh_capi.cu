@@ -8,6 +8,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <string>
 #include <vector>
 
@@ -22,8 +23,11 @@ namespace {
 thread_local std::string g_err;
 
 int fail(int code, const std::string& msg) { g_err = msg; return code; }
+// Also clears the runtime's last-error slot, where a failed runtime call may leave its error: the launchers end with
+// cudaGetLastError(), so the next launch on this thread would report it as its own.  A sticky error keeps failing.
 int cuda_fail(cudaError_t e, const char* what)
 {
+    cudaGetLastError();
     g_err = std::string(what) + ": " + cudaGetErrorString(e);
     return e == cudaErrorNoDevice || e == cudaErrorInsufficientDriver ? TXH_E_NODEVICE : TXH_E_CUDA;
 }
@@ -33,26 +37,28 @@ int cuda_fail(cudaError_t e, const char* what)
         if (e__ != cudaSuccess) return cuda_fail(e__, #call);      \
     } while (0)
 
-template <class T>
-int upload(T** dptr, const std::vector<T>& v)
-{
-    const size_t bytes = std::max<size_t>(v.size(), 1) * sizeof(T);
-    CU(cudaMalloc((void**)dptr, bytes));
-    if (!v.empty()) CU(cudaMemcpy(*dptr, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice));
-    return TXH_OK;
-}
+// Owners of the CUDA objects of a handle other than device memory (DevBuf, txh_kernels.cuh)
+template <auto Destroy>
+struct Destroyer {
+    template <class P> void operator()(P p) const { Destroy(p); }
+};
+using StreamOwner = std::unique_ptr<CUstream_st, Destroyer<cudaStreamDestroy>>;
+using EventOwner = std::unique_ptr<CUevent_st, Destroyer<cudaEventDestroy>>;
+using PinnedOwner = std::unique_ptr<int32_t[], Destroyer<cudaFreeHost>>;
 
-// Grow-only device buffer of a handle: reallocated when `count` elements do not fit, once the handle's stream has
-// drained (a queued launch may still read the old one); new memory is filled with the byte `fill` unless it is < 0.
-template <class T>
-int grow(T** buf, size_t* cap, size_t count, cudaStream_t st, int fill = -1)
+cudaError_t create_event(EventOwner& ev, unsigned flags)
 {
-    if (count <= *cap) return TXH_OK;
-    if (*buf) { CU(cudaStreamSynchronize(st)); CU(cudaFree(*buf)); *buf = nullptr; *cap = 0; }
-    CU(cudaMalloc((void**)buf, count * sizeof(T)));
-    *cap = count;
-    if (fill >= 0) CU(cudaMemsetAsync(*buf, fill, count * sizeof(T), st));
-    return TXH_OK;
+    cudaEvent_t e = nullptr;
+    const cudaError_t r = cudaEventCreateWithFlags(&e, flags);
+    if (r == cudaSuccess) ev.reset(e);
+    return r;
+}
+cudaError_t alloc_pinned(PinnedOwner& p, size_t count)
+{
+    int32_t* h = nullptr;
+    const cudaError_t r = cudaMallocHost((void**)&h, count * sizeof(int32_t));
+    p.reset(r == cudaSuccess ? h : nullptr);
+    return r;
 }
 
 // Development aid (TXH_TRACE_FILE, TXH_LANE_TRACE): when the environment variable `env` names a file, `launch` runs
@@ -65,13 +71,14 @@ int traced_launch(const char* env, unsigned long long*& trace, size_t words, con
     const char* file = getenv(env);
     trace = nullptr;
     if (!file || !*file) { CU(launch()); return TXH_OK; }
-    CU(cudaMalloc((void**)&trace, words * sizeof(unsigned long long)));
-    CU(cudaMemsetAsync(trace, 0, words * sizeof(unsigned long long), st));
+    DevBuf<unsigned long long> buf;
+    CU(buf.alloc(words));
+    CU(cudaMemsetAsync(buf, 0, words * sizeof(unsigned long long), st));
+    trace = buf;
     CU(launch());
     std::vector<unsigned long long> h(words);
-    CU(cudaMemcpyAsync(h.data(), trace, words * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(h.data(), buf, words * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
-    CU(cudaFree(trace));
     if (FILE* fp = fopen(file, "wb")) {
         fwrite(hd, sizeof(hd), 1, fp);
         if (extra_bytes) fwrite(extra, 1, extra_bytes, fp);
@@ -92,81 +99,82 @@ struct txh_net {
     bool dev_ready = false;
     int num_sms = 0;
     unsigned long long watchdog_ns = 10000000000ull;
-    TaskDesc* d_tasks = nullptr;
-    int32_t *d_notify = nullptr, *d_init_ready = nullptr, *d_up_off = nullptr, *d_up_pos = nullptr, *d_lvl_pos = nullptr,
-            *d_reach_of_pos = nullptr, *d_pos_of_reach = nullptr;
-    uint32_t *d_hdr = nullptr, *d_inw = nullptr;
-    uint8_t* d_outlet = nullptr;
-    int32_t* d_inner = nullptr; int64_t n_inner = 0;   // schedule positions that have upstream reaches
-    int4* d_inner_rec = nullptr;        // the same rows as {row, first three upstream rows | -1}; w == -2: more in the lists
-    double* d_coef = nullptr;           // same layout as coef_host
-    double* d_qtmp = nullptr;           // [n] schedule-order scratch for txh_route_step
-    int32_t* d_pending = nullptr; size_t pairs_cap = 0;
-    unsigned long long* d_queue = nullptr; size_t queue_cap = 0;
-    double* d_side = nullptr; size_t side_cap = 0;   // side buffer [n_side][ld]
-    unsigned long long* d_qctl = nullptr;     // [0] head, [1] tail, [2] completed, [4] status word
-    int32_t* d_status = nullptr;
-    StepInterp* d_steps = nullptr; size_t steps_cap = 0;
-    StepInterp* d_unit_step = nullptr;
-    int32_t* d_rec_slot = nullptr;
-    int32_t* d_rec_pos = nullptr; size_t rec_pos_cap = 0;   // positions of the recorded reaches (txh_run_assimilating_rec)
-    int32_t* d_tmp_idx = nullptr; size_t tmp_idx_cap = 0;
-    int32_t* h_status = nullptr;        // pinned mirror of d_status (word 0) and the solver info (word 1)
+    DevBuf<TaskDesc> d_tasks;
+    DevBuf<int32_t> d_notify, d_init_ready, d_up_off, d_up_pos, d_lvl_pos, d_reach_of_pos, d_pos_of_reach;
+    DevBuf<uint32_t> d_hdr, d_inw;
+    DevBuf<uint8_t> d_outlet;
+    DevBuf<int32_t> d_inner; int64_t n_inner = 0;   // schedule positions that have upstream reaches
+    DevBuf<int4> d_inner_rec;           // the same rows as {row, first three upstream rows | -1}; w == -2: more in the lists
+    DevBuf<double> d_coef;              // same layout as coef_host
+    DevBuf<double> d_qtmp;              // [n] schedule-order scratch for txh_route_step
+    DevBuf<int32_t> d_pending;          // [(task, member block) pairs]
+    DevBuf<unsigned long long> d_queue;
+    DevBuf<double> d_side;              // side buffer [n_side][ld]
+    DevBuf<unsigned long long> d_qctl;  // [0] head, [1] tail, [2] completed, [4] status word
+    int32_t* d_status = nullptr;        // points into d_qctl
+    DevBuf<StepInterp> d_steps;
+    DevBuf<StepInterp> d_unit_step;
+    DevBuf<int32_t> d_rec_slot;
+    DevBuf<int32_t> d_rec_pos;          // positions of the recorded reaches (txh_run_assimilating_rec)
+    DevBuf<int32_t> d_tmp_idx;
+    PinnedOwner h_status;               // pinned mirror of d_status (word 0) and the solver info (word 1)
     std::vector<int64_t> obs_cached;    // gauge list whose positions are resident in d_obs
-    int32_t* d_obs = nullptr; size_t obs_cap = 0;
-    int32_t* d_gauge_of_pos = nullptr;  // [n] gauge index of each schedule position, or -1
+    DevBuf<int32_t> d_obs;
+    DevBuf<int32_t> d_gauge_of_pos;     // [n] gauge index of each schedule position, or -1
     // ensemble update applied by the next window launch while it loads its tasks (txh_run_assimilating, txh_window.cu)
-    int32_t* d_gfix_off = nullptr;      // [window tasks + 1] gauge terms per task, for the gauges in obs_cached
-    int2* d_gfix = nullptr; size_t gfix_cap = 0; bool gfix_ok = false;
+    DevBuf<int32_t> d_gfix_off;         // [window tasks + 1] gauge terms per task, for the gauges in obs_cached
+    DevBuf<int2> d_gfix; bool gfix_ok = false;
     // window-mode kernel
-    WTaskDesc* d_wtasks = nullptr;
-    uint32_t *d_whdr = nullptr, *d_winw = nullptr;
-    int32_t* d_wprod = nullptr;
-    double* d_ring = nullptr; size_t ring_cap = 0; int ring_ld = 0;
+    DevBuf<WTaskDesc> d_wtasks;
+    DevBuf<uint32_t> d_whdr, d_winw;
+    DevBuf<int32_t> d_wprod;
+    DevBuf<double> d_ring; int ring_ld = 0;
     int route_kernel = 0;               // 0 auto (lane for small ensembles, else window), 1 dataflow, 2 window, 3 lane
     // lane kernel (txh_lane.cu): one schedule per member tile, built on first use
     struct LaneDev {
         LaneSchedule sched;
         bool built = false, ok = false, on_dev = false;
-        LaneRegionDesc* d_regions = nullptr;
-        int4* d_meta = nullptr;
-        int32_t* d_xbeg = nullptr;
-        uint16_t* d_child = nullptr;
+        DevBuf<LaneRegionDesc> d_regions;
+        DevBuf<int4> d_meta;
+        DevBuf<int32_t> d_xbeg;
+        DevBuf<uint16_t> d_child;
     };
-    LaneStep* d_lsteps = nullptr; size_t lsteps_cap = 0;
-    LaneStep* d_unit_lstep = nullptr;
+    DevBuf<LaneStep> d_lsteps;
+    DevBuf<LaneStep> d_unit_lstep;
     LaneDev lane[5];                    // member tiles 1, 2, 4, 8, 16
     int lane_cap_rows = 0;              // rows per region; 0 = from the size of the network and the SM count
-    double* d_lring = nullptr; size_t lring_cap = 0;
-    double* d_stage = nullptr; size_t stage_cap = 0;   // reach-order staging of txh_pack_host / txh_unpack_host
+    DevBuf<double> d_lring;
+    DevBuf<double> d_stage;             // reach-order staging of txh_pack_host / txh_unpack_host
     double* stats_rowsum = nullptr;     // txh_set_stats_output: row sums of the final outflows of every txh_route_run
     double stats_scale = 1.0;
     double* T_hist = nullptr;           // txh_set_transform_history: update k of a run_assimilating call solves into
     int64_t T_hist_cap = 0;             // T_hist + k*M*M (capacity in doubles)
     int enkf_kind = 0;                  // txh_set_enkf_transform: 0 stochastic, 1 ETKF (square root)
     double enkf_rtpp = 0.0;             // relaxation to prior perturbations, [0, 1)
-    std::vector<std::pair<cudaEvent_t, cudaEvent_t>> route_events;   // txh_run_assimilating(time_every > 0)
+    std::vector<std::pair<EventOwner, EventOwner>> route_events;   // txh_run_assimilating(time_every > 0)
 };
 
 struct txh_forcing {
     txh_net* net;
     int64_t R, M;
     std::vector<double> times;
-    double* d_times = nullptr;          // [R] the same on the device
-    double* d_F = nullptr;              // [R][n] schedule order
-    double* d_W = nullptr;              // [R][M] or nullptr
+    DevBuf<double> d_times;             // [R] the same on the device
+    DevBuf<double> d_F;                 // [R][n] schedule order
+    DevBuf<double> d_W;                 // [R][M] or empty
     // txh_forcing_update_async: the table arrives in row chunks on a copy stream of its own; a routing call waits
-    // (on its stream) for the chunks its steps read
-    cudaStream_t copy_stream = nullptr;
-    double* d_stage = nullptr;          // [R][n] reach order, private to the handle
-    cudaEvent_t reuse_ev = nullptr;
-    std::vector<cudaEvent_t> chunk_ev;
+    // (on its stream) for the chunks its steps read.  Set up by its first call, all at once.
+    StreamOwner copy_stream;
+    DevBuf<double> d_stage;             // [R][n] reach order, private to the handle
+    EventOwner reuse_ev;
+    std::vector<EventOwner> chunk_ev;
     std::vector<int64_t> chunk_begin;   // first row of each chunk
     size_t waited = 0;                  // chunks the routing stream has been made to wait for
 };
 
 namespace {
 
+// Uploads the schedule once.  A failed attempt may be retried: every buffer is assigned afresh, which frees what
+// the failed attempt left.
 int ensure_device(txh_net* net)
 {
     if (net->dev_ready) return TXH_OK;
@@ -180,51 +188,48 @@ int ensure_device(txh_net* net)
     CU(cudaGetDevice(&dev));
     CU(cudaDeviceGetAttribute(&net->num_sms, cudaDevAttrMultiProcessorCount, dev));
     const Schedule& s = net->sched;
-    int rc;
-    if ((rc = upload(&net->d_tasks, s.tasks))) return rc;
-    if ((rc = upload(&net->d_notify, s.notify))) return rc;
-    if ((rc = upload(&net->d_init_ready, s.init_ready))) return rc;
-    if ((rc = upload(&net->d_hdr, s.hdr))) return rc;
-    if ((rc = upload(&net->d_inw, s.inw))) return rc;
-    if ((rc = upload(&net->d_up_off, s.up_off))) return rc;
-    if ((rc = upload(&net->d_up_pos, s.up_pos))) return rc;
+    CU(net->d_tasks.upload(s.tasks));
+    CU(net->d_notify.upload(s.notify));
+    CU(net->d_init_ready.upload(s.init_ready));
+    CU(net->d_hdr.upload(s.hdr));
+    CU(net->d_inw.upload(s.inw));
+    CU(net->d_up_off.upload(s.up_off));
+    CU(net->d_up_pos.upload(s.up_pos));
     {
         std::vector<int32_t> inner;                            // rows with upstream reaches (inflow_gain_kernel)
         for (int64_t k = 0; k < net->topo.n; ++k) if (s.up_off[k + 1] > s.up_off[k]) inner.push_back((int32_t)k);
         net->n_inner = (int64_t)inner.size();
-        if ((rc = upload(&net->d_inner, inner))) return rc;
+        CU(net->d_inner.upload(inner));
         std::vector<int4> rec(inner.size());
         for (size_t e = 0; e < inner.size(); ++e) {
             const int32_t k = inner[e], u0 = s.up_off[k], cnt = s.up_off[k + 1] - u0;
             // the sum keeps the order of the lists (first upstream reach first), like nutils.py:84-85 does per visit
             rec[e] = make_int4(k, s.up_pos[u0], cnt > 1 ? s.up_pos[u0 + 1] : -1, cnt > 3 ? -2 : (cnt > 2 ? s.up_pos[u0 + 2] : -1));
         }
-        if ((rc = upload(&net->d_inner_rec, rec))) return rc;
+        CU(net->d_inner_rec.upload(rec));
     }
-    if ((rc = upload(&net->d_lvl_pos, s.lvl_pos))) return rc;
-    if ((rc = upload(&net->d_reach_of_pos, s.reach_of_pos))) return rc;
-    if ((rc = upload(&net->d_pos_of_reach, s.pos_of_reach))) return rc;
-    if ((rc = upload(&net->d_outlet, s.is_outlet_pos))) return rc;
-    if ((rc = upload(&net->d_wtasks, s.wtasks))) return rc;
-    if ((rc = upload(&net->d_whdr, s.whdr))) return rc;
-    if ((rc = upload(&net->d_winw, s.winw))) return rc;
-    if ((rc = upload(&net->d_wprod, s.wprod))) return rc;
+    CU(net->d_lvl_pos.upload(s.lvl_pos));
+    CU(net->d_reach_of_pos.upload(s.reach_of_pos));
+    CU(net->d_pos_of_reach.upload(s.pos_of_reach));
+    CU(net->d_outlet.upload(s.is_outlet_pos));
+    CU(net->d_wtasks.upload(s.wtasks));
+    CU(net->d_whdr.upload(s.whdr));
+    CU(net->d_winw.upload(s.winw));
+    CU(net->d_wprod.upload(s.wprod));
     if (const char* k = getenv("TXH_ROUTE_KERNEL")) {
         if (!strcmp(k, "dataflow")) net->route_kernel = 1;
         else if (!strcmp(k, "window")) net->route_kernel = 2;
         else if (!strcmp(k, "lane")) net->route_kernel = 3;
     }
-    CU(cudaMalloc((void**)&net->d_coef, sizeof(double) * (6 * net->topo.n + net->sched.link_last.size() + 1)));
-    CU(cudaMalloc((void**)&net->d_qtmp, sizeof(double) * net->topo.n));
-    CU(cudaMalloc((void**)&net->d_qctl, 64));
+    CU(net->d_coef.alloc(6 * net->topo.n + net->sched.link_last.size() + 1));
+    CU(net->d_qtmp.alloc(net->topo.n));
+    CU(net->d_qctl.alloc(8));
     net->d_status = reinterpret_cast<int32_t*>(net->d_qctl + 4);
     CU(cudaMemset(net->d_qctl, 0, 64));
-    CU(cudaMalloc((void**)&net->d_rec_slot, sizeof(int32_t) * net->topo.n));
-    CU(cudaMallocHost((void**)&net->h_status, 2 * sizeof(int32_t)));
+    CU(net->d_rec_slot.alloc(net->topo.n));
+    CU(alloc_pinned(net->h_status, 2));
     net->h_status[0] = net->h_status[1] = 0;
-    const StepInterp unit{0, 0, 1.0, 0.0};
-    CU(cudaMalloc((void**)&net->d_unit_step, sizeof(StepInterp)));
-    CU(cudaMemcpy(net->d_unit_step, &unit, sizeof(unit), cudaMemcpyHostToDevice));
+    CU(net->d_unit_step.upload({StepInterp{0, 0, 1.0, 0.0}}));
     if (const char* w = getenv("TXH_WATCHDOG_MS")) {
         const long ms = atol(w);
         if (ms > 0) net->watchdog_ns = (unsigned long long)ms * 1000000ull;
@@ -252,14 +257,14 @@ int ensure_coef(txh_net* net, cudaStream_t st)
 // (an abandoned launch leaves cells behind).
 int report_status(txh_net* net, cudaStream_t st)
 {
-    CU(cudaMemcpyAsync(net->h_status, net->d_status, 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(net->h_status.get(), net->d_status, 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     const int32_t status = net->h_status[0], info = net->h_status[1];
     if (status == 0 && info == 0) return TXH_OK;
     CU(cudaMemsetAsync(net->d_status, 0, 2 * sizeof(int32_t), st));
     if (status != 0) {
-        if (net->d_ring) CU(cudaMemsetAsync(net->d_ring, kEmptyByte, net->ring_cap * sizeof(double), st));
-        if (net->d_lring) CU(cudaMemsetAsync(net->d_lring, kEmptyByte, net->lring_cap * sizeof(double), st));
+        if (net->d_ring) CU(cudaMemsetAsync(net->d_ring, kEmptyByte, net->d_ring.capacity() * sizeof(double), st));
+        if (net->d_lring) CU(cudaMemsetAsync(net->d_lring, kEmptyByte, net->d_lring.capacity() * sizeof(double), st));
         CU(cudaMemsetAsync(net->d_qctl, 0, 32, st));                    // queue cursors, tickets
         CU(cudaMemsetAsync(net->d_qctl + 5, 0, 24, st));                // done counters, lane ticket
         CU(cudaStreamSynchronize(st));
@@ -329,12 +334,10 @@ int run_dataflow(txh_net* net, double* O, double* I, int64_t M, const double* F,
     // the ready queue never wraps: one slot per (pair, step); long runs go out in several launches
     const int64_t max_entries = int64_t(1) << 25;
     const int64_t steps_per_launch = std::max<int64_t>(1, std::min<int64_t>(nsteps, max_entries / (int64_t)pairs));
-    int rc;
-    if ((rc = grow(&net->d_pending, &net->pairs_cap, pairs, st)) ||
-        (rc = grow(&net->d_side, &net->side_cap, (size_t)std::max(1, s.n_side) * ld, st)) ||   // [n_side][ld]
-        (rc = grow(&net->d_queue, &net->queue_cap, pairs * (size_t)steps_per_launch, st)))
-        return rc;
-    if (plan.times && (rc = grow(&net->d_steps, &net->steps_cap, (size_t)steps_per_launch, st))) return rc;
+    CU(net->d_pending.grow(pairs, st));
+    CU(net->d_side.grow((size_t)std::max(1, s.n_side) * ld, st));   // [n_side][ld]
+    CU(net->d_queue.grow(pairs * (size_t)steps_per_launch, st));
+    if (plan.times) CU(net->d_steps.grow((size_t)steps_per_launch, st));
     const StepInterp* d_steps = plan.times ? net->d_steps : net->d_unit_step;
     for (int64_t s0 = 0; s0 < nsteps; s0 += steps_per_launch) {
         const int64_t ns = std::min<int64_t>(steps_per_launch, nsteps - s0);
@@ -373,8 +376,8 @@ int run_dataflow(txh_net* net, double* O, double* I, int64_t M, const double* F,
         a.smem_per_warp = a.off_ring + kRingBytes;
         // the per-task timeline of this launch
         const long long hd[4] = {(long long)pairs, (long long)ns, (long long)s.tasks.size(), (long long)nmb};
-        if ((rc = traced_launch("TXH_TRACE_FILE", a.trace, (size_t)a.total * 4, hd, nullptr, 0, st,
-                                [&] { return launch_route_dataflow(a, net->num_sms, st); })))
+        if (int rc = traced_launch("TXH_TRACE_FILE", a.trace, (size_t)a.total * 4, hd, nullptr, 0, st,
+                                   [&] { return launch_route_dataflow(a, net->num_sms, st); }))
             return rc;
     }
     return TXH_OK;
@@ -453,10 +456,9 @@ int run_window(txh_net* net, double* O, double* I, int64_t M, const double* F, c
     if (slot_row * spl * sizeof(double) >= (size_t(1) << 32)) return fail(TXH_E_INVALID, "window ring beyond 32-bit offsets");
     // every cell starts EMPTY (all bits set); consumers put EMPTY back, so a finished launch leaves the whole
     // ring EMPTY again whatever row stride the next launch lays over it
-    int rc;
-    if ((rc = grow(&net->d_ring, &net->ring_cap, slot_row * spl, st, kEmptyByte))) return rc;
+    CU(net->d_ring.grow(slot_row * spl, st, kEmptyByte));
     net->ring_ld = ld;
-    if (plan.times && (rc = grow(&net->d_steps, &net->steps_cap, (size_t)spl, st))) return rc;
+    if (plan.times) CU(net->d_steps.grow((size_t)spl, st));
     const StepInterp* d_steps = plan.times ? net->d_steps : net->d_unit_step;
     WinArgs a{};
     for (int64_t s0 = 0; s0 < nsteps; s0 += spl) {
@@ -492,8 +494,8 @@ int run_window(txh_net* net, double* O, double* I, int64_t M, const double* F, c
         a.nap_min = kWindowNapMin; a.nap_max = kWindowNapMax;
         // the per-task timeline of this launch
         const long long hd[4] = {(long long)pairs, (long long)ns, (long long)s.wtasks.size(), -(long long)nmb};
-        if ((rc = traced_launch("TXH_TRACE_FILE", a.trace, pairs * (size_t)(4 + ns), hd, nullptr, 0, st,
-                                [&] { return launch_route_window(a, a.upT ? fit.wpc_upd : fit.wpc, net->num_sms, st); })))
+        if (int rc = traced_launch("TXH_TRACE_FILE", a.trace, pairs * (size_t)(4 + ns), hd, nullptr, 0, st,
+                                   [&] { return launch_route_window(a, a.upT ? fit.wpc_upd : fit.wpc, net->num_sms, st); }))
             return rc;
     }
     return TXH_OK;
@@ -549,7 +551,6 @@ int run_lane(txh_net* net, double* O, double* I, int64_t M, const double* F, con
     txh_net::LaneDev* L = lane_schedule(net, ti, net->num_sms);
     if (!L->ok) return 1;
     const LaneSchedule& s = L->sched;
-    int rc;
     if (!L->on_dev) {
         std::vector<int4> meta(s.row_reach.size());
         for (size_t i = 0; i < meta.size(); ++i) {
@@ -557,17 +558,13 @@ int run_lane(txh_net* net, double* O, double* I, int64_t M, const double* F, con
             meta[i] = make_int4(j >= 0 ? net->sched.pos_of_reach[j] : -1, s.row_off[i] | (s.row_nx[i] << 16), s.row_c01[i],
                                 s.row_slot[i]);
         }
-        if ((rc = upload(&L->d_regions, s.regions))) return rc;
-        if ((rc = upload(&L->d_meta, meta))) return rc;
-        if ((rc = upload(&L->d_xbeg, s.row_xbeg))) return rc;
-        if ((rc = upload(&L->d_child, s.child))) return rc;
+        CU(L->d_regions.upload(s.regions));
+        CU(L->d_meta.upload(meta));
+        CU(L->d_xbeg.upload(s.row_xbeg));
+        CU(L->d_child.upload(s.child));
         L->on_dev = true;
     }
-    if (!net->d_unit_lstep) {
-        const LaneStep unit{1.0, 0.0, 0, 0, 0, 0};
-        CU(cudaMalloc((void**)&net->d_unit_lstep, sizeof(LaneStep)));
-        CU(cudaMemcpy(net->d_unit_lstep, &unit, sizeof(unit), cudaMemcpyHostToDevice));
-    }
+    if (!net->d_unit_lstep) CU(net->d_unit_lstep.upload({LaneStep{1.0, 0.0, 0, 0, 0, 0}}));
     const int ld = (int)txh_row_stride(M);
     // streams ring[slot][member][step]: one launch covers as many steps as fit 128 MiB
     const size_t streams = (size_t)std::max(1, s.n_slots) * (size_t)M;
@@ -575,9 +572,9 @@ int run_lane(txh_net* net, double* O, double* I, int64_t M, const double* F, con
     if (const char* k = getenv("TXH_LANE_SPL")) { const long v = atol(k); if (v > 0) spl = std::min<int64_t>(spl, v); }
     while (spl > 16 && streams * (size_t)((spl + 15) & ~int64_t(15)) * sizeof(double) > (size_t(128) << 20)) spl = (spl + 1) / 2;
     const size_t ring_need = streams * (size_t)((spl + 15) & ~int64_t(15));
-    if ((rc = grow(&net->d_lring, &net->lring_cap, ring_need, st, kEmptyByte))) return rc;   // every cell starts EMPTY
+    CU(net->d_lring.grow(ring_need, st, kEmptyByte));   // every cell starts EMPTY
     if (plan.times) {
-        if ((rc = grow(&net->d_lsteps, &net->lsteps_cap, (size_t)spl, st))) return rc;
+        CU(net->d_lsteps.grow((size_t)spl, st));
     } else if (nsteps != 1) {
         return fail(TXH_E_INVALID, "internal: a launch without a forcing table covers one step");
     }
@@ -615,9 +612,9 @@ int run_lane(txh_net* net, double* O, double* I, int64_t M, const double* F, con
         a.R = plan.times ? (int32_t)plan.R : 1;
         // the region timeline of this launch, behind the region descriptors
         const long long hd[4] = {(long long)s.regions.size(), (long long)ns, (long long)threads, (long long)grid};
-        if ((rc = traced_launch("TXH_LANE_TRACE", a.trace, 8 * s.regions.size(), hd, s.regions.data(),
-                                s.regions.size() * sizeof(LaneRegionDesc), st,
-                                [&] { return launch_route_lane(a, mt, threads, smem, grid, st); })))
+        if (int rc = traced_launch("TXH_LANE_TRACE", a.trace, 8 * s.regions.size(), hd, s.regions.data(),
+                                   s.regions.size() * sizeof(LaneRegionDesc), st,
+                                   [&] { return launch_route_lane(a, mt, threads, smem, grid, st); }))
             return rc;
     }
     return TXH_OK;
@@ -699,36 +696,7 @@ int txh_create(int64_t n, const int64_t* endnodes, const int32_t* sp, txh_net** 
     return TXH_OK;
 }
 
-void txh_destroy(txh_net* net)
-{
-    if (!net) return;
-    if (net->dev_ready) {
-        cudaFree(net->d_tasks); cudaFree(net->d_notify); cudaFree(net->d_init_ready); cudaFree(net->d_hdr); cudaFree(net->d_inw);
-        for (auto& ev : net->route_events) { cudaEventDestroy(ev.first); cudaEventDestroy(ev.second); }
-        cudaFree(net->d_up_off); cudaFree(net->d_up_pos); cudaFree(net->d_lvl_pos); cudaFree(net->d_inner); cudaFree(net->d_inner_rec);
-        cudaFree(net->d_reach_of_pos); cudaFree(net->d_pos_of_reach); cudaFree(net->d_outlet);
-        cudaFree(net->d_coef); cudaFree(net->d_qtmp); cudaFree(net->d_qctl); cudaFree(net->d_rec_slot);
-        cudaFree(net->d_unit_step);
-        if (net->d_rec_pos) cudaFree(net->d_rec_pos);
-        if (net->d_pending) cudaFree(net->d_pending);
-        if (net->d_queue) cudaFree(net->d_queue);
-        if (net->d_side) cudaFree(net->d_side);
-        if (net->d_steps) cudaFree(net->d_steps);
-        if (net->d_tmp_idx) cudaFree(net->d_tmp_idx);
-        if (net->d_obs) cudaFree(net->d_obs);
-        if (net->d_gauge_of_pos) cudaFree(net->d_gauge_of_pos);
-        cudaFree(net->d_gfix_off); cudaFree(net->d_gfix);
-        cudaFree(net->d_wtasks); cudaFree(net->d_whdr); cudaFree(net->d_winw); cudaFree(net->d_wprod);
-        if (net->d_ring) cudaFree(net->d_ring);
-        if (net->d_lring) cudaFree(net->d_lring);
-        for (auto& L : net->lane) { cudaFree(L.d_regions); cudaFree(L.d_meta); cudaFree(L.d_xbeg); cudaFree(L.d_child); }
-        if (net->d_lsteps) cudaFree(net->d_lsteps);
-        if (net->d_unit_lstep) cudaFree(net->d_unit_lstep);
-        if (net->d_stage) cudaFree(net->d_stage);
-        if (net->h_status) cudaFreeHost(net->h_status);
-    }
-    delete net;
-}
+void txh_destroy(txh_net* net) { delete net; }
 
 int64_t txh_n(const txh_net* net) { return net ? net->topo.n : 0; }
 
@@ -896,7 +864,7 @@ int txh_pack_host(txh_net* net, const double* src, int64_t M, int layout, double
     if ((rc = check_M(M)) || (rc = ensure_device(net))) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     const int64_t n = net->topo.n;
-    if ((rc = grow(&net->d_stage, &net->stage_cap, (size_t)n * M, st))) return rc;
+    CU(net->d_stage.grow((size_t)n * M, st));
     double* tmp = net->d_stage;
     CU(cudaMemcpyAsync(tmp, src, sizeof(double) * n * M, cudaMemcpyHostToDevice, st));
     CU(launch_pack(net->d_reach_of_pos, tmp, dst, n, (int)M, (int)txh_row_stride(M), layout, st));
@@ -910,7 +878,7 @@ int txh_unpack_host(txh_net* net, const double* src, int64_t M, int layout, doub
     if ((rc = check_M(M)) || (rc = ensure_device(net))) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     const int64_t n = net->topo.n;
-    if ((rc = grow(&net->d_stage, &net->stage_cap, (size_t)n * M, st))) return rc;
+    CU(net->d_stage.grow((size_t)n * M, st));
     double* tmp = net->d_stage;
     CU(launch_unpack(net->d_reach_of_pos, src, tmp, n, (int)M, (int)txh_row_stride(M), layout, st));
     CU(cudaMemcpyAsync(dst, tmp, sizeof(double) * n * M, cudaMemcpyDeviceToHost, st));
@@ -948,7 +916,7 @@ int txh_gather_rows(txh_net* net, const double* X, int64_t M, const int64_t* idx
         if (idx[k] < 0 || idx[k] >= net->topo.n) return fail(TXH_E_INVALID, "reach index out of range");
         pos[k] = net->sched.pos_of_reach[idx[k]];
     }
-    if ((rc = grow(&net->d_tmp_idx, &net->tmp_idx_cap, (size_t)count, st))) return rc;
+    CU(net->d_tmp_idx.grow((size_t)count, st));
     CU(cudaMemcpyAsync(net->d_tmp_idx, pos.data(), sizeof(int32_t) * count, cudaMemcpyHostToDevice, st));
     CU(cudaStreamSynchronize(st));      // `pos` is a stack-lifetime buffer
     CU(launch_gather_rows(net->d_tmp_idx, count, X, (int)txh_row_stride(M), (int)M, out, st));
@@ -975,27 +943,26 @@ int txh_forcing_create(txh_net* net, int64_t R, const double* times, const doubl
     for (int64_t r = 1; r < R; ++r)
         if (!(times[r] >= times[r - 1])) return fail(TXH_E_INVALID, "forcing times must be sorted ascending");
     const int64_t n = net->topo.n;
-    txh_forcing* f = new (std::nothrow) txh_forcing();
+    std::unique_ptr<txh_forcing> f(new (std::nothrow) txh_forcing());
     if (!f) return fail(TXH_E_INVALID, "out of memory");
     f->net = net; f->R = R; f->M = mul ? M : 0;
     f->times.assign(times, times + R);
     // one H2D copy of the table as given (pinned or pageable) into the handle's staging buffer, columns
     // permuted into schedule order on the device
-    if ((rc = grow(&net->d_stage, &net->stage_cap, (size_t)R * n, st))) { delete f; return rc; }
+    CU(net->d_stage.grow((size_t)R * n, st));
     double* tmp = net->d_stage;
-    cudaError_t e = cudaMalloc((void**)&f->d_F, sizeof(double) * R * n);
-    if (e == cudaSuccess) e = cudaMalloc((void**)&f->d_times, sizeof(double) * R);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(f->d_times, f->times.data(), sizeof(double) * R, cudaMemcpyHostToDevice, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(tmp, table, sizeof(double) * R * n, cudaMemcpyHostToDevice, st);
-    if (e == cudaSuccess) e = launch_permute_rows(net->d_reach_of_pos, tmp, f->d_F, n, R, st);
-    if (e == cudaSuccess && mul) {
-        if (M < 1) { cudaFree(f->d_F); cudaFree(f->d_times); delete f; return fail(TXH_E_INVALID, "member multipliers need M >= 1"); }
-        e = cudaMalloc((void**)&f->d_W, sizeof(double) * R * M);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(f->d_W, mul, sizeof(double) * R * M, cudaMemcpyHostToDevice, st);
+    CU(f->d_F.alloc((size_t)R * n));
+    CU(f->d_times.alloc((size_t)R));
+    CU(cudaMemcpyAsync(f->d_times, f->times.data(), sizeof(double) * R, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(tmp, table, sizeof(double) * R * n, cudaMemcpyHostToDevice, st));
+    CU(launch_permute_rows(net->d_reach_of_pos, tmp, f->d_F, n, R, st));
+    if (mul) {
+        if (M < 1) return fail(TXH_E_INVALID, "member multipliers need M >= 1");
+        CU(f->d_W.alloc((size_t)R * M));
+        CU(cudaMemcpyAsync(f->d_W, mul, sizeof(double) * R * M, cudaMemcpyHostToDevice, st));
     }
-    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-    if (e != cudaSuccess) { cudaFree(f->d_F); cudaFree(f->d_W); cudaFree(f->d_times); delete f; return cuda_fail(e, "forcing upload"); }
-    *out = f;
+    CU(cudaStreamSynchronize(st));
+    *out = f.release();
     return TXH_OK;
 }
 
@@ -1008,9 +975,8 @@ int txh_forcing_update(txh_forcing* f, const double* times, const double* table,
     const int64_t n = net->topo.n, R = f->R;
     for (int64_t r = 1; r < R; ++r)
         if (!(times[r] >= times[r - 1])) return fail(TXH_E_INVALID, "forcing times must be sorted ascending");
-    int rc;
-    if ((rc = txh_forcing_wait(f))) return rc;
-    if ((rc = grow(&net->d_stage, &net->stage_cap, (size_t)R * n, st))) return rc;
+    if (int rc = txh_forcing_wait(f)) return rc;
+    CU(net->d_stage.grow((size_t)R * n, st));
     double* tmp = net->d_stage;
     f->times.assign(times, times + R);
     CU(cudaMemcpyAsync(f->d_times, f->times.data(), sizeof(double) * R, cudaMemcpyHostToDevice, st));
@@ -1031,27 +997,36 @@ int txh_forcing_update_async(txh_forcing* f, const double* times, const double* 
     for (int64_t r = 1; r < R; ++r)
         if (!(times[r] >= times[r - 1])) return fail(TXH_E_INVALID, "forcing times must be sorted ascending");
     if (!f->copy_stream) {
-        CU(cudaStreamCreateWithFlags(&f->copy_stream, cudaStreamNonBlocking));
-        CU(cudaEventCreateWithFlags(&f->reuse_ev, cudaEventDisableTiming));
-        CU(cudaMalloc((void**)&f->d_stage, sizeof(double) * R * n));
+        // built aside and kept only when complete: copy_stream marks the set-up done
+        cudaStream_t cs = nullptr;
+        CU(cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking));
+        StreamOwner copy_stream(cs);
+        EventOwner reuse_ev;
+        CU(create_event(reuse_ev, cudaEventDisableTiming));
+        DevBuf<double> stage;
+        CU(stage.alloc((size_t)R * n));
         // a first chunk small enough that routing starts at once, then ~16 MiB pieces
         const int64_t rows_per = std::max<int64_t>(1, (int64_t)((size_t(16) << 20) / (sizeof(double) * n)));
-        for (int64_t r = 0; r < R; r += (r == 0 ? std::min<int64_t>(2, rows_per) : rows_per)) f->chunk_begin.push_back(r);
-        f->chunk_ev.resize(f->chunk_begin.size());
-        for (cudaEvent_t& e : f->chunk_ev) CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+        std::vector<int64_t> chunk_begin;
+        for (int64_t r = 0; r < R; r += (r == 0 ? std::min<int64_t>(2, rows_per) : rows_per)) chunk_begin.push_back(r);
+        std::vector<EventOwner> chunk_ev(chunk_begin.size());
+        for (EventOwner& e : chunk_ev) CU(create_event(e, cudaEventDisableTiming));
+        f->d_stage = std::move(stage); f->reuse_ev = std::move(reuse_ev);
+        f->chunk_begin = std::move(chunk_begin); f->chunk_ev = std::move(chunk_ev);
+        f->copy_stream = std::move(copy_stream);
     }
     f->times.assign(times, times + R);
     CU(cudaMemcpyAsync(f->d_times, f->times.data(), sizeof(double) * R, cudaMemcpyHostToDevice, st));
     if (mul) CU(cudaMemcpyAsync(f->d_W, mul, sizeof(double) * R * f->M, cudaMemcpyHostToDevice, st));
     // the table may still be read by launches already queued on `st`
-    CU(cudaEventRecord(f->reuse_ev, st));
-    CU(cudaStreamWaitEvent(f->copy_stream, f->reuse_ev, 0));
+    CU(cudaEventRecord(f->reuse_ev.get(), st));
+    CU(cudaStreamWaitEvent(f->copy_stream.get(), f->reuse_ev.get(), 0));
     for (size_t c = 0; c < f->chunk_begin.size(); ++c) {
         const int64_t r0 = f->chunk_begin[c], r1 = c + 1 < f->chunk_begin.size() ? f->chunk_begin[c + 1] : R;
         CU(cudaMemcpyAsync(f->d_stage + r0 * n, table + r0 * n, sizeof(double) * (r1 - r0) * n, cudaMemcpyHostToDevice,
-                           f->copy_stream));
-        CU(launch_permute_rows(net->d_reach_of_pos, f->d_stage + r0 * n, f->d_F + r0 * n, n, r1 - r0, f->copy_stream));
-        CU(cudaEventRecord(f->chunk_ev[c], f->copy_stream));
+                           f->copy_stream.get()));
+        CU(launch_permute_rows(net->d_reach_of_pos, f->d_stage + r0 * n, f->d_F + r0 * n, n, r1 - r0, f->copy_stream.get()));
+        CU(cudaEventRecord(f->chunk_ev[c].get(), f->copy_stream.get()));
     }
     f->waited = 0;
     return TXH_OK;
@@ -1060,7 +1035,7 @@ int txh_forcing_update_async(txh_forcing* f, const double* times, const double* 
 int txh_forcing_wait(txh_forcing* f)
 {
     if (!f) return fail(TXH_E_INVALID, "null argument");
-    if (f->copy_stream) CU(cudaStreamSynchronize(f->copy_stream));
+    if (f->copy_stream) CU(cudaStreamSynchronize(f->copy_stream.get()));
     f->waited = f->chunk_ev.size();
     return TXH_OK;
 }
@@ -1068,16 +1043,7 @@ int txh_forcing_wait(txh_forcing* f)
 void txh_forcing_destroy(txh_forcing* f)
 {
     if (!f) return;
-    if (f->copy_stream) {
-        cudaStreamSynchronize(f->copy_stream);
-        for (cudaEvent_t e : f->chunk_ev) cudaEventDestroy(e);
-        cudaEventDestroy(f->reuse_ev);
-        cudaStreamDestroy(f->copy_stream);
-        cudaFree(f->d_stage);
-    }
-    cudaFree(f->d_F);
-    if (f->d_times) cudaFree(f->d_times);
-    if (f->d_W) cudaFree(f->d_W);
+    if (f->copy_stream) cudaStreamSynchronize(f->copy_stream.get());
     delete f;
 }
 
@@ -1112,11 +1078,11 @@ int route_run_impl(txh_net* net, double* O, double* I, int64_t M, const txh_forc
         const double x_end = (double)(t0_ns + nsteps * dt_ns);
         const int64_t need = std::min<int64_t>(fo->R - 1, std::lower_bound(fo->times.begin(), fo->times.end(), x_end) - fo->times.begin());
         while (fw->waited < fw->chunk_ev.size() && fw->chunk_begin[fw->waited] <= need) {
-            CU(cudaStreamWaitEvent(st, fw->chunk_ev[fw->waited], 0));
+            CU(cudaStreamWaitEvent(st, fw->chunk_ev[fw->waited].get(), 0));
             ++fw->waited;
         }
     }
-    return run_routing(net, O, I, M, fo ? fo->d_F : nullptr, fo ? fo->d_W : nullptr, fo ? (int)fo->M : 0,
+    return run_routing(net, O, I, M, fo ? fo->d_F.get() : nullptr, fo ? fo->d_W.get() : nullptr, fo ? (int)fo->M : 0,
                        plan, nsteps, st, rec, rowsum, rowsum_scale, upd);
 }
 }  // namespace
@@ -1137,7 +1103,7 @@ int txh_route_run(txh_net* net, double* O, double* I, int64_t M, const txh_forci
     if ((rc = check_M(M)) || (rc = ensure_device(net)) || (rc = ensure_coef(net, st))) return rc;
     if (nsteps == 0) return TXH_OK;
     if (rec_count > 0 && (rc = upload_rec_slots(net, rec_reach, rec_count, st))) return rc;
-    const Recording rec{rec_count > 0 ? net->d_rec_slot : nullptr, rec_out, (int)rec_every, (int)rec_count, 0};
+    const Recording rec{rec_count > 0 ? net->d_rec_slot.get() : nullptr, rec_out, (int)rec_every, (int)rec_count, 0};
     return route_run_impl(net, O, I, M, fo, t0_ns, dt_ns, nsteps, method, rec, net->stats_rowsum, net->stats_scale,
                           nullptr, st);
 }
@@ -1149,7 +1115,7 @@ int txh_route_step(txh_net* net, double* O, double* I, int64_t M, const double* 
     cudaStream_t st = (cudaStream_t)stream;
     if ((rc = check_M(M)) || (rc = ensure_device(net)) || (rc = ensure_coef(net, st))) return rc;
     if (q) CU(launch_permute_vec(net->d_reach_of_pos, q, net->d_qtmp, net->topo.n, st));
-    return run_routing(net, O, I, M, q ? net->d_qtmp : nullptr, nullptr, 0, StepPlan(), 1, st);
+    return run_routing(net, O, I, M, q ? net->d_qtmp.get() : nullptr, nullptr, 0, StepPlan(), 1, st);
 }
 
 int txh_route_step_levels(txh_net* net, double* O, double* I, int64_t M, const double* q, void* stream)
@@ -1164,7 +1130,7 @@ int txh_route_step_levels(txh_net* net, double* O, double* I, int64_t M, const d
         LevelArgs a{};
         a.lvl_pos = net->d_lvl_pos + s.lvl_off[l]; a.count = s.lvl_off[l + 1] - s.lvl_off[l];
         a.up_off = net->d_up_off; a.up_pos = net->d_up_pos; a.coef = net->d_coef;
-        a.q = q ? net->d_qtmp : nullptr; a.O = O; a.I = I; a.ld = (int)txh_row_stride(M); a.M = (int)M;
+        a.q = q ? net->d_qtmp.get() : nullptr; a.O = O; a.I = I; a.ld = (int)txh_row_stride(M); a.M = (int)M;
         CU(launch_route_level(a, st));
     }
     return TXH_OK;
@@ -1216,11 +1182,10 @@ int obs_positions(txh_net* net, const int64_t* obs, int64_t m, cudaStream_t st, 
         if (k > 0 && obs[k] <= obs[k - 1]) return fail(TXH_E_INVALID, "gauge reach indices must be strictly ascending");
         pos[k] = net->sched.pos_of_reach[obs[k]];
     }
-    int rc;
-    if ((rc = grow(&net->d_obs, &net->obs_cap, (size_t)m, st))) return rc;
+    CU(net->d_obs.grow((size_t)m, st));
     std::vector<int32_t> gop(net->topo.n, -1);
     for (int64_t k = 0; k < m; ++k) gop[pos[k]] = (int32_t)k;
-    if (!net->d_gauge_of_pos) CU(cudaMalloc((void**)&net->d_gauge_of_pos, sizeof(int32_t) * net->topo.n));
+    CU(net->d_gauge_of_pos.grow(net->topo.n, st));
     CU(cudaMemcpyAsync(net->d_obs, pos.data(), sizeof(int32_t) * m, cudaMemcpyHostToDevice, st));
     CU(cudaMemcpyAsync(net->d_gauge_of_pos, gop.data(), sizeof(int32_t) * net->topo.n, cudaMemcpyHostToDevice, st));
     // gauge terms of the update per window task (route_window_kernel applies the update while it loads a task): the
@@ -1245,8 +1210,8 @@ int obs_positions(txh_net* net, const int64_t* obs, int64_t m, cudaStream_t st, 
     std::vector<int2> gfix;
     if (fix_ok)
         for (size_t k = 0; k < ntask; ++k) { gfix.insert(gfix.end(), per_task[k].begin(), per_task[k].end()); goff[k + 1] = (int32_t)gfix.size(); }
-    if (!net->d_gfix_off) CU(cudaMalloc((void**)&net->d_gfix_off, sizeof(int32_t) * (ntask + 1)));
-    if ((rc = grow(&net->d_gfix, &net->gfix_cap, std::max<size_t>(gfix.size(), 16), st))) return rc;
+    CU(net->d_gfix_off.grow(ntask + 1, st));
+    CU(net->d_gfix.grow(std::max<size_t>(gfix.size(), 16), st));
     net->gfix_ok = fix_ok;
     CU(cudaMemcpyAsync(net->d_gfix_off, goff.data(), sizeof(int32_t) * (ntask + 1), cudaMemcpyHostToDevice, st));
     if (!gfix.empty()) CU(cudaMemcpyAsync(net->d_gfix, gfix.data(), sizeof(int2) * gfix.size(), cudaMemcpyHostToDevice, st));
@@ -1483,9 +1448,8 @@ int txh_run_assimilating_rec(txh_net* net, double* O, double* I, int64_t M, cons
     if ((rc = ensure_device(net)) || (rc = ensure_coef(net, st))) return rc;
     if (rec) {
         // the slots and positions of the recorded reaches once per call
-        if ((rc = upload_rec_slots(net, rec_reach, rec_count, st)) ||
-            (rc = grow(&net->d_rec_pos, &net->rec_pos_cap, (size_t)rec_count, st)))
-            return rc;
+        if ((rc = upload_rec_slots(net, rec_reach, rec_count, st))) return rc;
+        CU(net->d_rec_pos.grow((size_t)rec_count, st));
         std::vector<int32_t> pos(rec_count);
         for (int64_t k = 0; k < rec_count; ++k) pos[k] = net->sched.pos_of_reach[rec_reach[k]];
         CU(cudaMemcpyAsync(net->d_rec_pos, pos.data(), sizeof(int32_t) * rec_count, cudaMemcpyHostToDevice, st));
@@ -1528,14 +1492,17 @@ int txh_run_assimilating_rec(txh_net* net, double* O, double* I, int64_t M, cons
     bool handed_over = false;
     int64_t t = t0_ns;
     for (int64_t k = 0; k < nseg; ++k) {
-        cudaEvent_t e0 = nullptr, e1 = nullptr;
+        EventOwner e0, e1;
         const bool timed = k < nwin && time_every > 0 && k % time_every == 0 && net->route_events.size() < 4096;
-        if (timed) { CU(cudaEventCreate(&e0)); CU(cudaEventCreate(&e1)); CU(cudaEventRecord(e0, st)); }
+        if (timed) {
+            CU(create_event(e0, cudaEventDefault)); CU(create_event(e1, cudaEventDefault));
+            CU(cudaEventRecord(e0.get(), st));
+        }
         const Recording rk = rec ? Recording{net->d_rec_slot, rec_out, (int)rec_every, (int)rec_count, k * every} : Recording();
         // the row sums of the forecast ride on the last step of every window (the mean of the update)
         rc = route_run_impl(net, O, I, M, fo, t, dt_ns, seg_steps(k), method, rk, k < nwin ? rowsum : nullptr,
                             1.0 / (double)M, handed_over ? &owed : nullptr, st);
-        if (timed) { CU(cudaEventRecord(e1, st)); net->route_events.emplace_back(e0, e1); }
+        if (timed) { CU(cudaEventRecord(e1.get(), st)); net->route_events.emplace_back(std::move(e0), std::move(e1)); }
         if (rc != TXH_OK) return rc;
         if (k == nwin) break;                              // the remaining steps: no update follows
         t += every * dt_ns;
@@ -1597,14 +1564,11 @@ int txh_get_route_timings(txh_net* net, double* ms_out, int64_t capacity, int64_
     *count = (int64_t)net->route_events.size();
     for (int64_t i = 0; i < *count && i < capacity; ++i) {
         float ms = 0.f;
-        CU(cudaEventSynchronize(net->route_events[i].second));
-        CU(cudaEventElapsedTime(&ms, net->route_events[i].first, net->route_events[i].second));
+        CU(cudaEventSynchronize(net->route_events[i].second.get()));
+        CU(cudaEventElapsedTime(&ms, net->route_events[i].first.get(), net->route_events[i].second.get()));
         ms_out[i] = ms;
     }
-    if (capacity >= *count) {                                  // read out: the events are done with
-        for (auto& ev : net->route_events) { cudaEventDestroy(ev.first); cudaEventDestroy(ev.second); }
-        net->route_events.clear();
-    }
+    if (capacity >= *count) net->route_events.clear();        // read out: the events are done with
     return TXH_OK;
 }
 
@@ -1624,14 +1588,13 @@ int txh_spd_solve(int64_t m, int64_t k, double* S, double* B, void* stream)
     if (!S || !B || m < 1 || k < 1) return fail(TXH_E_INVALID, "bad argument");
     if (txh_device_count() == 0) return fail(TXH_E_NODEVICE, "no CUDA device visible: libtxh has no CPU fallback");
     cudaStream_t st = (cudaStream_t)stream;
-    int* d_info = nullptr;
-    CU(cudaMalloc((void**)&d_info, sizeof(int)));
+    DevBuf<int> d_info;
+    CU(d_info.alloc(1));
     CU(cudaMemsetAsync(d_info, 0, sizeof(int), st));
     CU(launch_spd_solve(S, B, (int)m, (int)k, d_info, st));
     int info = 0;
     CU(cudaMemcpyAsync(&info, d_info, sizeof(int), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
-    cudaFree(d_info);
     if (info != 0) return fail(TXH_E_INVALID, "matrix is not positive definite");
     return TXH_OK;
 }
@@ -1641,14 +1604,13 @@ int txh_inverse(int64_t m, double* A, double* work, void* stream)
     if (!A || !work || m < 1) return fail(TXH_E_INVALID, "bad argument");
     if (txh_device_count() == 0) return fail(TXH_E_NODEVICE, "no CUDA device visible: libtxh has no CPU fallback");
     cudaStream_t st = (cudaStream_t)stream;
-    int* d_info = nullptr;
-    CU(cudaMalloc((void**)&d_info, sizeof(int)));
+    DevBuf<int> d_info;
+    CU(d_info.alloc(1));
     CU(cudaMemsetAsync(d_info, 0, sizeof(int), st));
     CU(launch_inverse(A, work, (int)m, d_info, st));
     int info = 0;
     CU(cudaMemcpyAsync(&info, d_info, sizeof(int), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
-    cudaFree(d_info);
     if (info != 0) return fail(TXH_E_INVALID, "matrix is singular");
     return TXH_OK;
 }
@@ -1714,11 +1676,9 @@ struct txh_kfb {
     std::vector<KfbBlock> blocks;
     int64_t n_u = 0, m_tot = 0, pp = 0, nm = 0, mm = 0;
     int max_n = 0, max_m = 0, ld = 0;
-    KfbBlock* d_blocks = nullptr;
-    int32_t *d_blk_of_reach = nullptr, *d_gl_of_reach = nullptr, *d_obs_reach = nullptr;
-    double *d_P = nullptr, *d_Pprev = nullptr, *d_Q = nullptr, *d_R = nullptr, *d_Pm = nullptr, *d_Ps = nullptr, *d_Prow = nullptr,
-           *d_S = nullptr, *d_K = nullptr, *d_z = nullptr, *d_dz = nullptr, *d_gain = nullptr, *d_Gp = nullptr, *d_X = nullptr,
-           *d_X2 = nullptr;
+    DevBuf<KfbBlock> d_blocks;
+    DevBuf<int32_t> d_blk_of_reach, d_gl_of_reach, d_obs_reach;
+    DevBuf<double> d_P, d_Pprev, d_Q, d_R, d_Pm, d_Ps, d_Prow, d_S, d_K, d_z, d_dz, d_gain, d_Gp, d_X, d_X2;
 };
 
 extern "C" {
@@ -1734,15 +1694,14 @@ int64_t txh_kfb_max_gauges(void)
 int txh_kfb_create(txh_net* net, int64_t nblocks, const int64_t* n_k, const int64_t* m_k, const int64_t* obs_local, txh_kfb** out)
 {
     if (!net || !n_k || !m_k || !obs_local || !out || nblocks < 1) return fail(TXH_E_INVALID, "bad argument");
-    int rc;
-    if ((rc = ensure_device(net))) return rc;
-    txh_kfb* b = new (std::nothrow) txh_kfb();
+    if (int rc = ensure_device(net)) return rc;
+    std::unique_ptr<txh_kfb> b(new (std::nothrow) txh_kfb());
     if (!b) return fail(TXH_E_INVALID, "out of memory");
     b->net = net;
     std::vector<int32_t> blk_of_reach, gl_of_reach, obs_reach;
     int64_t row0 = 0, g0 = 0;
     for (int64_t k = 0; k < nblocks; ++k) {
-        if (n_k[k] < 1 || m_k[k] < 1 || m_k[k] > n_k[k]) { delete b; return fail(TXH_E_INVALID, "bad block size"); }
+        if (n_k[k] < 1 || m_k[k] < 1 || m_k[k] > n_k[k]) return fail(TXH_E_INVALID, "bad block size");
         KfbBlock blk{};
         blk.n = (int32_t)n_k[k]; blk.m = (int32_t)m_k[k]; blk.row0 = (int32_t)row0; blk.g_off = (int32_t)g0; blk.active = 1;
         blk.p_off = b->pp; blk.nm_off = b->nm; blk.mm_off = b->mm;
@@ -1751,9 +1710,8 @@ int txh_kfb_create(txh_net* net, int64_t nblocks, const int64_t* n_k, const int6
         std::vector<int32_t> gl(n_k[k], -1);
         for (int64_t g = 0; g < m_k[k]; ++g) {
             const int64_t j = obs_local[g0 + g];
-            if (j < 0 || j >= n_k[k] || (g > 0 && j <= obs_local[g0 + g - 1])) {
-                delete b; return fail(TXH_E_INVALID, "gauge indices of a block must be strictly ascending local reaches");
-            }
+            if (j < 0 || j >= n_k[k] || (g > 0 && j <= obs_local[g0 + g - 1]))
+                return fail(TXH_E_INVALID, "gauge indices of a block must be strictly ascending local reaches");
             gl[j] = (int32_t)g;
             obs_reach.push_back((int32_t)(row0 + j));
         }
@@ -1762,37 +1720,26 @@ int txh_kfb_create(txh_net* net, int64_t nblocks, const int64_t* n_k, const int6
         b->blocks.push_back(blk);
         row0 += n_k[k]; g0 += m_k[k];
     }
-    if (row0 != net->topo.n) { delete b; return fail(TXH_E_INVALID, "block sizes do not add up to the union network"); }
-    if (b->max_m > txh_kfb_max_gauges()) {
-        delete b; return fail(TXH_E_INVALID, "a block has too many gauges for the batched inverse");
-    }
+    if (row0 != net->topo.n) return fail(TXH_E_INVALID, "block sizes do not add up to the union network");
+    if (b->max_m > txh_kfb_max_gauges()) return fail(TXH_E_INVALID, "a block has too many gauges for the batched inverse");
     b->n_u = row0; b->m_tot = g0;
     b->ld = (int)txh_row_stride(b->max_n);
-    if ((rc = upload(&b->d_blocks, b->blocks)) || (rc = upload(&b->d_blk_of_reach, blk_of_reach)) ||
-        (rc = upload(&b->d_gl_of_reach, gl_of_reach)) || (rc = upload(&b->d_obs_reach, obs_reach))) { delete b; return rc; }
-    auto dalloc = [](double** p, size_t count) { return cudaMalloc((void**)p, std::max<size_t>(count, 1) * sizeof(double)); };
-    cudaError_t e = cudaSuccess;
+    CU(b->d_blocks.upload(b->blocks));
+    CU(b->d_blk_of_reach.upload(blk_of_reach));
+    CU(b->d_gl_of_reach.upload(gl_of_reach));
+    CU(b->d_obs_reach.upload(obs_reach));
     for (auto pr : {std::make_pair(&b->d_P, (size_t)b->pp), std::make_pair(&b->d_Pprev, (size_t)b->pp), std::make_pair(&b->d_Q, (size_t)b->pp),
                     std::make_pair(&b->d_Pm, (size_t)b->pp), std::make_pair(&b->d_R, (size_t)b->mm), std::make_pair(&b->d_S, (size_t)b->mm),
                     std::make_pair(&b->d_Ps, (size_t)b->nm), std::make_pair(&b->d_Prow, (size_t)b->nm), std::make_pair(&b->d_K, (size_t)b->nm),
                     std::make_pair(&b->d_z, (size_t)b->m_tot), std::make_pair(&b->d_dz, (size_t)b->m_tot),
                     std::make_pair(&b->d_gain, (size_t)b->n_u), std::make_pair(&b->d_Gp, (size_t)b->n_u * 2),
                     std::make_pair(&b->d_X, (size_t)b->n_u * b->ld), std::make_pair(&b->d_X2, (size_t)b->n_u * b->ld)})
-        if (e == cudaSuccess) e = dalloc(pr.first, pr.second);
-    if (e != cudaSuccess) { txh_kfb_destroy(b); return cuda_fail(e, "batched filter buffers"); }
-    *out = b;
+        CU(pr.first->alloc(std::max<size_t>(pr.second, 1)));
+    *out = b.release();
     return TXH_OK;
 }
 
-void txh_kfb_destroy(txh_kfb* b)
-{
-    if (!b) return;
-    cudaFree(b->d_blocks); cudaFree(b->d_blk_of_reach); cudaFree(b->d_gl_of_reach); cudaFree(b->d_obs_reach);
-    for (double* p : {b->d_P, b->d_Pprev, b->d_Q, b->d_R, b->d_Pm, b->d_Ps, b->d_Prow, b->d_S, b->d_K, b->d_z, b->d_dz, b->d_gain,
-                      b->d_Gp, b->d_X, b->d_X2})
-        cudaFree(p);
-    delete b;
-}
+void txh_kfb_destroy(txh_kfb* b) { delete b; }
 
 // which: 0 P (posterior), 1 Q, 2 R, 3 P of the previous update, 4 K, 5 dz, 6 gain
 static int kfb_locate(txh_kfb* b, int64_t block, int which, double** ptr, size_t* count)

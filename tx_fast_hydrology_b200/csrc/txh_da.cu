@@ -1788,10 +1788,10 @@ cudaError_t launch_enkf_small_system(double* HX, const double* O, int ldo, const
         cudaGetLastError();
     }
     static const char* trace_file = getenv("TXH_SS_TRACE");
-    unsigned long long* d_trace = nullptr;
+    DevBuf<unsigned long long> trace;
     if (trace_file && *trace_file) {
-        if ((e = cudaMalloc((void**)&d_trace, 16 * 8 * sizeof(unsigned long long))) != cudaSuccess) return e;
-        cudaMemsetAsync(d_trace, 0, 16 * 8 * sizeof(unsigned long long), st);
+        if ((e = trace.alloc(16 * 8)) != cudaSuccess) return e;
+        cudaMemsetAsync(trace, 0, 16 * 8 * sizeof(unsigned long long), st);
     }
     cudaLaunchConfig_t cfg{};
     cfg.gridDim = dim3(nc); cfg.blockDim = dim3(256); cfg.dynamicSmemBytes = SS_SMEM; cfg.stream = st;
@@ -1800,15 +1800,14 @@ cudaError_t launch_enkf_small_system(double* HX, const double* O, int ldo, const
     attr[0].id = cudaLaunchAttributeClusterDimension; attr[0].val.clusterDim.x = nc; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
     attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization; attr[1].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr; cfg.numAttrs = pdl ? 2 : 1;
-    e = cudaLaunchKernelEx(&cfg, nc == 16 ? k16 : k8, HX, O, ldo, Zp, mean, obs_pos, dinv_diag, m, Mt, shift, T, W, info, d_trace);
+    e = cudaLaunchKernelEx(&cfg, nc == 16 ? k16 : k8, HX, O, ldo, Zp, mean, obs_pos, dinv_diag, m, Mt, shift, T, W, info, trace.get());
     count_launch();
     if (e == cudaSuccess) e = cudaGetLastError();
-    if (d_trace) {
+    if (trace) {
         // development aid: per-CTA phase stamps (ns relative to the first) appended to the file, synchronous
         unsigned long long h[16 * 8];
-        cudaMemcpyAsync(h, d_trace, sizeof(h), cudaMemcpyDeviceToHost, st);
+        cudaMemcpyAsync(h, trace, sizeof(h), cudaMemcpyDeviceToHost, st);
         cudaStreamSynchronize(st);
-        cudaFree(d_trace);
         if (FILE* fp = fopen(trace_file, "a")) {
             unsigned long long t0 = ~0ull;
             for (int r = 0; r < nc; ++r) if (h[r * 8] && h[r * 8] < t0) t0 = h[r * 8];

@@ -1,11 +1,70 @@
 // txh_kernels.cuh -- device-side argument blocks and launcher prototypes (sm_100a).
 #pragma once
 #include <cuda_runtime.h>
+#include <algorithm>
 #include <cstdint>
+#include <vector>
 
 #include "txh_topology.hpp"
 
 namespace txh {
+
+// The one owner of a device allocation: capacity() elements of T, move-only, freed on destruction.  It converts to
+// its pointer, so launch arguments read as they would from a raw one.  An allocation, copy or fill that fails leaves
+// it empty (nullptr, capacity 0).  An empty buffer makes no CUDA call, not even when it is destroyed.
+template <class T>
+class DevBuf {
+public:
+    DevBuf() = default;
+    DevBuf(DevBuf&& o) noexcept : p_(o.p_), cap_(o.cap_) { o.p_ = nullptr; o.cap_ = 0; }
+    DevBuf& operator=(DevBuf&& o) noexcept
+    {
+        if (this != &o) { reset(); p_ = o.p_; cap_ = o.cap_; o.p_ = nullptr; o.cap_ = 0; }
+        return *this;
+    }
+    ~DevBuf() { reset(); }
+    operator T*() const { return p_; }
+    T* get() const { return p_; }
+    size_t capacity() const { return cap_; }
+    void reset()
+    {
+        if (p_) cudaFree(p_);
+        p_ = nullptr; cap_ = 0;
+    }
+    // `count` elements of new, uninitialised memory in place of the old
+    cudaError_t alloc(size_t count)
+    {
+        reset();
+        const cudaError_t e = cudaMalloc((void**)&p_, count * sizeof(T));
+        if (e != cudaSuccess) { p_ = nullptr; return e; }
+        cap_ = count;
+        return cudaSuccess;
+    }
+    // a synchronous copy of `v` (one element when `v` is empty)
+    cudaError_t upload(const std::vector<T>& v)
+    {
+        cudaError_t e = alloc(std::max<size_t>(v.size(), 1));
+        if (e == cudaSuccess && !v.empty()) e = cudaMemcpy(p_, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice);
+        if (e != cudaSuccess) reset();
+        return e;
+    }
+    // Grow-only: reallocated when `count` elements do not fit, once `st` has drained (a queued launch may still read
+    // the old memory); new memory is filled with the byte `fill` unless it is < 0.
+    cudaError_t grow(size_t count, cudaStream_t st, int fill = -1)
+    {
+        if (count <= cap_) return cudaSuccess;
+        cudaError_t e = p_ ? cudaStreamSynchronize(st) : cudaSuccess;
+        if (e != cudaSuccess) return e;
+        e = alloc(count);
+        if (e == cudaSuccess && fill >= 0) e = cudaMemsetAsync(p_, fill, count * sizeof(T), st);
+        if (e != cudaSuccess) reset();
+        return e;
+    }
+
+private:
+    T* p_ = nullptr;
+    size_t cap_ = 0;
+};
 
 // Interpolation of the forcing table for one step, resolved on the host exactly as
 // nutils.py:21-34 does (searchsorted-left, clamped ends): q = w0*F[r0] + w1*F[r1].
